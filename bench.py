@@ -24,8 +24,12 @@ cpu_baseline  the reference's OpenCV path (oracle/cv2_pipeline.py: the reference
         the same cv2/numpy) on this box's host cores, bounded sample.
 --config3  BASELINE config 3 instead of the weak-scaling default: an 8-camera 1080p rig, --frames-per-stream frames per
         camera, whole streams sharded over the N ranks (8/N cameras per GPU, strong scaling), records gathered to rank 0.
+--dump-outputs DIR  after the timed steps, rank 0 writes what its last timed step returned to the caller (the per-frame
+        records of every native batch of that step, and the smoothing state after it) as DIR/<name>.npy, float64.  The
+        inputs are seeded, so two builds run with the same arguments can be compared array for array.
 """
 import argparse
+import collections
 import json
 import os
 import subprocess
@@ -40,6 +44,27 @@ import numpy as np  # noqa: E402
 
 H, W = 1080, 1920
 ALGO_BYTES_PER_FRAME = 4 * H * W          # SURVEY.md 8(d)
+DUMP_BYTES = 64 << 20                     # --dump-outputs: larger outputs are written as a seeded sample of frames
+
+
+# ------------------------------------------------------------------------------------ outputs
+def dump_outputs(path, recs, state_fit, state_valid, limit=DUMP_BYTES):
+    """Write the records ``recs`` (RECORD_DTYPE, one per frame) field by field as ``path/<field>.npy`` (the fields of
+    ``side`` as ``side_<field>.npy``, shaped [frames, 2, ...]), plus ``frame_index.npy`` (which records were written) and
+    the smoothing state ``state_fit.npy`` / ``state_valid.npy``; every array float64 (the int32 fields convert exactly).
+    If all frames would exceed ``limit`` bytes, a fixed seeded sample of frames is written instead."""
+    cols = {f"side_{k}": recs["side"][k] for k in recs.dtype["side"].base.names}
+    cols.update((k, recs[k]) for k in recs.dtype.names if k != "side")
+    per_frame = 8 * (1 + sum(int(np.prod(a.shape[1:], dtype=np.int64)) for a in cols.values()))
+    fixed = 8 * (state_fit.size + state_valid.size) + 1024 * (len(cols) + 3)      # + room for the .npy headers
+    keep = max(0, min(len(recs), (limit - fixed) // per_frame))
+    idx = np.arange(len(recs))
+    if keep < len(recs):
+        idx = np.sort(np.random.default_rng(0).choice(len(recs), keep, replace=False))
+    os.makedirs(path, exist_ok=True)
+    out = dict(((k, a[idx]) for k, a in cols.items()), frame_index=idx, state_fit=state_fit, state_valid=state_valid)
+    for k, a in out.items():
+        np.save(os.path.join(path, k + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 # ------------------------------------------------------------------------------------ CPU arm
@@ -201,7 +226,12 @@ def main():
     ap.add_argument("--skip-e2e", action="store_true", help="skip the e2e leg (profiling runs)")
     ap.add_argument("--config3", action="store_true", help="BASELINE config 3: 8 cameras sharded by stream (strong scaling)")
     ap.add_argument("--frames-per-stream", type=int, default=512, help="config 3: frames per camera per step")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -298,7 +328,8 @@ def main():
     # batches run in order on one stream.  The records of every batch are gathered to rank 0 (the path's only
     # collective, NCCL over NVLink) straight from the context's device copy: lane_ctx_records_device stays valid until the
     # batch after next is enqueued, and the context's stream waits for the gather before that slot is reused.
-    state = {"queued": 0, "next": 0, "first": True, "last_recs": None, "last_bufs": None}
+    state = {"queued": 0, "next": 0, "first": True, "last_recs": None, "last_bufs": None,
+             "step_recs": collections.deque(maxlen=S)}                # the batches of the last step, camera order
 
     def enqueue_next():
         k = state["next"] % S
@@ -321,6 +352,7 @@ def main():
             state["queued"] -= 1
             done += 1
             state["last_recs"] = recs
+            state["step_recs"].append(recs)
             if on_collect:
                 on_collect()
             if gatherer is not None:
@@ -366,6 +398,8 @@ def main():
     t1 = time.perf_counter()
     timed_window = (t0, t1)
     dev_ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, np.concatenate(state["step_recs"]), prev_fit, prev_valid)
     # ---- the same K steps once more with CUDA events between the stages (one stream): stage split, launch count and the
     # edge-path roofline come from this pass; its step time is reported beside the overlapped one
     ctx.set_profiling(True)

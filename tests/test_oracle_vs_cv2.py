@@ -31,6 +31,17 @@ def _frames():
 FRAMES = _frames()
 
 
+@pytest.fixture(autouse=True)
+def _cv2_single_thread():
+    """cv2 4.13's multi-threaded 8-bit GaussianBlur races on frames 6 to 11 rows tall: the 7x9 noise frame comes back with
+    a wrong row in a few percent of calls, with 8 threads or 128 alike.  On one thread its result is deterministic and
+    equals the exact 5x5 kernel, which is what the oracle restates."""
+    threads = cv2.getNumThreads()
+    cv2.setNumThreads(1)
+    yield
+    cv2.setNumThreads(threads)
+
+
 @pytest.mark.parametrize("name,frame", FRAMES, ids=[n for n, _ in FRAMES])
 def test_gray_blur_median_canny(name, frame):
     g = S.gray(frame)
