@@ -122,6 +122,22 @@ LANE_API int lane_detect_batch_nv12(lane_ctx *ctx, const uint8_t *frames_nv12, i
                            const int32_t *stream_id, int n_streams, double *prev_fit, uint8_t *prev_valid,
                            lane_record *out);
 
+/* Frame layouts a detect / ingest call accepts (what a decoder or VideoDataLoader hands out). */
+#define LANE_INPUT_BGR  0           /* uint8 [n][src_h][src_w][3] */
+#define LANE_INPUT_NV12 1           /* uint8 [n][src_h*3/2][src_w], Y then interleaved UV (hardware decoders) */
+#define LANE_INPUT_I420 2           /* uint8 [n][src_h*3/2][src_w], Y, then U plane, then V plane (software decoders) */
+
+/* lane_detect_batch on frames of another size and/or layout, as VideoDataLoader.read_frame delivers them
+ * (/root/reference/data/loaders/video_loader.py:96-131: decode, then cv2.resize(frame, target_size) at :108, :128) to
+ * LaneDetector.detect (lane_detector.py:178-218).  Each frame becomes the context's height x width BGR frame on the device
+ * -- cv2.resize(cv2.cvtColor(f, COLOR_YUV2BGR_NV12 | COLOR_YUV2BGR_I420), (width, height)) in one kernel for YUV, the
+ * lane_resize_batch kernel for BGR -- and the usual path runs on it: only the source bytes cross PCIe, and the records
+ * equal those of lane_detect_batch on the cv2-prepared frames.  format: LANE_INPUT_*; src_h / src_w: the frames' own
+ * size (even for NV12 / I420).  Other arguments as for lane_detect_batch. */
+LANE_API int lane_detect_batch_ingest(lane_ctx *ctx, const uint8_t *frames, int frames_on_device, int n, int format,
+                                      int src_h, int src_w, const int32_t *stream_id, int n_streams, double *prev_fit,
+                                      uint8_t *prev_valid, lane_record *out);
+
 /* Asynchronous split of the above for pipelined callers: enqueue (device frames only; records
  * land in an internal pinned buffer), then collect (waits for the OLDEST batch in flight and returns
  * its records and the EMA state after it).
@@ -225,6 +241,16 @@ LANE_API int lane_resize_batch(const uint8_t *src, int n, int src_h, int src_w, 
  * cuda_stream as for lane_resize_batch.  Needs no context; errors via lane_last_error(NULL). */
 LANE_API int lane_nv12_to_bgr_batch(const uint8_t *src, int n, int height, int width, uint8_t *dst, int on_device,
                                     int device, void *cuda_stream);
+
+/* Decoder output at camera resolution -> the frame VideoDataLoader.read_frame returns with target_size set
+ * (/root/reference/data/loaders/video_loader.py:96-131): per frame
+ * cv2.resize(cv2.cvtColor(f, COLOR_YUV2BGR_NV12 | COLOR_YUV2BGR_I420), (dst_w, dst_h)), bit-exact, in one pass that
+ * reads the 1.5 B/px source and writes only the destination (the full-resolution BGR frame is never stored).
+ * src: uint8 [n][src_h*3/2][src_w] in `format` (LANE_INPUT_NV12 or LANE_INPUT_I420), src_h / src_w even;
+ * dst: uint8 [n][dst_h][dst_w][3], any positive size (equal to the source size: conversion only).  on_device / device /
+ * cuda_stream as for lane_resize_batch.  Needs no context; errors via lane_last_error(NULL). */
+LANE_API int lane_yuv420_to_bgr_batch(const uint8_t *src, int format, int n, int src_h, int src_w, uint8_t *dst,
+                                      int dst_h, int dst_w, int on_device, int device, void *cuda_stream);
 
 /* ---- scene statistics (SURVEY.md 8f rank 2, second half) -----------------------------------------------------
  * Integer sums behind SceneClassifier's image cues (/root/reference/src/tagging/scene_classifier.py):

@@ -23,6 +23,7 @@ TAP_BLUR, TAP_HIST, TAP_CLASS, TAP_EDGES, TAP_POINTS, TAP_SEGMENTS, TAP_GRAY = 1
 FLAG_SEGMENTS_TRUNCATED, FLAG_POINTS_TRUNCATED = 1, 2
 PATH_FUSED_EDGE, PATH_CLUSTER_CANNY, PATH_PPHT_DSMEM = 1, 2, 4
 PATH_ALL_FAST = 7
+INPUT_BGR, INPUT_NV12, INPUT_I420 = 0, 1, 2          # LANE_INPUT_*: frame layouts the detect / ingest calls accept
 
 
 class LaneSide(C.Structure):
@@ -84,7 +85,11 @@ _PROTOS = {
                                     C.c_void_p, C.c_void_p]),
     "lane_detect_batch_nv12": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p,
                                          C.c_void_p, C.c_void_p]),
+    "lane_detect_batch_ingest": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                           C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "lane_nv12_to_bgr_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+    "lane_yuv420_to_bgr_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int,
+                                           C.c_int, C.c_int, C.c_void_p]),
     "lane_detect_enqueue": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "lane_detect_collect": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "lane_ctx_stream": (C.c_void_p, [C.c_void_p]),
@@ -235,17 +240,20 @@ class LaneContext:
 
     # ---- hot path
     def detect(self, frames, n: int, on_device: bool, stream_id, n_streams: int, prev_fit: np.ndarray,
-               prev_valid: np.ndarray, smoothing: float, one_minus: float, nv12: bool = False) -> np.ndarray:
-        """frames: int device pointer (on_device) or C-contiguous uint8 ndarray -- BGR [n,H,W,3], or with ``nv12`` the
-        decoder layout [n,H*3/2,W].  prev_fit float64[S,2,3] and prev_valid uint8[S,2] are updated in place.
-        Returns a RECORD_DTYPE array of n records (a copy)."""
+               prev_valid: np.ndarray, smoothing: float, one_minus: float, fmt: int = INPUT_BGR,
+               src_hw=None) -> np.ndarray:
+        """frames: int device pointer (on_device) or C-contiguous uint8 ndarray in layout ``fmt`` (INPUT_*) at size
+        ``src_hw`` = (h, w) (None: the context's) -- BGR [n,h,w,3] or the decoder layouts [n,h*3/2,w].  Frames of
+        another layout or size become the context's BGR frames on the device first (lane_detect_batch_ingest).
+        prev_fit float64[S,2,3] and prev_valid uint8[S,2] are updated in place.  Returns a RECORD_DTYPE array of n
+        records (a copy)."""
         L = lib()
         self._check(L.lane_set_smoothing(self._h, float(smoothing), float(one_minus)))
         fp = C.c_void_p(frames) if on_device else _ptr(frames)
         sid = None if stream_id is None else np.ascontiguousarray(stream_id, dtype=np.int32)
-        fn = L.lane_detect_batch_nv12 if nv12 else L.lane_detect_batch
-        self._check(fn(self._h, fp, int(on_device), n, _ptr(sid), n_streams, _ptr(prev_fit), _ptr(prev_valid),
-                       _ptr(self._records)))
+        sh, sw = (self.height, self.width) if src_hw is None else (int(src_hw[0]), int(src_hw[1]))
+        self._check(L.lane_detect_batch_ingest(self._h, fp, int(on_device), n, int(fmt), sh, sw, _ptr(sid), n_streams,
+                                               _ptr(prev_fit), _ptr(prev_valid), _ptr(self._records)))
         return self._records[:n].copy()
 
     def enqueue(self, frames_ptr: int, n: int, stream_id, n_streams, prev_fit, prev_valid, smoothing, one_minus):

@@ -7,38 +7,19 @@
 // cross PCIe per frame, which is what bounds the end-to-end rate.  Bit-exact against cv2 (oracle/nv12.py restates the
 // arithmetic: ITU-R BT.601 limited range, 20-bit fixed point, arithmetic shift, saturation).
 //
+// I420 (what software decoders hand out: U and V as separate quarter planes) carries the same samples and converts with
+// the same arithmetic; the kernels are templated on the chroma addressing (k0_common.cuh).
+//
 // HBM-bound: 1.5 B/px read + 3 B/px written.  A thread converts a 2 x 8 pixel block: one 8-byte load per luma row,
 // one 8-byte load of the four (U, V) pairs the block shares, three 8-byte stores per output row; a warp covers
 // 256 px of two rows, so every access is a full, aligned segment.
 #include <algorithm>
 
-#include "lane_common.cuh"
+#include "k0_common.cuh"
 
 namespace {
 
-constexpr int CY = 1220542, CUB = 2116026, CUG = -409993, CVG = -852492, CVR = 1673527, SHIFT = 20;
-
-__device__ __forceinline__ uint32_t sat8(int v) { return (uint32_t)min(max(v, 0), 255); }
-
-struct UV {
-    int r, g, b;                       // chroma terms of one 2x2 block (rounding constant included)
-};
-
-__device__ __forceinline__ UV uv_terms(int u, int v)
-{
-    u -= 128; v -= 128;
-    UV t;
-    t.r = (1 << (SHIFT - 1)) + CVR * v;
-    t.g = (1 << (SHIFT - 1)) + CVG * v + CUG * u;
-    t.b = (1 << (SHIFT - 1)) + CUB * u;
-    return t;
-}
-
-__device__ __forceinline__ void px(int yv, const UV &t, uint32_t &b, uint32_t &g, uint32_t &r)
-{
-    const int y = max(0, yv - 16) * CY;
-    b = sat8((y + t.b) >> SHIFT); g = sat8((y + t.g) >> SHIFT); r = sat8((y + t.r) >> SHIFT);
-}
+using namespace k0yuv;
 
 // 8 luma bytes of one row + the four chroma terms -> 24 BGR bytes (six words)
 __device__ __forceinline__ void row8(uint2 yy, const UV (&t)[4], uint32_t (&o)[6])
@@ -60,6 +41,7 @@ __device__ __forceinline__ void row8(uint2 yy, const UV (&t)[4], uint32_t (&o)[6
 }
 
 // W % 8 == 0, 8-byte aligned planes
+template <int FMT>
 __global__ void __launch_bounds__(256) k0_nv12_vec(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst, int n, int H,
                                                    int W)
 {
@@ -73,12 +55,20 @@ __global__ void __launch_bounds__(256) k0_nv12_vec(const uint8_t *__restrict__ s
         const uint8_t *s = src + f * src_frame;
         const uint2 y0 = __ldg(reinterpret_cast<const uint2 *>(s + (size_t)(2 * by) * W + 8 * bx));
         const uint2 y1 = __ldg(reinterpret_cast<const uint2 *>(s + (size_t)(2 * by + 1) * W + 8 * bx));
-        const uint2 uv = __ldg(reinterpret_cast<const uint2 *>(s + (size_t)(H + by) * W + 8 * bx));
         UV t[4];
-        t[0] = uv_terms((int)(uv.x & 0xFFu), (int)((uv.x >> 8) & 0xFFu));
-        t[1] = uv_terms((int)((uv.x >> 16) & 0xFFu), (int)(uv.x >> 24));
-        t[2] = uv_terms((int)(uv.y & 0xFFu), (int)((uv.y >> 8) & 0xFFu));
-        t[3] = uv_terms((int)((uv.y >> 16) & 0xFFu), (int)(uv.y >> 24));
+        if constexpr (FMT == LANE_INPUT_NV12) {
+            const uint2 uv = __ldg(reinterpret_cast<const uint2 *>(s + (size_t)(H + by) * W + 8 * bx));
+            t[0] = uv_terms((int)(uv.x & 0xFFu), (int)((uv.x >> 8) & 0xFFu));
+            t[1] = uv_terms((int)((uv.x >> 16) & 0xFFu), (int)(uv.x >> 24));
+            t[2] = uv_terms((int)(uv.y & 0xFFu), (int)((uv.y >> 8) & 0xFFu));
+            t[3] = uv_terms((int)((uv.y >> 16) & 0xFFu), (int)(uv.y >> 24));
+        } else {                       // four U bytes, four V bytes: 4-byte aligned when W % 8 == 0
+            const size_t P = (size_t)H * W, q = P + (size_t)by * (W / 2) + 4 * bx;
+            const uint32_t u = __ldg(reinterpret_cast<const uint32_t *>(s + q));
+            const uint32_t v = __ldg(reinterpret_cast<const uint32_t *>(s + q + P / 4));
+#pragma unroll
+            for (int i = 0; i < 4; i++) t[i] = uv_terms((int)((u >> (8 * i)) & 0xFFu), (int)((v >> (8 * i)) & 0xFFu));
+        }
         uint32_t o[6];
         uint8_t *d = dst + f * dst_frame + ((size_t)(2 * by) * W + 8 * bx) * 3;
         row8(y0, t, o);
@@ -91,6 +81,7 @@ __global__ void __launch_bounds__(256) k0_nv12_vec(const uint8_t *__restrict__ s
 }
 
 // any even W, H: one thread per 2x2 block
+template <int FMT>
 __global__ void __launch_bounds__(256) k0_nv12_generic(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst, int n, int H,
                                                        int W)
 {
@@ -102,8 +93,7 @@ __global__ void __launch_bounds__(256) k0_nv12_generic(const uint8_t *__restrict
         const long long q = i / bw;
         const int by = (int)(q % bh), f = (int)(q / bh);
         const uint8_t *s = src + f * src_frame;
-        const uint8_t *uvp = s + (size_t)(H + by) * W + 2 * bx;
-        const UV t = uv_terms(uvp[0], uvp[1]);
+        const UV t = chroma<FMT>(s, H, W, by, bx);
 #pragma unroll
         for (int dy = 0; dy < 2; dy++)
 #pragma unroll
@@ -117,53 +107,28 @@ __global__ void __launch_bounds__(256) k0_nv12_generic(const uint8_t *__restrict
     }
 }
 
-}  // namespace
-
-// device pointers; enqueued on st
-void launch_nv12_to_bgr(const uint8_t *src, uint8_t *dst, int n, int H, int W, cudaStream_t st)
+template <int FMT>
+void launch_fmt(const uint8_t *src, uint8_t *dst, int n, int H, int W, cudaStream_t st)
 {
     const int sms = lane_sm_count();
     if (W % 8 == 0 && (((uintptr_t)src | (uintptr_t)dst) % 8) == 0) {
         const long long total = (long long)n * (H / 2) * (W / 8);
         const int blocks = (int)std::min<long long>((total + 255) / 256, (long long)sms * 16);
-        k0_nv12_vec<<<std::max(blocks, 1), 256, 0, st>>>(src, dst, n, H, W);
+        k0_nv12_vec<FMT><<<std::max(blocks, 1), 256, 0, st>>>(src, dst, n, H, W);
     } else {
         const long long total = (long long)n * (H / 2) * (W / 2);
         const int blocks = (int)std::min<long long>((total + 255) / 256, (long long)sms * 16);
-        k0_nv12_generic<<<std::max(blocks, 1), 256, 0, st>>>(src, dst, n, H, W);
+        k0_nv12_generic<FMT><<<std::max(blocks, 1), 256, 0, st>>>(src, dst, n, H, W);
     }
 }
 
-extern "C" int lane_nv12_to_bgr_batch(const uint8_t *src, int n, int height, int width, uint8_t *dst, int on_device,
-                                      int device, void *cuda_stream)
+}  // namespace
+
+// YUV 4:2:0 (LANE_INPUT_NV12 / LANE_INPUT_I420) -> BGR at the same size; device pointers, enqueued on st
+void launch_yuv420_to_bgr(const uint8_t *src, int format, uint8_t *dst, int n, int H, int W, cudaStream_t st)
 {
-    auto fail = [](int code, const char *msg) { lane_set_global_error(msg); return code; };
-    if (!src || !dst || n < 1 || height < 2 || width < 2) return fail(LANE_ERR_INVALID, "lane_nv12_to_bgr_batch: bad arguments");
-    if ((height | width) & 1) return fail(LANE_ERR_INVALID, "lane_nv12_to_bgr_batch: NV12 needs even width and height");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-        return fail(LANE_ERR_NO_DEVICE, "no CUDA device visible: this library has no CPU fallback");
-    if (device < 0 || device >= ndev) return fail(LANE_ERR_INVALID, "lane_nv12_to_bgr_batch: device out of range");
-    if (cudaSetDevice(device) != cudaSuccess) return fail(LANE_ERR_CUDA, "cudaSetDevice failed");
-    cudaStream_t st = (cudaStream_t)cuda_stream;
-    const size_t in_bytes = (size_t)n * height * width * 3 / 2, out_bytes = (size_t)n * height * width * 3;
-    if (on_device) {
-        launch_nv12_to_bgr(src, dst, n, height, width, st);
-        if (cudaGetLastError() != cudaSuccess) return fail(LANE_ERR_CUDA, "k0_nv12 launch failed");
-        return LANE_OK;
-    }
-    uint8_t *d_in = nullptr, *d_out = nullptr;
-    if (cudaMalloc((void **)&d_in, in_bytes) != cudaSuccess || cudaMalloc((void **)&d_out, out_bytes) != cudaSuccess) {
-        cudaFree(d_in);
-        cudaGetLastError();
-        return fail(LANE_ERR_CUDA, "lane_nv12_to_bgr_batch: device allocation failed");
-    }
-    cudaMemcpyAsync(d_in, src, in_bytes, cudaMemcpyHostToDevice, st);
-    launch_nv12_to_bgr(d_in, d_out, n, height, width, st);
-    cudaMemcpyAsync(dst, d_out, out_bytes, cudaMemcpyDeviceToHost, st);
-    cudaError_t e = cudaStreamSynchronize(st);
-    if (e == cudaSuccess) e = cudaGetLastError();
-    cudaFree(d_in); cudaFree(d_out);
-    if (e != cudaSuccess) return fail(LANE_ERR_CUDA, cudaGetErrorString(e));
-    return LANE_OK;
+    if (format == LANE_INPUT_I420)
+        launch_fmt<LANE_INPUT_I420>(src, dst, n, H, W, st);
+    else
+        launch_fmt<LANE_INPUT_NV12>(src, dst, n, H, W, st);
 }

@@ -17,19 +17,12 @@
 #include <vector>
 
 #include "host_stage.h"
-#include "lane_common.cuh"
+#include "k0_common.cuh"
 
 namespace {
 
-struct Taps {
-    int *xofs = nullptr;        // [dw]   first source column
-    short2 *alpha = nullptr;    // [dw]   (a0, a1); the second tap is min(x0 + 1, sw - 1)
-    int2 *yofs = nullptr;       // [dh]   the two source rows, clamped one by one
-    short2 *beta = nullptr;     // [dh]   (b0, b1) from the unclamped fraction
-};
-
 std::mutex g_mu;
-std::map<std::tuple<int, int, int, int, int>, Taps> g_taps;
+std::map<std::tuple<int, int, int, int, int>, ResizeTaps> g_taps;
 
 void frac(int d, double scale, int *s, float *f)
 {
@@ -41,7 +34,7 @@ void frac(int d, double scale, int *s, float *f)
 
 short coef(float v) { return (short)lrintf(v * 2048.f); }      // cvRound (nearest even) of a float32 product
 
-cudaError_t build_taps(int sh, int sw, int dh, int dw, Taps *t)
+cudaError_t build_taps(int sh, int sw, int dh, int dw, ResizeTaps *t)
 {
     std::vector<int> xo(dw);
     std::vector<short2> al(dw), be(dh);
@@ -72,12 +65,6 @@ cudaError_t build_taps(int sh, int sw, int dh, int dw, Taps *t)
     return cudaMemcpy(t->beta, be.data(), sizeof(short2) * dh, cudaMemcpyHostToDevice);
 }
 
-__device__ __forceinline__ uint32_t vmix(int h0, int h1, int b0, int b1)
-{
-    const int v = (((b0 * (h0 >> 4)) >> 16) + ((b1 * (h1 >> 4)) >> 16) + 2) >> 2;
-    return (uint32_t)min(v, 255);
-}
-
 // One thread = PX consecutive destination pixels of one row (PX * CN bytes, written with the widest stores the
 // alignment allows); a warp covers a contiguous run of the row, so the source reads of a warp fall in two short
 // row segments that stay in L1 across the PX pixels.
@@ -103,7 +90,7 @@ __global__ void __launch_bounds__(256) k0_resize(const uint8_t *__restrict__ src
         for (int c = 0; c < CN; c++) {
             const int h0 = (int)__ldg(r0 + x0 * CN + c) * a.x + (int)__ldg(r0 + x1 * CN + c) * a.y;
             const int h1 = (int)__ldg(r1 + x0 * CN + c) * a.x + (int)__ldg(r1 + x1 * CN + c) * a.y;
-            px[k * CN + c] = (uint8_t)vmix(h0, h1, b.x, b.y);
+            px[k * CN + c] = (uint8_t)k0_vmix(h0, h1, b.x, b.y);
         }
     }
     if (dx0 + PX <= dw && ((uintptr_t)out & 3) == 0 && (PX * CN) % 4 == 0) {
@@ -127,6 +114,34 @@ int rfail(int code, const char *what, cudaError_t e)
 
 }  // namespace
 
+cudaError_t lane_resize_taps(int sh, int sw, int dh, int dw, ResizeTaps *t)
+{
+    int device = 0;
+    cudaError_t e;
+    if ((e = cudaGetDevice(&device))) return e;
+    std::lock_guard<std::mutex> lk(g_mu);
+    const auto key = std::make_tuple(device, sh, sw, dh, dw);
+    auto it = g_taps.find(key);
+    if (it != g_taps.end()) {
+        *t = it->second;
+        return cudaSuccess;
+    }
+    if ((e = build_taps(sh, sw, dh, dw, t))) return e;
+    g_taps[key] = *t;
+    return cudaSuccess;
+}
+
+void launch_resize(const uint8_t *src, uint8_t *dst, int n, int channels, int sh, int sw, int dh, int dw,
+                   const ResizeTaps &t, cudaStream_t st)
+{
+    constexpr int PX = 4;
+    dim3 grid((dw + 256 * PX - 1) / (256 * PX), dh, n);
+    if (channels == 3)
+        k0_resize<3, PX><<<grid, 256, 0, st>>>(src, dst, t.xofs, t.alpha, t.yofs, t.beta, sh, sw, dh, dw);
+    else
+        k0_resize<1, PX><<<grid, 256, 0, st>>>(src, dst, t.xofs, t.alpha, t.yofs, t.beta, sh, sw, dh, dw);
+}
+
 extern "C" int lane_resize_batch(const uint8_t *src, int n, int src_h, int src_w, int channels, uint8_t *dst, int dst_h,
                                  int dst_w, int on_device, int device, void *cuda_stream)
 {
@@ -138,18 +153,8 @@ extern "C" int lane_resize_batch(const uint8_t *src, int n, int src_h, int src_w
         return rfail(LANE_ERR_NO_DEVICE, "no usable CUDA device (there is no CPU fallback)", cudaSuccess);
     cudaError_t e;
     if ((e = cudaSetDevice(device))) return rfail(LANE_ERR_CUDA, "cudaSetDevice", e);
-    Taps t;
-    {
-        std::lock_guard<std::mutex> lk(g_mu);
-        const auto key = std::make_tuple(device, src_h, src_w, dst_h, dst_w);
-        auto it = g_taps.find(key);
-        if (it == g_taps.end()) {
-            if ((e = build_taps(src_h, src_w, dst_h, dst_w, &t))) return rfail(LANE_ERR_CUDA, "tap tables", e);
-            g_taps[key] = t;
-        } else {
-            t = it->second;
-        }
-    }
+    ResizeTaps t;
+    if ((e = lane_resize_taps(src_h, src_w, dst_h, dst_w, &t))) return rfail(LANE_ERR_CUDA, "tap tables", e);
     cudaStream_t st = (cudaStream_t)cuda_stream;
     const size_t sbytes = (size_t)n * src_h * src_w * channels, dbytes = (size_t)n * dst_h * dst_w * channels;
     const uint8_t *s_dev = src;
@@ -163,12 +168,7 @@ extern "C" int lane_resize_batch(const uint8_t *src, int n, int src_h, int src_w
         s_dev = tmp;
         d_dev = tmp + sbytes;
     }
-    constexpr int PX = 4;
-    dim3 grid((dst_w + 256 * PX - 1) / (256 * PX), dst_h, n);
-    if (channels == 3)
-        k0_resize<3, PX><<<grid, 256, 0, st>>>(s_dev, d_dev, t.xofs, t.alpha, t.yofs, t.beta, src_h, src_w, dst_h, dst_w);
-    else
-        k0_resize<1, PX><<<grid, 256, 0, st>>>(s_dev, d_dev, t.xofs, t.alpha, t.yofs, t.beta, src_h, src_w, dst_h, dst_w);
+    launch_resize(s_dev, d_dev, n, channels, src_h, src_w, dst_h, dst_w, t, st);
     if ((e = cudaGetLastError())) { if (tmp) cudaFree(tmp); return rfail(LANE_ERR_CUDA, "kernel launch", e); }
     if (!on_device) {
         e = cudaMemcpyAsync(dst, d_dev, dbytes, cudaMemcpyDeviceToHost, st);

@@ -10,7 +10,7 @@
 #include <thread>
 #include <vector>
 
-#include "lane_common.cuh"
+#include "k0_common.cuh"
 
 #define LANE_COPY_EVENTS 8
 
@@ -47,8 +47,9 @@ struct lane_ctx {
     std::string err;
 
     // device buffers
-    uint8_t *d_frames = nullptr;      // staging for host frames / BGR output of the NV12 conversion (lazy)
-    uint8_t *d_nv12 = nullptr;        // staging for host NV12 frames (lazy)
+    uint8_t *d_frames = nullptr;      // staging for host frames / BGR output of the ingest kernels (lazy)
+    uint8_t *d_src = nullptr;         // staging for host frames the ingest kernels convert / resize (lazy, grows)
+    size_t src_cap = 0;               // its size in bytes
     uint8_t *d_blur = nullptr;        // blurred plane: unfused path and verification taps only (lazy)
     uint32_t *d_kbits = nullptr;      // [B][H][WW] NMS survivors of the fused edge kernel
     uint8_t *d_vplane = nullptr;      // [B][H][W]  their magnitudes (sparse: only survivors' bytes are ever written / read)
@@ -154,7 +155,7 @@ cudaError_t dalloc(T **p, size_t count)
 void free_all(lane_ctx *c)
 {
     cudaSetDevice(c->device);
-    void *ptrs[] = {c->d_frames, c->d_nv12, c->d_blur, c->d_kbits, c->d_vplane, c->d_pre, c->d_cls, c->d_cls_dbg, c->d_roi, c->d_pmask, c->d_gray_dbg, c->d_hist,
+    void *ptrs[] = {c->d_frames, c->d_src, c->d_blur, c->d_kbits, c->d_vplane, c->d_pre, c->d_cls, c->d_cls_dbg, c->d_roi, c->d_pmask, c->d_gray_dbg, c->d_hist,
                     c->d_roi_bits, c->d_pmask_bits, c->d_edge_bits, c->d_dbg_c, c->d_dbg_s, c->d_accum16, c->d_win, c->d_win3, c->d_pmask_work, c->d_list_over,
                     c->d_points, c->d_points_dbg, c->d_lut, c->d_thr, c->d_seedsA, c->d_seedsB, c->d_seed_count,
                     c->d_n_edges, c->d_n_points, c->d_rounds, c->d_n_lines, c->d_accum, c->d_lines, c->fit.raw, c->fit.big,
@@ -205,6 +206,25 @@ int ensure_streams(lane_ctx *c, int S)
     }
     c->state_on_device = false;
     c->stream_cap = S;
+    return LANE_OK;
+}
+
+// Staging for max_batch source frames of `frame_bytes`.  A larger source replaces the buffer once the context's streams
+// are idle (an earlier batch may still be copying into it or converting out of it).
+int ensure_src(lane_ctx *c, size_t frame_bytes)
+{
+    const size_t need = (size_t)c->max_batch * frame_bytes;
+    if (need <= c->src_cap) return LANE_OK;
+    if (c->d_src) {
+        CU(cudaStreamSynchronize(c->st));
+        if (c->st2) CU(cudaStreamSynchronize(c->st2));
+        if (c->copy_st) CU(cudaStreamSynchronize(c->copy_st));
+        CU(cudaFree(c->d_src));
+        c->d_src = nullptr;
+        c->src_cap = 0;
+    }
+    CU(dalloc(&c->d_src, need));
+    c->src_cap = need;
     return LANE_OK;
 }
 
@@ -381,11 +401,18 @@ int run_stages(lane_ctx *c, const uint8_t *frames_dev, int off, int m, const int
     return stage_check(c, "fit");
 }
 
+// What the caller's frames are: layout (LANE_INPUT_*) and size.  Unless they already are the context's H x W BGR
+// frames, the ingest kernels (k0_common.cuh) make those from them on the device before the path runs.
+struct Ingest {
+    int format, h, w;
+    size_t frame_bytes() const { return format == LANE_INPUT_BGR ? (size_t)h * w * 3 : (size_t)h * w * 3 / 2; }
+};
+
 // Enqueue the whole batch.  Device-resident frames run as one chunk.  Host frames are cut into chunks that are
 // copied on a second stream while the previous chunk computes (the EMA state stays on the device across chunks,
 // which run in order on the compute stream).
 int enqueue(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int32_t *stream_id, int S,
-            const double *prev_fit, const uint8_t *prev_valid, bool nv12 = false)
+            const double *prev_fit, const uint8_t *prev_valid, Ingest in)
 {
     int rc = LANE_OK;
     lane_ctx::slot_t &sl = c->slots[c->cur];
@@ -408,20 +435,22 @@ int enqueue(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int
     const int32_t *sid = stream_id ? c->d_stream_id : nullptr;
     const uint8_t *frames_dev = frames;
     const size_t bgr_bytes = (size_t)c->g.H * c->g.W * 3;
-    if (nv12 && !c->d_frames) CU(dalloc(&c->d_frames, (size_t)c->max_batch * bgr_bytes));
+    const bool convert = in.format != LANE_INPUT_BGR || in.h != c->g.H || in.w != c->g.W;
+    if (convert && !c->d_frames) CU(dalloc(&c->d_frames, (size_t)c->max_batch * bgr_bytes));
     if (on_device) {
-        if (nv12) {                                  // decoder output already on the device: convert, then the usual path
-            launch_nv12_to_bgr(frames, c->d_frames, n, c->g.H, c->g.W, c->st);
+        if (convert) {                               // source already on the device: one ingest launch, then the usual path
+            CU(launch_ingest(frames, in.format, n, in.h, in.w, c->d_frames, c->g.H, c->g.W, c->st));
             frames_dev = c->d_frames;
         }
         rc = run_stages(c, frames_dev, 0, n, sid, S, c->profiling);
         if (rc) return rc;
     } else {
-        // bytes per frame that cross PCIe: 3 B/px for BGR, 1.5 B/px for NV12 (converted on the device, chunk by chunk)
-        const size_t bytes = nv12 ? bgr_bytes / 2 : bgr_bytes;
+        // bytes per frame that cross PCIe: the source's own (3 B/px BGR, 1.5 B/px YUV 4:2:0 at the decoder's size),
+        // converted / resized on the device chunk by chunk
+        const size_t bytes = in.frame_bytes();
         if (!c->d_frames) CU(dalloc(&c->d_frames, (size_t)c->max_batch * bgr_bytes));
-        if (nv12 && !c->d_nv12) CU(dalloc(&c->d_nv12, (size_t)c->max_batch * bytes));
-        uint8_t *d_in = nv12 ? c->d_nv12 : c->d_frames;
+        if (convert) { rc = ensure_src(c, bytes); if (rc) return rc; }
+        uint8_t *d_in = convert ? c->d_src : c->d_frames;
         if (!c->copy_st) {
             CU(cudaStreamCreateWithFlags(&c->copy_st, cudaStreamNonBlocking));
             for (auto &e : c->copy_ev) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
@@ -470,8 +499,9 @@ int enqueue(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int
             cudaEvent_t ev = c->copy_ev[k % LANE_COPY_EVENTS];
             CU(cudaEventRecord(ev, c->copy_st));
             CU(cudaStreamWaitEvent(c->st, ev, 0));
-            if (nv12)
-                launch_nv12_to_bgr(c->d_nv12 + (size_t)off * bytes, c->d_frames + (size_t)off * bgr_bytes, m, c->g.H, c->g.W, c->st);
+            if (convert)
+                CU(launch_ingest(c->d_src + (size_t)off * bytes, in.format, m, in.h, in.w, c->d_frames + (size_t)off * bgr_bytes,
+                                 c->g.H, c->g.W, c->st));
             rc = run_stages(c, c->d_frames, off, m, sid, S, false);
             if (rc) return rc;
         }
@@ -512,6 +542,28 @@ int check_call(lane_ctx *c, const void *frames, int n, int S, const void *pf, co
     c->cur = (c->q_first + c->q_count) & 1;
     memset(c->slots[c->cur].launches, 0, sizeof(c->slots[c->cur].launches));
     return LANE_OK;
+}
+
+// lane_detect_batch and its ingest forms: validate, enqueue, collect.
+int detect_blocking(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int32_t *stream_id, int n_streams,
+                    double *prev_fit, uint8_t *prev_valid, lane_record *out, Ingest in)
+{
+    if (in.format != LANE_INPUT_BGR && ((in.h | in.w) & 1))
+        return fail(c, LANE_ERR_INVALID, "NV12 / I420 needs even width and height (%dx%d)", in.w, in.h);
+    int rc = check_call(c, frames, n, n_streams, prev_fit, prev_valid);
+    if (rc) return rc;
+    if (!out) return fail(c, LANE_ERR_INVALID, "out is null");
+    if (n > 65535 && (in.h != c->g.H || in.w != c->g.W))           // the resize kernels put the batch on the grid's z
+        return fail(c, LANE_ERR_UNSUPPORTED, "batch %d above 65535", n);
+    CU(cudaSetDevice(c->device));
+    if (stream_id)
+        for (int i = 0; i < n; i++)
+            if (stream_id[i] < 0 || stream_id[i] >= n_streams)
+                return fail(c, LANE_ERR_INVALID, "stream_id[%d]=%d outside [0,%d)", i, stream_id[i], n_streams);
+    if (c->profiling) CU(cudaEventRecord(c->slots[c->cur].ev[LANE_STAGE_H2D], c->st));
+    rc = enqueue(c, frames, on_device, n, stream_id, n_streams, prev_fit, prev_valid, in);
+    if (rc) return rc;
+    return lane_detect_collect(c, prev_fit, prev_valid, out);
 }
 
 }  // namespace
@@ -808,7 +860,7 @@ int lane_detect_enqueue(lane_ctx *c, const uint8_t *frames_dev, int n, const int
             if (stream_id[i] < 0 || stream_id[i] >= n_streams)
                 return fail(c, LANE_ERR_INVALID, "stream_id[%d]=%d outside [0,%d)", i, stream_id[i], n_streams);
     if (c->profiling) CU(cudaEventRecord(c->slots[c->cur].ev[LANE_STAGE_H2D], c->st));
-    return enqueue(c, frames_dev, true, n, stream_id, n_streams, prev_fit, prev_valid);
+    return enqueue(c, frames_dev, true, n, stream_id, n_streams, prev_fit, prev_valid, Ingest{LANE_INPUT_BGR, c->g.H, c->g.W});
 }
 
 int lane_detect_collect(lane_ctx *c, double *prev_fit, uint8_t *prev_valid, lane_record *out)
@@ -833,36 +885,29 @@ int lane_detect_collect(lane_ctx *c, double *prev_fit, uint8_t *prev_valid, lane
 int lane_detect_batch(lane_ctx *c, const uint8_t *frames, int frames_on_device, int n, const int32_t *stream_id,
                       int n_streams, double *prev_fit, uint8_t *prev_valid, lane_record *out)
 {
-    int rc = check_call(c, frames, n, n_streams, prev_fit, prev_valid);
-    if (rc) return rc;
-    if (!out) return fail(c, LANE_ERR_INVALID, "out is null");
-    CU(cudaSetDevice(c->device));
-    if (stream_id)
-        for (int i = 0; i < n; i++)
-            if (stream_id[i] < 0 || stream_id[i] >= n_streams)
-                return fail(c, LANE_ERR_INVALID, "stream_id[%d]=%d outside [0,%d)", i, stream_id[i], n_streams);
-    if (c->profiling) CU(cudaEventRecord(c->slots[c->cur].ev[LANE_STAGE_H2D], c->st));
-    rc = enqueue(c, frames, frames_on_device != 0, n, stream_id, n_streams, prev_fit, prev_valid);
-    if (rc) return rc;
-    return lane_detect_collect(c, prev_fit, prev_valid, out);
+    if (!c) return LANE_ERR_INVALID;
+    return detect_blocking(c, frames, frames_on_device != 0, n, stream_id, n_streams, prev_fit, prev_valid, out,
+                           Ingest{LANE_INPUT_BGR, c->g.H, c->g.W});
 }
 
 int lane_detect_batch_nv12(lane_ctx *c, const uint8_t *frames_nv12, int frames_on_device, int n, const int32_t *stream_id,
                            int n_streams, double *prev_fit, uint8_t *prev_valid, lane_record *out)
 {
-    int rc = check_call(c, frames_nv12, n, n_streams, prev_fit, prev_valid);
-    if (rc) return rc;
-    if (!out) return fail(c, LANE_ERR_INVALID, "out is null");
-    if ((c->g.H | c->g.W) & 1) return fail(c, LANE_ERR_INVALID, "NV12 needs even width and height (%dx%d)", c->g.W, c->g.H);
-    CU(cudaSetDevice(c->device));
-    if (stream_id)
-        for (int i = 0; i < n; i++)
-            if (stream_id[i] < 0 || stream_id[i] >= n_streams)
-                return fail(c, LANE_ERR_INVALID, "stream_id[%d]=%d outside [0,%d)", i, stream_id[i], n_streams);
-    if (c->profiling) CU(cudaEventRecord(c->slots[c->cur].ev[LANE_STAGE_H2D], c->st));
-    rc = enqueue(c, frames_nv12, frames_on_device != 0, n, stream_id, n_streams, prev_fit, prev_valid, true);
-    if (rc) return rc;
-    return lane_detect_collect(c, prev_fit, prev_valid, out);
+    if (!c) return LANE_ERR_INVALID;
+    return detect_blocking(c, frames_nv12, frames_on_device != 0, n, stream_id, n_streams, prev_fit, prev_valid, out,
+                           Ingest{LANE_INPUT_NV12, c->g.H, c->g.W});
+}
+
+int lane_detect_batch_ingest(lane_ctx *c, const uint8_t *frames, int frames_on_device, int n, int format, int src_h,
+                             int src_w, const int32_t *stream_id, int n_streams, double *prev_fit, uint8_t *prev_valid,
+                             lane_record *out)
+{
+    if (!c) return LANE_ERR_INVALID;
+    if (format != LANE_INPUT_BGR && format != LANE_INPUT_NV12 && format != LANE_INPUT_I420)
+        return fail(c, LANE_ERR_INVALID, "unknown input format %d", format);
+    if (src_h < 1 || src_w < 1) return fail(c, LANE_ERR_INVALID, "bad source size %dx%d", src_w, src_h);
+    return detect_blocking(c, frames, frames_on_device != 0, n, stream_id, n_streams, prev_fit, prev_valid, out,
+                           Ingest{format, src_h, src_w});
 }
 
 int lane_get_stage_ms(lane_ctx *c, float ms[LANE_NUM_STAGES], int32_t launches[LANE_NUM_STAGES])

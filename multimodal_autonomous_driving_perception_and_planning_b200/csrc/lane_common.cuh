@@ -10,6 +10,8 @@
 //   K5  k5_fit.cu         side split (:105-134), polyfit + EMA + points (:136-176), offset (:253-272)
 // Adjacent rows (SURVEY.md 8f):
 //   K0  k0_resize.cu      cv2.resize of VideoDataLoader.read_frame (data/loaders/video_loader.py:108,128)
+//       k0_nv12.cu        decoder output (NV12 / I420) -> BGR at the same size
+//       k0_ingest.cu      decoder output -> BGR -> cv2.resize in one pass; the ingest launcher (k0_common.cuh)
 //   K6  k6_frame_stats.cu mean / Laplacian variance / HSV green ratio of SceneClassifier (src/tagging/scene_classifier.py)
 //   K7  k7_draw.cu        cv2-exact rasteriser: draw_lanes (:220-251), draw_lane_offset_indicator (visualization/overlays.py:103-148),
 //                         the synthetic generator's frames (draw_prims.h: host expansion + the geometry shared with the device)
@@ -68,9 +70,6 @@ bool launch_fused_edge_redo(const uint8_t *frames, const int *frame_list, const 
                             uint32_t *k_bits, uint8_t *v_plane, uint8_t *blur_dbg, int *task_counter, int n, int H, int W,
                             cudaStream_t st, int *launches);
 void launch_gray_debug(const uint8_t *frame, uint8_t *gray, int H, int W, cudaStream_t st);
-
-// ---- K0b: NV12 -> BGR (device pointers, enqueued on st) ---------------------------------
-void launch_nv12_to_bgr(const uint8_t *src, uint8_t *dst, int n, int H, int W, cudaStream_t st);
 
 // ---- K2 ---------------------------------------------------------------------------------
 // thr: int4 per frame = (median_x2, low, high, 0)

@@ -18,6 +18,7 @@ import cv2
 import numpy as np
 
 from .. import _native
+from ..loaders.frame_ingest import check_target_size, check_yuv420
 
 
 @dataclass
@@ -138,13 +139,16 @@ class LaneDetector:
             out.append((left, right))
         return out
 
-    def _run(self, frames, stream_id, n_streams, prev_fit, prev_valid, nv12: bool = False) -> np.ndarray:
-        """Chunked native calls over frames [N,H,W,3] (numpy or CUDA torch; [N,H*3/2,W] when ``nv12``); state arrays
-        updated in place."""
-        n, h, w = int(frames.shape[0]), int(frames.shape[1]), int(frames.shape[2])
-        if nv12:
-            h = h * 2 // 3
-        fbytes = h * w * 3 // 2 if nv12 else h * w * 3
+    def _run(self, frames, stream_id, n_streams, prev_fit, prev_valid, fmt: int = _native.INPUT_BGR,
+             target_size: Optional[Tuple[int, int]] = None) -> np.ndarray:
+        """Chunked native calls over frames [N,H,W,3] (numpy or CUDA torch; [N,H*3/2,W] for the YUV 4:2:0 layouts of
+        ``fmt``), detected at ``target_size`` = (width, height) when given (the device resizes every frame to it first);
+        state arrays updated in place."""
+        n, sh, sw = int(frames.shape[0]), int(frames.shape[1]), int(frames.shape[2])
+        if fmt != _native.INPUT_BGR:
+            sh = sh * 2 // 3
+        fbytes = sh * sw * 3 if fmt == _native.INPUT_BGR else sh * sw * 3 // 2
+        h, w = (sh, sw) if target_size is None else (target_size[1], target_size[0])
         ctx = self._context(h, w, n, frames)
         s, oms = self.smoothing_factor, 1 - self.smoothing_factor
         chunks = []
@@ -159,7 +163,7 @@ class LaneDetector:
         def call(c, a, b):
             sid = None if stream_id is None else stream_id[a:b]
             src = frames.data_ptr() + a * fbytes if on_device else frames[a:b]
-            return c.detect(src, b - a, on_device, sid, n_streams, prev_fit, prev_valid, s, oms, nv12=nv12)
+            return c.detect(src, b - a, on_device, sid, n_streams, prev_fit, prev_valid, s, oms, fmt=fmt, src_hw=(sh, sw))
 
         for a in range(0, n, ctx.max_batch):
             b = min(a + ctx.max_batch, n)
@@ -208,17 +212,23 @@ class LaneDetector:
         self._check_frames(frame, batched=False)
         return self.detect_batch(frame[None])[0]
 
-    def detect_batch(self, frames) -> List[LanePair]:
+    def detect_batch(self, frames, *, target_size: Optional[Tuple[int, int]] = None) -> List[LanePair]:
         """``frames`` uint8 [N,H,W,3] (numpy, or a CUDA torch tensor already on the device).
 
         Semantics: identical to calling ``detect`` on ``frames[0..N-1]`` in order on this instance --
         the temporal smoothing is carried through the batch and left in ``prev_*_fit``.
+
+        ``target_size`` = (width, height), as ``VideoDataLoader(..., target_size=...)`` and ``cv2.resize`` take it: every
+        frame is first resized to it on the device, so the call equals ``detect_batch`` of
+        ``np.stack([cv2.resize(f, target_size) for f in frames])`` (``roi_vertices`` are in target coordinates).
         """
         self._check_frames(frames, batched=True)
+        if target_size is not None:
+            target_size = check_target_size(target_size)
         if frames.shape[0] == 0:
             return []
         fit, valid = self._state_arrays()
-        recs = self._run(frames, None, 1, fit, valid)
+        recs = self._run(frames, None, 1, fit, valid, target_size=target_size)
         lanes = self._lanes_from_records(recs)
         self._adopt_state(lanes)
         return lanes
@@ -313,20 +323,31 @@ class LaneDetector:
                 self.prev_right_fit = right.polynomial
                 break
 
-    def detect_batch_nv12(self, frames) -> List[LanePair]:
+    def detect_batch_nv12(self, frames, *, target_size: Optional[Tuple[int, int]] = None) -> List[LanePair]:
         """``detect_batch`` for frames still in a video decoder's NV12 layout: uint8 ``[N, H*3/2, W]`` (Y plane, then
         the interleaved half-resolution UV plane), numpy or CUDA tensor.  Equal to ``detect_batch`` on
         ``cv2.cvtColor(f, cv2.COLOR_YUV2BGR_NV12)`` of every frame -- the conversion runs on the device, so a host batch
-        moves 1.5 B/px over PCIe instead of 3."""
-        shape = tuple(frames.shape)
-        if len(shape) != 3 or shape[1] % 3 or shape[2] % 2 or (shape[1] * 2 // 3) % 2:
-            raise cv2.error(f"LaneDetector: expected NV12 frames of shape [N, H*3/2, W] with even H and W, got {shape}")
-        if str(frames.dtype).replace("torch.", "") != "uint8":
-            raise cv2.error(f"LaneDetector: frames must be uint8, got {frames.dtype}")
-        if shape[0] == 0:
+        moves 1.5 B/px over PCIe instead of 3.
+
+        ``target_size`` = (width, height): the decoder's frames at camera resolution are detected at that size, equal to
+        ``detect_batch`` of ``cv2.resize(cv2.cvtColor(f, COLOR_YUV2BGR_NV12), target_size)`` (``VideoDataLoader`` with
+        ``target_size``); conversion and resize are one kernel and only the NV12 bytes cross PCIe."""
+        return self._detect_yuv420(frames, _native.INPUT_NV12, target_size)
+
+    def detect_batch_i420(self, frames, *, target_size: Optional[Tuple[int, int]] = None) -> List[LanePair]:
+        """``detect_batch_nv12`` for the planar layout software decoders hand out (FFmpeg / PyAV ``yuv420p``): uint8
+        ``[N, H*3/2, W]`` = Y plane, U plane, V plane; equal to ``detect_batch`` on
+        ``cv2.cvtColor(f, cv2.COLOR_YUV2BGR_I420)`` of every frame, resized to ``target_size`` when given."""
+        return self._detect_yuv420(frames, _native.INPUT_I420, target_size)
+
+    def _detect_yuv420(self, frames, fmt: int, target_size) -> List[LanePair]:
+        check_yuv420(frames, "LaneDetector")
+        if target_size is not None:
+            target_size = check_target_size(target_size)
+        if frames.shape[0] == 0:
             return []
         fit, valid = self._state_arrays()
-        recs = self._run(frames, None, 1, fit, valid, nv12=True)
+        recs = self._run(frames, None, 1, fit, valid, fmt=fmt, target_size=target_size)
         lanes = self._lanes_from_records(recs)
         self._adopt_state(lanes)
         return lanes
