@@ -4,13 +4,9 @@
 // counting half of np.median (lane_detector.py:79).  Integer-exact (SURVEY.md A.1-A.3):
 //   gray = (3735 B + 19235 G + 9798 R + 2^14) >> 15
 //   blur = (sum_ij w_i w_j gray[y+i-2][x+j-2] + 128) >> 8,  w = [1 4 6 4 1], BORDER_REFLECT_101
-#include <stdlib.h>
-#include <string.h>
-
 #include <algorithm>
 
 #include "lane_common.cuh"
-#include <type_traits>
 
 namespace {
 
@@ -28,7 +24,8 @@ __device__ __forceinline__ uint32_t gray_of(uint32_t b, uint32_t g, uint32_t r)
 
 constexpr int TW = 64, TH = 32, NT = 256;
 
-// Generic tile kernel: any H, W (also the reference implementation the strip kernel is checked against).
+// One CTA per 64 x 32 tile of a frame, any H, W.  Blurred frames of widths and heights the fused edge kernel
+// (k1_fused.cu) does not take run here.
 __global__ void __launch_bounds__(NT) k1_tile(const uint8_t *__restrict__ frames, uint8_t *__restrict__ blur,
                                               uint32_t *__restrict__ hist, int H, int W)
 {
@@ -67,271 +64,6 @@ __global__ void __launch_bounds__(NT) k1_tile(const uint8_t *__restrict__ frames
     if (lh[tid]) atomicAdd(&hist[f * 256 + tid], lh[tid]);
 }
 
-// ---------------------------------------------------------------------------------------------
-// Strip kernel (W % 16 == 0, 16-byte aligned frames): the HBM-roofline path.
-//
-// One warp owns a column strip of 512 pixels (16 px per lane: three 16-byte loads per lane per row)
-// and rolls down a band of rows keeping everything in registers:
-//   gray    : 2 IDP2A per pixel straight off the interleaved BGR words (Q16 coefficients = 2x the Q15
-//             ones, so the rounded result lands byte-aligned), packed as u16x2 pairs
-//   vertical: [1 4 6 4 1] as four chained pair-adds ([1 1]^4) on packed u16x2 (max 4080, carry-free)
-//   horizontal: neighbours' edge pairs by two shuffles, odd alignments by PRMT, u16x2 arithmetic
-//             (max 65408, carry-free), +128 >> 8 folded into the final byte pick (PRMT)
-//   store   : one 16-byte store per lane per row
-//   histogram: per-lane private byte counters in shared memory (no atomics, conflict-free in smooth
-//             regions), flushed every 15 rows into per-lane registers, one RED per bin per task
-// Lanes 0 and 31 only provide the 2-px halo (30 x 16 = 480 output px per warp); image borders are
-// REFLECT_101 on register pairs (columns) and on the row index (rows).  Warps pull (frame, band,
-// strip) tasks from a global counter, so the grid is persistent and there is no tail.
-constexpr int SPX = 16;                 // pixels per lane
-constexpr int STRIP_OUT = 30 * SPX;     // 480 output pixels per warp
-constexpr int SWARPS = 4;               // warps per CTA
-constexpr int FLUSH_ROWS = 15;          // 15 rows x 16 px = 240 < 256 increments per byte counter
-
-__device__ __forceinline__ uint32_t dp2a_lo(uint32_t a, uint32_t b, uint32_t c)
-{
-    uint32_t d;
-    asm("dp2a.lo.u32.u32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
-    return d;
-}
-__device__ __forceinline__ uint32_t dp2a_hi(uint32_t a, uint32_t b, uint32_t c)
-{
-    uint32_t d;
-    asm("dp2a.hi.u32.u32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
-    return d;
-}
-__device__ __forceinline__ uint32_t h2add(uint32_t a, uint32_t b)
-{
-    uint32_t d;
-    asm("add.f16x2 %0, %1, %2;" : "=r"(d) : "r"(a), "r"(b));
-    return d;
-}
-__device__ __forceinline__ uint4 ldg_stream(const uint4 *p)
-{
-    uint4 r;
-    asm volatile("ld.global.nc.v4.u32 {%0, %1, %2, %3}, [%4];"
-                 : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
-    return r;
-}
-
-
-// 16 interleaved BGR pixels (12 words) -> 8 packed u16x2 gray pairs
-__device__ __forceinline__ void gray16(const uint32_t (&w)[12], uint32_t (&g)[8])
-{
-    constexpr uint32_t CB = 2 * 3735, CG = 2 * 19235, CR = 2 * 9798, RND = 1u << 15;
-    constexpr uint32_t KBG = CB | (CG << 16), KR0 = CR, K0B = CB << 16, KGR = CG | (CR << 16);
-#pragma unroll
-    for (int q = 0; q < 4; q++) {       // 4 pixels per 3 words
-        const uint32_t w0 = w[3 * q], w1 = w[3 * q + 1], w2 = w[3 * q + 2];
-        uint32_t s0 = dp2a_hi(KR0, w0, dp2a_lo(KBG, w0, RND));   // B0 G0 R0 | .
-        uint32_t s1 = dp2a_lo(KGR, w1, dp2a_hi(K0B, w0, RND));   // . . . B1 | G1 R1
-        uint32_t s2 = dp2a_lo(KR0, w2, dp2a_hi(KBG, w1, RND));   // . . B2 G2 | R2
-        uint32_t s3 = dp2a_hi(KGR, w2, dp2a_lo(K0B, w2, RND));   // . B3 G3 R3
-        g[2 * q] = __byte_perm(s0, s1, 0x7632);                  // gray = bits 16..23 of each sum
-        g[2 * q + 1] = __byte_perm(s2, s3, 0x7632);
-    }
-}
-
-// TMA = true: every warp stages its strip rows in a private shared-memory ring with cp.async.bulk (one 1.5 KB
-// bulk copy per row, completion on an mbarrier), RING rows deep, so RING-1 rows of loads are in flight per warp
-// without holding registers; lanes then read their 48 bytes with three conflict-free LDS.128.
-// TMA = false (default) uses direct 16-byte ld.global.nc loads prefetched one row ahead in registers.
-constexpr int RING = 3;
-constexpr int ROW_BYTES = 32 * SPX * 3;          // 1536
-
-template <bool TMA, int MINB = 0>
-__global__ void __launch_bounds__(SWARPS * 32, MINB) k1_strip(const uint8_t *__restrict__ frames, uint8_t *__restrict__ blur,
-                                                        uint32_t *__restrict__ hist, int *__restrict__ task_counter,
-                                                        int n_frames, int H, int W, int band_rows, int tail_frames, int tail_rows)
-{
-    __shared__ uint32_t k1_tot[SWARPS][256];
-    extern __shared__ __align__(128) uint8_t k1_smem[];      // [SWARPS][8192] counters | [SWARPS][RING][1536] ring | barriers
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    uint8_t *wh = k1_smem + wid * (256 * 32);
-    uint8_t *ring = k1_smem + SWARPS * (256 * 32) + wid * (RING * ROW_BYTES);
-    unsigned long long *bars = reinterpret_cast<unsigned long long *>(k1_smem + SWARPS * (256 * 32) + SWARPS * RING * ROW_BYTES) + wid * RING;
-    uint32_t issued = 0, consumed = 0;             // monotonic per-warp ring counters (TMA)
-    if (TMA) {
-        if (lane == 0) {
-            for (int i = 0; i < RING; i++) mbar_init(smem_u32(&bars[i]), 1);
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        }
-        __syncwarp();
-    }
-    {   // zero this warp's private counters
-        uint4 *z = reinterpret_cast<uint4 *>(wh);
-        for (int i = lane; i < 256 * 32 / 16; i += 32) z[i] = make_uint4(0, 0, 0, 0);
-    }
-    __syncwarp();
-    const int n_strips = (W + STRIP_OUT - 1) / STRIP_OUT;
-    // tasks are handed out in order: the first n_frames - tail_frames frames in bands of band_rows rows, the last
-    // tail_frames frames in thinner bands, so the warps run dry within a short task of each other at the end
-    const int n_bands = (H + band_rows - 1) / band_rows, n_bands_t = (H + tail_rows - 1) / tail_rows;
-    const int n_main = (n_frames - tail_frames) * n_bands * n_strips;
-    const int n_tasks = n_main + tail_frames * n_bands_t * n_strips;
-    const size_t frame_px = (size_t)H * W;
-
-    for (;;) {
-        int task = 0;
-        if (lane == 0) task = atomicAdd(task_counter, 1);
-        task = __shfl_sync(0xffffffffu, task, 0);
-        if (task >= n_tasks) break;
-        const bool tail = task >= n_main;
-        const int tt = tail ? task - n_main : task, nb = tail ? n_bands_t : n_bands, br = tail ? tail_rows : band_rows;
-        const int strip = tt % n_strips;
-        const int band = (tt / n_strips) % nb;
-        const int f = tt / (n_strips * nb) + (tail ? n_frames - tail_frames : 0);
-        const int r0 = band * br, r1 = min(r0 + br, H);
-        const int xl = strip * STRIP_OUT - SPX + SPX * lane;          // first pixel of this lane
-        const bool in_img = xl >= 0 && xl < W;
-        const bool is_out = in_img && lane >= 1 && lane <= 30;
-        const bool left_edge = xl == 0, right_edge = xl + SPX == W;
-        const uint8_t *src = frames + f * frame_px * 3 + (size_t)max(xl, 0) * 3;
-        uint8_t *dst = blur + f * frame_px + max(xl, 0);
-
-        // column-filter state, two generations deep: rows alternate between slot 0 and slot 1 (the row loop is
-        // unrolled by two below) so "previous row" is the other slot and no register moves are needed
-        uint32_t sg[2][8], s1[2][8], s2[2][8], s3[2][8];
-#pragma unroll
-        for (int j = 0; j < 8; j++)
-            sg[0][j] = sg[1][j] = s1[0][j] = s1[1][j] = s2[0][j] = s2[1][j] = s3[0][j] = s3[1][j] = 0;
-        // per-task 32-bit totals live in shared memory (touched once per flush), not in 8 registers
-#pragma unroll
-        for (int b = 0; b < 8; b++) k1_tot[wid][b * 32 + lane] = 0;
-        int since_flush = 0;
-
-        auto flush = [&]() {
-            __syncwarp();
-#pragma unroll
-            for (int b = 0; b < 8; b++) {
-                uint4 *row = reinterpret_cast<uint4 *>(wh + (b * 32 + lane) * 32);
-                uint4 a = row[0], c = row[1];
-                uint32_t s = 0;
-                s = __dp4a(a.x, 0x01010101u, s); s = __dp4a(a.y, 0x01010101u, s);
-                s = __dp4a(a.z, 0x01010101u, s); s = __dp4a(a.w, 0x01010101u, s);
-                s = __dp4a(c.x, 0x01010101u, s); s = __dp4a(c.y, 0x01010101u, s);
-                s = __dp4a(c.z, 0x01010101u, s); s = __dp4a(c.w, 0x01010101u, s);
-                k1_tot[wid][b * 32 + lane] += s;
-                row[0] = make_uint4(0, 0, 0, 0); row[1] = make_uint4(0, 0, 0, 0);
-            }
-            __syncwarp();
-        };
-
-        // bulk-copy geometry of this strip: the in-image part of [strip_x0, strip_x0 + 512)
-        const int strip_x0 = strip * STRIP_OUT - SPX;
-        const int copy_x0 = max(strip_x0, 0);
-        const uint32_t copy_bytes = (uint32_t)(min(strip_x0 + 32 * SPX, W) - copy_x0) * 3u;
-        const uint32_t copy_off = (uint32_t)(copy_x0 - strip_x0) * 3u;
-        const uint8_t *frame_base = frames + f * frame_px * 3;
-        auto issue_row = [&](int y) {               // lane 0: arm the slot's barrier and start the copy
-            if (lane == 0) {
-                const uint32_t slot = issued % RING;
-                const uint32_t bar = smem_u32(&bars[slot]);
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // earlier LDS of this slot vs the async write
-                mbar_expect_tx(bar, copy_bytes);
-                bulk_g2s(smem_u32(ring + slot * ROW_BYTES) + copy_off,
-                         frame_base + ((size_t)fold101(y, H) * W + copy_x0) * 3, copy_bytes, bar);
-            }
-            issued++;
-        };
-        uint32_t w[12];
-        auto load_row = [&](int y) {
-            if (TMA) {
-                const uint32_t slot = consumed % RING;
-                mbar_wait(smem_u32(&bars[slot]), (consumed / RING) & 1u);
-                const uint4 *p = reinterpret_cast<const uint4 *>(ring + slot * ROW_BYTES) + 3 * lane;
-                uint4 a = p[0], b = p[1], c = p[2];
-                w[0] = a.x; w[1] = a.y; w[2] = a.z; w[3] = a.w; w[4] = b.x; w[5] = b.y; w[6] = b.z; w[7] = b.w;
-                w[8] = c.x; w[9] = c.y; w[10] = c.z; w[11] = c.w;
-                consumed++;
-                __syncwarp();                        // every lane has its copy: the slot may be refilled
-                if (y + RING < r1 + 2) issue_row(y + RING);
-                return;
-            }
-            // BORDER_REFLECT_101 for a two-row halo (H >= 4 on this path): |y|, then mirrored at the bottom; 32-bit
-            // byte offset inside the frame
-            const int ya = abs(y), yy = min(ya, 2 * H - 2 - ya);
-            if (in_img) {
-                const uint4 *p = reinterpret_cast<const uint4 *>(src + (uint32_t)(yy * W) * 3u);
-                uint4 a = ldg_stream(p), b = ldg_stream(p + 1), c = ldg_stream(p + 2);
-                w[0] = a.x; w[1] = a.y; w[2] = a.z; w[3] = a.w; w[4] = b.x; w[5] = b.y; w[6] = b.z; w[7] = b.w;
-                w[8] = c.x; w[9] = c.y; w[10] = c.z; w[11] = c.w;
-            }
-        };
-#pragma unroll
-        for (int j = 0; j < 12; j++) w[j] = 0;
-        if (TMA)
-            for (int i = 0; i < RING && r0 - 2 + i < r1 + 2; i++) issue_row(r0 - 2 + i);
-        load_row(r0 - 2);
-        const uint32_t hbase = smem_u32(wh) + lane;         // this lane's column of the private counters
-        auto row_step = [&](auto slot, int y) {
-            constexpr int c = decltype(slot)::value, o = c ^ 1;
-            gray16(w, sg[c]);
-            if (y + 1 < r1 + 2) load_row(y + 1);        // next row: from the ring (TMA) or prefetched into registers
-            uint32_t V[8];
-#pragma unroll
-            for (int j = 0; j < 8; j++) {               // [1 1]^4 down the column
-                // The first three stages stay below 2048, where binary16 (denormals included) is exact and its bit
-                // pattern is the integer itself, so they run as add.f16x2 on the FMA pipe; that takes 24 adds per
-                // row off the ALU pipe, which is the busiest one in this kernel.  The last stage (<= 4080) is integer.
-                s1[c][j] = h2add(sg[c][j], sg[o][j]);
-                s2[c][j] = h2add(s1[c][j], s1[o][j]);
-                s3[c][j] = h2add(s2[c][j], s2[o][j]);
-                V[j] = s3[c][j] + s3[o][j];
-            }
-            if (y < r0 + 2) return;                      // pipeline fill: V is the blur column sum of row y-2
-            const int yo = y - 2;
-            uint32_t L7 = __shfl_up_sync(0xffffffffu, V[7], 1);
-            uint32_t R0 = __shfl_down_sync(0xffffffffu, V[0], 1);
-            if (left_edge) L7 = __byte_perm(V[1], V[0], 0x7610);     // (x=-2,-1) := (x=2, 1)
-            if (right_edge) R0 = __byte_perm(V[7], V[6], 0x7610);    // (x=W, W+1) := (x=W-2, W-3)
-            uint32_t O[9];
-            O[0] = __byte_perm(L7, V[0], 0x5432);
-#pragma unroll
-            for (int j = 1; j < 8; j++) O[j] = __byte_perm(V[j - 1], V[j], 0x5432);
-            O[8] = __byte_perm(V[7], R0, 0x5432);
-            uint32_t Hs[8];
-#pragma unroll
-            for (int j = 0; j < 8; j++) {
-                const uint32_t vm = j == 0 ? L7 : V[j - 1], vp = j == 7 ? R0 : V[j + 1];
-                Hs[j] = vm + vp + 0x00800080u + 4u * (O[j] + O[j + 1]) + 6u * V[j];
-            }
-            uint4 ov;
-            ov.x = __byte_perm(Hs[0], Hs[1], 0x7531);
-            ov.y = __byte_perm(Hs[2], Hs[3], 0x7531);
-            ov.z = __byte_perm(Hs[4], Hs[5], 0x7531);
-            ov.w = __byte_perm(Hs[6], Hs[7], 0x7531);
-            if (is_out) {
-                *reinterpret_cast<uint4 *>(dst + (uint32_t)yo * (uint32_t)W) = ov;
-                const uint32_t ow[4] = {ov.x, ov.y, ov.z, ov.w};
-#pragma unroll
-                for (int q = 0; q < 4; q++) {
-#pragma unroll
-                    for (int k = 0; k < 4; k++) {
-                        // counter address = base + 32 * byte k of the word, in one dot-product instruction (FMA pipe)
-                        const uint32_t addr = __dp4a(ow[q], 0x20u << (8 * k), hbase);
-                        uint32_t t;
-                        asm volatile("ld.shared.u8 %0, [%1];" : "=r"(t) : "r"(addr));
-                        t += 1;
-                        asm volatile("st.shared.u8 [%0], %1;" ::"r"(addr), "r"(t) : "memory");
-                    }
-                }
-            }
-            if (++since_flush == FLUSH_ROWS) { flush(); since_flush = 0; }
-        };
-        for (int y = r0 - 2;;) {
-            row_step(std::integral_constant<int, 0>{}, y);
-            if (++y >= r1 + 2) break;
-            row_step(std::integral_constant<int, 1>{}, y);
-            if (++y >= r1 + 2) break;
-        }
-        flush();
-#pragma unroll
-        for (int b = 0; b < 8; b++)
-            if (const uint32_t t = k1_tot[wid][b * 32 + lane]) atomicAdd(&hist[f * 256 + b * 32 + lane], t);
-    }
-}
-
 // gray plane + histogram without the blur (scene_classifier.py:145-146 runs cv2.Canny on the plain grayscale frame)
 __global__ void __launch_bounds__(256) k1_gray_hist(const uint8_t *__restrict__ frames, uint8_t *__restrict__ out,
                                                     uint32_t *__restrict__ hist, int P)
@@ -360,51 +92,12 @@ __global__ void k_gray(const uint8_t *__restrict__ frame, uint8_t *__restrict__ 
 }  // namespace
 
 void launch_blur_hist(const uint8_t *frames, uint8_t *blur_out, uint32_t *hist, int n, int H, int W,
-                      cudaStream_t st, int *launches, int *task_counter, int force_tile, int blur)
+                      cudaStream_t st, int *launches, int blur)
 {
     cudaMemsetAsync(hist, 0, sizeof(uint32_t) * 256 * n, st);
     if (!blur) {
         dim3 grid(std::min((H * W + 255) / 256, 1184), n);
         k1_gray_hist<<<grid, 256, 0, st>>>(frames, blur_out, hist, H * W);
-        *launches += 1;
-        return;
-    }
-    const bool aligned = (W % 16 == 0) && (((uintptr_t)frames | (uintptr_t)blur_out) % 16 == 0);
-    if (aligned && !force_tile && H >= 4 && (size_t)H * W * 3 < ((size_t)1 << 32)) {
-        const int sms = lane_sm_count();
-        // band height: 102 rows (3.9 % halo rows) when there is plenty of work, thinner when a small batch would
-        // otherwise leave most of the sms*5*SWARPS warps without a task; the last sixteenth of the frames is cut into
-        // bands a third as high to shorten the end-of-kernel tail
-        const int n_strips = (W + STRIP_OUT - 1) / STRIP_OUT, warps = sms * 5 * SWARPS;
-        static const int band_env = getenv("LANE_K1_BAND") ? atoi(getenv("LANE_K1_BAND")) : 0;
-        static const int tail_env = getenv("LANE_K1_TAIL") ? atoi(getenv("LANE_K1_TAIL")) : -1;
-        int band_rows = band_env > 0 ? band_env : (H >= 540 ? 102 : (H >= 120 ? 60 : H));
-        {
-            const long rows_per_warp = ((long)n * H * n_strips + 2 * warps - 1) / (2 * warps);   // >= 2 tasks per warp
-            if (!band_env) band_rows = (int)std::max(12L, std::min((long)band_rows, rows_per_warp));
-        }
-        int tail_frames = tail_env >= 0 ? std::min(tail_env, n) : (n >= 16 ? n / 16 : 0);
-        const int tail_rows = std::max(12, band_rows / 3);
-        if (tail_rows >= band_rows) tail_frames = 0;
-        cudaMemsetAsync(task_counter, 0, sizeof(int), st);
-        // default: direct 16-byte loads.  LANE_B200_K1=tma selects the bulk-copy staged variant (measured slower on
-        // B200: 0.645 vs 0.546 ms per 256 1080p frames -- the kernel is ALU-issue bound, not load-latency bound)
-        static const bool use_ldg = !(getenv("LANE_B200_K1") && !strcmp(getenv("LANE_B200_K1"), "tma"));
-        const size_t smem_ldg = SWARPS * 256 * 32;
-        const size_t smem_tma = smem_ldg + SWARPS * RING * ROW_BYTES + SWARPS * RING * 8;
-        static bool configured[LANE_MAX_DEVICES];
-        if (!configured[lane_cur_device()]) {
-            cudaFuncSetAttribute(k1_strip<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_tma);
-            configured[lane_cur_device()] = true;
-        }
-        static const int minb = getenv("LANE_K1_MINB") ? atoi(getenv("LANE_K1_MINB")) : 5;
-        if (use_ldg && minb == 5) {
-            k1_strip<false, 5><<<sms * 5, SWARPS * 32, smem_ldg, st>>>(frames, blur_out, hist, task_counter, n, H, W, band_rows,
-                                                                     tail_frames, tail_rows);
-        } else if (use_ldg)
-            k1_strip<false, 0><<<sms * 4, SWARPS * 32, smem_ldg, st>>>(frames, blur_out, hist, task_counter, n, H, W, band_rows, tail_frames, tail_rows);
-        else
-            k1_strip<true><<<sms * 4, SWARPS * 32, smem_tma, st>>>(frames, blur_out, hist, task_counter, n, H, W, band_rows, tail_frames, tail_rows);
     } else {
         dim3 grid((W + TW - 1) / TW, (H + TH - 1) / TH, n);
         k1_tile<<<grid, NT, 0, st>>>(frames, blur_out, hist, H, W);

@@ -21,8 +21,11 @@
 // was too optimistic), flags the frame, and the frame is redone with pre = low (launch_fused_edge_redo): results never
 // depend on the estimate, only the time does.
 //
-// Data path (one warp = one 512-px column strip, 16 px per lane, rolling down a band of rows, as in k1_blur_hist.cu):
-//   gray / vertical [1 4 6 4 1] / horizontal pass: registers, packed u16x2 (see k1_blur_hist.cu)
+// Data path (one warp = one 512-px column strip, 16 px per lane, rolling down a band of rows; warps pull (frame, band,
+// strip) tasks from a global counter):
+//   gray: 2 IDP2A per pixel straight off the interleaved BGR words, packed as u16x2 pairs (gray16)
+//   vertical [1 4 6 4 1] as four chained pair-adds ([1 1]^4) on the packed pairs; horizontal pass: neighbours' edge pairs
+//     by two shuffles, odd alignments by PRMT, +128 >> 8 folded into the byte pick
 //   Sobel on the blurred row while it is still in registers: h1 = B(x+1) - B(x-1), h2 = B(x-1) + 2B(x) + B(x+1) per row,
 //     dx = h1(r-1) + 2 h1(r) + h1(r+1), dy = h2(r+1) - h2(r-1) down the column, all as exact packed f16x2 (every value
 //     is an integer below 2048 in units of 2^-24, where binary16 is exact and its bit pattern is the integer)
@@ -31,8 +34,8 @@
 //     puts its 3-4 candidate pixels into ONE lane's 16-px span; walking them in that lane would serialise the warp),
 //     each lane does the TG22 sector test and the asymmetric 3x3 comparison for its share and ORs survivors into a
 //     per-row bit string; fifteen lanes store the row's K words, survivors' V bytes go out as single byte stores
-//   histogram: per-lane private byte counters (k1_blur_hist.cu), with a one-update fast path for lanes whose sixteen
-//     blurred pixels are all equal (sky, asphalt)
+//   histogram: a per-warp table of 32-bit counters (shared-memory atomics), with a one-update fast path for lanes whose
+//     sixteen blurred pixels are all equal (sky, asphalt)
 #include <stdlib.h>
 #include <string.h>
 
@@ -48,6 +51,9 @@ namespace {
 constexpr int SPX = 16;                 // pixels per lane
 constexpr int STRIP_OUT = 30 * SPX;     // 480 output pixels per warp (lanes 0 and 31 are halo providers)
 constexpr int FWARPS = 4;               // warps per CTA
+// CTAs per SM: 3 leaves 168 registers per thread.  Measured on B200, 256 x 1080p: 3 -> 0.74 ms, 4 -> 0.88 ms (at 128
+// registers the spills cost more than four more warps hide).
+constexpr int FCTAS = 3;
 constexpr int RS = 512 + 16;            // M ring row stride in u16 (8 px of padding either side)
 
 // per-warp shared memory (bytes)
@@ -210,8 +216,7 @@ struct FusedArgs {
     int band_rows, tail_frames, tail_rows;
 };
 
-template <int MINB>
-__global__ void __launch_bounds__(FWARPS * 32, MINB) k1_fused(FusedArgs A)
+__global__ void __launch_bounds__(FWARPS * 32, FCTAS) k1_fused(FusedArgs A)
 {
     extern __shared__ __align__(128) uint8_t fsm[];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -568,30 +573,18 @@ bool lane_fused_edge_supported(int H, int W, const void *frames)
     return (W % 16 == 0) && H >= 16 && ((uintptr_t)frames % 16 == 0) && (size_t)H * W * 3 < ((size_t)1 << 32);
 }
 
-static int fused_minb()
-{
-    // CTAs (of four warps) per SM: 4 = 128 registers per thread, 3 = 168 (LANE_K1F_MINB, A/B knob)
-    // measured on B200, 256 x 1080p: 3 -> 0.74 ms, 4 -> 0.88 ms (the 160 bytes of spills cost more than four more warps hide)
-    static const int minb = getenv("LANE_K1F_MINB") ? atoi(getenv("LANE_K1F_MINB")) : 3;
-    return minb == 4 ? 4 : 3;
-}
-
 static void fused_config(int n, int H, int W, int *band_rows, int *tail_frames, int *tail_rows)
 {
     const int sms = lane_sm_count();
-    const int n_strips = (W + STRIP_OUT - 1) / STRIP_OUT, warps = sms * fused_minb() * FWARPS;
-    static const int band_env = getenv("LANE_K1F_BAND") ? atoi(getenv("LANE_K1F_BAND")) : 0;
-    static const int tail_env = getenv("LANE_K1F_TAIL") ? atoi(getenv("LANE_K1F_TAIL")) : -1;
+    const int n_strips = (W + STRIP_OUT - 1) / STRIP_OUT, warps = sms * FCTAS * FWARPS;
     // Every band re-reads 8 halo rows (7 % at 108 rows), but a task is also the unit the warps run dry by at the end of
     // the kernel (a row takes a warp ~1 us): measured on B200 (256 x 1080p) 108-row bands with the last eighth of the
     // frames cut into bands a third as high beat both taller bands (135: +1 %, 270: +15 %) and a shorter graded tail
     // (n/16: +4 %).  Small batches get thinner bands so that every resident warp has at least two tasks.
-    int br = band_env > 0 ? band_env : (H >= 540 ? 108 : (H >= 120 ? 60 : H));
-    if (!band_env) {
-        const long rows_per_warp = ((long)n * H * n_strips + 2 * warps - 1) / (2 * warps);
-        br = (int)std::max(16L, std::min((long)br, rows_per_warp));
-    }
-    int tf = tail_env >= 0 ? std::min(tail_env, n) : (n >= 16 ? n / 8 : 0);
+    int br = H >= 540 ? 108 : (H >= 120 ? 60 : H);
+    const long rows_per_warp = ((long)n * H * n_strips + 2 * warps - 1) / (2 * warps);
+    br = (int)std::max(16L, std::min((long)br, rows_per_warp));
+    int tf = n >= 16 ? n / 8 : 0;
     const int tr = std::max(16, br / 3);
     if (tr >= br) tf = 0;
     *band_rows = br; *tail_frames = tf; *tail_rows = tr;
@@ -601,16 +594,14 @@ static bool fused_launch(FusedArgs A, cudaStream_t st)
 {
     static bool configured[LANE_MAX_DEVICES];
     if (!configured[lane_cur_device()]) {
-        if (cudaFuncSetAttribute(k1_fused<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, FWARPS * SM_WARP) != cudaSuccess ||
-            cudaFuncSetAttribute(k1_fused<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, FWARPS * SM_WARP) != cudaSuccess) {
+        if (cudaFuncSetAttribute(k1_fused, cudaFuncAttributeMaxDynamicSharedMemorySize, FWARPS * SM_WARP) != cudaSuccess) {
             cudaGetLastError();
             return false;
         }
         configured[lane_cur_device()] = true;
     }
     cudaMemsetAsync(A.task_counter, 0, sizeof(int), st);
-    if (fused_minb() == 3) k1_fused<3><<<lane_sm_count() * 3, FWARPS * 32, FWARPS * SM_WARP, st>>>(A);
-    else k1_fused<4><<<lane_sm_count() * 4, FWARPS * 32, FWARPS * SM_WARP, st>>>(A);
+    k1_fused<<<lane_sm_count() * FCTAS, FWARPS * 32, FWARPS * SM_WARP, st>>>(A);
     return cudaPeekAtLastError() == cudaSuccess;
 }
 

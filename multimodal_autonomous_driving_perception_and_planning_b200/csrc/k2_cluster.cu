@@ -233,9 +233,9 @@ __device__ __forceinline__ void canny_rows(int H, int W, int WW, const uint8_t *
 // Warps pull (frame, band, strip) tasks from a global counter and write the candidate plane C and the
 // strong plane S (32 px per word) to global memory; perfectly load-balanced, no barriers at all.
 constexpr int K2A_WARPS = 4;
+constexpr int K2A_CTAS = 6;             // CTAs per SM
 
-template <int MINB>
-__global__ void __launch_bounds__(K2A_WARPS * 32, MINB) k2a_sobel_nms(const uint8_t *__restrict__ blur, const uint32_t *__restrict__ hist,
+__global__ void __launch_bounds__(K2A_WARPS * 32, K2A_CTAS) k2a_sobel_nms(const uint8_t *__restrict__ blur, const uint32_t *__restrict__ hist,
                                                                const uint8_t *__restrict__ lut_low,
                                                                const uint8_t *__restrict__ lut_high, int4 *__restrict__ thr,
                                                                uint32_t *__restrict__ c_bits, uint32_t *__restrict__ s_bits,
@@ -247,7 +247,7 @@ __global__ void __launch_bounds__(K2A_WARPS * 32, MINB) k2a_sobel_nms(const uint
     const int WW = (W + 31) / 32;
     const int n_strips = (W + STRIP_OUT - 1) / STRIP_OUT;
     // tasks in hand-out order: the first n_frames - tail_frames frames in bands of band_rows rows, the rest in thinner
-    // bands so the end-of-kernel tail is short (same scheme as K1)
+    // bands so the end-of-kernel tail is short (same scheme as K1F)
     const int n_bands = (H + band_rows - 1) / band_rows, n_bands_t = (H + tail_rows - 1) / tail_rows;
     const int n_main = (n_frames - tail_frames) * n_bands * n_strips;
     const int n_tasks = n_main + tail_frames * n_bands_t * n_strips;
@@ -726,8 +726,7 @@ static bool k2b_plan(int H, int W, int *G_out, int *R_out, size_t *smem_out)
 {
     const int WW = (W + 31) / 32;
     int G = 1;
-    const int rows_per_band = getenv("LANE_K2_ROWS") ? atoi(getenv("LANE_K2_ROWS")) : 160;   // tuning knob
-    while (G < 16 && H > rows_per_band * G) G *= 2;
+    while (G < 16 && H > 160 * G) G *= 2;                // bands of up to 160 rows
     size_t smem = 0;
     int R = 0;
     for (;; G *= 2) {
@@ -776,24 +775,15 @@ bool launch_canny_cluster(const uint8_t *blur, const uint32_t *hist, const uint8
     const int sms = lane_sm_count();
     cudaMemsetAsync(task_counter, 0, sizeof(int), st);
     {
-        static const int band_env = getenv("LANE_K2A_BAND") ? atoi(getenv("LANE_K2A_BAND")) : 0;
-        static const int tail_env = getenv("LANE_K2A_TAIL") ? atoi(getenv("LANE_K2A_TAIL")) : -1;
-        static const int minb = getenv("LANE_K2A_MINB") ? atoi(getenv("LANE_K2A_MINB")) : 6;
-        const int n_strips = (W + STRIP_OUT - 1) / STRIP_OUT, warps = sms * minb * K2A_WARPS;
-        int band_rows = band_env > 0 ? band_env : 64;
-        if (!band_env) {        // small batches: at least two tasks per resident warp, bands no thinner than 12 rows
-            const long rows_per_warp = ((long)n * H * n_strips + 2 * warps - 1) / (2 * warps);
-            band_rows = (int)std::max(12L, std::min((long)band_rows, rows_per_warp));
-        }
-        int tail_frames = tail_env >= 0 ? std::min(tail_env, n) : (n >= 16 ? n / 16 : 0);
+        const int n_strips = (W + STRIP_OUT - 1) / STRIP_OUT, warps = sms * K2A_CTAS * K2A_WARPS;
+        // small batches: at least two tasks per resident warp, bands no thinner than 12 rows
+        const long rows_per_warp = ((long)n * H * n_strips + 2 * warps - 1) / (2 * warps);
+        const int band_rows = (int)std::max(12L, std::min(64L, rows_per_warp));
+        int tail_frames = n >= 16 ? n / 16 : 0;
         const int tail_rows = std::max(12, band_rows / 3);
         if (tail_rows >= band_rows) tail_frames = 0;
-        if (minb == 6)
-            k2a_sobel_nms<6><<<sms * 6, K2A_WARPS * 32, 0, st>>>(blur, hist, lut_low, lut_high, thr, c_bits, s_bits, task_counter,
-                                                                 n, H, W, band_rows, tail_frames, tail_rows);
-        else
-            k2a_sobel_nms<5><<<sms * 5, K2A_WARPS * 32, 0, st>>>(blur, hist, lut_low, lut_high, thr, c_bits, s_bits, task_counter,
-                                                                 n, H, W, band_rows, tail_frames, tail_rows);
+        k2a_sobel_nms<<<sms * K2A_CTAS, K2A_WARPS * 32, 0, st>>>(blur, hist, lut_low, lut_high, thr, c_bits, s_bits, task_counter,
+                                                                  n, H, W, band_rows, tail_frames, tail_rows);
     }
     K2Args A{};
     A.c_bits = c_bits; A.s_bits = s_bits; A.roi_bits = roi_bits;

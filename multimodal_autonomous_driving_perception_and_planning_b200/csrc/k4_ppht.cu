@@ -4,11 +4,12 @@
 // from the row-major list with the MWC generator RNG(0xFFFFFFFFFFFFFFFF), each votes 180 bins
 // (float32 rho = x*cos + y*sin, separate multiply/add, round-half-even), and the first bin to reach
 // the threshold triggers a fixed-point line walk that removes (and, for a good line, un-votes) the
-// pixels on it.  One CTA owns one frame.  Thread n < 180 owns angle n and its accumulator row, so
-// its in-order atomics see exactly the sequential vote counts; points are drawn in batches (the
-// draw order never depends on the accumulator or the mask) and voted speculatively: the first
-// triggering point of a batch is exact, later votes of the batch are rolled back and replayed
-// after the walk.
+// pixels on it.  Every angle is voted by exactly one thread, in point order, so it sees exactly the
+// sequential vote counts; points are drawn in batches (the draw order never depends on the
+// accumulator or the mask) and voted speculatively: the first triggering point of a batch is exact,
+// later votes of the batch are rolled back and replayed after the walk.  Two kernels:
+//   k4_ppht_v3  a cluster of CTAs per frame, accumulator in distributed shared memory (default)
+//   k4_ppht_v2  one CTA per frame, accumulator in global memory (frames and ROIs v3 cannot take)
 #include "lane_common.cuh"
 
 #include <math.h>
@@ -34,11 +35,8 @@ void lane_upload_tables()
 
 namespace {
 
-constexpr int NT = 192;           // 6 warps; threads 0..179 own one angle each
-constexpr int BATCH = 32;         // points drawn per selection round
 constexpr int LIST_CAP = 8192;    // point list kept in shared memory when it fits
 constexpr unsigned SKIP = 0xFFFFFFFFu;
-constexpr int HIT_CAP = 192;
 
 __device__ __forceinline__ int rho_of(int x, int y, float cs, float sn)
 {
@@ -62,210 +60,15 @@ __device__ __forceinline__ void step_pixel(const WalkSetup &w, int k, int s, int
     if (w.xflag) { j1 = x; i1 = y >> 16; } else { j1 = x >> 16; i1 = y; }
 }
 
-__global__ void __launch_bounds__(NT) k4_ppht(uint32_t *__restrict__ points_all, const int *__restrict__ n_points,
-                                              uint32_t *__restrict__ pmask_all, int32_t *__restrict__ accum_all,
-                                              int32_t *__restrict__ lines_all, int *__restrict__ n_lines,
-                                              LaneGeom g, LaneHoughParams hp)
-{
-    __shared__ uint32_t s_list[LIST_CAP];
-    __shared__ uint32_t s_batch[BATCH];
-    __shared__ int s_P, s_trig;
-    __shared__ int s_redv[NT / 32], s_redn[NT / 32];
-    __shared__ int s_end[2][2];       // line_end[k] = (x, y)
-    __shared__ int s_nsteps[2];
-    __shared__ int s_good;
-    __shared__ uint32_t s_hits[HIT_CAP];
-    __shared__ int s_nhits;
-    __shared__ WalkSetup s_walk;
-
-    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5, f = blockIdx.x;
-    const bool active = tid < LANE_NUM_ANGLES;
-    const int WW = (g.W + 31) / 32;
-    uint32_t *pm = pmask_all + (size_t)f * g.bh * WW;     // mask word of (x, y): pm[(y-by0)*WW + (x>>5)], bit x&31
-    int32_t *lines = lines_all + (size_t)f * g.max_segments * 4;
-    const int rho_off = (g.numrho - 1) / 2;
-    int32_t *acc = accum_all + ((size_t)f * LANE_NUM_ANGLES + (active ? tid : 0)) * g.numrho + rho_off;
-    const float cs = active ? c_ppht_cos[tid] : 0.f, sn = active ? c_ppht_sin[tid] : 0.f;
-
-    int count = n_points[f];
-    uint32_t *list = points_all + (size_t)f * g.max_points;
-    if (count <= LIST_CAP) {
-        for (int i = tid; i < count; i += NT) s_list[i] = list[i];
-        list = s_list;
-    }
-    uint64_t rng = 0xFFFFFFFFFFFFFFFFull;   // used by thread 0 only
-    int nl = 0;                             // thread 0 only
-    __syncthreads();
-
-    while (count > 0) {
-        // ---- draw the next batch (sequential by construction; independent of mask/accumulator)
-        if (tid == 0) {
-            int P = count < BATCH ? count : BATCH;
-            for (int k = 0; k < P; k++) {
-                rng = (uint64_t)(uint32_t)rng * 4164903690ull + (uint32_t)(rng >> 32);
-                int idx = (int)((uint32_t)rng % (uint32_t)(count - k));
-                s_batch[k] = list[idx];
-                list[idx] = list[count - k - 1];
-            }
-            s_P = P;
-        }
-        __syncthreads();
-        const int P = s_P;
-        count -= P;
-        int k0 = 0;
-        while (k0 < P) {
-            // ---- drop points already removed by an earlier walk
-            if (tid == 0) s_trig = BATCH;
-            if (tid >= k0 && tid < P) {
-                uint32_t pt = s_batch[tid];
-                if (pt != SKIP) {
-                    int x = pt & 0xFFFF, y = pt >> 16;
-                    if (!((__ldcg(&pm[(y - g.by0) * WW + (x >> 5)]) >> (x & 31)) & 1u)) s_batch[tid] = SKIP;
-                }
-            }
-            __syncthreads();
-            // ---- vote: thread n applies the batch to its own row, in order
-            if (active) {
-                for (int k = k0; k < P; k++) {
-                    uint32_t pt = s_batch[k];
-                    if (pt == SKIP) continue;
-                    int r = rho_of(pt & 0xFFFF, pt >> 16, cs, sn);
-                    int v = atomicAdd(&acc[r], 1) + 1;
-                    if (v >= hp.threshold) atomicMin(&s_trig, k);
-                }
-            }
-            __syncthreads();
-            const int t = s_trig;
-            if (t == BATCH) break;          // whole batch consumed, nothing reached the threshold
-            // ---- roll back the speculative votes after the first trigger
-            if (active) {
-                for (int k = t + 1; k < P; k++) {
-                    uint32_t pt = s_batch[k];
-                    if (pt == SKIP) continue;
-                    atomicSub(&acc[rho_of(pt & 0xFFFF, pt >> 16, cs, sn)], 1);
-                }
-            }
-            // ---- arg-max over the 180 bins of the trigger point (first n wins ties)
-            const uint32_t tp = s_batch[t];
-            const int px = tp & 0xFFFF, py = tp >> 16;
-            int bv = -2147483647, bn = 0x7fffffff;
-            if (active) { bv = atomicAdd(&acc[rho_of(px, py, cs, sn)], 0); bn = tid; }   // read at L2, after own atomics
-            for (int o = 16; o; o >>= 1) {
-                int ov = __shfl_xor_sync(0xffffffffu, bv, o), on = __shfl_xor_sync(0xffffffffu, bn, o);
-                if (ov > bv || (ov == bv && on < bn)) { bv = ov; bn = on; }
-            }
-            if (lane == 0) { s_redv[wid] = bv; s_redn[wid] = bn; }
-            __syncthreads();
-            if (tid == 0) {
-                int mv = s_redv[0], mn = s_redn[0];
-                for (int w = 1; w < NT / 32; w++)
-                    if (s_redv[w] > mv || (s_redv[w] == mv && s_redn[w] < mn)) { mv = s_redv[w]; mn = s_redn[w]; }
-                // ---- walk setup (float32, as cv2)
-                float a = -c_ppht_sin[mn], b = c_ppht_cos[mn];
-                WalkSetup w;
-                w.x0 = px; w.y0 = py;
-                if (fabsf(a) > fabsf(b)) {
-                    w.xflag = 1;
-                    w.dx0 = a > 0 ? 1 : -1;
-                    w.dy0 = __float2int_rn(__fdiv_rn(__fmul_rn(b, 65536.0f), fabsf(a)));
-                    w.y0 = (py << 16) + 32768;
-                } else {
-                    w.xflag = 0;
-                    w.dy0 = b > 0 ? 1 : -1;
-                    w.dx0 = __float2int_rn(__fdiv_rn(__fmul_rn(a, 65536.0f), fabsf(b)));
-                    w.x0 = (px << 16) + 32768;
-                }
-                s_walk = w;
-            }
-            __syncthreads();
-            const WalkSetup w = s_walk;
-            // ---- pass 1: warps 0 and 1 walk the two directions, 32 steps per ballot
-            if (wid < 2) {
-                const int k = wid;
-                int last = 0;
-                bool done = false;
-                for (int base = 0; !done; base += 32) {
-                    int j1, i1;
-                    step_pixel(w, k, base + lane, j1, i1);
-                    bool ib = j1 >= 0 && j1 < g.W && i1 >= 0 && i1 < g.H;
-                    bool hit = false;
-                    if (ib && j1 >= g.bx0 && j1 < g.bx1 && i1 >= g.by0 && i1 < g.by1)
-                        hit = ((__ldcg(&pm[(i1 - g.by0) * WW + (j1 >> 5)]) >> (j1 & 31)) & 1u) != 0;
-                    unsigned IB = __ballot_sync(0xffffffffu, ib), Hh = __ballot_sync(0xffffffffu, hit);
-                    int limit = (~IB) ? __ffs(~IB) - 1 : 32;       // valid steps of this chunk: [0, limit)
-                    if (limit < 32) Hh &= (1u << limit) - 1u;
-                    while (Hh) {
-                        int p = base + __ffs(Hh) - 1;
-                        if (p - last > hp.max_gap + 1) { done = true; break; }
-                        last = p;
-                        Hh &= Hh - 1;
-                    }
-                    if (!done) {
-                        if (limit < 32) done = true;
-                        else if (base + 31 - last > hp.max_gap) done = true;
-                    }
-                }
-                if (lane == 0) {
-                    int j1, i1;
-                    step_pixel(w, k, last, j1, i1);
-                    s_end[k][0] = j1; s_end[k][1] = i1;
-                    s_nsteps[k] = last + 1;
-                }
-            }
-            __syncthreads();
-            if (tid == 0) {
-                int good = abs(s_end[1][0] - s_end[0][0]) >= hp.min_len || abs(s_end[1][1] - s_end[0][1]) >= hp.min_len;
-                s_good = good;
-                if (good) {
-                    if (nl < g.max_segments) {
-                        lines[4 * nl + 0] = s_end[0][0]; lines[4 * nl + 1] = s_end[0][1];
-                        lines[4 * nl + 2] = s_end[1][0]; lines[4 * nl + 3] = s_end[1][1];
-                    }
-                    nl++;
-                }
-            }
-            // ---- pass 2: clear the pixels on the segment; for a good line every one of them is un-voted
-            for (int k = 0; k < 2; k++) {
-                const int ns = s_nsteps[k];
-                for (int base = 0; base < ns; base += NT) {
-                    if (tid == 0) s_nhits = 0;
-                    __syncthreads();
-                    int s = base + tid;
-                    if (s < ns) {
-                        int j1, i1;
-                        step_pixel(w, k, s, j1, i1);
-                        if (j1 >= g.bx0 && j1 < g.bx1 && i1 >= g.by0 && i1 < g.by1) {
-                            const uint32_t bit = 1u << (j1 & 31);
-                            if (atomicAnd(&pm[(i1 - g.by0) * WW + (j1 >> 5)], ~bit) & bit)
-                                s_hits[atomicAdd(&s_nhits, 1)] = ((uint32_t)i1 << 16) | (uint32_t)j1;
-                        }
-                    }
-                    __syncthreads();
-                    if (s_good && active) {
-                        const int nh = s_nhits;
-                        for (int h = 0; h < nh; h++) {
-                            uint32_t pt = s_hits[h];
-                            atomicSub(&acc[rho_of(pt & 0xFFFF, pt >> 16, cs, sn)], 1);
-                        }
-                    }
-                    __syncthreads();
-                }
-            }
-            k0 = t + 1;
-        }
-    }
-    if (tid == 0) n_lines[f] = nl;
-}
-
-
 // ---------------------------------------------------------------------------------------------
-// v2: same exact algorithm, reorganised for latency.
+// v2: one CTA per frame; voter thread n < 180 owns angle n and its accumulator row.
 //   * a producer warp draws the points (RNG + swap-remove on the shared-memory list) one batch
 //     ahead of the six voter warps (double-buffered batches, one CTA barrier per batch);
 //   * votes are issued eight deep before any result is inspected, so the L2 round trips overlap;
 //   * accumulator cells are biased 16-bit counters packed two per word, and every angle only owns
 //     the rho window the ROI can reach (host-computed from the mask's row spans with the same
-//     float32 arithmetic), so a 1080p frame needs ~0.45 MB instead of 4.3 MB and stays in L2.
+//     float32 arithmetic), so a 1080p frame needs ~0.45 MB instead of the 4.3 MB of int32 cells over
+//     the full rho range, and stays in L2.
 constexpr int NV = 192;            // voter threads (180 active)
 constexpr int NT2 = NV + 32;       // + producer warp
 constexpr int BATCH2 = 64;
@@ -1152,15 +955,13 @@ int lane_ppht_plan_v3(const int2 *win, int cells_total, int2 *win3, int *cells_m
     int width[LANE_NUM_ANGLES];
     for (int n = 0; n < LANE_NUM_ANGLES; n++)
         width[n] = (n + 1 < LANE_NUM_ANGLES ? win[n + 1].y : cells_total) - win[n].y;
-    const int forced = getenv("LANE_PPHT_G") ? atoi(getenv("LANE_PPHT_G")) : 0;      // tuning knob
     // A smaller cluster means more frames in flight and fewer exchange partners, so a shorter shared point list is
     // accepted when that is all a cluster size lacks (4K: 8 CTAs with 2560 list entries instead of 16 CTAs -- 37 frames in
     // flight instead of 18, 1.76 ms against 3.6 ms per 128 frames; longer lists continue in the global extension).
     static const int caps[3] = {LIST_CAP3, 2560, 2048};
     for (int pass = 0; pass < 2; pass++)
     for (int G = 1; G <= 16; G *= 2) {
-        if (forced && G != forced) continue;
-        const size_t budget = pass == 0 && !forced ? 112 * 1024 : 226 * 1024;   // first try to fit two CTAs per SM
+        const size_t budget = pass == 0 ? 112 * 1024 : 226 * 1024;   // first try to fit two CTAs per SM
         int off[16] = {0};
         for (int n = 0; n < LANE_NUM_ANGLES; n++) {
             win3[n] = make_int2(win[n].x, off[n % G]);
@@ -1207,12 +1008,4 @@ int lane_ppht_windows(const uint8_t *mask, int H, int W, int2 *win)
         cells += (rmax[n] - rmin[n] + 1 + 1) & ~1;      // rows start on word boundaries
     }
     return cells;
-}
-
-void launch_ppht(uint32_t *points, const int *n_points, uint32_t *pmask, int32_t *accum, int32_t *lines,
-                 int *n_lines, LaneGeom g, LaneHoughParams hp, int n, cudaStream_t st, int *launches)
-{
-    cudaMemsetAsync(accum, 0, sizeof(int32_t) * (size_t)n * LANE_NUM_ANGLES * g.numrho, st);
-    k4_ppht<<<n, NT, 0, st>>>(points, n_points, pmask, accum, lines, n_lines, g, hp);
-    *launches += 1;
 }

@@ -98,7 +98,7 @@ __global__ void __launch_bounds__(K6T) k6_frame_stats(const uint8_t *__restrict_
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// Strip form (W % 16 == 0, 16-byte aligned frames): the same sums with K1's data path.  A warp owns a 512-px column
+// Strip form (W % 16 == 0, 16-byte aligned frames): the same sums with K1F's data path.  A warp owns a 512-px column
 // strip (16 px per lane, three 16-byte loads per lane per row, lanes 0 / 31 are the one-pixel halo) and rolls down a
 // band of rows in registers.  gray = 2 IDP2A per pixel as packed u16x2 pairs; the Laplacian is formed on the pairs as
 // L' = up + down + left + right + 1020 - 4*centre (0..2040, carry-free), two rows of state alternating between two
@@ -329,8 +329,7 @@ extern "C" int lane_frame_stats(const uint8_t *frames, int on_device, int n, int
     if (e) { if (owned) cudaFree(scratch); return sfail(LANE_ERR_CUDA, "upload", e); }
     dim3 grid((width + TC - 1) / TC, (height + TR - 1) / TR, n);
     if (grid.y > 65535) { if (owned) cudaFree(scratch); return sfail(LANE_ERR_UNSUPPORTED, "frame too tall", cudaSuccess); }
-    static const bool force_tile = getenv("LANE_K6_TILE") != nullptr;
-    const bool strip = !force_tile && width % 16 == 0 && ((uintptr_t)d_frames % 16) == 0 && height >= 2 &&
+    const bool strip = width % 16 == 0 && ((uintptr_t)d_frames % 16) == 0 && height >= 2 &&
                        (size_t)height * width * 3 < ((size_t)1 << 32);
     if (strip) {
         int sms = 0;

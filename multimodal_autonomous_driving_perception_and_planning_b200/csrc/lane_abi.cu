@@ -42,7 +42,7 @@ struct lane_ctx {
     // that cross from the edge half to the back half are kept per result slot (see `two`).
     cudaStream_t st2 = nullptr;
     cudaEvent_t edge_done[2] = {};
-    bool overlap_ok = true, overlap_now = false;    // LANE_B200_OVERLAP=0: one stream (A/B)
+    bool overlap_now = false;                       // the batch being enqueued runs its back half on st2
     cudaEvent_t copy_ev[LANE_COPY_EVENTS] = {}, start_ev = nullptr;
     std::string err;
 
@@ -54,7 +54,6 @@ struct lane_ctx {
     uint32_t *d_kbits = nullptr;      // [B][H][WW] NMS survivors of the fused edge kernel
     uint8_t *d_vplane = nullptr;      // [B][H][W]  their magnitudes (sparse: only survivors' bytes are ever written / read)
     int *d_pre = nullptr;             // [B] magnitude floor per frame | [B] floor of the redo pass | [B] redo list | count
-    int force_unfused = 0;            // LANE_B200_K1=unfused pins the round-1 K1 + K2a kernels (A/B checks)
     uint32_t *d_roi_bits = nullptr;   // [H][WW] bit-plane of the ROI mask
     uint32_t *d_pmask_bits = nullptr; // [B][bh][WW] ROI-masked edges (the HoughLinesP mask)
     uint32_t *d_edge_bits = nullptr;  // [B][H][WW] Canny map
@@ -64,7 +63,6 @@ struct lane_ctx {
     uint8_t *h_roi = nullptr;
     bool fallback_ready = false, last_cluster = false;
     int last_paths = 0;               // LANE_PATH_* of the chunk that ran last
-    int force_generic_k2 = 0;         // LANE_B200_K2=generic forces the byte-map kernels (A/B checks)
     uint8_t *d_gray_dbg = nullptr;
     uint32_t *d_hist = nullptr, *d_points = nullptr, *d_points_dbg = nullptr;
     uint8_t *d_lut = nullptr;         // low[511] | high[511]
@@ -72,13 +70,12 @@ struct lane_ctx {
     int *d_seedsA = nullptr, *d_seedsB = nullptr, *d_seed_count = nullptr;
     int seed_cap = 0;
     int *d_n_edges = nullptr, *d_n_points = nullptr, *d_rounds = nullptr, *d_n_lines = nullptr;
-    int32_t *d_accum = nullptr, *d_lines = nullptr;   // d_accum: v1 PPHT only (LANE_B200_K4=v1), lazy
+    int32_t *d_lines = nullptr;
     uint32_t *d_accum16 = nullptr;    // [B][cells_per_frame] biased 16-bit cells, two per word
     int2 *d_win = nullptr;            // [180] (rmin, first cell) per angle
     int cells_per_frame = 0;
-    int ppht_v1 = 0, ppht_v2 = 0;     // LANE_B200_K4=v1|v2 pins an older PPHT kernel (A/B checks)
-    int k4_lpt = 1;                   // frames with the most points first (LANE_B200_K4_ORDER=0: launch order, A/B)
-    int *d_order = nullptr;
+    int ppht_v2 = 0;                  // LANE_B200_K4=v2 pins the global-memory PPHT kernel (tests)
+    int *d_order = nullptr;           // [B] frames with the most points first (v3 launch order)
     int2 *d_win3 = nullptr;           // v3 layout: (rmin, first cell inside the owning CTA)
     uint32_t *d_pmask_work = nullptr; // [B][G3][bh][WW] private mask copies of the v3 cluster CTAs
     uint32_t *d_list_over = nullptr;  // [B][G3][over_cap] private extensions of the v3 point list (ROIs with many pixels)
@@ -99,7 +96,6 @@ struct lane_ctx {
     int2 *d_peaks = nullptr;
     int *d_n_peaks = nullptr;
     int *d_task_counter = nullptr;
-    int force_tile = 0;               // LANE_B200_K1=tile forces the generic K1 kernel (A/B checks)
     int peaks_cap = 0;
 
     // Up to two batches may be in flight on the context's stream (enqueue, enqueue, collect, enqueue, collect ...): the
@@ -158,7 +154,7 @@ void free_all(lane_ctx *c)
     void *ptrs[] = {c->d_frames, c->d_src, c->d_blur, c->d_kbits, c->d_vplane, c->d_pre, c->d_cls, c->d_cls_dbg, c->d_roi, c->d_pmask, c->d_gray_dbg, c->d_hist,
                     c->d_roi_bits, c->d_pmask_bits, c->d_edge_bits, c->d_dbg_c, c->d_dbg_s, c->d_accum16, c->d_win, c->d_win3, c->d_pmask_work, c->d_list_over,
                     c->d_points, c->d_points_dbg, c->d_lut, c->d_thr, c->d_seedsA, c->d_seedsB, c->d_seed_count,
-                    c->d_n_edges, c->d_n_points, c->d_rounds, c->d_n_lines, c->d_accum, c->d_lines, c->fit.raw, c->fit.big,
+                    c->d_n_edges, c->d_n_points, c->d_rounds, c->d_n_lines, c->d_lines, c->fit.raw, c->fit.big,
                     c->fit.side_n, c->fit.side_flags, c->d_stream_id, c->d_prev_fit, c->d_prev_valid,
                     c->slots[0].d_records, c->slots[1].d_records, c->d_std_accum, c->d_hb_accum, c->d_hb_sorted, c->d_hb_tmp, c->d_hb_count, c->d_peaks, c->d_n_peaks, c->d_task_counter, c->d_order};
     for (void *p : ptrs)
@@ -293,7 +289,7 @@ int run_stages(lane_ctx *c, const uint8_t *frames_dev, int off, int m, const int
     // cluster kernel; the blurred plane is only written for the verification taps.
     bool fused = false;
     c->last_cluster = false;
-    if (!c->force_unfused && !c->force_tile && !c->force_generic_k2 && c->blur && lane_fused_edge_supported(H, W, fr)) {
+    if (c->blur && lane_fused_edge_supported(H, W, fr)) {
         if (!c->d_kbits) {
             CU(dalloc(&c->d_kbits, (size_t)c->max_batch * planes));
             CU(dalloc(&c->d_vplane, (size_t)c->max_batch * P));
@@ -334,10 +330,9 @@ int run_stages(lane_ctx *c, const uint8_t *frames_dev, int off, int m, const int
         rc = ensure_blur(c); if (rc) return rc;
         uint8_t *blur = c->d_blur + o * P;
         if (timed) { rc = mark(c, LANE_STAGE_BLUR_HIST); if (rc) return rc; }
-        launch_blur_hist(fr, blur, hist, m, H, W, c->st, &L[LANE_STAGE_BLUR_HIST], c->d_task_counter, c->force_tile,
-                         c->blur);
+        launch_blur_hist(fr, blur, hist, m, H, W, c->st, &L[LANE_STAGE_BLUR_HIST], c->blur);
         if (timed) { rc = mark(c, LANE_STAGE_CANNY); if (rc) return rc; }
-        c->last_cluster = !c->force_generic_k2 &&
+        c->last_cluster =
             launch_canny_cluster(blur, hist, c->d_lut, c->d_lut + 511, c->d_roi_bits, thr, n_edges, rounds, points, n_points,
                                  pmask_bits, edge_bits, cb, sb, c->d_task_counter, g, m, c->st, &L[LANE_STAGE_CANNY]);
     }
@@ -372,21 +367,15 @@ int run_stages(lane_ctx *c, const uint8_t *frames_dev, int off, int m, const int
         CU(cudaEventRecord(c->edge_done[c->cur], c->st));
         CU(cudaStreamWaitEvent(hs, c->edge_done[c->cur], 0));
     }
-    if (c->ppht_v1) {
-        if (!c->d_accum) CU(dalloc(&c->d_accum, (size_t)c->max_batch * LANE_NUM_ANGLES * g.numrho));
-        launch_ppht(points, n_points, pmask_bits, c->d_accum + o * LANE_NUM_ANGLES * g.numrho, lines, n_lines, g, c->hp, m,
-                    hs, &L[LANE_STAGE_PPHT]);
-    } else {
-        // v3 (cells in distributed shared memory) takes every frame it can; v2 (global 16-bit cells) then sweeps
-        // up the frames v3 flagged (point list larger than its shared-memory list), or runs alone if v3 cannot launch.
-        bool v3 = !c->ppht_v2 && c->G3 > 0 &&
-                  launch_ppht_v3(points, n_points, pmask_bits, c->d_pmask_work + o * c->G3 * std::max(g.bh, 1) * WW,
-                                 c->d_list_over ? c->d_list_over + o * c->G3 * (size_t)c->over_cap3 : nullptr, c->d_win3, c->cells_max3, c->list_cap3, c->over_cap3, c->G3, lines, n_lines, g, c->hp, m, hs, &L[LANE_STAGE_PPHT],
-                                 c->k4_lpt ? c->d_order + o : nullptr);
-        launch_ppht_v2(points, n_points, pmask_bits, c->d_accum16 + o * (c->cells_per_frame / 2), c->d_win,
-                       c->cells_per_frame, lines, n_lines, g, c->hp, m, hs, &L[LANE_STAGE_PPHT], v3 ? 1 : 0);
-        if (v3) c->last_paths |= LANE_PATH_PPHT_DSMEM;
-    }
+    // v3 (cells in distributed shared memory) takes every frame it can; v2 (global 16-bit cells) then sweeps
+    // up the frames v3 flagged (point list larger than its shared-memory list), or runs alone if v3 cannot launch.
+    bool v3 = !c->ppht_v2 && c->G3 > 0 &&
+              launch_ppht_v3(points, n_points, pmask_bits, c->d_pmask_work + o * c->G3 * std::max(g.bh, 1) * WW,
+                             c->d_list_over ? c->d_list_over + o * c->G3 * (size_t)c->over_cap3 : nullptr, c->d_win3, c->cells_max3, c->list_cap3, c->over_cap3, c->G3, lines, n_lines, g, c->hp, m, hs, &L[LANE_STAGE_PPHT],
+                             c->d_order + o);
+    launch_ppht_v2(points, n_points, pmask_bits, c->d_accum16 + o * (c->cells_per_frame / 2), c->d_win,
+                   c->cells_per_frame, lines, n_lines, g, c->hp, m, hs, &L[LANE_STAGE_PPHT], v3 ? 1 : 0);
+    if (v3) c->last_paths |= LANE_PATH_PPHT_DSMEM;
 
     rc = stage_check(c, "ppht"); if (rc) return rc;
     if (timed) { rc = mark(c, LANE_STAGE_FIT); if (rc) return rc; }
@@ -419,7 +408,7 @@ int enqueue(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int
     // back half on its own stream: device-resident batches outside profiling / debug mode (stage events and taps assume
     // one stream).  Everything only the back half touches (stream ids, EMA state, records) is ordered on that stream.
     const bool was_overlap = c->overlap_now;
-    c->overlap_now = c->overlap_ok && on_device && !c->profiling && !c->debug && c->st2 != nullptr;
+    c->overlap_now = on_device && !c->profiling && !c->debug;
     if (was_overlap != c->overlap_now && c->q_count) {       // mode change with a batch in flight: order the two streams once
         CU(cudaEventRecord(c->edge_done[c->cur ^ 1], was_overlap ? c->st2 : c->st));
         CU(cudaStreamWaitEvent(was_overlap ? c->st : c->st2, c->edge_done[c->cur ^ 1], 0));
@@ -461,9 +450,8 @@ int enqueue(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int
         cudaPointerAttributes pa{};
         bool pageable = cudaPointerGetAttributes(&pa, frames) != cudaSuccess || pa.type == cudaMemoryTypeUnregistered;
         cudaGetLastError();
-        static const bool no_stage = getenv("LANE_B200_NO_STAGING") != nullptr;       // A/B knob
         // small transfers (a single frame) are quicker through the driver's own path than through worker wake-ups
-        if (no_stage || bytes * (size_t)n < ((size_t)24 << 20)) pageable = false;
+        if (bytes * (size_t)n < ((size_t)24 << 20)) pageable = false;
         if (pageable && !c->pool) {
             const unsigned hc = std::thread::hardware_concurrency();
             c->pool = new CopyPool((int)std::max(1u, std::min(8u, hc ? hc / 2 : 4u)));
@@ -613,17 +601,11 @@ int lane_ctx_create(int device, int height, int width, int max_batch, int max_se
     } while (0)
     CUB(cudaStreamCreateWithFlags(&ctx->st, cudaStreamNonBlocking));
     {
-        int lo = 0, hi = 0;                          // the back half first: its clusters keep their slots, the edge kernels fill in
+        // the back half first: its clusters keep their slots, the edge kernels fill in (DESIGN.md §4, "Two streams")
+        int lo = 0, hi = 0;
         cudaDeviceGetStreamPriorityRange(&lo, &hi);
-        const char *pr = getenv("LANE_B200_BACK_PRIORITY");          // A/B knob: "low" = the edge kernels first
-        CUB(cudaStreamCreateWithPriority(&ctx->st2, cudaStreamNonBlocking, pr && !strcmp(pr, "low") ? lo : hi));
-        if (pr && !strcmp(pr, "low")) {                              // then the edge stream gets the high priority
-            cudaStreamDestroy(ctx->st);
-            CUB(cudaStreamCreateWithPriority(&ctx->st, cudaStreamNonBlocking, hi));
-        }
+        CUB(cudaStreamCreateWithPriority(&ctx->st2, cudaStreamNonBlocking, hi));
         for (auto &e : ctx->edge_done) CUB(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        const char *ov = getenv("LANE_B200_OVERLAP");
-        ctx->overlap_ok = !(ov && !strcmp(ov, "0"));
     }
     for (auto &sl : ctx->slots) {
         for (auto &e : sl.ev) CUB(cudaEventCreate(&e));
@@ -658,16 +640,8 @@ int lane_ctx_create(int device, int height, int width, int max_batch, int max_se
     }
     CUB(dalloc(&ctx->d_task_counter, 4));
     {
-        const char *e = getenv("LANE_B200_K1");
-        ctx->force_tile = e && !strcmp(e, "tile");
-        ctx->force_unfused = e && (!strcmp(e, "unfused") || !strcmp(e, "tma"));
-        e = getenv("LANE_B200_K4");
-        ctx->ppht_v1 = e && !strcmp(e, "v1");
+        const char *e = getenv("LANE_B200_K4");
         ctx->ppht_v2 = e && !strcmp(e, "v2");
-        const char *ord = getenv("LANE_B200_K4_ORDER");
-        ctx->k4_lpt = !(ord && !strcmp(ord, "0"));
-        e = getenv("LANE_B200_K2");
-        ctx->force_generic_k2 = e && !strcmp(e, "generic");
     }
     for (auto &sl : ctx->slots) CUB(cudaMallocHost((void **)&sl.h_records, sizeof(lane_record) * B));
     lane_upload_tables();
@@ -735,9 +709,7 @@ int lane_set_roi_mask(lane_ctx *c, const uint8_t *mask)
             // cells leave room for: 74 at 1080p (G = 4, two CTAs per SM) but only 18 at 4K (G = 16), where the
             // global-memory kernel with every frame of the batch in flight is faster (measured on B200, 128 x 4K:
             // v3 3.55 ms, v2 2.47 ms).  Take v3 only when it can keep at least 32 frames going.
-            const char *e = getenv("LANE_B200_K4");
-            const bool forced = e && !strcmp(e, "v3");
-            if (c->G3 > 0 && !forced) {
+            if (c->G3 > 0) {
                 const size_t per_cta = (size_t)c->cells_max3 * 2 + sizeof(uint32_t) * (size_t)c->list_cap3 + 4700;
                 const int ctas = per_cta <= 112 * 1024 ? 2 : 1;
                 if (lane_sm_count() * ctas / c->G3 < 32) c->G3 = 0;

@@ -59,7 +59,7 @@ void lane_set_global_error(const char *msg);
 
 // ---- K1 ---------------------------------------------------------------------------------
 void launch_blur_hist(const uint8_t *frames, uint8_t *blur, uint32_t *hist, int n, int H, int W,
-                      cudaStream_t st, int *launches, int *task_counter, int force_tile, int gaussian_blur);
+                      cudaStream_t st, int *launches, int gaussian_blur);
 // fused edge kernel (k1_fused.cu): probe + gray + blur + histogram + Sobel + NMS -> K bit-plane, V byte plane
 bool lane_fused_edge_supported(int H, int W, const void *frames);
 bool launch_fused_edge(const uint8_t *frames, const uint8_t *lut_low, const uint8_t *lut_high, uint32_t *hist, int4 *thr,
@@ -117,11 +117,8 @@ void lane_upload_tables();       // trig tables -> __constant__ (both Hough vari
 void lane_upload_tables_std();
 
 // ---- K4 ---------------------------------------------------------------------------------
-// accum: int32 [n][180][numrho] zeroed by the launcher; lines: int32 [n][max_segments][4]
+// lines: int32 [n][max_segments][4]
 // pmask_bits: [n][bh][WW] bit-plane of the ROI-masked edges (bit x&31 of word x>>5), cleared as lines are found
-void launch_ppht(uint32_t *points, const int *n_points, uint32_t *pmask_bits, int32_t *accum, int32_t *lines,
-                 int *n_lines, LaneGeom g, LaneHoughParams hp, int n, cudaStream_t st, int *launches);
-
 // v2: 16-bit biased cells inside per-angle rho windows (win[n] = (rmin, first cell)), producer warp, deep votes
 void launch_ppht_v2(uint32_t *points, const int *n_points, uint32_t *pmask_bits, uint32_t *accum16, const int2 *win,
                     int cells_per_frame, int32_t *lines, int *n_lines, LaneGeom g, LaneHoughParams hp, int n,

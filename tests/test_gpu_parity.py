@@ -84,7 +84,8 @@ def test_stage_taps_generator_640x480():
     _run_stage_checks(gen_frames(640, 480, 6), hough=True)
 
 
-@pytest.mark.parametrize("shape", [(7, 9), (5, 5), (3, 3), (33, 65), (64, 64), (481, 643), (240, 320)])
+# (8, 64) and (12, 1936): widths the fused kernel takes but fewer than 16 rows -> k1_tile + k2a_sobel_nms + the cluster
+@pytest.mark.parametrize("shape", [(7, 9), (5, 5), (3, 3), (33, 65), (64, 64), (481, 643), (240, 320), (8, 64), (12, 1936)])
 def test_stage_taps_noise(shape):
     rng = np.random.default_rng(shape[0] * 1000 + shape[1])
     frames = [rng.integers(0, 256, shape + (3,), dtype=np.uint8) for _ in range(2)]
@@ -92,8 +93,8 @@ def test_stage_taps_noise(shape):
 
 
 @pytest.mark.parametrize("shape", [(16, 16), (48, 64), (135, 480), (271, 976), (137, 1936), (1080, 1920)])
-def test_k1_strip_kernel_noise(shape):
-    """K1 fast path (W % 16 == 0): blur plane, histogram and thresholds on uniform noise, every
+def test_fused_kernel_blur_hist_thresholds_noise(shape):
+    """Fused edge kernel (W % 16 == 0, H >= 16): blur plane, histogram and thresholds on uniform noise, every
     strip/band/edge-lane layout (1, 2, 3 and 5 strips; partial last strip; odd band heights)."""
     rng = np.random.default_rng(shape[0] + shape[1])
     frames = np.stack([rng.integers(0, 256, shape + (3,), dtype=np.uint8) for _ in range(3)])

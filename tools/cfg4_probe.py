@@ -1,4 +1,5 @@
-"""GPU-box probe: config 4 (128 x 3840x2160) stage times, for A/B of PPHT kernel choices (LANE_B200_K4, LANE_PPHT_G)."""
+"""GPU-box probe: config 4 (128 x 3840x2160) stage times, for A/B of PPHT kernel choices (LANE_B200_K4=v2, or
+another build of the library through LANE_B200_LIB)."""
 import json, os, sys, time
 sys.path.insert(0, '.')
 import numpy as np, torch
@@ -18,5 +19,5 @@ for _ in range(3):
     ms, _ = ctx.stage_ms()
     for k, v in ms.items():
         tot[k] = tot.get(k, 0) + v / 3
-print(json.dumps({"env": {k: os.environ.get(k) for k in ("LANE_B200_K4", "LANE_PPHT_G", "LANE_B200_LIB")}, "paths": ctx.last_paths(),
+print(json.dumps({"env": {k: os.environ.get(k) for k in ("LANE_B200_K4", "LANE_B200_LIB")}, "paths": ctx.last_paths(),
                   "stage_ms": {k: round(v, 4) for k, v in tot.items()}, "segments_mean": float(recs["n_segments"].mean())}))

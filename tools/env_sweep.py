@@ -1,5 +1,6 @@
-"""Run bench.py (device-resident leg only) once per value of an environment knob and print the stage split.
-usage: python tools/env_sweep.py VAR v1 v2 ... [-- extra bench args]"""
+"""Run bench.py (device-resident leg only) once per value of an environment variable and print the stage split.
+usage: python tools/env_sweep.py VAR v1 v2 ... [-- extra bench args]
+("-" leaves VAR unset), e.g. this build against another one: python tools/env_sweep.py LANE_B200_LIB - OTHER/liblane_b200.so"""
 import json, os, subprocess, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 args = sys.argv[1:]
