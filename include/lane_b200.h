@@ -122,7 +122,8 @@ LANE_API int lane_detect_batch_nv12(lane_ctx *ctx, const uint8_t *frames_nv12, i
                            const int32_t *stream_id, int n_streams, double *prev_fit, uint8_t *prev_valid,
                            lane_record *out);
 
-/* Frame layouts a detect / ingest call accepts (what a decoder or VideoDataLoader hands out). */
+/* Frame layouts a detect / ingest call accepts (what a decoder or VideoDataLoader hands out); lane_bgr_to_yuv420_batch
+ * produces the two YUV ones (what an encoder takes). */
 #define LANE_INPUT_BGR  0           /* uint8 [n][src_h][src_w][3] */
 #define LANE_INPUT_NV12 1           /* uint8 [n][src_h*3/2][src_w], Y then interleaved UV (hardware decoders) */
 #define LANE_INPUT_I420 2           /* uint8 [n][src_h*3/2][src_w], Y, then U plane, then V plane (software decoders) */
@@ -251,6 +252,18 @@ LANE_API int lane_nv12_to_bgr_batch(const uint8_t *src, int n, int height, int w
  * cuda_stream as for lane_resize_batch.  Needs no context; errors via lane_last_error(NULL). */
 LANE_API int lane_yuv420_to_bgr_batch(const uint8_t *src, int format, int n, int src_h, int src_w, uint8_t *dst,
                                       int dst_h, int dst_w, int on_device, int device, void *cuda_stream);
+
+/* ---- frame egress (SURVEY.md 8f rank 3: the step after the overlays when annotated video is written) ---------------
+ * cv2.cvtColor(f, COLOR_BGR2YUV_I420) per frame (NV12: the same samples, U and V interleaved), for annotated frames
+ * that are in device memory -- what LaneDetector.draw_lanes (lane_detector.py:220-251) and the offset indicator leave in
+ * HBM, ready for an encoder (libx264 -pix_fmt yuv420p, a hardware encoder's NV12 surface) at 1.5 B/px.
+ * src_dev: device uint8 [n][height][width][3]; dst: uint8 [n][height*3/2][width],
+ * device memory (dst_on_device = 1: enqueued on cuda_stream, returns without synchronising) or host memory
+ * (dst_on_device = 0: converted chunk by chunk, each chunk copied out while the next is converted; blocking).
+ * format: LANE_INPUT_I420 or LANE_INPUT_NV12; height, width even; n = 0 does nothing.  Host sources are not taken
+ * (cv2.cvtColor converts those where they are).  Needs no context; errors via lane_last_error(NULL). */
+LANE_API int lane_bgr_to_yuv420_batch(const uint8_t *src_dev, int format, int n, int height, int width, uint8_t *dst,
+                                      int dst_on_device, int device, void *cuda_stream);
 
 /* ---- scene statistics (SURVEY.md 8f rank 2, second half) -----------------------------------------------------
  * Integer sums behind SceneClassifier's image cues (/root/reference/src/tagging/scene_classifier.py):

@@ -24,6 +24,7 @@ FLAG_SEGMENTS_TRUNCATED, FLAG_POINTS_TRUNCATED = 1, 2
 PATH_FUSED_EDGE, PATH_CLUSTER_CANNY, PATH_PPHT_DSMEM = 1, 2, 4
 PATH_ALL_FAST = 7
 INPUT_BGR, INPUT_NV12, INPUT_I420 = 0, 1, 2          # LANE_INPUT_*: frame layouts the detect / ingest calls accept
+#                                                     (and NV12 / I420: what lane_bgr_to_yuv420_batch writes)
 
 
 class LaneSide(C.Structure):
@@ -90,6 +91,8 @@ _PROTOS = {
     "lane_nv12_to_bgr_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "lane_yuv420_to_bgr_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int,
                                            C.c_int, C.c_int, C.c_void_p]),
+    "lane_bgr_to_yuv420_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int,
+                                           C.c_void_p]),
     "lane_detect_enqueue": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "lane_detect_collect": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "lane_ctx_stream": (C.c_void_p, [C.c_void_p]),

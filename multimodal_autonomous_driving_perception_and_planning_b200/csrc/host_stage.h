@@ -1,4 +1,4 @@
-// Host-side staging of ordinary (pageable) memory for H2D copies.
+// Host-side staging of ordinary (pageable) memory for H2D and D2H copies.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -66,7 +66,7 @@ struct CopyPool {
 };
 
 
-// Context-free entry points (resize, frame statistics) share one staging ring per device.  h2d() is blocking on the
+// Context-free entry points (resize, frame statistics, egress) share one staging ring per device.  h2d() is blocking on the
 // host side only as far as the memcpy into pinned memory goes; the DMA itself is asynchronous on `st`.
 struct HostStager {
     static constexpr int SLOTS = 3;
@@ -105,6 +105,38 @@ struct HostStager {
             if ((e = cudaMemcpyAsync(dst + done, stage[slot], nb, cudaMemcpyHostToDevice, st))) return e;
             if ((e = cudaEventRecord(ev[slot], st))) return e;
             used[slot] = true;
+        }
+        return cudaSuccess;
+    }
+    // The reverse direction, for a pageable destination (the caller has checked pageable()): the DMA on `st` fills a
+    // slot, and the pool copies the slot into `dst` once the slot's event has fired, while the DMA of the next pieces
+    // is under way.  Pieces are a quarter slot so that even one 32 MB chunk overlaps the two copies.  Blocking: returns
+    // when all `bytes` are in `dst`.
+    cudaError_t d2h(uint8_t *dst, const uint8_t *src, size_t bytes, cudaStream_t st)
+    {
+        cudaError_t e;
+        if (!ok) return (e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, st)) ? e : cudaStreamSynchronize(st);
+        constexpr size_t D2H_PIECE = PIECE / 4;
+        std::lock_guard<std::mutex> lk(mu);
+        const size_t pieces = (bytes + D2H_PIECE - 1) / D2H_PIECE;
+        auto issue = [&](size_t p) {
+            const int slot = (int)(p % SLOTS);
+            cudaError_t r;
+            if (used[slot] && (r = cudaEventSynchronize(ev[slot]))) return r;      // an h2d() may still read it
+            const size_t off = p * D2H_PIECE;
+            if ((r = cudaMemcpyAsync(stage[slot], src + off, std::min(D2H_PIECE, bytes - off), cudaMemcpyDeviceToHost, st)))
+                return r;
+            used[slot] = true;
+            return cudaEventRecord(ev[slot], st);
+        };
+        for (size_t p = 0; p < std::min(pieces, (size_t)SLOTS); p++)
+            if ((e = issue(p))) return e;
+        for (size_t p = 0; p < pieces; p++) {
+            const int slot = (int)(p % SLOTS);
+            if ((e = cudaEventSynchronize(ev[slot]))) return e;
+            const size_t off = p * D2H_PIECE;
+            pool.run(dst + off, stage[slot], std::min(D2H_PIECE, bytes - off));
+            if (p + SLOTS < pieces && (e = issue(p + SLOTS))) return e;
         }
         return cudaSuccess;
     }

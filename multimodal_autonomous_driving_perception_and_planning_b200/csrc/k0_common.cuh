@@ -1,5 +1,5 @@
-// Shared pieces of the frame-ingest kernels (K0): the YUV 4:2:0 -> BGR arithmetic of k0_nv12.cu / k0_ingest.cu and
-// the INTER_LINEAR tap tables and vertical step of k0_resize.cu.
+// Shared pieces of the frame-ingest kernels (K0): the YUV 4:2:0 -> BGR arithmetic of k0_nv12.cu / k0_ingest.cu, its
+// inverse for the egress kernel (k8_egress.cu) and the INTER_LINEAR tap tables and vertical step of k0_resize.cu.
 #pragma once
 #include "lane_common.cuh"
 
@@ -47,6 +47,18 @@ __device__ __forceinline__ UV chroma(const uint8_t *s, int H, int W, int by, int
         return uv_terms(__ldg(s + q), __ldg(s + q + P / 4));
     }
 }
+
+// ---- BGR -> YUV 4:2:0, bit-exact with cv2.cvtColor(f, COLOR_BGR2YUV_I420) (k8_egress.cu) ---------------------------
+// The same BT.601 limited range in 20-bit fixed point with a round-half constant; Y from every pixel, U and V from the
+// top-left pixel of each 2x2 block (no averaging).  All sums are non-negative, so >> is a floor.
+constexpr int EYR = 269484, EYG = 528482, EYB = 102760;
+constexpr int EUR = -155188, EUG = -305135, EUB = 460324;
+constexpr int EVR = 460324, EVG = -385875, EVB = -74448;
+constexpr int EY0 = (16 << SHIFT) + (1 << (SHIFT - 1)), EC0 = (128 << SHIFT) + (1 << (SHIFT - 1));
+
+__device__ __forceinline__ uint32_t bgr_y(int b, int g, int r) { return sat8((EYR * r + EYG * g + EYB * b + EY0) >> SHIFT); }
+__device__ __forceinline__ uint32_t bgr_u(int b, int g, int r) { return sat8((EUR * r + EUG * g + EUB * b + EC0) >> SHIFT); }
+__device__ __forceinline__ uint32_t bgr_v(int b, int g, int r) { return sat8((EVR * r + EVG * g + EVB * b + EC0) >> SHIFT); }
 
 }  // namespace k0yuv
 

@@ -252,21 +252,3 @@ def multi_camera_batch(num_streams: int, frames_per_stream: int, width: int = 19
         for t in range(distinct, frames_per_stream):
             out[s, t] = out[s, t % distinct]
     return out
-
-
-def bgr_to_nv12(frames: np.ndarray) -> np.ndarray:
-    """``uint8[N,H,W,3]`` BGR frames -> ``uint8[N,H*3/2,W]`` in a video decoder's NV12 layout (Y plane followed by the
-    interleaved half-resolution UV plane), via cv2's BGR -> I420 conversion.  Makes decoder-shaped inputs for
-    ``LaneDetector.detect_batch_nv12`` / ``FrameIngest.from_nv12`` out of the synthetic frames; H and W must be even."""
-    frames = np.asarray(frames)
-    n, h, w = frames.shape[:3]
-    if h % 2 or w % 2:
-        raise ValueError("NV12 needs even width and height")
-    out = np.empty((n, h * 3 // 2, w), np.uint8)
-    for i in range(n):
-        i420 = cv2.cvtColor(frames[i], cv2.COLOR_BGR2YUV_I420)
-        out[i, :h] = i420[:h]
-        u = i420[h:h + h // 4].reshape(h // 2, w // 2)
-        v = i420[h + h // 4:].reshape(h // 2, w // 2)
-        out[i, h:] = np.stack([u, v], axis=-1).reshape(h // 2, w)
-    return out
