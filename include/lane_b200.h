@@ -35,9 +35,9 @@ extern "C" {
 
 typedef enum lane_status {
     LANE_OK = 0,
-    LANE_ERR_INVALID = -1,          /* bad argument (shape, null pointer, batch too large) */
+    LANE_ERR_INVALID = -1,          /* bad argument (shape, null pointer, batch too large, device index out of range) */
     LANE_ERR_CUDA = -2,             /* a CUDA runtime call or kernel failed; see lane_last_error */
-    LANE_ERR_NO_DEVICE = -3,        /* no usable sm_100 device: there is NO CPU fallback */
+    LANE_ERR_NO_DEVICE = -3,        /* no CUDA device visible, or (lane_ctx_create) not sm_100: there is NO CPU fallback */
     LANE_ERR_STATE = -4,            /* ROI / LUT not set before detect */
     LANE_ERR_UNSUPPORTED = -5       /* frame larger than this build supports */
 } lane_status;

@@ -56,6 +56,13 @@ class LaneError(RuntimeError):
         self.code = code
 
 
+def check_global(rc: int) -> None:
+    """Raise LaneError for a non-zero code from a call that reports through lane_last_error(NULL): context creation
+    and the context-free entry points."""
+    if rc:
+        raise LaneError(rc, (lib().lane_last_error(None) or b"").decode())
+
+
 def build(verbose: bool = False) -> str:
     """Compile the CUDA sources for sm_100a in-tree (nvcc cross-compiles without a GPU)."""
     out = subprocess.run(["make", "-C", CSRC, "-j8"], capture_output=True, text=True)
@@ -163,9 +170,7 @@ class LaneContext:
         self._h = None
         L = lib()
         h = C.c_void_p()
-        rc = L.lane_ctx_create(device, height, width, max_batch, max_segments, C.byref(h))
-        if rc != 0:
-            raise LaneError(rc, (L.lane_last_error(None) or b"").decode())
+        check_global(L.lane_ctx_create(device, height, width, max_batch, max_segments, C.byref(h)))
         self._h = h
         self.height, self.width, self.max_batch, self.device = height, width, max_batch, device
         self.max_segments = max_segments

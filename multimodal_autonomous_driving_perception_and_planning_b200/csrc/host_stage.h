@@ -1,7 +1,9 @@
-// Host-side staging of ordinary (pageable) memory for H2D and D2H copies.
+// The host/device boundary of the context-free entry points: error reporting, device selection, and host memory in and
+// out (staging of ordinary pageable memory for H2D and D2H copies, per-device scratch).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <stdio.h>
 #include <string.h>
 
 #include <algorithm>
@@ -10,8 +12,10 @@
 #include <thread>
 #include <vector>
 
+#include "lane_common.cuh"
+
 // Host frames in ordinary (pageable) memory: cudaMemcpy from such memory runs at ~11 GB/s on this platform (the
-// driver stages it single-threaded).  The context stages them itself instead: a few worker threads copy 32 MB
+// driver stages it single-threaded).  The library stages them itself instead: a few worker threads copy 32 MB
 // pieces into a small ring of pinned buffers while the previous piece is on its way over PCIe.
 struct CopyPool {
     std::vector<std::thread> th;
@@ -66,24 +70,34 @@ struct CopyPool {
 };
 
 
-// Context-free entry points (resize, frame statistics, egress) share one staging ring per device.  h2d() is blocking on the
-// host side only as far as the memcpy into pinned memory goes; the DMA itself is asynchronous on `st`.
+// One staging ring per device, shared by the contexts and the context-free entry points on it; the worker threads and
+// pinned buffers are created by the first staged copy.  h2d() is blocking on the host side only as far as the memcpy
+// into pinned memory goes; the DMA itself is asynchronous on `st`.
 struct HostStager {
     static constexpr int SLOTS = 3;
     static constexpr size_t PIECE = (size_t)32 << 20;
-    CopyPool pool;
+    CopyPool *pool = nullptr;
     uint8_t *stage[SLOTS] = {};
     cudaEvent_t ev[SLOTS] = {};
     bool used[SLOTS] = {};
+    int next = 0;                     // slot of the next h2d() piece: consecutive calls go round the ring
     std::mutex mu;
     bool ok = true;
 
-    HostStager() : pool((int)std::max(1u, std::min(8u, std::thread::hardware_concurrency() ? std::thread::hardware_concurrency() / 2 : 4u)))
+    bool ready()                      // under mu; false: the ring could not be allocated, copies take the DMA directly
     {
+        if (pool) return ok;
+        const unsigned hc = std::thread::hardware_concurrency();
+        pool = new CopyPool((int)std::max(1u, std::min(8u, hc ? hc / 2 : 4u)));
         for (int i = 0; i < SLOTS; i++)
             ok = ok && cudaHostAlloc((void **)&stage[i], PIECE, cudaHostAllocDefault) == cudaSuccess &&
                  cudaEventCreateWithFlags(&ev[i], cudaEventDisableTiming) == cudaSuccess;
+        cudaGetLastError();
+        return ok;
     }
+    // Whether a transfer of `bytes` to or from host `p` should go through the ring: ordinary memory, 24 MB or more.
+    // Pinned or registered memory goes straight to the copy engine, and small transfers (a single frame) are quicker
+    // through the driver's own path than through worker wake-ups.
     static bool pageable(const void *p, size_t bytes)
     {
         cudaPointerAttributes pa{};
@@ -91,17 +105,18 @@ struct HostStager {
         cudaGetLastError();
         return un && bytes >= ((size_t)24 << 20);
     }
+    // Through the ring, whatever the size (the caller has decided with pageable()).
     cudaError_t h2d(uint8_t *dst, const uint8_t *src, size_t bytes, cudaStream_t st)
     {
-        if (!ok || !pageable(src, bytes)) return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st);
         std::lock_guard<std::mutex> lk(mu);
-        int piece = 0;
-        for (size_t done = 0; done < bytes; done += PIECE, piece++) {
-            const int slot = piece % SLOTS;
+        if (!ready()) return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st);
+        for (size_t done = 0; done < bytes; done += PIECE) {
+            const int slot = next;
+            next = (next + 1) % SLOTS;
             const size_t nb = std::min(PIECE, bytes - done);
             cudaError_t e;
-            if (used[slot] && (e = cudaEventSynchronize(ev[slot]))) return e;
-            pool.run(stage[slot], src + done, nb);
+            if (used[slot] && (e = cudaEventSynchronize(ev[slot]))) return e;    // its last DMA has left
+            pool->run(stage[slot], src + done, nb);
             if ((e = cudaMemcpyAsync(dst + done, stage[slot], nb, cudaMemcpyHostToDevice, st))) return e;
             if ((e = cudaEventRecord(ev[slot], st))) return e;
             used[slot] = true;
@@ -115,9 +130,9 @@ struct HostStager {
     cudaError_t d2h(uint8_t *dst, const uint8_t *src, size_t bytes, cudaStream_t st)
     {
         cudaError_t e;
-        if (!ok) return (e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, st)) ? e : cudaStreamSynchronize(st);
-        constexpr size_t D2H_PIECE = PIECE / 4;
         std::lock_guard<std::mutex> lk(mu);
+        if (!ready()) return (e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, st)) ? e : cudaStreamSynchronize(st);
+        constexpr size_t D2H_PIECE = PIECE / 4;
         const size_t pieces = (bytes + D2H_PIECE - 1) / D2H_PIECE;
         auto issue = [&](size_t p) {
             const int slot = (int)(p % SLOTS);
@@ -135,19 +150,101 @@ struct HostStager {
             const int slot = (int)(p % SLOTS);
             if ((e = cudaEventSynchronize(ev[slot]))) return e;
             const size_t off = p * D2H_PIECE;
-            pool.run(dst + off, stage[slot], std::min(D2H_PIECE, bytes - off));
+            pool->run(dst + off, stage[slot], std::min(D2H_PIECE, bytes - off));
             if (p + SLOTS < pieces && (e = issue(p + SLOTS))) return e;
         }
         return cudaSuccess;
     }
 };
 
-inline HostStager *lane_host_stager(int device)      // one per device, created on first use, lives until exit
+// Everything the context-free entry points keep per device, until exit.  `mu` serialises the blocking calls that use
+// the scratch buffer or the copy stream; each returns with both idle.
+struct LaneDeviceHost {
+    std::mutex mu;
+    HostStager stager;
+    uint8_t *scratch = nullptr;       // grow-only: host round trips, frame statistics' sums, egress's conversion slots
+    size_t cap = 0;
+    cudaStream_t copy_st = nullptr;   // egress to host memory: copies out beside the conversions on the caller's stream
+    cudaEvent_t converted[2] = {}, copied[2] = {};
+
+    cudaError_t reserve(size_t bytes)
+    {
+        if (cap >= bytes) return cudaSuccess;
+        cudaFree(scratch);
+        scratch = nullptr;
+        cap = 0;
+        cudaError_t e = cudaMalloc((void **)&scratch, bytes);
+        if (!e) cap = bytes;
+        return e;
+    }
+    cudaError_t init_copy_stream()
+    {
+        if (copy_st) return cudaSuccess;
+        cudaError_t e;
+        for (int i = 0; i < 2; i++)
+            if ((e = cudaEventCreateWithFlags(&converted[i], cudaEventDisableTiming)) ||
+                (e = cudaEventCreateWithFlags(&copied[i], cudaEventDisableTiming)))
+                return e;
+        return cudaStreamCreateWithFlags(&copy_st, cudaStreamNonBlocking);
+    }
+};
+
+inline LaneDeviceHost &lane_device_host(int device)      // device: checked by lane_api_device; created on first use
 {
     static std::mutex mu;
-    static HostStager *all[64] = {};
-    if (device < 0 || device >= 64) return nullptr;
+    static LaneDeviceHost *all[LANE_MAX_DEVICES] = {};
     std::lock_guard<std::mutex> lk(mu);
-    if (!all[device]) all[device] = new HostStager();
-    return all[device];
+    if (!all[device]) all[device] = new LaneDeviceHost();
+    return *all[device];
+}
+
+// Reports a context-free call's failure: lane_last_error(NULL) reads "<who>: <what>[: <CUDA error>]".
+inline int lane_api_fail(int code, const char *who, const char *what, cudaError_t e = cudaSuccess)
+{
+    char buf[256];
+    snprintf(buf, sizeof buf, "%s: %s%s%s", who, what, e ? ": " : "", e ? cudaGetErrorString(e) : "");
+    lane_set_global_error(buf);
+    return code;
+}
+
+// Selects `device` for a context-free call, after its argument checks.
+inline int lane_api_device(const char *who, int device)
+{
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+        return lane_api_fail(LANE_ERR_NO_DEVICE, who, "no CUDA device visible: this library has no CPU fallback");
+    if (device < 0 || device >= std::min(ndev, LANE_MAX_DEVICES)) return lane_api_fail(LANE_ERR_INVALID, who, "device out of range");
+    const cudaError_t e = cudaSetDevice(device);
+    return e ? lane_api_fail(LANE_ERR_CUDA, who, "cudaSetDevice", e) : LANE_OK;
+}
+
+// The blocking host round trip of a context-free call, through the device's scratch buffer: `in_bytes` from host `in`
+// to d_in, launch(d_in, d_out) on `st`, `out_bytes` from d_out back to host `out`, synchronise.  No upload when `in` is
+// null (the generator clears its frames on the device), no download when `out` is null (frame statistics copy their
+// few sums themselves), and d_out == d_in when in == out (drawing on host frames).  Pageable buffers of 24 MB or more
+// go through the staging ring, all others straight to the DMA.  launch returns LANE_OK or a code it has reported.
+template <class Launch>
+int lane_host_round_trip(const char *who, int device, cudaStream_t st, const void *in, size_t in_bytes, void *out,
+                         size_t out_bytes, Launch &&launch)
+{
+    LaneDeviceHost &h = lane_device_host(device);
+    std::lock_guard<std::mutex> lk(h.mu);
+    const size_t in_span = in && in != out ? (in_bytes + 255) & ~(size_t)255 : 0;
+    cudaError_t e;
+    if ((e = h.reserve(std::max<size_t>(in_span + out_bytes, 1)))) return lane_api_fail(LANE_ERR_CUDA, who, "scratch allocation", e);
+    uint8_t *d_in = h.scratch, *d_out = h.scratch + in_span;
+    int rc = LANE_OK;
+    if (in) {
+        e = HostStager::pageable(in, in_bytes) ? h.stager.h2d(d_in, (const uint8_t *)in, in_bytes, st)
+                                               : cudaMemcpyAsync(d_in, in, in_bytes, cudaMemcpyHostToDevice, st);
+        if (e) rc = lane_api_fail(LANE_ERR_CUDA, who, "H2D", e);
+    }
+    if (!rc) rc = launch(d_in, d_out);
+    if (!rc && out) {
+        e = HostStager::pageable(out, out_bytes) ? h.stager.d2h((uint8_t *)out, d_out, out_bytes, st)
+                                                 : cudaMemcpyAsync(out, d_out, out_bytes, cudaMemcpyDeviceToHost, st);
+        if (e) rc = lane_api_fail(LANE_ERR_CUDA, who, "D2H", e);
+    }
+    if ((e = cudaStreamSynchronize(st)) && !rc) rc = lane_api_fail(LANE_ERR_CUDA, who, "host round trip", e);
+    return rc;
 }

@@ -8,8 +8,7 @@
 // and the 2x2 block's (U, V), k0_common.cuh) and apply k0_resize's 11-bit horizontal taps and vertical step to them:
 // the full-resolution BGR frame is never written.  HBM-bound: reads the touched 1.5 B/px of the source once, writes
 // 3 B per destination pixel.
-#include <stdio.h>
-
+#include "host_stage.h"
 #include "k0_common.cuh"
 
 namespace {
@@ -61,14 +60,6 @@ __global__ void __launch_bounds__(256) k0_yuv420_resize(const uint8_t *__restric
     }
 }
 
-int gfail(int code, const char *what, cudaError_t e = cudaSuccess)
-{
-    char buf[256];
-    snprintf(buf, sizeof buf, "lane_yuv420_to_bgr_batch: %s%s%s", what, e ? ": " : "", e ? cudaGetErrorString(e) : "");
-    lane_set_global_error(buf);
-    return code;
-}
-
 }  // namespace
 
 cudaError_t launch_ingest(const uint8_t *src, int format, int n, int sh, int sw, uint8_t *dst, int dh, int dw,
@@ -94,46 +85,42 @@ cudaError_t launch_ingest(const uint8_t *src, int format, int n, int sh, int sw,
     return cudaGetLastError();
 }
 
+namespace {
+
+int yuv420_to_bgr(const char *who, const uint8_t *src, int format, int n, int src_h, int src_w, uint8_t *dst, int dst_h,
+                  int dst_w, int on_device, int device, void *cuda_stream)
+{
+    if (!src || !dst || n < 1 || src_h < 1 || src_w < 1 || dst_h < 1 || dst_w < 1)
+        return lane_api_fail(LANE_ERR_INVALID, who, "bad arguments (non-null pointers, positive sizes)");
+    if (format != LANE_INPUT_NV12 && format != LANE_INPUT_I420)
+        return lane_api_fail(LANE_ERR_INVALID, who, "format must be LANE_INPUT_NV12 or LANE_INPUT_I420");
+    if ((src_h | src_w) & 1) return lane_api_fail(LANE_ERR_INVALID, who, "YUV 4:2:0 needs even width and height");
+    const bool resize = dst_h != src_h || dst_w != src_w;
+    if (resize && (dst_h > 65535 || n > 65535))
+        return lane_api_fail(LANE_ERR_UNSUPPORTED, who, "destination height / batch above 65535");
+    if (int rc = lane_api_device(who, device)) return rc;
+    cudaStream_t st = (cudaStream_t)cuda_stream;
+    auto launch = [&](const uint8_t *s, uint8_t *d) {
+        const cudaError_t e = launch_ingest(s, format, n, src_h, src_w, d, dst_h, dst_w, st);
+        return e ? lane_api_fail(LANE_ERR_CUDA, who, "launch", e) : LANE_OK;
+    };
+    if (on_device) return launch(src, dst);
+    return lane_host_round_trip(who, device, st, src, (size_t)n * src_h * src_w * 3 / 2, dst, (size_t)n * dst_h * dst_w * 3,
+                                launch);
+}
+
+}  // namespace
+
 extern "C" int lane_yuv420_to_bgr_batch(const uint8_t *src, int format, int n, int src_h, int src_w, uint8_t *dst,
                                         int dst_h, int dst_w, int on_device, int device, void *cuda_stream)
 {
-    if (!src || !dst || n < 1 || src_h < 1 || src_w < 1 || dst_h < 1 || dst_w < 1)
-        return gfail(LANE_ERR_INVALID, "bad arguments (non-null pointers, positive sizes)");
-    if (format != LANE_INPUT_NV12 && format != LANE_INPUT_I420)
-        return gfail(LANE_ERR_INVALID, "format must be LANE_INPUT_NV12 or LANE_INPUT_I420");
-    if ((src_h | src_w) & 1) return gfail(LANE_ERR_INVALID, "YUV 4:2:0 needs even width and height");
-    const bool resize = dst_h != src_h || dst_w != src_w;
-    if (resize && (dst_h > 65535 || n > 65535)) return gfail(LANE_ERR_UNSUPPORTED, "destination height / batch above 65535");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-        return gfail(LANE_ERR_NO_DEVICE, "no CUDA device visible: this library has no CPU fallback");
-    if (device < 0 || device >= ndev) return gfail(LANE_ERR_INVALID, "device out of range");
-    cudaError_t e;
-    if ((e = cudaSetDevice(device))) return gfail(LANE_ERR_CUDA, "cudaSetDevice", e);
-    cudaStream_t st = (cudaStream_t)cuda_stream;
-    if (on_device) {
-        if ((e = launch_ingest(src, format, n, src_h, src_w, dst, dst_h, dst_w, st))) return gfail(LANE_ERR_CUDA, "launch", e);
-        return LANE_OK;
-    }
-    const size_t in_bytes = (size_t)n * src_h * src_w * 3 / 2, out_bytes = (size_t)n * dst_h * dst_w * 3;
-    uint8_t *d_in = nullptr, *d_out = nullptr;
-    if ((e = cudaMalloc((void **)&d_in, in_bytes)) || (e = cudaMalloc((void **)&d_out, out_bytes))) {
-        cudaFree(d_in);
-        cudaGetLastError();
-        return gfail(LANE_ERR_CUDA, "device allocation", e);
-    }
-    e = cudaMemcpyAsync(d_in, src, in_bytes, cudaMemcpyHostToDevice, st);
-    if (!e) e = launch_ingest(d_in, format, n, src_h, src_w, d_out, dst_h, dst_w, st);
-    if (!e) e = cudaMemcpyAsync(dst, d_out, out_bytes, cudaMemcpyDeviceToHost, st);
-    if (!e) e = cudaStreamSynchronize(st);
-    cudaFree(d_in); cudaFree(d_out);
-    if (e) return gfail(LANE_ERR_CUDA, "host round trip", e);
-    return LANE_OK;
+    return yuv420_to_bgr("lane_yuv420_to_bgr_batch", src, format, n, src_h, src_w, dst, dst_h, dst_w, on_device, device,
+                         cuda_stream);
 }
 
 extern "C" int lane_nv12_to_bgr_batch(const uint8_t *src, int n, int height, int width, uint8_t *dst, int on_device,
                                       int device, void *cuda_stream)
 {
-    return lane_yuv420_to_bgr_batch(src, LANE_INPUT_NV12, n, height, width, dst, height, width, on_device, device,
-                                    cuda_stream);
+    return yuv420_to_bgr("lane_nv12_to_bgr_batch", src, LANE_INPUT_NV12, n, height, width, dst, height, width, on_device,
+                         device, cuda_stream);
 }

@@ -8,7 +8,6 @@
 //
 // Bound: HBM (reads the touched source pixels once, writes the destination once; no arithmetic to speak of).
 #include <math.h>
-#include <stdio.h>
 
 #include <map>
 #include <mutex>
@@ -104,14 +103,6 @@ __global__ void __launch_bounds__(256) k0_resize(const uint8_t *__restrict__ src
     }
 }
 
-int rfail(int code, const char *what, cudaError_t e)
-{
-    char buf[256];
-    snprintf(buf, sizeof buf, "lane_resize_batch: %s%s%s", what, e ? ": " : "", e ? cudaGetErrorString(e) : "");
-    lane_set_global_error(buf);
-    return code;
-}
-
 }  // namespace
 
 cudaError_t lane_resize_taps(int sh, int sw, int dh, int dw, ResizeTaps *t)
@@ -145,36 +136,21 @@ void launch_resize(const uint8_t *src, uint8_t *dst, int n, int channels, int sh
 extern "C" int lane_resize_batch(const uint8_t *src, int n, int src_h, int src_w, int channels, uint8_t *dst, int dst_h,
                                  int dst_w, int on_device, int device, void *cuda_stream)
 {
+    constexpr const char *who = "lane_resize_batch";
     if (!src || !dst || n <= 0 || src_h <= 0 || src_w <= 0 || dst_h <= 0 || dst_w <= 0 || (channels != 1 && channels != 3))
-        return rfail(LANE_ERR_INVALID, "bad arguments (uint8 frames with 1 or 3 channels, positive sizes)", cudaSuccess);
-    if (dst_h > 65535 || n > 65535) return rfail(LANE_ERR_UNSUPPORTED, "destination height / batch above 65535", cudaSuccess);
-    int count = 0;
-    if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0 || device < 0 || device >= count)
-        return rfail(LANE_ERR_NO_DEVICE, "no usable CUDA device (there is no CPU fallback)", cudaSuccess);
+        return lane_api_fail(LANE_ERR_INVALID, who, "bad arguments (uint8 frames with 1 or 3 channels, positive sizes)");
+    if (dst_h > 65535 || n > 65535) return lane_api_fail(LANE_ERR_UNSUPPORTED, who, "destination height / batch above 65535");
+    if (int rc = lane_api_device(who, device)) return rc;
     cudaError_t e;
-    if ((e = cudaSetDevice(device))) return rfail(LANE_ERR_CUDA, "cudaSetDevice", e);
     ResizeTaps t;
-    if ((e = lane_resize_taps(src_h, src_w, dst_h, dst_w, &t))) return rfail(LANE_ERR_CUDA, "tap tables", e);
+    if ((e = lane_resize_taps(src_h, src_w, dst_h, dst_w, &t))) return lane_api_fail(LANE_ERR_CUDA, who, "tap tables", e);
     cudaStream_t st = (cudaStream_t)cuda_stream;
-    const size_t sbytes = (size_t)n * src_h * src_w * channels, dbytes = (size_t)n * dst_h * dst_w * channels;
-    const uint8_t *s_dev = src;
-    uint8_t *d_dev = dst;
-    uint8_t *tmp = nullptr;
-    if (!on_device) {
-        if ((e = cudaMalloc(&tmp, sbytes + dbytes))) return rfail(LANE_ERR_CUDA, "staging allocation", e);
-        HostStager *hs = lane_host_stager(device);
-        e = hs ? hs->h2d(tmp, src, sbytes, st) : cudaMemcpyAsync(tmp, src, sbytes, cudaMemcpyHostToDevice, st);
-        if (e) { cudaFree(tmp); return rfail(LANE_ERR_CUDA, "H2D", e); }
-        s_dev = tmp;
-        d_dev = tmp + sbytes;
-    }
-    launch_resize(s_dev, d_dev, n, channels, src_h, src_w, dst_h, dst_w, t, st);
-    if ((e = cudaGetLastError())) { if (tmp) cudaFree(tmp); return rfail(LANE_ERR_CUDA, "kernel launch", e); }
-    if (!on_device) {
-        e = cudaMemcpyAsync(dst, d_dev, dbytes, cudaMemcpyDeviceToHost, st);
-        if (!e) e = cudaStreamSynchronize(st);
-        cudaFree(tmp);
-        if (e) return rfail(LANE_ERR_CUDA, "D2H", e);
-    }
-    return LANE_OK;
+    auto launch = [&](const uint8_t *s, uint8_t *d) {
+        launch_resize(s, d, n, channels, src_h, src_w, dst_h, dst_w, t, st);
+        const cudaError_t r = cudaGetLastError();
+        return r ? lane_api_fail(LANE_ERR_CUDA, who, "kernel launch", r) : LANE_OK;
+    };
+    if (on_device) return launch(src, dst);
+    return lane_host_round_trip(who, device, st, src, (size_t)n * src_h * src_w * channels, dst,
+                                (size_t)n * dst_h * dst_w * channels, launch);
 }

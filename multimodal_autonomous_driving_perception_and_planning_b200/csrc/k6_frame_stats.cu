@@ -16,11 +16,9 @@
 // Bound: HBM (3 B/px read, nothing written).  A CTA takes a 64x128 tile: gray of the tile and its one-pixel frame
 // goes to shared memory once (gray sum and green test on the way), the Laplacian reads it back.
 #include <math.h>
-#include <stdio.h>
 #include <stdlib.h>
 
 #include <algorithm>
-#include <mutex>
 #include <type_traits>
 
 #include <vector>
@@ -270,27 +268,15 @@ __global__ void __launch_bounds__(K6_WARPS * 32, 5) k6_strip(const uint8_t *__re
     }
 }
 
-int sfail(int code, const char *what, cudaError_t e)
-{
-    char buf[256];
-    snprintf(buf, sizeof buf, "lane_frame_stats: %s%s%s", what, e ? ": " : "", e ? cudaGetErrorString(e) : "");
-    lane_set_global_error(buf);
-    return code;
-}
-
 }  // namespace
 
 extern "C" int lane_frame_stats(const uint8_t *frames, int on_device, int n, int height, int width, lane_frame_stat *out,
                                 int device, void *cuda_stream)
 {
-    if (!frames || !out || n <= 0 || height <= 0 || width <= 0)
-        return sfail(LANE_ERR_INVALID, "bad arguments", cudaSuccess);
-    if (n > 65535) return sfail(LANE_ERR_UNSUPPORTED, "batch above 65535", cudaSuccess);
-    int count = 0;
-    if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0 || device < 0 || device >= count)
-        return sfail(LANE_ERR_NO_DEVICE, "no usable CUDA device (there is no CPU fallback)", cudaSuccess);
-    cudaError_t e;
-    if ((e = cudaSetDevice(device))) return sfail(LANE_ERR_CUDA, "cudaSetDevice", e);
+    constexpr const char *who = "lane_frame_stats";
+    if (!frames || !out || n <= 0 || height <= 0 || width <= 0) return lane_api_fail(LANE_ERR_INVALID, who, "bad arguments");
+    if (n > 65535) return lane_api_fail(LANE_ERR_UNSUPPORTED, who, "batch above 65535");
+    if (int rc = lane_api_device(who, device)) return rc;
     cudaStream_t st = (cudaStream_t)cuda_stream;
     // OpenCV's tables: sdiv[i] = round(255*4096 / i), hdiv180[i] = round(180*4096 / (6*i)), entry 0 unused
     int h_tab[512] = {0};
@@ -298,58 +284,42 @@ extern "C" int lane_frame_stats(const uint8_t *frames, int on_device, int n, int
         h_tab[i] = (int)lrint((255 << 12) / (1. * i));
         h_tab[256 + i] = (int)lrint((180 << 12) / (6. * i));
     }
-    const size_t fbytes = (size_t)n * height * width * 3;
-    // grow-only scratch per device (tables, sums, staging for host frames); calls are serialised by the mutex
-    static std::mutex mu;
-    static uint8_t *cache[64] = {nullptr};
-    static size_t cache_bytes[64] = {0};
-    std::lock_guard<std::mutex> lk(mu);
-    uint8_t *scratch = nullptr;
-    const size_t acc_bytes = ((size_t)n * 4 + 2) * sizeof(unsigned long long);   // sums + the strip kernel's task counter
-    const size_t need = 512 * sizeof(int) + acc_bytes + 256 + (on_device ? 0 : fbytes);
-    if (device < 64 && cache_bytes[device] >= need) {
-        scratch = cache[device];
-    } else {
-        if (device < 64 && cache[device]) { cudaFree(cache[device]); cache[device] = nullptr; cache_bytes[device] = 0; }
-        if ((e = cudaMalloc(&scratch, need))) return sfail(LANE_ERR_CUDA, "scratch allocation", e);
-        if (device < 64) { cache[device] = scratch; cache_bytes[device] = need; }
-    }
-    const bool owned = device >= 64;
-    int *d_tab = reinterpret_cast<int *>(scratch);
-    unsigned long long *d_acc = reinterpret_cast<unsigned long long *>(scratch + 512 * sizeof(int));
-    const uint8_t *d_frames = frames;
-    e = cudaMemcpyAsync(d_tab, h_tab, sizeof h_tab, cudaMemcpyHostToDevice, st);
-    if (!e) e = cudaMemsetAsync(d_acc, 0, (size_t)n * 4 * sizeof(unsigned long long), st);
-    if (!e && !on_device) {
-        uint8_t *df = scratch + ((512 * sizeof(int) + acc_bytes + 255) & ~(size_t)255);
-        HostStager *hs = lane_host_stager(device);
-        e = hs ? hs->h2d(df, frames, fbytes, st) : cudaMemcpyAsync(df, frames, fbytes, cudaMemcpyHostToDevice, st);
-        d_frames = df;
-    }
-    if (e) { if (owned) cudaFree(scratch); return sfail(LANE_ERR_CUDA, "upload", e); }
-    dim3 grid((width + TC - 1) / TC, (height + TR - 1) / TR, n);
-    if (grid.y > 65535) { if (owned) cudaFree(scratch); return sfail(LANE_ERR_UNSUPPORTED, "frame too tall", cudaSuccess); }
-    const bool strip = width % 16 == 0 && ((uintptr_t)d_frames % 16) == 0 && height >= 2 &&
-                       (size_t)height * width * 3 < ((size_t)1 << 32);
-    if (strip) {
-        int sms = 0;
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-        int *d_counter = reinterpret_cast<int *>(d_acc + (size_t)n * 4);       // task counter, right behind the sums
-        e = cudaMemsetAsync(d_counter, 0, sizeof(int), st);
-        const int n_strips = (width + K6_STRIP - 1) / K6_STRIP, warps = sms * 5 * K6_WARPS;
-        const long rows_per_warp = ((long)n * height * n_strips + 2 * warps - 1) / (2 * warps);
-        const int band_rows = (int)std::max(12L, std::min(102L, rows_per_warp));
-        k6_strip<<<sms * 5, K6_WARPS * 32, 0, st>>>(d_frames, d_acc, d_counter, n, height, width, band_rows, d_tab, d_tab + 256,
-                                                    35, 85, 40, 40);
-    } else {
-        k6_frame_stats<<<grid, K6T, 0, st>>>(d_frames, d_acc, height, width, d_tab, d_tab + 256, 35, 85, 40, 40);
-    }
     std::vector<unsigned long long> h_acc((size_t)n * 4);
-    e = cudaGetLastError();
-    if (!e) e = cudaMemcpyAsync(h_acc.data(), d_acc, h_acc.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st);
-    if (!e) e = cudaStreamSynchronize(st);
-    if (owned) cudaFree(scratch);
-    if (e) return sfail(LANE_ERR_CUDA, "kernel / download", e);
+    bool strip = false;
+    // device scratch: the tables, then the sums and the strip kernel's task counter
+    const size_t scratch_bytes = 512 * sizeof(int) + ((size_t)n * 4 + 2) * sizeof(unsigned long long);
+    auto launch = [&](const uint8_t *staged, uint8_t *scratch) {
+        int *d_tab = reinterpret_cast<int *>(scratch);
+        unsigned long long *d_acc = reinterpret_cast<unsigned long long *>(scratch + 512 * sizeof(int));
+        const uint8_t *d_frames = on_device ? frames : staged;
+        cudaError_t e = cudaMemcpyAsync(d_tab, h_tab, sizeof h_tab, cudaMemcpyHostToDevice, st);
+        if (!e) e = cudaMemsetAsync(d_acc, 0, (size_t)n * 4 * sizeof(unsigned long long), st);
+        if (e) return lane_api_fail(LANE_ERR_CUDA, who, "upload", e);
+        dim3 grid((width + TC - 1) / TC, (height + TR - 1) / TR, n);
+        if (grid.y > 65535) return lane_api_fail(LANE_ERR_UNSUPPORTED, who, "frame too tall");
+        strip = width % 16 == 0 && ((uintptr_t)d_frames % 16) == 0 && height >= 2 &&
+                (size_t)height * width * 3 < ((size_t)1 << 32);
+        if (strip) {
+            int sms = 0;
+            cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+            int *d_counter = reinterpret_cast<int *>(d_acc + (size_t)n * 4);       // task counter, right behind the sums
+            e = cudaMemsetAsync(d_counter, 0, sizeof(int), st);
+            const int n_strips = (width + K6_STRIP - 1) / K6_STRIP, warps = sms * 5 * K6_WARPS;
+            const long rows_per_warp = ((long)n * height * n_strips + 2 * warps - 1) / (2 * warps);
+            const int band_rows = (int)std::max(12L, std::min(102L, rows_per_warp));
+            k6_strip<<<sms * 5, K6_WARPS * 32, 0, st>>>(d_frames, d_acc, d_counter, n, height, width, band_rows, d_tab, d_tab + 256,
+                                                        35, 85, 40, 40);
+        } else {
+            k6_frame_stats<<<grid, K6T, 0, st>>>(d_frames, d_acc, height, width, d_tab, d_tab + 256, 35, 85, 40, 40);
+        }
+        e = cudaGetLastError();
+        if (!e) e = cudaMemcpyAsync(h_acc.data(), d_acc, h_acc.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st);
+        return e ? lane_api_fail(LANE_ERR_CUDA, who, "kernel / download", e) : LANE_OK;
+    };
+    // host frames go in ahead of the scratch; the few sums come back in launch
+    const int rc = lane_host_round_trip(who, device, st, on_device ? nullptr : frames, on_device ? 0 : (size_t)n * height * width * 3,
+                                        nullptr, scratch_bytes, launch);
+    if (rc) return rc;
     for (int i = 0; i < n; i++) {
         out[i].sum_gray = h_acc[4 * i];
         if (strip) {                                         // the strip kernel sums L' = L + 1020

@@ -39,7 +39,7 @@
 #include <vector>
 
 #include "draw_prims.h"
-#include "lane_common.cuh"
+#include "host_stage.h"
 
 using namespace lane_draw;
 
@@ -476,14 +476,25 @@ struct Chunk {
 inline int band_lo(const Prim &p) { return p.y0 / BAND_ROWS; }
 inline int band_hi(const Prim &p) { return p.y1 / BAND_ROWS; }
 
+// launch(d_frames, d_frames) on frames that are drawn on in place: device frames directly, host frames through the
+// device's scratch (cleared there instead of uploaded when `clear_first`).  Blocking either way.
+template <class Launch>
+int draw_frames(const char *who, uint8_t *frames, int on_device, size_t bytes, int device, cudaStream_t st, bool clear_first,
+                Launch &&launch)
+{
+    if (!on_device) return lane_host_round_trip(who, device, st, clear_first ? nullptr : frames, bytes, frames, bytes, launch);
+    const int rc = launch(frames, frames);
+    const cudaError_t e = cudaStreamSynchronize(st);
+    return rc ? rc : e ? lane_api_fail(LANE_ERR_CUDA, who, "synchronise", e) : LANE_OK;
+}
+
 // The host half, frames in parallel: worker t expands the drawing calls of its frames into primitives and counts them per
 // band; the lists are then laid out in one pinned block (band offsets | primitives | side tables | per-band index lists),
 // filled by the same workers, and uploaded with one copy.  build_frame(Builder&, int f, const char **err) -> bool.
 template <class BuildFrame>
-int draw_driver(uint8_t *frames, int on_device, int n, int H, int W, int device, cudaStream_t st, float *device_ms,
-                BuildFrame build_frame, bool clear_first = false)
+int draw_driver(const char *who, uint8_t *frames, int on_device, int n, int H, int W, int device, cudaStream_t st,
+                float *device_ms, BuildFrame build_frame, bool clear_first = false)
 {
-    auto fail = [](int code, const char *msg) { lane_set_global_error(msg); return code; };
     const int bands = (H + BAND_ROWS - 1) / BAND_ROWS;
     const int T = std::max(1, std::min({n / 8, (int)std::thread::hardware_concurrency(), 16}));
     std::vector<Chunk> chunks(T);
@@ -511,7 +522,7 @@ int draw_driver(uint8_t *frames, int on_device, int n, int H, int W, int device,
         c.b.begin.push_back((int64_t)c.b.prims.size());
     });
     for (const Chunk &c : chunks)
-        if (c.err) return fail(LANE_ERR_INVALID, c.err);
+        if (c.err) return lane_api_fail(LANE_ERR_INVALID, who, c.err);
     int64_t n_prims = 0, n_side = 0;
     for (Chunk &c : chunks) {
         c.prim_base = n_prims;
@@ -533,7 +544,7 @@ int draw_driver(uint8_t *frames, int on_device, int n, int H, int W, int device,
                  off_idx = (off_side + nb_side + 63) & ~(size_t)63, total = off_idx + nb_idx;
 
     std::lock_guard<std::mutex> lk(g_draw_mutex);
-    DrawCache &c = g_draw_cache[device & (LANE_MAX_DEVICES - 1)];
+    DrawCache &c = g_draw_cache[device];
     if (c.cap < total) {
         if (c.d) cudaFree(c.d);
         if (c.h) cudaFreeHost(c.h);
@@ -547,7 +558,7 @@ int draw_driver(uint8_t *frames, int on_device, int n, int H, int W, int device,
             if (c.d) cudaFree(c.d);
             c = DrawCache{};
             cudaGetLastError();
-            return fail(LANE_ERR_CUDA, "lane_draw: staging allocation failed");
+            return lane_api_fail(LANE_ERR_CUDA, who, "staging allocation failed");
         }
         c.cap = cap;
     }
@@ -575,60 +586,39 @@ int draw_driver(uint8_t *frames, int on_device, int n, int H, int W, int device,
         if (!local.empty()) memcpy(hi + idx0, local.data(), local.size() * 4);
     });
 
-    const size_t frame_bytes = (size_t)n * H * W * 3;
-    uint8_t *d_frames = frames;
-    if (!on_device) {
-        if (cudaMalloc((void **)&d_frames, frame_bytes) != cudaSuccess) { cudaGetLastError(); return fail(LANE_ERR_CUDA, "lane_draw: device allocation failed"); }
-        if (!clear_first) cudaMemcpyAsync(d_frames, frames, frame_bytes, cudaMemcpyHostToDevice, st);
-    }
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    if (device_ms) { cudaEventCreate(&e0); cudaEventCreate(&e1); cudaEventRecord(e0, st); }
-    if (clear_first) cudaMemsetAsync(d_frames, 0, frame_bytes, st);
-    cudaMemcpyAsync(d, h, total, cudaMemcpyHostToDevice, st);
+    cudaEvent_t e0 = nullptr, e1 = nullptr, ec = nullptr;
     static const bool dbg = getenv("LANE_B200_DRAW_DEBUG") != nullptr;
-    cudaEvent_t ec = nullptr;
-    if (dbg && device_ms) { cudaEventCreate(&ec); cudaEventRecord(ec, st); }
-    const int WW = (W + 31) >> 5;
-    const size_t mask_words = (size_t)BAND_ROWS * WW;
-    const size_t smem = (mask_words + (mask_words & 1)) * 4 + (size_t)(DRAW_THREADS / 32) * MAX_ROW_EDGES * 8;
-    static bool configured[LANE_MAX_DEVICES];
-    if (smem > 48 * 1024 && !configured[device & (LANE_MAX_DEVICES - 1)]) {
-        cudaFuncSetAttribute(k7_draw, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        configured[device & (LANE_MAX_DEVICES - 1)] = true;
-    }
-    if (smem > 200 * 1024) {
-        if (!on_device) cudaFree(d_frames);
-        return fail(LANE_ERR_UNSUPPORTED, "lane_draw: frame too wide for the band mask");
-    }
-    k7_draw<<<dim3(bands, n), DRAW_THREADS, smem, st>>>(d_frames, (const Prim *)(d + off_prims), (const int64_t *)d,
-                                                        (const int32_t *)(d + off_idx), (const int64_t *)(d + off_side), H, W);
-    cudaError_t e = cudaGetLastError();
-    if (device_ms) cudaEventRecord(e1, st);
-    if (e == cudaSuccess && !on_device) cudaMemcpyAsync(frames, d_frames, frame_bytes, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    if (e == cudaSuccess && device_ms) cudaEventElapsedTime(device_ms, e0, e1);
+    auto launch = [&](uint8_t *d_frames, uint8_t *) {
+        if (device_ms) { cudaEventCreate(&e0); cudaEventCreate(&e1); cudaEventRecord(e0, st); }
+        if (clear_first) cudaMemsetAsync(d_frames, 0, (size_t)n * H * W * 3, st);
+        cudaMemcpyAsync(d, h, total, cudaMemcpyHostToDevice, st);
+        if (dbg && device_ms) { cudaEventCreate(&ec); cudaEventRecord(ec, st); }
+        const int WW = (W + 31) >> 5;
+        const size_t mask_words = (size_t)BAND_ROWS * WW;
+        const size_t smem = (mask_words + (mask_words & 1)) * 4 + (size_t)(DRAW_THREADS / 32) * MAX_ROW_EDGES * 8;
+        static bool configured[LANE_MAX_DEVICES];
+        if (smem > 48 * 1024 && !configured[device]) {
+            cudaFuncSetAttribute(k7_draw, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+            configured[device] = true;
+        }
+        if (smem > 200 * 1024) return lane_api_fail(LANE_ERR_UNSUPPORTED, who, "frame too wide for the band mask");
+        k7_draw<<<dim3(bands, n), DRAW_THREADS, smem, st>>>(d_frames, (const Prim *)(d + off_prims), (const int64_t *)d,
+                                                            (const int32_t *)(d + off_idx), (const int64_t *)(d + off_side), H, W);
+        const cudaError_t e = cudaGetLastError();
+        if (device_ms) cudaEventRecord(e1, st);
+        return e ? lane_api_fail(LANE_ERR_CUDA, who, "k7_draw launch", e) : LANE_OK;
+    };
+    int rc = draw_frames(who, frames, on_device, (size_t)n * H * W * 3, device, st, clear_first, launch);
+    if (rc == LANE_OK && device_ms) cudaEventElapsedTime(device_ms, e0, e1);
     if (ec) {
         float cms = 0;
-        if (e == cudaSuccess) cudaEventElapsedTime(&cms, e0, ec);
+        if (rc == LANE_OK) cudaEventElapsedTime(&cms, e0, ec);
         fprintf(stderr, "lane_draw: %lld primitives, %lld band entries, %.2f MB uploaded in %.3f ms, upload + kernel %.3f ms, %d host threads\n",
                 (long long)n_prims, (long long)n_idx, total / 1e6, cms, device_ms ? *device_ms : 0.f, T);
         cudaEventDestroy(ec);
     }
     if (e0) { cudaEventDestroy(e0); cudaEventDestroy(e1); }
-    if (!on_device) cudaFree(d_frames);
-    if (e != cudaSuccess) return fail(LANE_ERR_CUDA, cudaGetErrorString(e));
-    return LANE_OK;
-}
-
-int prepare_device(int device)
-{
-    auto fail = [](int code, const char *msg) { lane_set_global_error(msg); return code; };
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-        return fail(LANE_ERR_NO_DEVICE, "no CUDA device visible: this library has no CPU fallback");
-    if (device < 0 || device >= ndev) return fail(LANE_ERR_INVALID, "lane_draw: device out of range");
-    if (cudaSetDevice(device) != cudaSuccess) return fail(LANE_ERR_CUDA, "cudaSetDevice failed");
-    return LANE_OK;
+    return rc;
 }
 
 }  // namespace
@@ -636,14 +626,14 @@ int prepare_device(int device)
 extern "C" int lane_draw_commands(uint8_t *frames, int on_device, int n, int height, int width, const int32_t *commands,
                                   const int64_t *command_begin, int device, void *cuda_stream, float *device_ms)
 {
-    auto fail = [](int code, const char *msg) { lane_set_global_error(msg); return code; };
+    constexpr const char *who = "lane_draw_commands";
     if (!frames || !commands || !command_begin || n < 1 || height < 1 || width < 1)
-        return fail(LANE_ERR_INVALID, "lane_draw_commands: bad arguments");
-    if (height > 32767 || width > 32767) return fail(LANE_ERR_UNSUPPORTED, "lane_draw_commands: frame larger than 32767 px");
+        return lane_api_fail(LANE_ERR_INVALID, who, "bad arguments");
+    if (height > 32767 || width > 32767) return lane_api_fail(LANE_ERR_UNSUPPORTED, who, "frame larger than 32767 px");
     for (int f = 0; f < n; f++)
-        if (command_begin[f + 1] < command_begin[f]) return fail(LANE_ERR_INVALID, "lane_draw_commands: command_begin must not decrease");
-    if (int rc = prepare_device(device)) return rc;
-    return draw_driver(frames, on_device, n, height, width, device, (cudaStream_t)cuda_stream, device_ms,
+        if (command_begin[f + 1] < command_begin[f]) return lane_api_fail(LANE_ERR_INVALID, who, "command_begin must not decrease");
+    if (int rc = lane_api_device(who, device)) return rc;
+    return draw_driver(who, frames, on_device, n, height, width, device, (cudaStream_t)cuda_stream, device_ms,
                        [&](Builder &b, int f, const char **err) {
                            return parse_commands(b, commands + command_begin[f], command_begin[f + 1] - command_begin[f], err);
                        });
@@ -656,21 +646,23 @@ struct LaneItem {                    // what k7_lanes reads per frame when the l
     int32_t valid[2];
 };
 
-int launch_lanes(uint8_t *d_frames, const LaneSrc &src, int n, int H, int W, int fill_lane, cudaStream_t st, int device)
+int launch_lanes(const char *who, uint8_t *d_frames, const LaneSrc &src, int n, int H, int W, int fill_lane, cudaStream_t st,
+                 int device)
 {
     const int bands = (H + BAND_ROWS - 1) / BAND_ROWS, WW = (W + 31) >> 5;
     const size_t mask_words = (size_t)BAND_ROWS * WW;
     const size_t smem = (mask_words + (mask_words & 1)) * 4 + (size_t)(DRAW_THREADS / 32) * MAX_ROW_EDGES * 8;
     static bool configured[LANE_MAX_DEVICES];
-    if (smem > 44 * 1024 && !configured[device & (LANE_MAX_DEVICES - 1)]) {
+    if (smem > 44 * 1024 && !configured[device]) {
         cudaFuncSetAttribute(k7_lanes, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        configured[device & (LANE_MAX_DEVICES - 1)] = true;
+        configured[device] = true;
     }
-    if (smem > 200 * 1024) return LANE_ERR_UNSUPPORTED;
+    if (smem > 200 * 1024) return lane_api_fail(LANE_ERR_UNSUPPORTED, who, "frame too wide for the band mask");
     // (0, 255, 100) at weight 0.3 over 0.7 (lane_detector.py:243-244), left (255, 0, 0) :248, right (0, 0, 255) :251
     k7_lanes<<<dim3(bands, n), DRAW_THREADS, smem, st>>>(d_frames, src, H, W, fill_lane, 0u | 255u << 8 | 100u << 16, 255u, 255u << 16,
                                                         0.7f, 0.3f);
-    return cudaGetLastError() == cudaSuccess ? LANE_OK : LANE_ERR_CUDA;
+    const cudaError_t e = cudaGetLastError();
+    return e ? lane_api_fail(LANE_ERR_CUDA, who, "k7_lanes launch", e) : LANE_OK;
 }
 
 bool lanes_by_primitives()           // LANE_B200_DRAW_LANES=prims: the host-expanded primitive lists (A/B, and the tests run both)
@@ -685,23 +677,23 @@ extern "C" int lane_draw_lanes_batch(uint8_t *frames, int on_device, int n, int 
                                      const uint8_t *left_valid, const int32_t *right_points, const uint8_t *right_valid,
                                      int fill_lane, int device, void *cuda_stream, float *device_ms)
 {
-    auto fail = [](int code, const char *msg) { lane_set_global_error(msg); return code; };
+    constexpr const char *who = "lane_draw_lanes_batch";
     if (!frames || !left_points || !right_points || !left_valid || !right_valid || n < 1 || height < 1 || width < 1)
-        return fail(LANE_ERR_INVALID, "lane_draw_lanes_batch: bad arguments");
-    if (height > 32767 || width > 32767) return fail(LANE_ERR_UNSUPPORTED, "lane_draw_lanes_batch: frame larger than 32767 px");
-    if (int rc = prepare_device(device)) return rc;
+        return lane_api_fail(LANE_ERR_INVALID, who, "bad arguments");
+    if (height > 32767 || width > 32767) return lane_api_fail(LANE_ERR_UNSUPPORTED, who, "frame larger than 32767 px");
+    if (int rc = lane_api_device(who, device)) return rc;
     cudaStream_t st = (cudaStream_t)cuda_stream;
     if (lanes_by_primitives())
-        return draw_driver(frames, on_device, n, height, width, device, st, device_ms,
+        return draw_driver(who, frames, on_device, n, height, width, device, st, device_ms,
                            [&](Builder &b, int f, const char **) {
                                build_draw_lanes_frame(b, left_points + (size_t)f * LANE_NUM_POINTS * 2, left_valid[f],
                                                       right_points + (size_t)f * LANE_NUM_POINTS * 2, right_valid[f], fill_lane);
                                return true;
                            });
     // default: the geometry runs on the device (k7_lanes); only the 100 points per frame are uploaded
-    const size_t item_bytes = (size_t)n * sizeof(LaneItem), frame_bytes = (size_t)n * height * width * 3;
+    const size_t item_bytes = (size_t)n * sizeof(LaneItem);
     std::lock_guard<std::mutex> lk(g_draw_mutex);
-    DrawCache &c = g_draw_cache[device & (LANE_MAX_DEVICES - 1)];
+    DrawCache &c = g_draw_cache[device];
     if (c.cap < item_bytes) {
         if (c.d) cudaFree(c.d);
         if (c.h) cudaFreeHost(c.h);
@@ -711,7 +703,7 @@ extern "C" int lane_draw_lanes_batch(uint8_t *frames, int on_device, int n, int 
             if (c.d) cudaFree(c.d);
             c = DrawCache{};
             cudaGetLastError();
-            return fail(LANE_ERR_CUDA, "lane_draw_lanes_batch: staging allocation failed");
+            return lane_api_fail(LANE_ERR_CUDA, who, "staging allocation failed");
         }
         c.cap = cap;
     }
@@ -722,53 +714,43 @@ extern "C" int lane_draw_lanes_batch(uint8_t *frames, int on_device, int n, int 
         items[f].valid[0] = left_valid[f] != 0;
         items[f].valid[1] = right_valid[f] != 0;
     }
-    uint8_t *d_frames = frames;
-    if (!on_device) {
-        if (cudaMalloc((void **)&d_frames, frame_bytes) != cudaSuccess) { cudaGetLastError(); return fail(LANE_ERR_CUDA, "lane_draw_lanes_batch: device allocation failed"); }
-        cudaMemcpyAsync(d_frames, frames, frame_bytes, cudaMemcpyHostToDevice, st);
-    }
     cudaEvent_t e0 = nullptr, e1 = nullptr;
-    if (device_ms) { cudaEventCreate(&e0); cudaEventCreate(&e1); cudaEventRecord(e0, st); }
-    cudaMemcpyAsync(c.d, c.h, item_bytes, cudaMemcpyHostToDevice, st);
-    LaneSrc src{(const char *)c.d, sizeof(LaneItem), {offsetof(LaneItem, pts), offsetof(LaneItem, pts) + sizeof(items[0].pts[0])},
-                {offsetof(LaneItem, valid), offsetof(LaneItem, valid) + 4}, 4};
-    int rc = launch_lanes(d_frames, src, n, height, width, fill_lane, st, device);
-    if (device_ms) cudaEventRecord(e1, st);
-    cudaError_t e = cudaSuccess;
-    if (rc == LANE_OK && !on_device) cudaMemcpyAsync(frames, d_frames, frame_bytes, cudaMemcpyDeviceToHost, st);
-    e = cudaStreamSynchronize(st);
-    if (e == cudaSuccess && rc == LANE_OK && device_ms) cudaEventElapsedTime(device_ms, e0, e1);
+    auto launch = [&](uint8_t *d_frames, uint8_t *) {
+        if (device_ms) { cudaEventCreate(&e0); cudaEventCreate(&e1); cudaEventRecord(e0, st); }
+        cudaMemcpyAsync(c.d, c.h, item_bytes, cudaMemcpyHostToDevice, st);
+        LaneSrc src{(const char *)c.d, sizeof(LaneItem), {offsetof(LaneItem, pts), offsetof(LaneItem, pts) + sizeof(items[0].pts[0])},
+                    {offsetof(LaneItem, valid), offsetof(LaneItem, valid) + 4}, 4};
+        const int rc = launch_lanes(who, d_frames, src, n, height, width, fill_lane, st, device);
+        if (device_ms) cudaEventRecord(e1, st);
+        return rc;
+    };
+    const int rc = draw_frames(who, frames, on_device, (size_t)n * height * width * 3, device, st, false, launch);
+    if (rc == LANE_OK && device_ms) cudaEventElapsedTime(device_ms, e0, e1);
     if (e0) { cudaEventDestroy(e0); cudaEventDestroy(e1); }
-    if (!on_device) cudaFree(d_frames);
-    if (rc == LANE_ERR_UNSUPPORTED) return fail(rc, "lane_draw_lanes_batch: frame too wide for the band mask");
-    if (rc != LANE_OK || e != cudaSuccess) return fail(LANE_ERR_CUDA, cudaGetErrorString(e != cudaSuccess ? e : cudaGetLastError()));
-    return LANE_OK;
+    return rc;
 }
 
 extern "C" int lane_draw_lanes_records(uint8_t *frames_dev, int n, int height, int width, const lane_record *records_dev,
                                        int fill_lane, int device, void *cuda_stream)
 {
-    auto fail = [](int code, const char *msg) { lane_set_global_error(msg); return code; };
-    if (!frames_dev || !records_dev || n < 1 || height < 1 || width < 1) return fail(LANE_ERR_INVALID, "lane_draw_lanes_records: bad arguments");
-    if (height > 32767 || width > 32767) return fail(LANE_ERR_UNSUPPORTED, "lane_draw_lanes_records: frame larger than 32767 px");
-    if (int rc = prepare_device(device)) return rc;
+    constexpr const char *who = "lane_draw_lanes_records";
+    if (!frames_dev || !records_dev || n < 1 || height < 1 || width < 1) return lane_api_fail(LANE_ERR_INVALID, who, "bad arguments");
+    if (height > 32767 || width > 32767) return lane_api_fail(LANE_ERR_UNSUPPORTED, who, "frame larger than 32767 px");
+    if (int rc = lane_api_device(who, device)) return rc;
     LaneSrc src{(const char *)records_dev, sizeof(lane_record),
                 {offsetof(lane_record, side) + offsetof(lane_side, points), offsetof(lane_record, side) + sizeof(lane_side) + offsetof(lane_side, points)},
                 {offsetof(lane_record, side) + offsetof(lane_side, valid), offsetof(lane_record, side) + sizeof(lane_side) + offsetof(lane_side, valid)}, 4};
-    const int rc = launch_lanes(frames_dev, src, n, height, width, fill_lane, (cudaStream_t)cuda_stream, device);
-    if (rc == LANE_ERR_UNSUPPORTED) return fail(rc, "lane_draw_lanes_records: frame too wide for the band mask");
-    if (rc != LANE_OK) return fail(LANE_ERR_CUDA, "k7_lanes launch failed");
-    return LANE_OK;
+    return launch_lanes(who, frames_dev, src, n, height, width, fill_lane, (cudaStream_t)cuda_stream, device);
 }
 
 extern "C" int lane_generate_frames(uint8_t *frames, int on_device, int n, int height, int width, int64_t frame_count0,
                                     int device, void *cuda_stream, float *device_ms)
 {
-    auto fail = [](int code, const char *msg) { lane_set_global_error(msg); return code; };
-    if (!frames || n < 1 || height < 1 || width < 1 || frame_count0 < 0) return fail(LANE_ERR_INVALID, "lane_generate_frames: bad arguments");
-    if (height > 32767 || width > 32767) return fail(LANE_ERR_UNSUPPORTED, "lane_generate_frames: frame larger than 32767 px");
-    if (int rc = prepare_device(device)) return rc;
-    return draw_driver(frames, on_device, n, height, width, device, (cudaStream_t)cuda_stream, device_ms,
+    constexpr const char *who = "lane_generate_frames";
+    if (!frames || n < 1 || height < 1 || width < 1 || frame_count0 < 0) return lane_api_fail(LANE_ERR_INVALID, who, "bad arguments");
+    if (height > 32767 || width > 32767) return lane_api_fail(LANE_ERR_UNSUPPORTED, who, "frame larger than 32767 px");
+    if (int rc = lane_api_device(who, device)) return rc;
+    return draw_driver(who, frames, on_device, n, height, width, device, (cudaStream_t)cuda_stream, device_ms,
                        [&](Builder &b, int f, const char **) {
                            build_generator_frame(b, frame_count0 + f);
                            return true;

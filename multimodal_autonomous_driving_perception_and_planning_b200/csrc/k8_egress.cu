@@ -10,10 +10,7 @@
 // HBM-bound: 3 B/px read + 1.5 B/px written.  The vector kernel converts a 2 x 8 pixel block per thread: three 8-byte
 // loads per BGR row, one 8-byte Y store per row, then four U and four V bytes (I420) or eight interleaved bytes (NV12).
 // The scalar kernel takes one 2x2 block per thread, for any other even width or a misaligned pointer.
-#include <stdio.h>
-
 #include <algorithm>
-#include <mutex>
 
 #include "host_stage.h"
 #include "k0_common.cuh"
@@ -138,14 +135,6 @@ void launch_bgr_to_yuv420(const uint8_t *src, int format, uint8_t *dst, int n, i
         launch_fmt<LANE_INPUT_NV12>(src, dst, n, H, W, st);
 }
 
-int efail(int code, const char *what, cudaError_t e = cudaSuccess)
-{
-    char buf[256];
-    snprintf(buf, sizeof buf, "lane_bgr_to_yuv420_batch: %s%s%s", what, e ? ": " : "", e ? cudaGetErrorString(e) : "");
-    lane_set_global_error(buf);
-    return code;
-}
-
 bool device_memory_on(const void *p, int device)
 {
     cudaPointerAttributes pa{};
@@ -155,114 +144,70 @@ bool device_memory_on(const void *p, int device)
     return ok;
 }
 
-// Host destinations: chunks of CHUNK output bytes are converted into one of two device scratch slots on the caller's
-// stream while the previous chunk is copied out on the copy stream.  One per device, created on first use; the mutex
-// serialises host-destination calls, each of which returns with both slots idle.
-struct Egress {
-    static constexpr size_t CHUNK = (size_t)32 << 20;
-    std::mutex mu;
-    uint8_t *scratch = nullptr;
-    size_t cap = 0;
-    cudaStream_t cs = nullptr;
-    cudaEvent_t converted[2] = {}, copied[2] = {};
-
-    cudaError_t init()
-    {
-        if (cs) return cudaSuccess;
-        cudaError_t e;
-        for (int i = 0; i < 2; i++)
-            if ((e = cudaEventCreateWithFlags(&converted[i], cudaEventDisableTiming)) ||
-                (e = cudaEventCreateWithFlags(&copied[i], cudaEventDisableTiming)))
-                return e;
-        return cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking);
-    }
-    cudaError_t reserve(size_t bytes)
-    {
-        if (cap >= bytes) return cudaSuccess;
-        cudaFree(scratch);
-        scratch = nullptr;
-        cap = 0;
-        cudaError_t e = cudaMalloc((void **)&scratch, bytes);
-        if (!e) cap = bytes;
-        return e;
-    }
-};
-
-Egress *egress_of(int device)         // one per device, lives until exit
-{
-    static std::mutex mu;
-    static Egress *all[64] = {};
-    if (device < 0 || device >= 64) return nullptr;
-    std::lock_guard<std::mutex> lk(mu);
-    if (!all[device]) all[device] = new Egress();
-    return all[device];
-}
-
 }  // namespace
 
 extern "C" int lane_bgr_to_yuv420_batch(const uint8_t *src_dev, int format, int n, int height, int width, uint8_t *dst,
                                         int dst_on_device, int device, void *cuda_stream)
 {
-    if (!src_dev || !dst) return efail(LANE_ERR_INVALID, "null pointer");
+    constexpr const char *who = "lane_bgr_to_yuv420_batch";
+    if (!src_dev || !dst) return lane_api_fail(LANE_ERR_INVALID, who, "null pointer");
     if (format != LANE_INPUT_NV12 && format != LANE_INPUT_I420)
-        return efail(LANE_ERR_INVALID, "format must be LANE_INPUT_NV12 or LANE_INPUT_I420");
-    if (n < 0 || height < 1 || width < 1) return efail(LANE_ERR_INVALID, "bad sizes (n >= 0, positive height and width)");
-    if ((height | width) & 1) return efail(LANE_ERR_INVALID, "YUV 4:2:0 needs even width and height");
+        return lane_api_fail(LANE_ERR_INVALID, who, "format must be LANE_INPUT_NV12 or LANE_INPUT_I420");
+    if (n < 0 || height < 1 || width < 1) return lane_api_fail(LANE_ERR_INVALID, who, "bad sizes (n >= 0, positive height and width)");
+    if ((height | width) & 1) return lane_api_fail(LANE_ERR_INVALID, who, "YUV 4:2:0 needs even width and height");
     // the kernels grid-stride over 64-bit block indices: the only bound on n is that byte offsets stay below 2^62
-    if ((double)n * height * width * 3 > 0x1p62) return efail(LANE_ERR_INVALID, "batch above 2^62 bytes");
+    if ((double)n * height * width * 3 > 0x1p62) return lane_api_fail(LANE_ERR_INVALID, who, "batch above 2^62 bytes");
     if (n == 0) return LANE_OK;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-        return efail(LANE_ERR_NO_DEVICE, "no CUDA device visible: this library has no CPU fallback");
-    if (device < 0 || device >= ndev) return efail(LANE_ERR_INVALID, "device out of range");
-    cudaError_t e;
-    if ((e = cudaSetDevice(device))) return efail(LANE_ERR_CUDA, "cudaSetDevice", e);
+    if (int rc = lane_api_device(who, device)) return rc;
     if (!device_memory_on(src_dev, device))
-        return efail(LANE_ERR_INVALID, "src_dev must be device memory on `device` (host frames: cv2.cvtColor)");
+        return lane_api_fail(LANE_ERR_INVALID, who, "src_dev must be device memory on `device` (host frames: cv2.cvtColor)");
     if (dst_on_device && !device_memory_on(dst, device))
-        return efail(LANE_ERR_INVALID, "dst_on_device = 1 needs device memory on `device`");
+        return lane_api_fail(LANE_ERR_INVALID, who, "dst_on_device = 1 needs device memory on `device`");
     cudaStream_t st = (cudaStream_t)cuda_stream;
+    cudaError_t e;
     if (dst_on_device) {
         launch_bgr_to_yuv420(src_dev, format, dst, n, height, width, st);
-        if ((e = cudaGetLastError())) return efail(LANE_ERR_CUDA, "launch", e);
+        if ((e = cudaGetLastError())) return lane_api_fail(LANE_ERR_CUDA, who, "launch", e);
         return LANE_OK;
     }
 
-    Egress *eg = egress_of(device);
-    if (!eg) return efail(LANE_ERR_INVALID, "device index above 63");
-    std::lock_guard<std::mutex> lk(eg->mu);
-    if ((e = eg->init())) return efail(LANE_ERR_CUDA, "copy stream", e);
+    // Host destinations: chunks of CHUNK output bytes are converted into one of two slots of the device's scratch on the
+    // caller's stream while the previous chunk is copied out on the device's copy stream.
+    constexpr size_t CHUNK = (size_t)32 << 20;
+    LaneDeviceHost &h = lane_device_host(device);
+    std::lock_guard<std::mutex> lk(h.mu);
+    if ((e = h.init_copy_stream())) return lane_api_fail(LANE_ERR_CUDA, who, "copy stream", e);
     const size_t in_frame = (size_t)height * width * 3, out_frame = in_frame / 2;
-    const int chunk = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, Egress::CHUNK / out_frame));
+    const int chunk = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, CHUNK / out_frame));
     const size_t slot_bytes = (size_t)chunk * out_frame;
-    if ((e = eg->reserve(2 * slot_bytes))) return efail(LANE_ERR_CUDA, "scratch allocation", e);
+    if ((e = h.reserve(2 * slot_bytes))) return lane_api_fail(LANE_ERR_CUDA, who, "scratch allocation", e);
     // pinned / registered destinations and small pageable ones take the DMA directly; large pageable ones the ring
-    HostStager *hs = HostStager::pageable(dst, (size_t)n * out_frame) ? lane_host_stager(device) : nullptr;
+    const bool staged = HostStager::pageable(dst, (size_t)n * out_frame);
     const int chunks = (n + chunk - 1) / chunk;
     auto convert = [&](int k) {
         const int slot = k & 1, f0 = k * chunk;
         cudaError_t r;
-        if (k >= 2 && (r = cudaStreamWaitEvent(st, eg->copied[slot], 0))) return r;
-        launch_bgr_to_yuv420(src_dev + (size_t)f0 * in_frame, format, eg->scratch + slot * slot_bytes,
+        if (k >= 2 && (r = cudaStreamWaitEvent(st, h.copied[slot], 0))) return r;
+        launch_bgr_to_yuv420(src_dev + (size_t)f0 * in_frame, format, h.scratch + slot * slot_bytes,
                              std::min(chunk, n - f0), height, width, st);
         if ((r = cudaGetLastError())) return r;
-        return cudaEventRecord(eg->converted[slot], st);
+        return cudaEventRecord(h.converted[slot], st);
     };
     e = convert(0);
     for (int k = 0; !e && k < chunks; k++) {
         const int slot = k & 1, f0 = k * chunk;
         if (k + 1 < chunks && (e = convert(k + 1))) break;
-        if ((e = cudaStreamWaitEvent(eg->cs, eg->converted[slot], 0))) break;
+        if ((e = cudaStreamWaitEvent(h.copy_st, h.converted[slot], 0))) break;
         uint8_t *to = dst + (size_t)f0 * out_frame;
-        const uint8_t *from = eg->scratch + slot * slot_bytes;
+        const uint8_t *from = h.scratch + slot * slot_bytes;
         const size_t nb = (size_t)std::min(chunk, n - f0) * out_frame;
-        e = hs ? hs->d2h(to, from, nb, eg->cs) : cudaMemcpyAsync(to, from, nb, cudaMemcpyDeviceToHost, eg->cs);
-        if (!e) e = cudaEventRecord(eg->copied[slot], eg->cs);
+        e = staged ? h.stager.d2h(to, from, nb, h.copy_st) : cudaMemcpyAsync(to, from, nb, cudaMemcpyDeviceToHost, h.copy_st);
+        if (!e) e = cudaEventRecord(h.copied[slot], h.copy_st);
     }
     // the copy stream waited for every conversion it copied; after a failure the caller's stream may still hold one
-    const cudaError_t s = cudaStreamSynchronize(eg->cs);
+    const cudaError_t s = cudaStreamSynchronize(h.copy_st);
     if (e) cudaStreamSynchronize(st);
     if (!e) e = s;
-    if (e) return efail(LANE_ERR_CUDA, "conversion to host memory", e);
+    if (e) return lane_api_fail(LANE_ERR_CUDA, who, "conversion to host memory", e);
     return LANE_OK;
 }

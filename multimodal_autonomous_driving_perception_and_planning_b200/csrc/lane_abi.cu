@@ -4,10 +4,8 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
-#include <condition_variable>
 #include <mutex>
 #include <string>
-#include <thread>
 #include <vector>
 
 #include "k0_common.cuh"
@@ -19,15 +17,8 @@ void lane_set_global_error(const char *msg) { g_create_error = msg ? msg : ""; }
 
 #include "host_stage.h"
 
-#define LANE_STAGE_SLOTS 3
-#define LANE_STAGE_BYTES ((size_t)32 << 20)
-
 struct lane_ctx {
     int device = 0;
-    CopyPool *pool = nullptr;                          // lazy: first batch of pageable host frames
-    uint8_t *h_stage[LANE_STAGE_SLOTS] = {};           // pinned staging ring
-    cudaEvent_t stage_ev[LANE_STAGE_SLOTS] = {};
-    bool stage_used[LANE_STAGE_SLOTS] = {};
     int max_batch = 0;
     LaneGeom g{};
     LaneHoughParams hp{50, 50, 150};
@@ -173,11 +164,6 @@ void free_all(lane_ctx *c)
         if (e) cudaEventDestroy(e);
     if (c->start_ev) cudaEventDestroy(c->start_ev);
     for (auto &e : c->hb_ev)
-        if (e) cudaEventDestroy(e);
-    delete c->pool;
-    for (auto &p : c->h_stage)
-        if (p) cudaFreeHost(p);
-    for (auto &e : c->stage_ev)
         if (e) cudaEventDestroy(e);
     if (c->copy_st) cudaStreamDestroy(c->copy_st);
     if (c->own_stream && c->st) cudaStreamDestroy(c->st);
@@ -446,21 +432,9 @@ int enqueue(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int
             CU(cudaEventCreateWithFlags(&c->start_ev, cudaEventDisableTiming));
         }
         frames_dev = c->d_frames;
-        // pinned (or registered) host memory goes straight to the copy engine; ordinary memory through the staging ring
-        cudaPointerAttributes pa{};
-        bool pageable = cudaPointerGetAttributes(&pa, frames) != cudaSuccess || pa.type == cudaMemoryTypeUnregistered;
-        cudaGetLastError();
-        // small transfers (a single frame) are quicker through the driver's own path than through worker wake-ups
-        if (bytes * (size_t)n < ((size_t)24 << 20)) pageable = false;
-        if (pageable && !c->pool) {
-            const unsigned hc = std::thread::hardware_concurrency();
-            c->pool = new CopyPool((int)std::max(1u, std::min(8u, hc ? hc / 2 : 4u)));
-            for (int i = 0; i < LANE_STAGE_SLOTS; i++) {
-                CU(cudaHostAlloc((void **)&c->h_stage[i], LANE_STAGE_BYTES, cudaHostAllocDefault));
-                CU(cudaEventCreateWithFlags(&c->stage_ev[i], cudaEventDisableTiming));
-            }
-        }
-        int piece = 0;
+        // pinned (or registered) host memory goes straight to the copy engine; ordinary memory through the device's
+        // staging ring.  Decided once for the whole batch: every chunk of a large pageable batch is staged.
+        HostStager *ring = HostStager::pageable(frames, bytes * (size_t)n) ? &lane_device_host(c->device).stager : nullptr;
         // chunk so that a copy (~50 GB/s) and the compute of the previous chunk overlap; >= 4 chunks when possible
         const int chunk = std::max(1, std::min(64, (n + 3) / 4));
         CU(cudaEventRecord(c->start_ev, c->st));                 // the staging buffer is free once earlier work is done
@@ -468,22 +442,12 @@ int enqueue(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int
         int k = 0;
         for (int off = 0; off < n; off += chunk, k++) {
             const int m = std::min(chunk, n - off);
-            if (!pageable) {
-                CU(cudaMemcpyAsync(d_in + (size_t)off * bytes, frames + (size_t)off * bytes, bytes * m,
-                                   cudaMemcpyHostToDevice, c->copy_st));
-            } else {
-                const size_t total = bytes * m;
-                for (size_t done = 0; done < total; done += LANE_STAGE_BYTES, piece++) {
-                    const int slot = piece % LANE_STAGE_SLOTS;
-                    const size_t nb = std::min(LANE_STAGE_BYTES, total - done);
-                    if (c->stage_used[slot]) CU(cudaEventSynchronize(c->stage_ev[slot]));   // its last DMA has left
-                    c->pool->run(c->h_stage[slot], frames + (size_t)off * bytes + done, nb);
-                    CU(cudaMemcpyAsync(d_in + (size_t)off * bytes + done, c->h_stage[slot], nb, cudaMemcpyHostToDevice,
-                                       c->copy_st));
-                    CU(cudaEventRecord(c->stage_ev[slot], c->copy_st));
-                    c->stage_used[slot] = true;
-                }
-            }
+            uint8_t *to = d_in + (size_t)off * bytes;
+            const uint8_t *from = frames + (size_t)off * bytes;
+            if (ring)
+                CU(ring->h2d(to, from, bytes * m, c->copy_st));
+            else
+                CU(cudaMemcpyAsync(to, from, bytes * m, cudaMemcpyHostToDevice, c->copy_st));
             cudaEvent_t ev = c->copy_ev[k % LANE_COPY_EVENTS];
             CU(cudaEventRecord(ev, c->copy_st));
             CU(cudaStreamWaitEvent(c->st, ev, 0));
@@ -572,7 +536,8 @@ int lane_ctx_create(int device, int height, int width, int max_batch, int max_se
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
         return fail(c, LANE_ERR_NO_DEVICE, "no CUDA device visible: this library has no CPU fallback");
-    if (device < 0 || device >= ndev) return fail(c, LANE_ERR_INVALID, "device %d out of range (%d visible)", device, ndev);
+    if (device < 0 || device >= std::min(ndev, LANE_MAX_DEVICES))
+        return fail(c, LANE_ERR_INVALID, "device %d out of range (%d visible)", device, ndev);
     cudaDeviceProp prop;
     if (cudaGetDeviceProperties(&prop, device) != cudaSuccess || prop.major != 10)
         return fail(c, LANE_ERR_NO_DEVICE, "device %d is sm_%d%d; this build holds sm_100a code only", device, prop.major, prop.minor);

@@ -231,8 +231,7 @@ class SyntheticDataGenerator:
             stream = torch.cuda.current_stream(out.device).cuda_stream
             rc = lib.lane_generate_frames(C.c_void_p(out.data_ptr()), 1, num_frames, self.height, self.width,
                                           int(self.frame_count), out.device.index, C.c_void_p(stream), C.byref(ms))
-        if rc:
-            raise _native.LaneError(rc, (lib.lane_last_error(None) or b"").decode())
+        _native.check_global(rc)
         self.frame_count += num_frames
         return (out, ms.value) if return_ms else out
 

@@ -55,8 +55,7 @@ class FrameIngest:
             dst = np.empty(out_shape, np.uint8)
             rc = lib.lane_resize_batch(src.ctypes.data_as(C.c_void_p), n, sh, sw, cn, dst.ctypes.data_as(C.c_void_p), dh, dw,
                                        0, self._device_index(), None)
-            if rc:
-                raise _native.LaneError(rc, (lib.lane_last_error(None) or b"").decode())
+            _native.check_global(rc)
             return dst
         import torch
         if not frames.is_cuda:
@@ -66,8 +65,7 @@ class FrameIngest:
         stream = torch.cuda.current_stream(src.device).cuda_stream
         rc = lib.lane_resize_batch(C.c_void_p(src.data_ptr()), n, sh, sw, cn, C.c_void_p(dst.data_ptr()), dh, dw, 1,
                                    src.device.index, C.c_void_p(stream))
-        if rc:
-            raise _native.LaneError(rc, (lib.lane_last_error(None) or b"").decode())
+        _native.check_global(rc)
         return dst
 
     def from_nv12(self, frames):
@@ -102,8 +100,7 @@ class FrameIngest:
             stream = torch.cuda.current_stream(src.device).cuda_stream
             rc = lib.lane_yuv420_to_bgr_batch(C.c_void_p(src.data_ptr()), fmt, n, h, w, C.c_void_p(dst.data_ptr()), dh, dw,
                                               1, src.device.index, C.c_void_p(stream))
-        if rc:
-            raise _native.LaneError(rc, (lib.lane_last_error(None) or b"").decode())
+        _native.check_global(rc)
         return dst
 
     def resize(self, frame: np.ndarray) -> np.ndarray:

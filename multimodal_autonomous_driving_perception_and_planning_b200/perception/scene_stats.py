@@ -78,8 +78,7 @@ class SceneStatsAnalyzer:
             src = frames.contiguous()
             stream = torch.cuda.current_stream(src.device).cuda_stream
             rc = lib.lane_frame_stats(C.c_void_p(src.data_ptr()), 1, n, h, w, out, src.device.index, C.c_void_p(stream))
-        if rc:
-            raise _native.LaneError(rc, (lib.lane_last_error(None) or b"").decode())
+        _native.check_global(rc)
         px = h * w
         res = []
         for s in out:

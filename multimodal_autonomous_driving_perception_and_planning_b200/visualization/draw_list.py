@@ -135,6 +135,5 @@ def run_commands(frames, words: np.ndarray, begin: np.ndarray, device: Optional[
         stream = torch.cuda.current_stream(frames.device).cuda_stream
         rc = lib.lane_draw_commands(C.c_void_p(frames.data_ptr()), 1, n, h, w, words.ctypes.data_as(C.c_void_p),
                                     begin.ctypes.data_as(C.c_void_p), frames.device.index, C.c_void_p(stream), C.byref(ms))
-    if rc:
-        raise _native.LaneError(rc, (lib.lane_last_error(None) or b"").decode())
+    _native.check_global(rc)
     return (frames, ms.value) if return_ms else frames

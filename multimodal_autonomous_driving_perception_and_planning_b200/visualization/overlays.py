@@ -92,8 +92,7 @@ def draw_lanes_arrays(frames, left_points, left_valid, right_points, right_valid
         stream = torch.cuda.current_stream(frames.device).cuda_stream
         rc = lib.lane_draw_lanes_batch(C.c_void_p(frames.data_ptr()), 1, n, h, w, *args, frames.device.index,
                                        C.c_void_p(stream), C.byref(ms))
-    if rc:
-        raise _native.LaneError(rc, (lib.lane_last_error(None) or b"").decode())
+    _native.check_global(rc)
     return (frames, ms.value) if return_ms else frames
 
 
@@ -109,8 +108,7 @@ def draw_lanes_records(frames, records_device_ptr: int, fill_lane: bool = True):
     stream = torch.cuda.current_stream(frames.device).cuda_stream
     rc = lib.lane_draw_lanes_records(C.c_void_p(frames.data_ptr()), n, h, w, C.c_void_p(records_device_ptr), int(bool(fill_lane)),
                                      frames.device.index, C.c_void_p(stream))
-    if rc:
-        raise _native.LaneError(rc, (lib.lane_last_error(None) or b"").decode())
+    _native.check_global(rc)
     return frames
 
 

@@ -117,6 +117,5 @@ def _device(frames, out, fmt, who):
     stream = torch.cuda.current_stream(src.device).cuda_stream
     rc = lib.lane_bgr_to_yuv420_batch(C.c_void_p(src.data_ptr()), fmt, n, h, w, C.c_void_p(dst), int(on_device),
                                       src.device.index, C.c_void_p(stream))
-    if rc:
-        raise _native.LaneError(rc, (lib.lane_last_error(None) or b"").decode())
+    _native.check_global(rc)
     return out
