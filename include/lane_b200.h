@@ -84,7 +84,8 @@ LANE_API int lane_abi_version(void);
 
 /* ---- static per-detector inputs ------------------------------------------------------- */
 /* ROI mask produced once on the host by cv2.fillPoly (lane_detector.py:47-64): uint8[height*width],
- * non-zero = inside.  Replaces the per-frame _get_roi_mask/_apply_roi (:86-90). */
+ * non-zero = inside.  Replaces the per-frame _get_roi_mask/_apply_roi (:86-90).  May be called again on a live
+ * context; if such a call fails, detect calls return LANE_ERR_STATE until one succeeds. */
 LANE_API int lane_set_roi_mask(lane_ctx *ctx, const uint8_t *mask);
 /* low/high Canny thresholds for every possible 2*median (index 0..510), filled by evaluating the
  * reference's own float64 expressions (lane_detector.py:80-81). */

@@ -12,6 +12,7 @@
 #include <thread>
 #include <vector>
 
+#include "cuda_owned.h"
 #include "lane_common.cuh"
 
 // Host frames in ordinary (pageable) memory: cudaMemcpy from such memory runs at ~11 GB/s on this platform (the
@@ -162,34 +163,42 @@ struct HostStager {
 struct LaneDeviceHost {
     std::mutex mu;
     HostStager stager;
-    uint8_t *scratch = nullptr;       // grow-only: host round trips, frame statistics' sums, egress's conversion slots
-    size_t cap = 0;
-    cudaStream_t copy_st = nullptr;   // egress to host memory: copies out beside the conversions on the caller's stream
-    cudaEvent_t converted[2] = {}, copied[2] = {};
+    DeviceArray<uint8_t> scratch;     // grow-only: host round trips, frame statistics' sums, egress's conversion slots
+    CudaStream copy_st;               // egress to host memory: copies out beside the conversions on the caller's stream
+    CudaEvent converted[2], copied[2];
+    // Drawing's upload block (primitive lists or lane points), written by the host into write-combined pinned memory and
+    // copied to the device in one piece; grow-only.  Its own lock: a draw call holds it across lane_host_round_trip,
+    // which takes `mu`.
+    std::mutex draw_mu;
+    DeviceArray<uint8_t> draw_d;
+    PinnedArray<uint8_t> draw_h;
 
-    cudaError_t reserve(size_t bytes)
-    {
-        if (cap >= bytes) return cudaSuccess;
-        cudaFree(scratch);
-        scratch = nullptr;
-        cap = 0;
-        cudaError_t e = cudaMalloc((void **)&scratch, bytes);
-        if (!e) cap = bytes;
-        return e;
-    }
     cudaError_t init_copy_stream()
     {
         if (copy_st) return cudaSuccess;
         cudaError_t e;
         for (int i = 0; i < 2; i++)
-            if ((e = cudaEventCreateWithFlags(&converted[i], cudaEventDisableTiming)) ||
-                (e = cudaEventCreateWithFlags(&copied[i], cudaEventDisableTiming)))
-                return e;
-        return cudaStreamCreateWithFlags(&copy_st, cudaStreamNonBlocking);
+            if ((e = converted[i].create(cudaEventDisableTiming)) || (e = copied[i].create(cudaEventDisableTiming))) return e;
+        return copy_st.create(cudaStreamNonBlocking);
+    }
+    // Under draw_mu: `cap` bytes on both sides unless `need` are already there.
+    cudaError_t reserve_draw(size_t need, size_t cap)
+    {
+        if (draw_d.size() >= need) return cudaSuccess;
+        draw_h.reset();
+        cudaError_t e = draw_d.alloc(cap);
+        if (!e) e = draw_h.alloc(cap, cudaHostAllocWriteCombined);
+        if (e) {
+            draw_d.reset();
+            cudaGetLastError();
+        }
+        return e;
     }
 };
 
-inline LaneDeviceHost &lane_device_host(int device)      // device: checked by lane_api_device; created on first use
+// One record per device, created on first use and never destroyed: no CUDA call may run from a static destructor at
+// process exit.
+inline LaneDeviceHost &lane_device_host(int device)      // device: checked by lane_api_device
 {
     static std::mutex mu;
     static LaneDeviceHost *all[LANE_MAX_DEVICES] = {};
@@ -231,7 +240,7 @@ int lane_host_round_trip(const char *who, int device, cudaStream_t st, const voi
     std::lock_guard<std::mutex> lk(h.mu);
     const size_t in_span = in && in != out ? (in_bytes + 255) & ~(size_t)255 : 0;
     cudaError_t e;
-    if ((e = h.reserve(std::max<size_t>(in_span + out_bytes, 1)))) return lane_api_fail(LANE_ERR_CUDA, who, "scratch allocation", e);
+    if ((e = h.scratch.grow(std::max<size_t>(in_span + out_bytes, 1)))) return lane_api_fail(LANE_ERR_CUDA, who, "scratch allocation", e);
     uint8_t *d_in = h.scratch, *d_out = h.scratch + in_span;
     int rc = LANE_OK;
     if (in) {

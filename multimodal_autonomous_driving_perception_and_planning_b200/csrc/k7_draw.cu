@@ -457,14 +457,6 @@ __global__ void __launch_bounds__(DRAW_THREADS) k7_lanes(uint8_t *frames, LaneSr
     }
 }
 
-// grow-only device / pinned staging per device; the entry points are blocking, so one set per device is enough
-struct DrawCache {
-    void *d = nullptr, *h = nullptr;
-    size_t cap = 0;
-};
-std::mutex g_draw_mutex;
-DrawCache g_draw_cache[LANE_MAX_DEVICES];
-
 struct Chunk {
     Builder b;
     int f0 = 0, f1 = 0;
@@ -543,26 +535,15 @@ int draw_driver(const char *who, uint8_t *frames, int on_device, int n, int H, i
     const size_t off_prims = (nb_begin + 63) & ~(size_t)63, off_side = (off_prims + nb_prims + 63) & ~(size_t)63,
                  off_idx = (off_side + nb_side + 63) & ~(size_t)63, total = off_idx + nb_idx;
 
-    std::lock_guard<std::mutex> lk(g_draw_mutex);
-    DrawCache &c = g_draw_cache[device];
-    if (c.cap < total) {
-        if (c.d) cudaFree(c.d);
-        if (c.h) cudaFreeHost(c.h);
-        c = DrawCache{};
-        const size_t cap = std::max(total + total / 2, (size_t)1 << 20);
-        // write-combined: the block is written once, front to back, by up to 16 host threads and then read by the copy
-        // engine only.  (Measured on the B200 box: the upload that follows the fill runs at ~11 GB/s with write-combined
-        // and with ordinary pinned memory alike, a repeated upload of the same block at 46 GB/s -- the hand-over from the
-        // CPU's writes to the DMA reads is what costs, 2 ms per 22 MB; LANE_B200_DRAW_DEBUG=1 prints it.)
-        if (cudaMalloc(&c.d, cap) != cudaSuccess || cudaHostAlloc(&c.h, cap, cudaHostAllocWriteCombined) != cudaSuccess) {
-            if (c.d) cudaFree(c.d);
-            c = DrawCache{};
-            cudaGetLastError();
-            return lane_api_fail(LANE_ERR_CUDA, who, "staging allocation failed");
-        }
-        c.cap = cap;
-    }
-    uint8_t *h = (uint8_t *)c.h, *d = (uint8_t *)c.d;
+    LaneDeviceHost &dh = lane_device_host(device);
+    std::lock_guard<std::mutex> lk(dh.draw_mu);
+    // write-combined: the block is written once, front to back, by up to 16 host threads and then read by the copy
+    // engine only.  (Measured on the B200 box: the upload that follows the fill runs at ~11 GB/s with write-combined
+    // and with ordinary pinned memory alike, a repeated upload of the same block at 46 GB/s -- the hand-over from the
+    // CPU's writes to the DMA reads is what costs, 2 ms per 22 MB; LANE_B200_DRAW_DEBUG=1 prints it.)
+    if (dh.reserve_draw(total, std::max(total + total / 2, (size_t)1 << 20)))
+        return lane_api_fail(LANE_ERR_CUDA, who, "staging allocation failed");
+    uint8_t *h = dh.draw_h, *d = dh.draw_d;
     memcpy(h, band_begin.data(), nb_begin);
     for_chunks([&](Chunk &ck) {
         Prim *hp = (Prim *)(h + off_prims) + ck.prim_base;
@@ -586,13 +567,13 @@ int draw_driver(const char *who, uint8_t *frames, int on_device, int n, int H, i
         if (!local.empty()) memcpy(hi + idx0, local.data(), local.size() * 4);
     });
 
-    cudaEvent_t e0 = nullptr, e1 = nullptr, ec = nullptr;
+    CudaEvent e0, e1, ec;
     static const bool dbg = getenv("LANE_B200_DRAW_DEBUG") != nullptr;
     auto launch = [&](uint8_t *d_frames, uint8_t *) {
-        if (device_ms) { cudaEventCreate(&e0); cudaEventCreate(&e1); cudaEventRecord(e0, st); }
+        if (device_ms) { e0.create(); e1.create(); cudaEventRecord(e0, st); }
         if (clear_first) cudaMemsetAsync(d_frames, 0, (size_t)n * H * W * 3, st);
         cudaMemcpyAsync(d, h, total, cudaMemcpyHostToDevice, st);
-        if (dbg && device_ms) { cudaEventCreate(&ec); cudaEventRecord(ec, st); }
+        if (dbg && device_ms) { ec.create(); cudaEventRecord(ec, st); }
         const int WW = (W + 31) >> 5;
         const size_t mask_words = (size_t)BAND_ROWS * WW;
         const size_t smem = (mask_words + (mask_words & 1)) * 4 + (size_t)(DRAW_THREADS / 32) * MAX_ROW_EDGES * 8;
@@ -615,9 +596,7 @@ int draw_driver(const char *who, uint8_t *frames, int on_device, int n, int H, i
         if (rc == LANE_OK) cudaEventElapsedTime(&cms, e0, ec);
         fprintf(stderr, "lane_draw: %lld primitives, %lld band entries, %.2f MB uploaded in %.3f ms, upload + kernel %.3f ms, %d host threads\n",
                 (long long)n_prims, (long long)n_idx, total / 1e6, cms, device_ms ? *device_ms : 0.f, T);
-        cudaEventDestroy(ec);
     }
-    if (e0) { cudaEventDestroy(e0); cudaEventDestroy(e1); }
     return rc;
 }
 
@@ -692,33 +671,23 @@ extern "C" int lane_draw_lanes_batch(uint8_t *frames, int on_device, int n, int 
                            });
     // default: the geometry runs on the device (k7_lanes); only the 100 points per frame are uploaded
     const size_t item_bytes = (size_t)n * sizeof(LaneItem);
-    std::lock_guard<std::mutex> lk(g_draw_mutex);
-    DrawCache &c = g_draw_cache[device];
-    if (c.cap < item_bytes) {
-        if (c.d) cudaFree(c.d);
-        if (c.h) cudaFreeHost(c.h);
-        c = DrawCache{};
-        const size_t cap = std::max(item_bytes * 2, (size_t)1 << 20);
-        if (cudaMalloc(&c.d, cap) != cudaSuccess || cudaHostAlloc(&c.h, cap, cudaHostAllocWriteCombined) != cudaSuccess) {
-            if (c.d) cudaFree(c.d);
-            c = DrawCache{};
-            cudaGetLastError();
-            return lane_api_fail(LANE_ERR_CUDA, who, "staging allocation failed");
-        }
-        c.cap = cap;
-    }
-    LaneItem *items = (LaneItem *)c.h;
+    LaneDeviceHost &dh = lane_device_host(device);
+    std::lock_guard<std::mutex> lk(dh.draw_mu);
+    if (dh.reserve_draw(item_bytes, std::max(item_bytes * 2, (size_t)1 << 20)))
+        return lane_api_fail(LANE_ERR_CUDA, who, "staging allocation failed");
+    uint8_t *h = dh.draw_h, *d = dh.draw_d;
+    LaneItem *items = (LaneItem *)h;
     for (int f = 0; f < n; f++) {
         memcpy(items[f].pts[0], left_points + (size_t)f * LANE_PTS * 2, sizeof(items[f].pts[0]));
         memcpy(items[f].pts[1], right_points + (size_t)f * LANE_PTS * 2, sizeof(items[f].pts[1]));
         items[f].valid[0] = left_valid[f] != 0;
         items[f].valid[1] = right_valid[f] != 0;
     }
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    CudaEvent e0, e1;
     auto launch = [&](uint8_t *d_frames, uint8_t *) {
-        if (device_ms) { cudaEventCreate(&e0); cudaEventCreate(&e1); cudaEventRecord(e0, st); }
-        cudaMemcpyAsync(c.d, c.h, item_bytes, cudaMemcpyHostToDevice, st);
-        LaneSrc src{(const char *)c.d, sizeof(LaneItem), {offsetof(LaneItem, pts), offsetof(LaneItem, pts) + sizeof(items[0].pts[0])},
+        if (device_ms) { e0.create(); e1.create(); cudaEventRecord(e0, st); }
+        cudaMemcpyAsync(d, h, item_bytes, cudaMemcpyHostToDevice, st);
+        LaneSrc src{(const char *)d, sizeof(LaneItem), {offsetof(LaneItem, pts), offsetof(LaneItem, pts) + sizeof(items[0].pts[0])},
                     {offsetof(LaneItem, valid), offsetof(LaneItem, valid) + 4}, 4};
         const int rc = launch_lanes(who, d_frames, src, n, height, width, fill_lane, st, device);
         if (device_ms) cudaEventRecord(e1, st);
@@ -726,7 +695,6 @@ extern "C" int lane_draw_lanes_batch(uint8_t *frames, int on_device, int n, int 
     };
     const int rc = draw_frames(who, frames, on_device, (size_t)n * height * width * 3, device, st, false, launch);
     if (rc == LANE_OK && device_ms) cudaEventElapsedTime(device_ms, e0, e1);
-    if (e0) { cudaEventDestroy(e0); cudaEventDestroy(e1); }
     return rc;
 }
 

@@ -180,7 +180,7 @@ extern "C" int lane_bgr_to_yuv420_batch(const uint8_t *src_dev, int format, int 
     const size_t in_frame = (size_t)height * width * 3, out_frame = in_frame / 2;
     const int chunk = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, CHUNK / out_frame));
     const size_t slot_bytes = (size_t)chunk * out_frame;
-    if ((e = h.reserve(2 * slot_bytes))) return lane_api_fail(LANE_ERR_CUDA, who, "scratch allocation", e);
+    if ((e = h.scratch.grow(2 * slot_bytes))) return lane_api_fail(LANE_ERR_CUDA, who, "scratch allocation", e);
     // pinned / registered destinations and small pageable ones take the DMA directly; large pageable ones the ring
     const bool staged = HostStager::pageable(dst, (size_t)n * out_frame);
     const int chunks = (n + chunk - 1) / chunk;

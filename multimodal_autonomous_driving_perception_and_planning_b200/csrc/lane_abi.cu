@@ -4,10 +4,12 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <vector>
 
+#include "cuda_owned.h"
 #include "k0_common.cuh"
 
 #define LANE_COPY_EVENTS 8
@@ -24,81 +26,77 @@ struct lane_ctx {
     LaneHoughParams hp{50, 50, 150};
     double smooth = 0.7, one_minus_smooth = 1 - 0.7;
     bool have_roi = false, have_lut = false, debug = false, profiling = false;
-    bool own_stream = true;
     int blur = 1;                     // 0: Canny runs on the plain grayscale plane (lane_set_preprocess)
-    cudaStream_t st = nullptr, copy_st = nullptr;   // compute stream; H2D stream for chunked host batches
+    CudaStream st, copy_st;           // compute stream (or the caller's, lane_ctx_set_stream); H2D stream for chunked host batches
     // Second compute stream for the back half of the path (PPHT + fit + record copies) of device-resident batches: the
     // PPHT kernel runs in waves of whole frames (71 clusters at 1080p) and its last wave leaves 40 % of the SMs idle for a
     // frame's latency; with the edge kernels of the NEXT queued batch on the first stream those SMs are used.  The buffers
     // that cross from the edge half to the back half are kept per result slot (see `two`).
-    cudaStream_t st2 = nullptr;
-    cudaEvent_t edge_done[2] = {};
+    CudaStream st2;
+    CudaEvent edge_done[2];
     bool overlap_now = false;                       // the batch being enqueued runs its back half on st2
-    cudaEvent_t copy_ev[LANE_COPY_EVENTS] = {}, start_ev = nullptr;
+    CudaEvent copy_ev[LANE_COPY_EVENTS], start_ev;
     std::string err;
 
     // device buffers
-    uint8_t *d_frames = nullptr;      // staging for host frames / BGR output of the ingest kernels (lazy)
-    uint8_t *d_src = nullptr;         // staging for host frames the ingest kernels convert / resize (lazy, grows)
-    size_t src_cap = 0;               // its size in bytes
-    uint8_t *d_blur = nullptr;        // blurred plane: unfused path and verification taps only (lazy)
-    uint32_t *d_kbits = nullptr;      // [B][H][WW] NMS survivors of the fused edge kernel
-    uint8_t *d_vplane = nullptr;      // [B][H][W]  their magnitudes (sparse: only survivors' bytes are ever written / read)
-    int *d_pre = nullptr;             // [B] magnitude floor per frame | [B] floor of the redo pass | [B] redo list | count
-    uint32_t *d_roi_bits = nullptr;   // [H][WW] bit-plane of the ROI mask
-    uint32_t *d_pmask_bits = nullptr; // [B][bh][WW] ROI-masked edges (the HoughLinesP mask)
-    uint32_t *d_edge_bits = nullptr;  // [B][H][WW] Canny map
-    uint32_t *d_dbg_c = nullptr, *d_dbg_s = nullptr;   // [B][H][WW] candidate / strong planes before hysteresis
+    DeviceArray<uint8_t> d_frames;    // staging for host frames / BGR output of the ingest kernels (lazy)
+    DeviceArray<uint8_t> d_src;       // staging for host frames the ingest kernels convert / resize (lazy, grows)
+    DeviceArray<uint8_t> d_blur;      // blurred plane: unfused path and verification taps only (lazy)
+    DeviceArray<uint32_t> d_kbits;    // [B][H][WW] NMS survivors of the fused edge kernel
+    DeviceArray<uint8_t> d_vplane;    // [B][H][W]  their magnitudes (sparse: only survivors' bytes are ever written / read)
+    DeviceArray<int> d_pre;           // [B] magnitude floor per frame | [B] floor of the redo pass | [B] redo list | count
+    DeviceArray<uint32_t> d_roi_bits;     // [H][WW] bit-plane of the ROI mask
+    DeviceArray<uint32_t> d_pmask_bits;   // [B][bh][WW] ROI-masked edges (the HoughLinesP mask)
+    DeviceArray<uint32_t> d_edge_bits;    // [B][H][WW] Canny map
+    DeviceArray<uint32_t> d_cand_bits, d_strong_bits;   // [B][H][WW] candidate / strong planes before hysteresis
     // generic-width fallback (byte maps), allocated on first use
-    uint8_t *d_cls = nullptr, *d_cls_dbg = nullptr, *d_roi = nullptr, *d_pmask = nullptr;
-    uint8_t *h_roi = nullptr;
+    DeviceArray<uint8_t> d_cls, d_cls_dbg, d_roi, d_pmask;
+    std::vector<uint8_t> h_roi;
     bool fallback_ready = false, last_cluster = false;
     int last_paths = 0;               // LANE_PATH_* of the chunk that ran last
-    uint8_t *d_gray_dbg = nullptr;
-    uint32_t *d_hist = nullptr, *d_points = nullptr, *d_points_dbg = nullptr;
-    uint8_t *d_lut = nullptr;         // low[511] | high[511]
-    int4 *d_thr = nullptr;
-    int *d_seedsA = nullptr, *d_seedsB = nullptr, *d_seed_count = nullptr;
+    DeviceArray<uint8_t> d_gray_dbg;
+    DeviceArray<uint32_t> d_hist, d_points, d_points_dbg;
+    DeviceArray<uint8_t> d_lut;       // low[511] | high[511]
+    DeviceArray<int4> d_thr;
+    DeviceArray<int> d_seedsA, d_seedsB, d_seed_count;
     int seed_cap = 0;
-    int *d_n_edges = nullptr, *d_n_points = nullptr, *d_rounds = nullptr, *d_n_lines = nullptr;
-    int32_t *d_lines = nullptr;
-    uint32_t *d_accum16 = nullptr;    // [B][cells_per_frame] biased 16-bit cells, two per word
-    int2 *d_win = nullptr;            // [180] (rmin, first cell) per angle
+    DeviceArray<int> d_n_edges, d_n_points, d_rounds, d_n_lines;
+    DeviceArray<int32_t> d_lines;
+    DeviceArray<uint32_t> d_accum16;  // [B][cells_per_frame] biased 16-bit cells, two per word
+    DeviceArray<int2> d_win;          // [180] (rmin, first cell) per angle
     int cells_per_frame = 0;
     int ppht_v2 = 0;                  // LANE_B200_K4=v2 pins the global-memory PPHT kernel (tests)
-    int *d_order = nullptr;           // [B] frames with the most points first (v3 launch order)
-    int2 *d_win3 = nullptr;           // v3 layout: (rmin, first cell inside the owning CTA)
-    uint32_t *d_pmask_work = nullptr; // [B][G3][bh][WW] private mask copies of the v3 cluster CTAs
-    uint32_t *d_list_over = nullptr;  // [B][G3][over_cap] private extensions of the v3 point list (ROIs with many pixels)
+    DeviceArray<int> d_order;         // [B] frames with the most points first (v3 launch order)
+    DeviceArray<int2> d_win3;         // v3 layout: (rmin, first cell inside the owning CTA)
+    DeviceArray<uint32_t> d_pmask_work;   // [B][G3][bh][WW] private mask copies of the v3 cluster CTAs
+    DeviceArray<uint32_t> d_list_over;    // [B][G3][over_cap] private extensions of the v3 point list (ROIs with many pixels)
     int G3 = 0, cells_max3 = 0, list_cap3 = 0, over_cap3 = 0;   // v3 plan: cluster size, cells / shared list entries per CTA, list extension
-    LaneFitScratch fit{};
-    int *d_stream_id = nullptr;
-    double *d_prev_fit = nullptr;
-    uint8_t *d_prev_valid = nullptr;
+    DeviceArray<double> d_fit_raw, d_fit_big;             // LaneFitScratch
+    DeviceArray<int> d_fit_side_n, d_fit_side_flags;
+    DeviceArray<int> d_stream_id;
+    DeviceArray<double> d_prev_fit;
+    DeviceArray<uint8_t> d_prev_valid;
     int stream_cap = 0;
-    int32_t *d_std_accum = nullptr;
+    DeviceArray<int32_t> d_std_accum;
     // batched standard Hough (lane_hough_lines_batch), allocated on first use
-    int32_t *d_hb_accum = nullptr, *d_hb_sorted = nullptr;
-    int2 *d_hb_tmp = nullptr;
-    int *d_hb_count = nullptr;
-    int hb_cap = 0;
-    bool hb_accum_ready = false;
-    cudaEvent_t hb_ev[2] = {};
-    int2 *d_peaks = nullptr;
-    int *d_n_peaks = nullptr;
-    int *d_task_counter = nullptr;
-    int peaks_cap = 0;
+    DeviceArray<int32_t> d_hb_accum, d_hb_sorted;
+    DeviceArray<int2> d_hb_tmp;
+    DeviceArray<int> d_hb_count;
+    CudaEvent hb_ev[2];
+    DeviceArray<int2> d_peaks;
+    DeviceArray<int> d_n_peaks;
+    DeviceArray<int> d_task_counter;
 
     // Up to two batches may be in flight on the context's stream (enqueue, enqueue, collect, enqueue, collect ...): the
     // device never waits for the host between them.  Each has its own pinned result buffers and timing events.
     struct slot_t {
-        lane_record *h_records = nullptr;            // pinned
-        lane_record *d_records = nullptr;            // device copy, alive until this slot is enqueued again
-        double *h_prev_fit = nullptr;                // pinned: state in (explicit mode) and state out
-        uint8_t *h_prev_valid = nullptr;
-        cudaEvent_t ev[LANE_NUM_STAGES + 1] = {};
-        cudaEvent_t done = nullptr;
-        cudaEvent_t reader_done = nullptr;           // lane_ctx_fence_records: an outside reader of d_records ends here
+        PinnedArray<lane_record> h_records;
+        DeviceArray<lane_record> d_records;          // alive until this slot is enqueued again
+        PinnedArray<double> h_prev_fit;              // state in (explicit mode) and state out
+        PinnedArray<uint8_t> h_prev_valid;
+        CudaEvent ev[LANE_NUM_STAGES + 1];
+        CudaEvent done;
+        CudaEvent reader_done;                       // lane_ctx_fence_records: an outside reader of d_records ends here
         bool has_reader = false;
         int n = 0, S = 0;
         bool timed = false;
@@ -110,6 +108,20 @@ struct lane_ctx {
     const uint8_t *last_frames_dev = nullptr;
     float stage_ms[LANE_NUM_STAGES] = {};            // of the batch collected last
     int32_t stage_launches[LANE_NUM_STAGES] = {};
+
+    // Waits for all work on the context's streams: what they may still read or write can then be released.
+    cudaError_t sync() const
+    {
+        cudaError_t e = cudaStreamSynchronize(st);
+        if (!e && st2) e = cudaStreamSynchronize(st2);
+        if (!e && copy_st) e = cudaStreamSynchronize(copy_st);
+        return e;
+    }
+    ~lane_ctx()                                      // the members release their resources after this
+    {
+        cudaSetDevice(device);
+        sync();
+    }
 };
 
 namespace {
@@ -133,58 +145,14 @@ int fail(lane_ctx *c, int code, const char *fmt, ...)
                         __FILE__, __LINE__);                                                       \
     } while (0)
 
-template <typename T>
-cudaError_t dalloc(T **p, size_t count)
-{
-    return cudaMalloc((void **)p, std::max<size_t>(count, 1) * sizeof(T) + 64);
-}
-
-void free_all(lane_ctx *c)
-{
-    cudaSetDevice(c->device);
-    void *ptrs[] = {c->d_frames, c->d_src, c->d_blur, c->d_kbits, c->d_vplane, c->d_pre, c->d_cls, c->d_cls_dbg, c->d_roi, c->d_pmask, c->d_gray_dbg, c->d_hist,
-                    c->d_roi_bits, c->d_pmask_bits, c->d_edge_bits, c->d_dbg_c, c->d_dbg_s, c->d_accum16, c->d_win, c->d_win3, c->d_pmask_work, c->d_list_over,
-                    c->d_points, c->d_points_dbg, c->d_lut, c->d_thr, c->d_seedsA, c->d_seedsB, c->d_seed_count,
-                    c->d_n_edges, c->d_n_points, c->d_rounds, c->d_n_lines, c->d_lines, c->fit.raw, c->fit.big,
-                    c->fit.side_n, c->fit.side_flags, c->d_stream_id, c->d_prev_fit, c->d_prev_valid,
-                    c->slots[0].d_records, c->slots[1].d_records, c->d_std_accum, c->d_hb_accum, c->d_hb_sorted, c->d_hb_tmp, c->d_hb_count, c->d_peaks, c->d_n_peaks, c->d_task_counter, c->d_order};
-    for (void *p : ptrs)
-        if (p) cudaFree(p);
-    free(c->h_roi);
-    for (auto &sl : c->slots) {
-        if (sl.h_records) cudaFreeHost(sl.h_records);
-        if (sl.h_prev_fit) cudaFreeHost(sl.h_prev_fit);
-        if (sl.h_prev_valid) cudaFreeHost(sl.h_prev_valid);
-        for (auto &e : sl.ev)
-            if (e) cudaEventDestroy(e);
-        if (sl.done) cudaEventDestroy(sl.done);
-        if (sl.reader_done) cudaEventDestroy(sl.reader_done);
-    }
-    for (auto &e : c->copy_ev)
-        if (e) cudaEventDestroy(e);
-    if (c->start_ev) cudaEventDestroy(c->start_ev);
-    for (auto &e : c->hb_ev)
-        if (e) cudaEventDestroy(e);
-    if (c->copy_st) cudaStreamDestroy(c->copy_st);
-    if (c->own_stream && c->st) cudaStreamDestroy(c->st);
-    if (c->st2) cudaStreamDestroy(c->st2);
-    for (auto &e : c->edge_done) if (e) cudaEventDestroy(e);
-}
-
 int ensure_streams(lane_ctx *c, int S)
 {
     if (S <= c->stream_cap) return LANE_OK;
-    if (c->d_prev_fit) cudaFree(c->d_prev_fit);
-    if (c->d_prev_valid) cudaFree(c->d_prev_valid);
-    c->d_prev_fit = nullptr; c->d_prev_valid = nullptr;
-    CU(dalloc(&c->d_prev_fit, (size_t)S * 6));
-    CU(dalloc(&c->d_prev_valid, (size_t)S * 2));
+    CU(c->d_prev_fit.grow((size_t)S * 6));
+    CU(c->d_prev_valid.grow((size_t)S * 2));
     for (auto &sl : c->slots) {
-        if (sl.h_prev_fit) cudaFreeHost(sl.h_prev_fit);
-        if (sl.h_prev_valid) cudaFreeHost(sl.h_prev_valid);
-        sl.h_prev_fit = nullptr; sl.h_prev_valid = nullptr;
-        CU(cudaMallocHost((void **)&sl.h_prev_fit, sizeof(double) * S * 6));
-        CU(cudaMallocHost((void **)&sl.h_prev_valid, (size_t)S * 2));
+        CU(sl.h_prev_fit.alloc((size_t)S * 6));
+        CU(sl.h_prev_valid.alloc((size_t)S * 2));
     }
     c->state_on_device = false;
     c->stream_cap = S;
@@ -196,23 +164,8 @@ int ensure_streams(lane_ctx *c, int S)
 int ensure_src(lane_ctx *c, size_t frame_bytes)
 {
     const size_t need = (size_t)c->max_batch * frame_bytes;
-    if (need <= c->src_cap) return LANE_OK;
-    if (c->d_src) {
-        CU(cudaStreamSynchronize(c->st));
-        if (c->st2) CU(cudaStreamSynchronize(c->st2));
-        if (c->copy_st) CU(cudaStreamSynchronize(c->copy_st));
-        CU(cudaFree(c->d_src));
-        c->d_src = nullptr;
-        c->src_cap = 0;
-    }
-    CU(dalloc(&c->d_src, need));
-    c->src_cap = need;
-    return LANE_OK;
-}
-
-int ensure_blur(lane_ctx *c)
-{
-    if (!c->d_blur) CU(dalloc(&c->d_blur, (size_t)c->max_batch * c->g.H * c->g.W));
+    if (c->d_src && need > c->d_src.size()) CU(c->sync());
+    CU(c->d_src.grow(need));
     return LANE_OK;
 }
 
@@ -221,14 +174,14 @@ int ensure_fallback(lane_ctx *c)
 {
     if (c->fallback_ready) return LANE_OK;
     const size_t P = (size_t)c->g.H * c->g.W, B = (size_t)c->max_batch;
-    CU(dalloc(&c->d_cls, B * P));
-    if (c->debug) CU(dalloc(&c->d_cls_dbg, B * P));
-    CU(dalloc(&c->d_roi, P));
-    CU(dalloc(&c->d_pmask, B * std::max(c->g.bw * c->g.bh, 1)));
-    CU(dalloc(&c->d_seedsA, B * c->seed_cap));
-    CU(dalloc(&c->d_seedsB, B * c->seed_cap));
-    CU(dalloc(&c->d_seed_count, B));
-    CU(cudaMemcpyAsync(c->d_roi, c->h_roi, P, cudaMemcpyHostToDevice, c->st));
+    CU(c->d_cls.alloc(B * P));
+    if (c->debug) CU(c->d_cls_dbg.alloc(B * P));
+    CU(c->d_roi.alloc(P));
+    CU(c->d_pmask.alloc(B * std::max(c->g.bw * c->g.bh, 1)));
+    CU(c->d_seedsA.alloc(B * c->seed_cap));
+    CU(c->d_seedsB.alloc(B * c->seed_cap));
+    CU(c->d_seed_count.alloc(B));
+    CU(cudaMemcpyAsync(c->d_roi, c->h_roi.data(), P, cudaMemcpyHostToDevice, c->st));
     c->fallback_ready = true;
     return LANE_OK;
 }
@@ -267,7 +220,7 @@ int run_stages(lane_ctx *c, const uint8_t *frames_dev, int off, int m, const int
     int *n_edges = c->d_n_edges + two, *n_points = c->d_n_points + two, *rounds = c->d_rounds + two, *n_lines = c->d_n_lines + o;
     uint32_t *points = c->d_points + two * g.max_points;
     uint32_t *pmask_bits = c->d_pmask_bits + two * std::max(g.bh, 1) * WW;
-    uint32_t *edge_bits = c->d_edge_bits + o * planes, *cb = c->d_dbg_c + o * planes, *sb = c->d_dbg_s + o * planes;
+    uint32_t *edge_bits = c->d_edge_bits + o * planes, *cb = c->d_cand_bits + o * planes, *sb = c->d_strong_bits + o * planes;
     int32_t *lines = c->d_lines + o * g.max_segments * 4;
 
     if (timed) { rc = mark(c, LANE_STAGE_BLUR_HIST); if (rc) return rc; }
@@ -276,12 +229,10 @@ int run_stages(lane_ctx *c, const uint8_t *frames_dev, int off, int m, const int
     bool fused = false;
     c->last_cluster = false;
     if (c->blur && lane_fused_edge_supported(H, W, fr)) {
-        if (!c->d_kbits) {
-            CU(dalloc(&c->d_kbits, (size_t)c->max_batch * planes));
-            CU(dalloc(&c->d_vplane, (size_t)c->max_batch * P));
-            CU(dalloc(&c->d_pre, (size_t)c->max_batch * 5 + 4));
-        }
-        if (c->debug) { rc = ensure_blur(c); if (rc) return rc; }
+        CU(c->d_kbits.lazy((size_t)c->max_batch * planes));
+        CU(c->d_vplane.lazy((size_t)c->max_batch * P));
+        CU(c->d_pre.lazy((size_t)c->max_batch * 5 + 4));
+        if (c->debug) CU(c->d_blur.lazy((size_t)c->max_batch * P));
         const size_t B = (size_t)c->max_batch;
         int *pre = c->d_pre + o, *pre_redo = c->d_pre + B + o, *redo_list = c->d_pre + 2 * B + o, *redo_flag = c->d_pre + 3 * B + o,
             *frame_done = c->d_pre + 4 * B + o, *redo_count = c->d_pre + 5 * B;
@@ -313,7 +264,7 @@ int run_stages(lane_ctx *c, const uint8_t *frames_dev, int off, int m, const int
     }
     c->last_paths = fused ? LANE_PATH_FUSED_EDGE : 0;
     if (!fused) {
-        rc = ensure_blur(c); if (rc) return rc;
+        CU(c->d_blur.lazy((size_t)c->max_batch * P));
         uint8_t *blur = c->d_blur + o * P;
         if (timed) { rc = mark(c, LANE_STAGE_BLUR_HIST); if (rc) return rc; }
         launch_blur_hist(fr, blur, hist, m, H, W, c->st, &L[LANE_STAGE_BLUR_HIST], c->blur);
@@ -369,8 +320,8 @@ int run_stages(lane_ctx *c, const uint8_t *frames_dev, int off, int m, const int
         CU(cudaStreamWaitEvent(hs, c->slots[c->cur].reader_done, 0));
         c->slots[c->cur].has_reader = false;
     }
-    LaneFitScratch fs{c->fit.raw + o * 6, c->fit.side_n + o * 2, c->fit.side_flags + o,
-                      c->fit.big ? c->fit.big + o * 2 * 5 * 2 * (size_t)g.max_segments : nullptr};
+    LaneFitScratch fs{c->d_fit_raw + o * 6, c->d_fit_side_n + o * 2, c->d_fit_side_flags + o,
+                      c->d_fit_big ? c->d_fit_big + o * 2 * 5 * 2 * (size_t)g.max_segments : nullptr};
     launch_fit(lines, n_lines, fs, stream_id_dev ? stream_id_dev + o : nullptr, S, c->d_prev_fit, c->d_prev_valid, c->smooth,
                c->one_minus_smooth, thr, n_edges, n_points, rounds, c->slots[c->cur].d_records + o, g, m, hs, &L[LANE_STAGE_FIT]);
     return stage_check(c, "fit");
@@ -407,11 +358,11 @@ int enqueue(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int
         CU(cudaMemcpyAsync(c->d_prev_fit, sl.h_prev_fit, sizeof(double) * S * 6, cudaMemcpyHostToDevice, hs));
         CU(cudaMemcpyAsync(c->d_prev_valid, sl.h_prev_valid, (size_t)S * 2, cudaMemcpyHostToDevice, hs));
     }
-    const int32_t *sid = stream_id ? c->d_stream_id : nullptr;
+    const int32_t *sid = stream_id ? c->d_stream_id.get() : nullptr;
     const uint8_t *frames_dev = frames;
     const size_t bgr_bytes = (size_t)c->g.H * c->g.W * 3;
     const bool convert = in.format != LANE_INPUT_BGR || in.h != c->g.H || in.w != c->g.W;
-    if (convert && !c->d_frames) CU(dalloc(&c->d_frames, (size_t)c->max_batch * bgr_bytes));
+    if (convert) CU(c->d_frames.lazy((size_t)c->max_batch * bgr_bytes));
     if (on_device) {
         if (convert) {                               // source already on the device: one ingest launch, then the usual path
             CU(launch_ingest(frames, in.format, n, in.h, in.w, c->d_frames, c->g.H, c->g.W, c->st));
@@ -423,13 +374,13 @@ int enqueue(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int
         // bytes per frame that cross PCIe: the source's own (3 B/px BGR, 1.5 B/px YUV 4:2:0 at the decoder's size),
         // converted / resized on the device chunk by chunk
         const size_t bytes = in.frame_bytes();
-        if (!c->d_frames) CU(dalloc(&c->d_frames, (size_t)c->max_batch * bgr_bytes));
+        CU(c->d_frames.lazy((size_t)c->max_batch * bgr_bytes));
         if (convert) { rc = ensure_src(c, bytes); if (rc) return rc; }
         uint8_t *d_in = convert ? c->d_src : c->d_frames;
         if (!c->copy_st) {
-            CU(cudaStreamCreateWithFlags(&c->copy_st, cudaStreamNonBlocking));
-            for (auto &e : c->copy_ev) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-            CU(cudaEventCreateWithFlags(&c->start_ev, cudaEventDisableTiming));
+            for (auto &e : c->copy_ev) CU(e.create(cudaEventDisableTiming));
+            CU(c->start_ev.create(cudaEventDisableTiming));
+            CU(c->copy_st.create(cudaStreamNonBlocking));
         }
         frames_dev = c->d_frames;
         // pinned (or registered) host memory goes straight to the copy engine; ordinary memory through the device's
@@ -474,7 +425,9 @@ int enqueue(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int
     return LANE_OK;
 }
 
-int check_call(lane_ctx *c, const void *frames, int n, int S, const void *pf, const void *pv)
+// What every detect call checks and sets up before it enqueues: arguments and context state, the context's device, the
+// stream state buffers, the batch's result slot and, when profiling, the mark where the batch starts.
+int check_call(lane_ctx *c, const void *frames, int n, const int32_t *stream_id, int S, const void *pf, const void *pv)
 {
     if (!c) return LANE_ERR_INVALID;
     if (!frames || n <= 0 || n > c->max_batch) return fail(c, LANE_ERR_INVALID, "bad batch: n=%d (max_batch=%d)", n, c->max_batch);
@@ -487,12 +440,18 @@ int check_call(lane_ctx *c, const void *frames, int n, int S, const void *pf, co
         if (!c->state_on_device || S > c->stream_cap)
             return fail(c, LANE_ERR_STATE, "no state on the device for %d streams: pass prev_fit / prev_valid once", S);
     }
-    {
-        int rc = c->q_count ? LANE_OK : ensure_streams(c, S);
+    if (stream_id)
+        for (int i = 0; i < n; i++)
+            if (stream_id[i] < 0 || stream_id[i] >= S)
+                return fail(c, LANE_ERR_INVALID, "stream_id[%d]=%d outside [0,%d)", i, stream_id[i], S);
+    CU(cudaSetDevice(c->device));
+    if (!c->q_count) {
+        const int rc = ensure_streams(c, S);
         if (rc) return rc;
     }
     c->cur = (c->q_first + c->q_count) & 1;
     memset(c->slots[c->cur].launches, 0, sizeof(c->slots[c->cur].launches));
+    if (c->profiling) CU(cudaEventRecord(c->slots[c->cur].ev[LANE_STAGE_H2D], c->st));
     return LANE_OK;
 }
 
@@ -502,20 +461,76 @@ int detect_blocking(lane_ctx *c, const uint8_t *frames, bool on_device, int n, c
 {
     if (in.format != LANE_INPUT_BGR && ((in.h | in.w) & 1))
         return fail(c, LANE_ERR_INVALID, "NV12 / I420 needs even width and height (%dx%d)", in.w, in.h);
-    int rc = check_call(c, frames, n, n_streams, prev_fit, prev_valid);
+    int rc = check_call(c, frames, n, stream_id, n_streams, prev_fit, prev_valid);
     if (rc) return rc;
     if (!out) return fail(c, LANE_ERR_INVALID, "out is null");
     if (n > 65535 && (in.h != c->g.H || in.w != c->g.W))           // the resize kernels put the batch on the grid's z
         return fail(c, LANE_ERR_UNSUPPORTED, "batch %d above 65535", n);
-    CU(cudaSetDevice(c->device));
-    if (stream_id)
-        for (int i = 0; i < n; i++)
-            if (stream_id[i] < 0 || stream_id[i] >= n_streams)
-                return fail(c, LANE_ERR_INVALID, "stream_id[%d]=%d outside [0,%d)", i, stream_id[i], n_streams);
-    if (c->profiling) CU(cudaEventRecord(c->slots[c->cur].ev[LANE_STAGE_H2D], c->st));
     rc = enqueue(c, frames, on_device, n, stream_id, n_streams, prev_fit, prev_valid, in);
     if (rc) return rc;
     return lane_detect_collect(c, prev_fit, prev_valid, out);
+}
+
+// The queries on the last batch (taps, Hough, edge counts) need it collected and, when they name one of its frames,
+// that frame to exist; otherwise it must hold a frame at all.  Returns the batch's size or a LANE_ERR_* code.
+int last_batch(lane_ctx *c, const int *frame_index = nullptr)
+{
+    if (c->q_count) return fail(c, LANE_ERR_STATE, "collect the last batch first");
+    const int n = c->slots[c->cur].n;
+    if (frame_index && (*frame_index < 0 || *frame_index >= n))
+        return fail(c, LANE_ERR_INVALID, "frame_index %d outside the last batch (%d frames)", *frame_index, n);
+    if (n < 1) return fail(c, LANE_ERR_STATE, "no batch has run on this context");
+    return n;
+}
+
+// The streams, events and buffers a context has from its creation on; the rest are created on first use.
+int create_resources(lane_ctx *c)
+{
+    const size_t B = (size_t)c->max_batch, H = (size_t)c->g.H, WW = (c->g.W + 31) / 32;
+    CU(c->st.create(cudaStreamNonBlocking));
+    {
+        // the back half first: its clusters keep their slots, the edge kernels fill in (DESIGN.md §4, "Two streams")
+        int lo = 0, hi = 0;
+        cudaDeviceGetStreamPriorityRange(&lo, &hi);
+        CU(c->st2.create(cudaStreamNonBlocking, hi));
+        for (auto &e : c->edge_done) CU(e.create(cudaEventDisableTiming));
+    }
+    for (auto &sl : c->slots) {
+        for (auto &e : sl.ev) CU(e.create());
+        CU(sl.done.create(cudaEventDisableTiming));
+        CU(sl.reader_done.create(cudaEventDisableTiming));
+    }
+    CU(c->d_roi_bits.alloc(H * WW));
+    CU(c->d_edge_bits.alloc(B * H * WW));
+    CU(c->d_cand_bits.alloc(B * H * WW));
+    CU(c->d_strong_bits.alloc(B * H * WW));
+    CU(c->d_hist.alloc(B * 256));
+    CU(c->d_lut.alloc(1022));
+    CU(c->d_thr.alloc(2 * B));
+    CU(c->d_n_edges.alloc(2 * B));
+    CU(c->d_n_points.alloc(2 * B));
+    CU(c->d_rounds.alloc(2 * B));
+    CU(c->d_n_lines.alloc(B));
+    CU(c->d_order.alloc(B));
+    CU(c->d_win.alloc(LANE_NUM_ANGLES));
+    CU(c->d_win3.alloc(LANE_NUM_ANGLES));
+    CU(c->d_lines.alloc(B * c->g.max_segments * 4));
+    CU(c->d_fit_raw.alloc(B * 6));
+    CU(c->d_fit_side_n.alloc(B * 2));
+    CU(c->d_fit_side_flags.alloc(B));
+    if (c->g.max_segments > LANE_MAX_SIDE_SEGMENTS)      // a side can hold every segment: work columns in global memory
+        CU(c->d_fit_big.alloc(B * 2 * 5 * 2 * (size_t)c->g.max_segments));
+    CU(c->d_stream_id.alloc(B));
+    for (auto &sl : c->slots) {
+        CU(sl.d_records.alloc(B));
+        CU(cudaMemset(sl.d_records, 0, sizeof(lane_record) * B));
+    }
+    CU(c->d_task_counter.alloc(4));
+    for (auto &sl : c->slots) CU(sl.h_records.alloc(B));
+    lane_upload_tables();
+    CU(cudaGetLastError());
+    CU(cudaDeviceSynchronize());
+    return LANE_OK;
 }
 
 }  // namespace
@@ -543,93 +558,44 @@ int lane_ctx_create(int device, int height, int width, int max_batch, int max_se
         return fail(c, LANE_ERR_NO_DEVICE, "device %d is sm_%d%d; this build holds sm_100a code only", device, prop.major, prop.minor);
     if (cudaSetDevice(device) != cudaSuccess) return fail(c, LANE_ERR_CUDA, "cudaSetDevice(%d) failed", device);
 
-    lane_ctx *ctx = new lane_ctx();
+    auto ctx = std::make_unique<lane_ctx>();
     ctx->device = device;
     ctx->max_batch = max_batch;
     LaneGeom &g = ctx->g;
     g.H = height; g.W = width;
     g.numrho = 2 * (width + height) + 1;
     g.max_segments = max_segments > 0 ? max_segments : 256;
-    g.bx0 = g.by0 = g.bx1 = g.by1 = g.bw = g.bh = 0;
-    g.max_points = 0;
-    const size_t P = (size_t)height * width, B = (size_t)max_batch;
-    ctx->seed_cap = (int)std::min<size_t>(P, (size_t)1 << 17);
-    c = ctx;
-    auto bail = [&](int code) { std::string e = ctx->err; free_all(ctx); delete ctx; g_create_error = e; return code; };
-#define CUB(call)                                                                                       \
-    do {                                                                                                \
-        cudaError_t e_ = (call);                                                                        \
-        if (e_ != cudaSuccess) {                                                                        \
-            fail(c, LANE_ERR_CUDA, "%s failed: %s", #call, cudaGetErrorString(e_));                     \
-            return bail(LANE_ERR_CUDA);                                                                 \
-        }                                                                                               \
-    } while (0)
-    CUB(cudaStreamCreateWithFlags(&ctx->st, cudaStreamNonBlocking));
-    {
-        // the back half first: its clusters keep their slots, the edge kernels fill in (DESIGN.md §4, "Two streams")
-        int lo = 0, hi = 0;
-        cudaDeviceGetStreamPriorityRange(&lo, &hi);
-        CUB(cudaStreamCreateWithPriority(&ctx->st2, cudaStreamNonBlocking, hi));
-        for (auto &e : ctx->edge_done) CUB(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    }
-    for (auto &sl : ctx->slots) {
-        for (auto &e : sl.ev) CUB(cudaEventCreate(&e));
-        CUB(cudaEventCreateWithFlags(&sl.done, cudaEventDisableTiming));
-        CUB(cudaEventCreateWithFlags(&sl.reader_done, cudaEventDisableTiming));
-    }
-    const size_t WW = (width + 31) / 32;
-    CUB(dalloc(&ctx->d_roi_bits, (size_t)height * WW));
-    CUB(dalloc(&ctx->d_edge_bits, B * height * WW));
-    CUB(dalloc(&ctx->d_dbg_c, B * height * WW));
-    CUB(dalloc(&ctx->d_dbg_s, B * height * WW));
-    CUB(dalloc(&ctx->d_hist, B * 256));
-    CUB(dalloc(&ctx->d_lut, 1022));
-    CUB(dalloc(&ctx->d_thr, 2 * B));
-    CUB(dalloc(&ctx->d_n_edges, 2 * B));
-    CUB(dalloc(&ctx->d_n_points, 2 * B));
-    CUB(dalloc(&ctx->d_rounds, 2 * B));
-    CUB(dalloc(&ctx->d_n_lines, B));
-    CUB(dalloc(&ctx->d_order, B));
-    CUB(dalloc(&ctx->d_win, LANE_NUM_ANGLES));
-    CUB(dalloc(&ctx->d_win3, LANE_NUM_ANGLES));
-    CUB(dalloc(&ctx->d_lines, B * g.max_segments * 4));
-    CUB(dalloc(&ctx->fit.raw, B * 6));
-    CUB(dalloc(&ctx->fit.side_n, B * 2));
-    CUB(dalloc(&ctx->fit.side_flags, B));
-    if (g.max_segments > LANE_MAX_SIDE_SEGMENTS)      // a side can hold every segment: work columns in global memory
-        CUB(dalloc(&ctx->fit.big, B * 2 * 5 * 2 * (size_t)g.max_segments));
-    CUB(dalloc(&ctx->d_stream_id, B));
-    for (auto &sl : ctx->slots) {
-        CUB(dalloc(&sl.d_records, B));
-        CUB(cudaMemset(sl.d_records, 0, sizeof(lane_record) * B));
-    }
-    CUB(dalloc(&ctx->d_task_counter, 4));
+    ctx->seed_cap = (int)std::min<size_t>((size_t)height * width, (size_t)1 << 17);
     {
         const char *e = getenv("LANE_B200_K4");
         ctx->ppht_v2 = e && !strcmp(e, "v2");
     }
-    for (auto &sl : ctx->slots) CUB(cudaMallocHost((void **)&sl.h_records, sizeof(lane_record) * B));
-    lane_upload_tables();
-    CUB(cudaGetLastError());
-    CUB(cudaDeviceSynchronize());
-#undef CUB
-    *out = ctx;
+    if (const int rc = create_resources(ctx.get())) {
+        g_create_error = std::move(ctx->err);        // the context goes; lane_last_error(NULL) reads why
+        cudaGetLastError();                          // reported: not left behind for the next call's own check
+        return rc;
+    }
+    *out = ctx.release();
     return LANE_OK;
 }
 
-void lane_ctx_destroy(lane_ctx *ctx)
-{
-    if (!ctx) return;
-    cudaSetDevice(ctx->device);
-    if (ctx->st) cudaStreamSynchronize(ctx->st);
-    free_all(ctx);
-    delete ctx;
-}
+void lane_ctx_destroy(lane_ctx *ctx) { delete ctx; }
 
 int lane_set_roi_mask(lane_ctx *c, const uint8_t *mask)
 {
     if (!c || !mask) return LANE_ERR_INVALID;
     CU(cudaSetDevice(c->device));
+    // Detect calls are refused until every buffer made from the ROI is rebuilt below, so a re-set that fails part way
+    // leaves a context without a ROI, not one whose kernels would read released buffers.  The old buffers go before the
+    // new ones are allocated: the two sets are never held at once.
+    c->have_roi = false;
+    CU(c->sync());
+    c->fallback_ready = false;                       // the generic-width buffers are rebuilt on next use
+    c->d_cls.reset(); c->d_cls_dbg.reset(); c->d_roi.reset(); c->d_pmask.reset();
+    c->d_seedsA.reset(); c->d_seedsB.reset(); c->d_seed_count.reset();
+    c->d_pmask_bits.reset(); c->d_points.reset(); c->d_points_dbg.reset();
+    c->d_accum16.reset(); c->d_pmask_work.reset(); c->d_list_over.reset();
+
     LaneGeom &g = c->g;
     int x0 = g.W, y0 = g.H, x1 = -1, y1 = -1, cnt = 0;
     for (int y = 0; y < g.H; y++)
@@ -642,31 +608,18 @@ int lane_set_roi_mask(lane_ctx *c, const uint8_t *mask)
     g.bx0 = x0; g.by0 = y0; g.bx1 = x1 + 1; g.by1 = y1 + 1;
     g.bw = g.bx1 - g.bx0; g.bh = g.by1 - g.by0;
     g.max_points = cnt;
-    CU(cudaStreamSynchronize(c->st));
     const size_t P = (size_t)g.H * g.W, WW = (g.W + 31) / 32;
-    free(c->h_roi);
-    c->h_roi = (uint8_t *)malloc(P);
-    memcpy(c->h_roi, mask, P);
+    c->h_roi.assign(mask, mask + P);
     std::vector<uint32_t> bits((size_t)g.H * WW, 0u);
     for (int y = 0; y < g.H; y++)
         for (int x = 0; x < g.W; x++)
             if (mask[(size_t)y * g.W + x]) bits[(size_t)y * WW + (x >> 5)] |= 1u << (x & 31);
     CU(cudaMemcpy(c->d_roi_bits, bits.data(), sizeof(uint32_t) * bits.size(), cudaMemcpyHostToDevice));
-    // geometry changed: the lazily-built fallback buffers are rebuilt on next use
-    for (void **p : {(void **)&c->d_pmask, (void **)&c->d_roi, (void **)&c->d_cls, (void **)&c->d_cls_dbg,
-                     (void **)&c->d_seedsA, (void **)&c->d_seedsB, (void **)&c->d_seed_count,
-                     (void **)&c->d_pmask_bits, (void **)&c->d_points, (void **)&c->d_points_dbg}) {
-        if (*p) cudaFree(*p);
-        *p = nullptr;
-    }
-    c->fallback_ready = false;
     {
         int2 win[LANE_NUM_ANGLES];
         c->cells_per_frame = lane_ppht_windows(mask, g.H, g.W, win);
         CU(cudaMemcpy(c->d_win, win, sizeof(win), cudaMemcpyHostToDevice));
-        if (c->d_accum16) cudaFree(c->d_accum16);
-        c->d_accum16 = nullptr;
-        CU(dalloc(&c->d_accum16, (size_t)c->max_batch * (c->cells_per_frame / 2)));
+        CU(c->d_accum16.alloc((size_t)c->max_batch * (c->cells_per_frame / 2)));
         int2 win3[LANE_NUM_ANGLES];
         c->G3 = lane_ppht_plan_v3(win, c->cells_per_frame, win3, &c->cells_max3, &c->list_cap3);
         {
@@ -681,25 +634,21 @@ int lane_set_roi_mask(lane_ctx *c, const uint8_t *mask)
             }
         }
         CU(cudaMemcpy(c->d_win3, win3, sizeof(win3), cudaMemcpyHostToDevice));
-        if (c->d_pmask_work) cudaFree(c->d_pmask_work);
-        c->d_pmask_work = nullptr;
-        if (c->d_list_over) cudaFree(c->d_list_over);
-        c->d_list_over = nullptr;
         if (c->G3 > 0) {
-            CU(dalloc(&c->d_pmask_work, (size_t)c->max_batch * c->G3 * std::max(g.bh, 1) * WW));
+            CU(c->d_pmask_work.alloc((size_t)c->max_batch * c->G3 * std::max(g.bh, 1) * WW));
             // the ROI can hold more edge pixels than the shared-memory list: every CTA of a cluster gets a private global
             // extension, sized by the ROI up to lane_ppht_over_cap_v3() points (busier frames go to the global-memory kernel)
             c->over_cap3 = 0;
             if (cnt > c->list_cap3) {
                 c->over_cap3 = (int)std::min<long long>((long long)cnt - c->list_cap3, lane_ppht_over_cap_v3());
                 c->over_cap3 = (c->over_cap3 + 63) & ~63;
-                CU(dalloc(&c->d_list_over, (size_t)c->max_batch * c->G3 * (size_t)c->over_cap3));
+                CU(c->d_list_over.alloc((size_t)c->max_batch * c->G3 * (size_t)c->over_cap3));
             }
         }
     }
-    CU(dalloc(&c->d_pmask_bits, 2 * (size_t)c->max_batch * std::max(g.bh, 1) * WW));      // per result slot
-    CU(dalloc(&c->d_points, 2 * (size_t)c->max_batch * g.max_points));
-    if (c->debug) CU(dalloc(&c->d_points_dbg, (size_t)c->max_batch * g.max_points));
+    CU(c->d_pmask_bits.alloc(2 * (size_t)c->max_batch * std::max(g.bh, 1) * WW));      // per result slot
+    CU(c->d_points.alloc(2 * (size_t)c->max_batch * g.max_points));
+    if (c->debug) CU(c->d_points_dbg.alloc((size_t)c->max_batch * g.max_points));
     c->have_roi = true;
     return LANE_OK;
 }
@@ -743,12 +692,9 @@ int lane_set_debug(lane_ctx *c, int keep)
     c->debug = keep != 0;
     if (c->debug) {
         const size_t P = (size_t)c->g.H * c->g.W;
-        const size_t WW = (c->g.W + 31) / 32;
-        if (!c->d_dbg_c) CU(dalloc(&c->d_dbg_c, (size_t)c->max_batch * c->g.H * WW));
-        if (!c->d_dbg_s) CU(dalloc(&c->d_dbg_s, (size_t)c->max_batch * c->g.H * WW));
-        if (c->fallback_ready && !c->d_cls_dbg) CU(dalloc(&c->d_cls_dbg, (size_t)c->max_batch * P));
-        if (!c->d_gray_dbg) CU(dalloc(&c->d_gray_dbg, P));
-        if (!c->d_points_dbg && c->have_roi) CU(dalloc(&c->d_points_dbg, (size_t)c->max_batch * c->g.max_points));
+        if (c->fallback_ready) CU(c->d_cls_dbg.lazy((size_t)c->max_batch * P));
+        CU(c->d_gray_dbg.lazy(P));
+        if (c->have_roi) CU(c->d_points_dbg.lazy((size_t)c->max_batch * c->g.max_points));
     }
     return LANE_OK;
 }
@@ -764,7 +710,7 @@ void *lane_ctx_stream(lane_ctx *c) { return c ? (void *)c->st : nullptr; }
 
 int lane_ctx_last_paths(lane_ctx *c) { return c ? c->last_paths : 0; }
 
-const lane_record *lane_ctx_records_device(lane_ctx *c) { return c ? c->slots[c->last_collected].d_records : nullptr; }
+const lane_record *lane_ctx_records_device(lane_ctx *c) { return c ? c->slots[c->last_collected].d_records.get() : nullptr; }
 
 int lane_ctx_fence_records(lane_ctx *c, void *reader_stream)
 {
@@ -780,23 +726,16 @@ int lane_ctx_set_stream(lane_ctx *c, void *cuda_stream)
 {
     if (!c) return LANE_ERR_INVALID;
     if (c->q_count) return fail(c, LANE_ERR_STATE, "cannot switch streams with a batch in flight");
-    if (c->own_stream && c->st) { cudaStreamSynchronize(c->st); cudaStreamDestroy(c->st); }
-    c->st = (cudaStream_t)cuda_stream;
-    c->own_stream = false;
+    if (c->st) cudaStreamSynchronize(c->st);
+    c->st.borrow((cudaStream_t)cuda_stream);
     return LANE_OK;
 }
 
 int lane_detect_enqueue(lane_ctx *c, const uint8_t *frames_dev, int n, const int32_t *stream_id, int n_streams,
                         const double *prev_fit, const uint8_t *prev_valid)
 {
-    int rc = check_call(c, frames_dev, n, n_streams, prev_fit, prev_valid);
+    const int rc = check_call(c, frames_dev, n, stream_id, n_streams, prev_fit, prev_valid);
     if (rc) return rc;
-    CU(cudaSetDevice(c->device));
-    if (stream_id)
-        for (int i = 0; i < n; i++)
-            if (stream_id[i] < 0 || stream_id[i] >= n_streams)
-                return fail(c, LANE_ERR_INVALID, "stream_id[%d]=%d outside [0,%d)", i, stream_id[i], n_streams);
-    if (c->profiling) CU(cudaEventRecord(c->slots[c->cur].ev[LANE_STAGE_H2D], c->st));
     return enqueue(c, frames_dev, true, n, stream_id, n_streams, prev_fit, prev_valid, Ingest{LANE_INPUT_BGR, c->g.H, c->g.W});
 }
 
@@ -858,9 +797,7 @@ int lane_get_stage_ms(lane_ctx *c, float ms[LANE_NUM_STAGES], int32_t launches[L
 int lane_debug_tap(lane_ctx *c, int what, int fi, void *host_out, size_t capacity, size_t *bytes_written)
 {
     if (!c || !host_out) return LANE_ERR_INVALID;
-    if (c->q_count) return fail(c, LANE_ERR_STATE, "collect the batch before reading taps");
-    const int last_n = c->slots[c->cur].n;
-    if (fi < 0 || fi >= last_n) return fail(c, LANE_ERR_INVALID, "frame_index %d outside last batch (%d)", fi, last_n);
+    if (const int n = last_batch(c, &fi); n < 0) return n;
     CU(cudaSetDevice(c->device));
     const LaneGeom &g = c->g;
     const size_t P = (size_t)g.H * g.W;
@@ -887,8 +824,8 @@ int lane_debug_tap(lane_ctx *c, int what, int fi, void *host_out, size_t capacit
             return fail(c, LANE_ERR_STATE, "LANE_TAP_CLASS needs lane_set_debug(ctx,1) before detect");
         } else if (c->last_cluster) {
             std::vector<uint32_t> cc(words), ss(words);
-            CU(cudaMemcpy(cc.data(), c->d_dbg_c + fi * words, sizeof(uint32_t) * words, cudaMemcpyDeviceToHost));
-            CU(cudaMemcpy(ss.data(), c->d_dbg_s + fi * words, sizeof(uint32_t) * words, cudaMemcpyDeviceToHost));
+            CU(cudaMemcpy(cc.data(), c->d_cand_bits + fi * words, sizeof(uint32_t) * words, cudaMemcpyDeviceToHost));
+            CU(cudaMemcpy(ss.data(), c->d_strong_bits + fi * words, sizeof(uint32_t) * words, cudaMemcpyDeviceToHost));
             for (int y = 0; y < g.H; y++)
                 for (int x = 0; x < g.W; x++) {
                     const uint32_t cb = (cc[y * WW + (x >> 5)] >> (x & 31)) & 1u, sb = (ss[y * WW + (x >> 5)] >> (x & 31)) & 1u;
@@ -932,26 +869,19 @@ int lane_hough_accumulator(lane_ctx *c, int fi, int32_t *accum_host, int thresho
                            int max_peaks, int *n_peaks)
 {
     if (!c) return LANE_ERR_INVALID;
-    if (c->q_count) return fail(c, LANE_ERR_STATE, "collect the batch first");
-    const int last_n = c->slots[c->cur].n;
-    if (fi < 0 || fi >= last_n) return fail(c, LANE_ERR_INVALID, "frame_index %d outside last batch (%d)", fi, last_n);
+    if (const int n = last_batch(c, &fi); n < 0) return n;
     if (!c->debug || !c->d_points_dbg) return fail(c, LANE_ERR_STATE, "lane_hough_accumulator needs lane_set_debug(ctx,1) before detect");
     CU(cudaSetDevice(c->device));
     const LaneGeom &g = c->g;
     const size_t cells = (size_t)(LANE_NUM_ANGLES + 2) * (g.numrho + 2);
-    if (!c->d_std_accum) CU(dalloc(&c->d_std_accum, cells));
+    CU(c->d_std_accum.lazy(cells));
     launch_hough_accum(c->d_points_dbg + (size_t)fi * g.max_points, c->d_n_points + (size_t)c->cur * c->max_batch + fi, c->d_std_accum, g, c->st);
     CU(cudaGetLastError());
     if (accum_host) CU(cudaMemcpyAsync(accum_host, c->d_std_accum, sizeof(int32_t) * cells, cudaMemcpyDeviceToHost, c->st));
     int found = 0;
     if (peaks_host && max_peaks > 0) {
-        if (max_peaks > c->peaks_cap) {
-            if (c->d_peaks) cudaFree(c->d_peaks);
-            c->d_peaks = nullptr;
-            CU(dalloc(&c->d_peaks, (size_t)max_peaks));
-            c->peaks_cap = max_peaks;
-        }
-        if (!c->d_n_peaks) CU(dalloc(&c->d_n_peaks, 1));
+        CU(c->d_peaks.grow((size_t)max_peaks));
+        CU(c->d_n_peaks.lazy(1));
         launch_hough_peaks(c->d_std_accum, g.numrho, threshold, c->d_peaks, max_peaks, c->d_n_peaks, c->st);
         CU(cudaGetLastError());
         CU(cudaMemcpyAsync(&found, c->d_n_peaks, sizeof(int), cudaMemcpyDeviceToHost, c->st));
@@ -975,9 +905,8 @@ int lane_hough_accumulator(lane_ctx *c, int fi, int32_t *accum_host, int thresho
 int lane_edge_count_rect(lane_ctx *c, int x0, int y0, int x1, int y1, int32_t *counts_host)
 {
     if (!c || !counts_host) return LANE_ERR_INVALID;
-    if (c->q_count) return fail(c, LANE_ERR_STATE, "collect the batch first");
-    const int n = c->slots[c->cur].n;
-    if (n < 1) return fail(c, LANE_ERR_STATE, "no batch has run on this context");
+    const int n = last_batch(c);
+    if (n < 0) return n;
     if (x0 < 0 || y0 < 0 || x1 > c->g.W || y1 > c->g.H || x0 >= x1 || y0 >= y1)
         return fail(c, LANE_ERR_INVALID, "bad rectangle [%d,%d) x [%d,%d)", x0, x1, y0, y1);
     CU(cudaSetDevice(c->device));
@@ -993,29 +922,20 @@ int lane_hough_lines_batch(lane_ctx *c, int threshold, int max_peaks, int32_t *p
                            int32_t *accum_host, float *device_ms)
 {
     if (!c || max_peaks < 1 || !peaks_host || !n_peaks_host) return LANE_ERR_INVALID;
-    if (c->q_count) return fail(c, LANE_ERR_STATE, "collect the batch first");
-    const int n = c->slots[c->cur].n;
-    if (n < 1) return fail(c, LANE_ERR_STATE, "no batch has run on this context");
+    const int n = last_batch(c);
+    if (n < 0) return n;
     CU(cudaSetDevice(c->device));
     const LaneGeom &g = c->g;
     const size_t cells = (size_t)(LANE_NUM_ANGLES + 2) * (g.numrho + 2), B = (size_t)c->max_batch;
-    if (max_peaks > c->hb_cap) {
-        for (void **p : {(void **)&c->d_hb_sorted, (void **)&c->d_hb_tmp}) {
-            if (*p) cudaFree(*p);
-            *p = nullptr;
-        }
-        CU(dalloc(&c->d_hb_sorted, B * max_peaks * 3));
-        CU(dalloc(&c->d_hb_tmp, B * max_peaks));
-        c->hb_cap = max_peaks;
-    }
+    CU(c->d_hb_sorted.grow(B * max_peaks * 3));
+    CU(c->d_hb_tmp.grow(B * max_peaks));
     if (!c->d_hb_count) {
-        CU(dalloc(&c->d_hb_count, B));
-        CU(cudaEventCreate(&c->hb_ev[0]));
-        CU(cudaEventCreate(&c->hb_ev[1]));
+        for (auto &e : c->hb_ev) CU(e.create());
+        CU(c->d_hb_count.alloc(B));
     }
-    if (accum_host && !c->d_hb_accum) CU(dalloc(&c->d_hb_accum, B * cells));
+    if (accum_host) CU(c->d_hb_accum.lazy(B * cells));
     CU(cudaEventRecord(c->hb_ev[0], c->st));
-    if (!launch_hough_batch(c->d_edge_bits, c->d_roi_bits, accum_host ? c->d_hb_accum : nullptr, c->d_hb_tmp, c->d_hb_sorted,
+    if (!launch_hough_batch(c->d_edge_bits, c->d_roi_bits, accum_host ? c->d_hb_accum.get() : nullptr, c->d_hb_tmp, c->d_hb_sorted,
                             c->d_hb_count, g, threshold, max_peaks, n, c->st))
         return fail(c, LANE_ERR_UNSUPPORTED, "frame %dx%d: a Hough row does not fit shared memory", g.W, g.H);
     CU(cudaEventRecord(c->hb_ev[1], c->st));
