@@ -87,6 +87,12 @@ LANE_API int lane_abi_version(void);
  * non-zero = inside.  Replaces the per-frame _get_roi_mask/_apply_roi (:86-90).  May be called again on a live
  * context; if such a call fails, detect calls return LANE_ERR_STATE until one succeeds. */
 LANE_API int lane_set_roi_mask(lane_ctx *ctx, const uint8_t *mask);
+/* One ROI mask per camera of a rig (lane_detector.py:47-64, one LaneDetector(roi_vertices=...) per camera):
+ * uint8[n_masks][height*width], non-zero = inside.  Mask r belongs to stream r: with n_masks > 1 frame f of a detect
+ * call uses mask stream_id[f] (mask 0 when stream_id is NULL), and a call with n_streams > n_masks is refused with
+ * LANE_ERR_INVALID.  A frame's records, taps and Hough outputs equal those of a context set with its mask alone.
+ * n_masks = 1 is lane_set_roi_mask.  Re-setting and failures behave as for lane_set_roi_mask. */
+LANE_API int lane_set_roi_masks(lane_ctx *ctx, const uint8_t *masks, int n_masks);
 /* low/high Canny thresholds for every possible 2*median (index 0..510), filled by evaluating the
  * reference's own float64 expressions (lane_detector.py:80-81). */
 LANE_API int lane_set_threshold_lut(lane_ctx *ctx, const uint8_t *low511, const uint8_t *high511);

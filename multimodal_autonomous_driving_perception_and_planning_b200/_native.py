@@ -84,6 +84,7 @@ _PROTOS = {
     "lane_ctx_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "lane_ctx_destroy": (None, [C.c_void_p]),
     "lane_set_roi_mask": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "lane_set_roi_masks": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int]),
     "lane_set_threshold_lut": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "lane_set_hough_params": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int]),
     "lane_set_smoothing": (C.c_int, [C.c_void_p, C.c_double, C.c_double]),
@@ -163,7 +164,10 @@ def _ptr(a):
 
 
 class LaneContext:
-    """One native context: fixed (H, W), up to max_batch frames per call, one CUDA stream."""
+    """One native context: fixed (H, W), up to max_batch frames per call, one CUDA stream.
+
+    ``roi_mask`` is uint8 ``(H, W)``, or ``(R, H, W)`` for one mask per camera stream: mask r is stream r's, and every
+    call then takes at most R streams (see lane_set_roi_masks)."""
 
     def __init__(self, height: int, width: int, max_batch: int, roi_mask: np.ndarray, device: int = 0,
                  max_segments: int = 256, debug: bool = False):
@@ -178,9 +182,13 @@ class LaneContext:
             self._check(L.lane_set_debug(self._h, 1))
         self.debug = debug
         mask = np.ascontiguousarray(roi_mask, dtype=np.uint8)
-        if mask.shape != (height, width):
-            raise ValueError(f"roi mask shape {mask.shape} != {(height, width)}")
-        self._check(L.lane_set_roi_mask(self._h, _ptr(mask)))
+        if mask.ndim == 3 and mask.shape[0] >= 1 and mask.shape[1:] == (height, width):
+            self._check(L.lane_set_roi_masks(self._h, _ptr(mask), mask.shape[0]))
+        elif mask.shape == (height, width):
+            self._check(L.lane_set_roi_mask(self._h, _ptr(mask)))
+        else:
+            raise ValueError(f"roi mask shape {mask.shape} is neither {(height, width)} nor (R, {height}, {width})")
+        self.n_roi = mask.shape[0] if mask.ndim == 3 else 1
         low, high = threshold_lut()
         self._check(L.lane_set_threshold_lut(self._h, _ptr(low), _ptr(high)))
         self.settings = {"hough": (50, 50, 150), "lut": (low, high), "blur": True}   # what copy_settings_to replays

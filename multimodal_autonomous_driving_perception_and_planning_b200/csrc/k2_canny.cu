@@ -197,6 +197,7 @@ __global__ void k_finalize(uint8_t *__restrict__ cls, int *__restrict__ n_edges,
 
 // ---- ROI mask + ordered compaction: one CTA per frame walks the ROI bounding box row-major -------
 __global__ void __launch_bounds__(1024) k_compact(const uint8_t *__restrict__ edges, const uint8_t *__restrict__ roi,
+                                                  const int *__restrict__ roi_index, size_t roi_stride,
                                                   uint8_t *__restrict__ pmask, uint32_t *__restrict__ points,
                                                   int *__restrict__ n_points, LaneGeom g)
 {
@@ -204,6 +205,7 @@ __global__ void __launch_bounds__(1024) k_compact(const uint8_t *__restrict__ ed
     __shared__ int s_total;
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5, f = blockIdx.x;
     const uint8_t *e = edges + (size_t)f * g.H * g.W;
+    if (roi_index) roi += (size_t)roi_index[f] * roi_stride;
     const int area = g.bw * g.bh;
     uint8_t *pm = pmask + (size_t)f * area;
     uint32_t *out = points + (size_t)f * g.max_points;
@@ -273,9 +275,9 @@ void launch_finalize_edges(uint8_t *cls_edges, int *n_edges, int n, int H, int W
     *launches += 1;
 }
 
-void launch_compact(const uint8_t *edges, const uint8_t *roi, uint8_t *pmask, uint32_t *points, int *n_points,
-                    LaneGeom g, int n, cudaStream_t st, int *launches)
+void launch_compact(const uint8_t *edges, const uint8_t *roi, const int *roi_index, size_t roi_stride, uint8_t *pmask,
+                    uint32_t *points, int *n_points, LaneGeom g, int n, cudaStream_t st, int *launches)
 {
-    k_compact<<<n, 1024, 0, st>>>(edges, roi, pmask, points, n_points, g);
+    k_compact<<<n, 1024, 0, st>>>(edges, roi, roi_index, roi_stride, pmask, points, n_points, g);
     *launches += 1;
 }

@@ -39,13 +39,15 @@ struct K2Args {
     const uint32_t *c_bits, *s_bits;   // [n][H][WW] candidate / strong planes (from k2a_sobel_nms or k2t_threshold)
     const int *skip_flag;              // [n] or null: frames waiting for the redo pass (fused path) are skipped
     const int *frame_list, *n_list;    // redo pass: the frames to process (null = all)
-    const uint32_t *roi_bits;      // [H][WW]
+    const uint32_t *roi_bits;      // [R][roi_stride] ROI planes, each [H][WW]
     int *n_edges, *rounds, *n_points;
     uint32_t *points;              // [n][max_points]
     uint32_t *pmask_bits;          // [n][bh][WW]
     uint32_t *edge_bits;           // [n][H][WW]
     int H, W, WW, R;               // R = rows per band
     LaneGeom g;
+    const int *roi_index;          // [n] ROI plane of each frame, or null: every frame uses plane 0
+    size_t roi_stride;             // words between planes (0 with a null roi_index)
 };
 
 __device__ __forceinline__ uint32_t h2add(uint32_t a, uint32_t b)
@@ -561,7 +563,7 @@ __global__ void __launch_bounds__(K2T, 3) k2_canny_cluster(K2Args A)
     // row-major point list below never waits on global memory.
     const LaneGeom &g = A.g;
     const int y0 = max(b0, g.by0), y1 = min(b1, g.by1);
-    const uint32_t *roi = A.roi_bits;
+    const uint32_t *roi = A.roi_bits + (A.roi_index ? (size_t)A.roi_index[f] * A.roi_stride : 0);
     uint32_t *Mk = C;                                     // [Rv][WW] masked edges of this band
     int cnt = 0;
     uint32_t *eb = A.edge_bits + ((size_t)f * H + b0) * WW;
@@ -707,11 +709,13 @@ __global__ void k_bytes_to_bits(const uint8_t *__restrict__ bytes, uint32_t *__r
     }
 }
 
-// pmask[f][y-by0][w] = edge_bits[f][y][w] & roi_bits[y][w]  (generic-width fallback path)
+// pmask[f][y-by0][w] = edge_bits[f][y][w] & roi_bits[roi_index[f]][y][w]  (generic-width fallback path)
 __global__ void k_mask_rows(const uint32_t *__restrict__ edge_bits, const uint32_t *__restrict__ roi_bits,
-                            uint32_t *__restrict__ pmask_bits, int H, int WW, int by0, int bh)
+                            const int *__restrict__ roi_index, size_t roi_stride, uint32_t *__restrict__ pmask_bits, int H,
+                            int WW, int by0, int bh)
 {
     const int f = blockIdx.y;
+    if (roi_index) roi_bits += (size_t)roi_index[f] * roi_stride;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < bh * WW; i += gridDim.x * blockDim.x) {
         const int y = by0 + i / WW, w = i % WW;
         pmask_bits[(size_t)f * bh * WW + i] = edge_bits[((size_t)f * H + y) * WW + w] & roi_bits[(size_t)y * WW + w];
@@ -763,7 +767,7 @@ static cudaError_t k2b_launch(const K2Args &A, int G, size_t smem, int n, cudaSt
 // Unfused form: K2a (Sobel + NMS + thresholds from the blurred plane) then K2b.  Returns false when this frame geometry
 // cannot take the cluster path (caller falls back to the generic byte-map kernels).
 bool launch_canny_cluster(const uint8_t *blur, const uint32_t *hist, const uint8_t *lut_low, const uint8_t *lut_high,
-                          const uint32_t *roi_bits, int4 *thr, int *n_edges, int *rounds, uint32_t *points,
+                          const uint32_t *roi_bits, const int *roi_index, size_t roi_stride, int4 *thr, int *n_edges, int *rounds, uint32_t *points,
                           int *n_points, uint32_t *pmask_bits, uint32_t *edge_bits, uint32_t *c_bits, uint32_t *s_bits,
                           int *task_counter, LaneGeom g, int n, cudaStream_t st, int *launches)
 {
@@ -786,7 +790,7 @@ bool launch_canny_cluster(const uint8_t *blur, const uint32_t *hist, const uint8
                                                                   n, H, W, band_rows, tail_frames, tail_rows);
     }
     K2Args A{};
-    A.c_bits = c_bits; A.s_bits = s_bits; A.roi_bits = roi_bits;
+    A.c_bits = c_bits; A.s_bits = s_bits; A.roi_bits = roi_bits; A.roi_index = roi_index; A.roi_stride = roi_stride;
     A.n_edges = n_edges; A.rounds = rounds; A.n_points = n_points; A.points = points;
     A.pmask_bits = pmask_bits; A.edge_bits = edge_bits;
     A.H = H; A.W = W; A.WW = WW; A.R = R; A.g = g;
@@ -803,10 +807,11 @@ bool launch_canny_cluster(const uint8_t *blur, const uint32_t *hist, const uint8
 // are flagged, listed in redo_list and skipped.  frame_list == redo_list: the redo pass, after launch_fused_edge_redo
 // has rebuilt those frames' planes with the exact floor.
 bool launch_canny_cluster_fused(const uint32_t *k_bits, const uint8_t *v_plane, const uint32_t *hist, const uint8_t *lut_low,
-                                const uint8_t *lut_high, const uint32_t *roi_bits, int4 *thr, const int *pre, int *pre_redo,
-                                int *redo_list, int *redo_count, int *redo_flag, const int *frame_list, int *n_edges,
-                                int *rounds, uint32_t *points, int *n_points, uint32_t *pmask_bits, uint32_t *edge_bits,
-                                uint32_t *c_bits, uint32_t *s_bits, LaneGeom g, int n, cudaStream_t st, int *launches)
+                                const uint8_t *lut_high, const uint32_t *roi_bits, const int *roi_index, size_t roi_stride,
+                                int4 *thr, const int *pre, int *pre_redo, int *redo_list, int *redo_count, int *redo_flag,
+                                const int *frame_list, int *n_edges, int *rounds, uint32_t *points, int *n_points,
+                                uint32_t *pmask_bits, uint32_t *edge_bits, uint32_t *c_bits, uint32_t *s_bits, LaneGeom g, int n,
+                                cudaStream_t st, int *launches)
 {
     const int H = g.H, W = g.W, WW = (W + 31) / 32;
     int G = 1, R = 0;
@@ -825,7 +830,8 @@ bool launch_canny_cluster_fused(const uint32_t *k_bits, const uint8_t *v_plane, 
     k2t_threshold<<<tgrid, 256, 0, st>>>(T);
     K2Args A{};
     A.c_bits = c_bits; A.s_bits = s_bits; A.skip_flag = redo_flag;
-    A.frame_list = frame_list; A.n_list = frame_list ? redo_count : nullptr; A.roi_bits = roi_bits;
+    A.frame_list = frame_list; A.n_list = frame_list ? redo_count : nullptr;
+    A.roi_bits = roi_bits; A.roi_index = roi_index; A.roi_stride = roi_stride;
     A.n_edges = n_edges; A.rounds = rounds; A.n_points = n_points; A.points = points;
     A.pmask_bits = pmask_bits; A.edge_bits = edge_bits;
     A.H = H; A.W = W; A.WW = WW; A.R = R; A.g = g;
@@ -879,12 +885,12 @@ void launch_bytes_to_bits(const uint8_t *bytes, uint32_t *bits, int n, int rows,
     if (launches) *launches += 1;
 }
 
-void launch_mask_rows(const uint32_t *edge_bits, const uint32_t *roi_bits, uint32_t *pmask_bits, LaneGeom g, int n,
-                      cudaStream_t st, int *launches)
+void launch_mask_rows(const uint32_t *edge_bits, const uint32_t *roi_bits, const int *roi_index, size_t roi_stride,
+                      uint32_t *pmask_bits, LaneGeom g, int n, cudaStream_t st, int *launches)
 {
     const int WW = (g.W + 31) / 32;
     if (g.bh <= 0) return;
     dim3 grid((g.bh * WW + 255) / 256, n);
-    k_mask_rows<<<grid, 256, 0, st>>>(edge_bits, roi_bits, pmask_bits, g.H, WW, g.by0, g.bh);
+    k_mask_rows<<<grid, 256, 0, st>>>(edge_bits, roi_bits, roi_index, roi_stride, pmask_bits, g.H, WW, g.by0, g.bh);
     if (launches) *launches += 1;
 }

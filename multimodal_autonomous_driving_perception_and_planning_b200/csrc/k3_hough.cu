@@ -80,11 +80,13 @@ constexpr int K3_CAP = 2048;           // points per voting round (a quarter of 
 
 struct K3Args {
     const uint32_t *edge_bits;         // [n][H][WW]
-    const uint32_t *roi_bits;          // [H][WW]
+    const uint32_t *roi_bits;          // [R][roi_stride] ROI planes, each [H][WW]
     int32_t *accum;                    // [n][182][numrho+2] or null
     int2 *peaks;                       // [n][max_peaks] (flat padded index, votes), unordered
     int *n_peaks;                      // [n]
     int H, WW, by0, by1, numrho, TB, threshold, max_peaks;
+    const int *roi_index;              // [n] ROI plane of each frame, or null: every frame uses plane 0
+    size_t roi_stride;
 };
 
 __device__ __forceinline__ int k3_cell(const uint32_t *row, int c) { return (int)((row[c >> 1] >> ((c & 1) * 16)) & 0xFFFFu); }
@@ -104,6 +106,7 @@ __global__ void __launch_bounds__(K3T) k3_batch(K3Args A)
     __syncthreads();
     const int off = (A.numrho - 1) / 2 + 1;
     const uint32_t *eb = A.edge_bits + (size_t)f * A.H * A.WW;
+    const uint32_t *roi = A.roi_bits + (A.roi_index ? (size_t)A.roi_index[f] * A.roi_stride : 0);
     const int n_words = (A.by1 - A.by0) * A.WW;
 
     // vote the s_cnt points in pts[]: a warp per angle row, 32 consecutive points per step, equal cells merged
@@ -152,7 +155,7 @@ __global__ void __launch_bounds__(K3T) k3_batch(K3Args A)
         int y = 0, w = 0;
         if (i < n_words) {
             y = A.by0 + i / A.WW; w = i % A.WW;
-            m = eb[(size_t)y * A.WW + w] & A.roi_bits[(size_t)y * A.WW + w];
+            m = eb[(size_t)y * A.WW + w] & roi[(size_t)y * A.WW + w];
         }
         if (m) atomicAdd(&s_round[par], __popc(m));
         __syncthreads();
@@ -250,9 +253,9 @@ void launch_hough_peaks(const int32_t *accum_padded, int numrho, int threshold, 
 // Batched standard Hough over the n frames whose edge planes are in edge_bits.  accum (optional) receives the padded
 // int32 accumulators [n][182][numrho+2]; peaks_sorted [n][max_peaks][3] = (rho index, angle index, votes) in cv2 order,
 // n_peaks[n] = peaks found (may exceed max_peaks; only that many are kept).  peaks_tmp: [n][max_peaks] int2 scratch.
-bool launch_hough_batch(const uint32_t *edge_bits, const uint32_t *roi_bits, int32_t *accum, int2 *peaks_tmp,
-                        int32_t *peaks_sorted, int *n_peaks, LaneGeom g, int threshold, int max_peaks, int n,
-                        cudaStream_t st)
+bool launch_hough_batch(const uint32_t *edge_bits, const uint32_t *roi_bits, const int *roi_index, size_t roi_stride,
+                        int32_t *accum, int2 *peaks_tmp, int32_t *peaks_sorted, int *n_peaks, LaneGeom g, int threshold,
+                        int max_peaks, int n, cudaStream_t st)
 {
     const int row_words = (g.numrho + 2 + 1) / 2;
     const size_t row_bytes = (size_t)row_words * 4, fixed = sizeof(uint32_t) * K3_CAP;
@@ -268,7 +271,7 @@ bool launch_hough_batch(const uint32_t *edge_bits, const uint32_t *roi_bits, int
         configured[lane_cur_device()] = true;
     }
     K3Args A{};
-    A.edge_bits = edge_bits; A.roi_bits = roi_bits; A.accum = accum; A.peaks = peaks_tmp; A.n_peaks = n_peaks;
+    A.edge_bits = edge_bits; A.roi_bits = roi_bits; A.roi_index = roi_index; A.roi_stride = roi_stride; A.accum = accum; A.peaks = peaks_tmp; A.n_peaks = n_peaks;
     A.H = g.H; A.WW = (g.W + 31) / 32; A.by0 = g.by0; A.by1 = g.by1; A.numrho = g.numrho; A.TB = TB;
     A.threshold = threshold; A.max_peaks = max_peaks;
     cudaMemsetAsync(n_peaks, 0, sizeof(int) * n, st);

@@ -45,13 +45,16 @@ struct lane_ctx {
     DeviceArray<uint32_t> d_kbits;    // [B][H][WW] NMS survivors of the fused edge kernel
     DeviceArray<uint8_t> d_vplane;    // [B][H][W]  their magnitudes (sparse: only survivors' bytes are ever written / read)
     DeviceArray<int> d_pre;           // [B] magnitude floor per frame | [B] floor of the redo pass | [B] redo list | count
-    DeviceArray<uint32_t> d_roi_bits;     // [H][WW] bit-plane of the ROI mask
+    DeviceArray<uint32_t> d_roi_bits;     // [n_roi][roi_stride] bit-planes of the ROI masks, each [H][WW]
+    int n_roi = 0;                        // ROI masks; with more than one, frame f uses mask stream_id[f]
+    size_t roi_stride = 0;                // words between ROI planes: H*WW rounded up to 128 bytes (bulk-copy sources)
+    DeviceArray<int> d_roi_idx;           // [2][B] ROI plane of each frame, per result slot (n_roi > 1 only)
     DeviceArray<uint32_t> d_pmask_bits;   // [B][bh][WW] ROI-masked edges (the HoughLinesP mask)
     DeviceArray<uint32_t> d_edge_bits;    // [B][H][WW] Canny map
     DeviceArray<uint32_t> d_cand_bits, d_strong_bits;   // [B][H][WW] candidate / strong planes before hysteresis
     // generic-width fallback (byte maps), allocated on first use
-    DeviceArray<uint8_t> d_cls, d_cls_dbg, d_roi, d_pmask;
-    std::vector<uint8_t> h_roi;
+    DeviceArray<uint8_t> d_cls, d_cls_dbg, d_roi, d_pmask;   // d_roi: [n_roi][H*W]
+    std::vector<uint8_t> h_roi;                               // [n_roi][H*W]
     bool fallback_ready = false, last_cluster = false;
     int last_paths = 0;               // LANE_PATH_* of the chunk that ran last
     DeviceArray<uint8_t> d_gray_dbg;
@@ -94,6 +97,7 @@ struct lane_ctx {
         DeviceArray<lane_record> d_records;          // alive until this slot is enqueued again
         PinnedArray<double> h_prev_fit;              // state in (explicit mode) and state out
         PinnedArray<uint8_t> h_prev_valid;
+        PinnedArray<int32_t> h_roi_idx;              // staging of d_roi_idx (n_roi > 1 only)
         CudaEvent ev[LANE_NUM_STAGES + 1];
         CudaEvent done;
         CudaEvent reader_done;                       // lane_ctx_fence_records: an outside reader of d_records ends here
@@ -176,12 +180,12 @@ int ensure_fallback(lane_ctx *c)
     const size_t P = (size_t)c->g.H * c->g.W, B = (size_t)c->max_batch;
     CU(c->d_cls.alloc(B * P));
     if (c->debug) CU(c->d_cls_dbg.alloc(B * P));
-    CU(c->d_roi.alloc(P));
+    CU(c->d_roi.alloc(P * c->n_roi));
     CU(c->d_pmask.alloc(B * std::max(c->g.bw * c->g.bh, 1)));
     CU(c->d_seedsA.alloc(B * c->seed_cap));
     CU(c->d_seedsB.alloc(B * c->seed_cap));
     CU(c->d_seed_count.alloc(B));
-    CU(cudaMemcpyAsync(c->d_roi, c->h_roi.data(), P, cudaMemcpyHostToDevice, c->st));
+    CU(cudaMemcpyAsync(c->d_roi, c->h_roi.data(), P * c->n_roi, cudaMemcpyHostToDevice, c->st));
     c->fallback_ready = true;
     return LANE_OK;
 }
@@ -222,6 +226,9 @@ int run_stages(lane_ctx *c, const uint8_t *frames_dev, int off, int m, const int
     uint32_t *pmask_bits = c->d_pmask_bits + two * std::max(g.bh, 1) * WW;
     uint32_t *edge_bits = c->d_edge_bits + o * planes, *cb = c->d_cand_bits + o * planes, *sb = c->d_strong_bits + o * planes;
     int32_t *lines = c->d_lines + o * g.max_segments * 4;
+    // ROI plane per frame: null (plane 0 for every frame) on a single-ROI context
+    const int *roi_idx = c->n_roi > 1 ? c->d_roi_idx + two : nullptr;
+    const size_t roi_stride = roi_idx ? c->roi_stride : 0;
 
     if (timed) { rc = mark(c, LANE_STAGE_BLUR_HIST); if (rc) return rc; }
     // Fused edge path (aligned widths, Gaussian blur on): one kernel from BGR frames to NMS survivors, then the
@@ -243,14 +250,14 @@ int run_stages(lane_ctx *c, const uint8_t *frames_dev, int off, int m, const int
                               kb, vp, bd, c->d_task_counter, m, H, W, c->st, LK)) {
             rc = stage_check(c, "k1_fused"); if (rc) return rc;
             if (timed) { rc = mark(c, LANE_STAGE_CANNY); if (rc) return rc; }
-            fused = launch_canny_cluster_fused(kb, vp, hist, c->d_lut, c->d_lut + 511, c->d_roi_bits, thr, pre, pre_redo,
-                                               redo_list, redo_count, redo_flag, nullptr, n_edges, rounds, points, n_points,
+            fused = launch_canny_cluster_fused(kb, vp, hist, c->d_lut, c->d_lut + 511, c->d_roi_bits, roi_idx, roi_stride, thr,
+                                               pre, pre_redo, redo_list, redo_count, redo_flag, nullptr, n_edges, rounds, points, n_points,
                                                pmask_bits, edge_bits, cb, sb, g, m, c->st, LC) &&
                     // frames whose sampled floor was above their true low (normally none): rebuild K / V with the exact
                     // floor and finish them; both kernels return at once when the list is empty
                     launch_fused_edge_redo(fr, redo_list, redo_count, pre_redo, kb, vp, bd, c->d_task_counter, m, H, W, c->st, LC) &&
-                    launch_canny_cluster_fused(kb, vp, hist, c->d_lut, c->d_lut + 511, c->d_roi_bits, thr, pre, pre_redo,
-                                               redo_list, redo_count, redo_flag, redo_list, n_edges, rounds, points, n_points,
+                    launch_canny_cluster_fused(kb, vp, hist, c->d_lut, c->d_lut + 511, c->d_roi_bits, roi_idx, roi_stride, thr,
+                                               pre, pre_redo, redo_list, redo_count, redo_flag, redo_list, n_edges, rounds, points, n_points,
                                                pmask_bits, edge_bits, cb, sb, g, m, c->st, LC);
         }
         if (!fused) fprintf(stderr, "lane_b200: fused edge path rejected by device %d, using the unfused kernels\n", c->device);
@@ -270,7 +277,8 @@ int run_stages(lane_ctx *c, const uint8_t *frames_dev, int off, int m, const int
         launch_blur_hist(fr, blur, hist, m, H, W, c->st, &L[LANE_STAGE_BLUR_HIST], c->blur);
         if (timed) { rc = mark(c, LANE_STAGE_CANNY); if (rc) return rc; }
         c->last_cluster =
-            launch_canny_cluster(blur, hist, c->d_lut, c->d_lut + 511, c->d_roi_bits, thr, n_edges, rounds, points, n_points,
+            launch_canny_cluster(blur, hist, c->d_lut, c->d_lut + 511, c->d_roi_bits, roi_idx, roi_stride, thr, n_edges, rounds,
+                                 points, n_points,
                                  pmask_bits, edge_bits, cb, sb, c->d_task_counter, g, m, c->st, &L[LANE_STAGE_CANNY]);
     }
     if (c->last_cluster) {
@@ -286,10 +294,10 @@ int run_stages(lane_ctx *c, const uint8_t *frames_dev, int off, int m, const int
         launch_hysteresis(cls, seedsA, seedsB, seed_count, c->seed_cap, rounds, m, H, W, c->st, &L[LANE_STAGE_CANNY]);
         launch_finalize_edges(cls, n_edges, m, H, W, c->st, &L[LANE_STAGE_CANNY]);
         if (timed) { rc = mark(c, LANE_STAGE_COMPACT); if (rc) return rc; }
-        launch_compact(cls, c->d_roi, c->d_pmask + o * std::max(g.bw * g.bh, 1), points, n_points, g, m, c->st,
-                       &L[LANE_STAGE_COMPACT]);
+        launch_compact(cls, c->d_roi, roi_idx, roi_idx ? P : 0, c->d_pmask + o * std::max(g.bw * g.bh, 1), points, n_points,
+                       g, m, c->st, &L[LANE_STAGE_COMPACT]);
         launch_bytes_to_bits(cls, edge_bits, m, H, W, W, c->st, &L[LANE_STAGE_COMPACT]);
-        launch_mask_rows(edge_bits, c->d_roi_bits, pmask_bits, g, m, c->st, &L[LANE_STAGE_COMPACT]);
+        launch_mask_rows(edge_bits, c->d_roi_bits, roi_idx, roi_stride, pmask_bits, g, m, c->st, &L[LANE_STAGE_COMPACT]);
     }
     c->last_paths |= c->last_cluster ? LANE_PATH_CLUSTER_CANNY : 0;
     if (c->debug)
@@ -352,6 +360,14 @@ int enqueue(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int
     }
     cudaStream_t hs = c->overlap_now ? c->st2 : c->st;
     if (stream_id) CU(cudaMemcpyAsync(c->d_stream_id, stream_id, sizeof(int) * n, cudaMemcpyHostToDevice, hs));
+    if (c->n_roi > 1) {
+        // The edge kernels read each frame's ROI plane from their own copy of the stream ids, made on the compute stream:
+        // d_stream_id is written on the back half's stream while the fit of the batch before may still read it.
+        if (stream_id) memcpy(sl.h_roi_idx, stream_id, sizeof(int32_t) * n);
+        else memset(sl.h_roi_idx, 0, sizeof(int32_t) * n);
+        CU(cudaMemcpyAsync(c->d_roi_idx + (size_t)c->cur * c->max_batch, sl.h_roi_idx, sizeof(int32_t) * n,
+                           cudaMemcpyHostToDevice, c->st));
+    }
     if (prev_fit) {                                  // explicit state: the caller's; otherwise what the last batch left on the device
         memcpy(sl.h_prev_fit, prev_fit, sizeof(double) * S * 6);
         memcpy(sl.h_prev_valid, prev_valid, (size_t)S * 2);
@@ -433,6 +449,8 @@ int check_call(lane_ctx *c, const void *frames, int n, const int32_t *stream_id,
     if (!frames || n <= 0 || n > c->max_batch) return fail(c, LANE_ERR_INVALID, "bad batch: n=%d (max_batch=%d)", n, c->max_batch);
     if (S <= 0 || (!pf) != (!pv)) return fail(c, LANE_ERR_INVALID, "bad stream state: n_streams=%d", S);
     if (!c->have_roi || !c->have_lut) return fail(c, LANE_ERR_STATE, "lane_set_roi_mask and lane_set_threshold_lut must be called first");
+    if (c->n_roi > 1 && S > c->n_roi)
+        return fail(c, LANE_ERR_INVALID, "n_streams=%d but the context holds %d ROI masks (one per stream)", S, c->n_roi);
     if (pf) {          // explicit state is staged through host buffers: one batch at a time
         if (c->q_count) return fail(c, LANE_ERR_STATE, "a batch is already in flight; call lane_detect_collect");
     } else {           // state carried on the device: a second batch may queue behind the first
@@ -483,6 +501,9 @@ int last_batch(lane_ctx *c, const int *frame_index = nullptr)
     return n;
 }
 
+// Words of one ROI bit-plane: [H][WW], padded to 128 bytes so that every plane's rows are aligned bulk-copy sources.
+size_t roi_plane_words(const LaneGeom &g) { return ((size_t)g.H * ((g.W + 31) / 32) + 31) & ~(size_t)31; }
+
 // The streams, events and buffers a context has from its creation on; the rest are created on first use.
 int create_resources(lane_ctx *c)
 {
@@ -500,7 +521,7 @@ int create_resources(lane_ctx *c)
         CU(sl.done.create(cudaEventDisableTiming));
         CU(sl.reader_done.create(cudaEventDisableTiming));
     }
-    CU(c->d_roi_bits.alloc(H * WW));
+    CU(c->d_roi_bits.alloc(roi_plane_words(c->g)));           // one plane; more are made by lane_set_roi_masks
     CU(c->d_edge_bits.alloc(B * H * WW));
     CU(c->d_cand_bits.alloc(B * H * WW));
     CU(c->d_strong_bits.alloc(B * H * WW));
@@ -581,9 +602,11 @@ int lane_ctx_create(int device, int height, int width, int max_batch, int max_se
 
 void lane_ctx_destroy(lane_ctx *ctx) { delete ctx; }
 
-int lane_set_roi_mask(lane_ctx *c, const uint8_t *mask)
+int lane_set_roi_mask(lane_ctx *c, const uint8_t *mask) { return lane_set_roi_masks(c, mask, 1); }
+
+int lane_set_roi_masks(lane_ctx *c, const uint8_t *masks, int n_masks)
 {
-    if (!c || !mask) return LANE_ERR_INVALID;
+    if (!c || !masks || n_masks < 1) return LANE_ERR_INVALID;
     CU(cudaSetDevice(c->device));
     // Detect calls are refused until every buffer made from the ROI is rebuilt below, so a re-set that fails part way
     // leaves a context without a ROI, not one whose kernels would read released buffers.  The old buffers go before the
@@ -595,29 +618,50 @@ int lane_set_roi_mask(lane_ctx *c, const uint8_t *mask)
     c->d_seedsA.reset(); c->d_seedsB.reset(); c->d_seed_count.reset();
     c->d_pmask_bits.reset(); c->d_points.reset(); c->d_points_dbg.reset();
     c->d_accum16.reset(); c->d_pmask_work.reset(); c->d_list_over.reset();
+    c->d_roi_idx.reset();
+    for (auto &sl : c->slots) sl.h_roi_idx.reset();
+    if (n_masks > 1) c->d_roi_bits.reset();         // one plane stays where lane_ctx_create put it
 
+    // Every buffer and window made from the ROI below comes from the union of the masks: a frame's point list and
+    // HoughLinesP mask hold only its own mask's pixels, and rows or rho windows beyond its own mask's reach stay empty.
+    // The point lists are sized by the largest mask.
     LaneGeom &g = c->g;
+    const size_t P = (size_t)g.H * g.W, WW = (g.W + 31) / 32;
+    const size_t stride = roi_plane_words(g);
+    std::vector<uint8_t> uni(masks, masks + P);
+    std::vector<uint32_t> bits(stride * n_masks, 0u);
     int x0 = g.W, y0 = g.H, x1 = -1, y1 = -1, cnt = 0;
-    for (int y = 0; y < g.H; y++)
-        for (int x = 0; x < g.W; x++)
-            if (mask[(size_t)y * g.W + x]) {
-                x0 = std::min(x0, x); x1 = std::max(x1, x); y0 = std::min(y0, y); y1 = std::max(y1, y);
-                cnt++;
-            }
-    if (cnt == 0) { x0 = y0 = 0; x1 = y1 = -1; }
+    for (int r = 0; r < n_masks; r++) {
+        const uint8_t *mask = masks + r * P;
+        uint32_t *plane = bits.data() + r * stride;
+        int mask_cnt = 0;
+        for (int y = 0; y < g.H; y++)
+            for (int x = 0; x < g.W; x++)
+                if (mask[(size_t)y * g.W + x]) {
+                    x0 = std::min(x0, x); x1 = std::max(x1, x); y0 = std::min(y0, y); y1 = std::max(y1, y);
+                    mask_cnt++;
+                    uni[(size_t)y * g.W + x] = 1;
+                    plane[(size_t)y * WW + (x >> 5)] |= 1u << (x & 31);
+                }
+        cnt = std::max(cnt, mask_cnt);
+    }
+    if (x1 < 0) { x0 = y0 = 0; x1 = y1 = -1; }
     g.bx0 = x0; g.by0 = y0; g.bx1 = x1 + 1; g.by1 = y1 + 1;
     g.bw = g.bx1 - g.bx0; g.bh = g.by1 - g.by0;
     g.max_points = cnt;
-    const size_t P = (size_t)g.H * g.W, WW = (g.W + 31) / 32;
-    c->h_roi.assign(mask, mask + P);
-    std::vector<uint32_t> bits((size_t)g.H * WW, 0u);
-    for (int y = 0; y < g.H; y++)
-        for (int x = 0; x < g.W; x++)
-            if (mask[(size_t)y * g.W + x]) bits[(size_t)y * WW + (x >> 5)] |= 1u << (x & 31);
+    c->n_roi = n_masks;
+    c->roi_stride = stride;
+    c->h_roi.assign(masks, masks + P * n_masks);
+    CU(c->d_roi_bits.grow(bits.size()));
     CU(cudaMemcpy(c->d_roi_bits, bits.data(), sizeof(uint32_t) * bits.size(), cudaMemcpyHostToDevice));
+    if (n_masks > 1) {
+        CU(c->d_roi_idx.alloc(2 * (size_t)c->max_batch));
+        CU(cudaMemset(c->d_roi_idx, 0, sizeof(int) * 2 * (size_t)c->max_batch));   // valid planes for taps of an older batch
+        for (auto &sl : c->slots) CU(sl.h_roi_idx.alloc((size_t)c->max_batch));
+    }
     {
         int2 win[LANE_NUM_ANGLES];
-        c->cells_per_frame = lane_ppht_windows(mask, g.H, g.W, win);
+        c->cells_per_frame = lane_ppht_windows(uni.data(), g.H, g.W, win);
         CU(cudaMemcpy(c->d_win, win, sizeof(win), cudaMemcpyHostToDevice));
         CU(c->d_accum16.alloc((size_t)c->max_batch * (c->cells_per_frame / 2)));
         int2 win3[LANE_NUM_ANGLES];
@@ -935,8 +979,10 @@ int lane_hough_lines_batch(lane_ctx *c, int threshold, int max_peaks, int32_t *p
     }
     if (accum_host) CU(c->d_hb_accum.lazy(B * cells));
     CU(cudaEventRecord(c->hb_ev[0], c->st));
-    if (!launch_hough_batch(c->d_edge_bits, c->d_roi_bits, accum_host ? c->d_hb_accum.get() : nullptr, c->d_hb_tmp, c->d_hb_sorted,
-                            c->d_hb_count, g, threshold, max_peaks, n, c->st))
+    const int *roi_idx = c->n_roi > 1 ? c->d_roi_idx + (size_t)c->cur * B : nullptr;
+    if (!launch_hough_batch(c->d_edge_bits, c->d_roi_bits, roi_idx, roi_idx ? c->roi_stride : 0,
+                            accum_host ? c->d_hb_accum.get() : nullptr, c->d_hb_tmp, c->d_hb_sorted, c->d_hb_count, g, threshold,
+                            max_peaks, n, c->st))
         return fail(c, LANE_ERR_UNSUPPORTED, "frame %dx%d: a Hough row does not fit shared memory", g.W, g.H);
     CU(cudaEventRecord(c->hb_ev[1], c->st));
     CU(cudaMemcpyAsync(n_peaks_host, c->d_hb_count, sizeof(int) * n, cudaMemcpyDeviceToHost, c->st));

@@ -26,10 +26,10 @@
 
 struct LaneGeom {
     int H, W;
-    int bx0, by0, bx1, by1;   // ROI bounding box [bx0,bx1) x [by0,by1); empty => bx1 <= bx0
+    int bx0, by0, bx1, by1;   // bounding box [bx0,bx1) x [by0,by1) of the ROI (of all ROI planes); empty => bx1 <= bx0
     int bw, bh;               // bbox size
     int numrho;               // 2*(W+H)+1
-    int max_points;           // non-zero pixels of the ROI mask (upper bound of the point list)
+    int max_points;           // non-zero pixels of the largest ROI mask (upper bound of the point list)
     int max_segments;
 };
 
@@ -83,26 +83,30 @@ void launch_hysteresis(uint8_t *cls, int *seeds, int *seeds2, const int *seed_co
                        int *rounds, int n, int H, int W, cudaStream_t st, int *launches);
 // cls (>=2) -> edges 0/255 in place, n_edges per frame
 void launch_finalize_edges(uint8_t *cls_edges, int *n_edges, int n, int H, int W, cudaStream_t st, int *launches);
-// ROI mask + ordered compaction: points[f][k] = (y<<16)|x in row-major order; pmask = bbox-sized byte mask
-void launch_compact(const uint8_t *edges, const uint8_t *roi, uint8_t *pmask, uint32_t *points, int *n_points,
-                    LaneGeom g, int n, cudaStream_t st, int *launches);
+// ROI mask + ordered compaction: points[f][k] = (y<<16)|x in row-major order; pmask = bbox-sized byte mask.
+// ROI planes (here and in every launcher below): frame f uses roi + roi_index[f] * roi_stride; a null roi_index means
+// plane 0 for every frame.  The bounding box in g covers every plane.
+void launch_compact(const uint8_t *edges, const uint8_t *roi, const int *roi_index, size_t roi_stride, uint8_t *pmask,
+                    uint32_t *points, int *n_points, LaneGeom g, int n, cudaStream_t st, int *launches);
 
 // cluster form of K2 (bit-planes in distributed shared memory); false => geometry not supported, use the kernels above
 bool launch_canny_cluster(const uint8_t *blur, const uint32_t *hist, const uint8_t *lut_low, const uint8_t *lut_high,
-                          const uint32_t *roi_bits, int4 *thr, int *n_edges, int *rounds, uint32_t *points,
+                          const uint32_t *roi_bits, const int *roi_index, size_t roi_stride, int4 *thr, int *n_edges,
+                          int *rounds, uint32_t *points,
                           int *n_points, uint32_t *pmask_bits, uint32_t *edge_bits, uint32_t *c_bits, uint32_t *s_bits,
                           int *task_counter, LaneGeom g, int n, cudaStream_t st, int *launches);
 bool launch_canny_cluster_fused(const uint32_t *k_bits, const uint8_t *v_plane, const uint32_t *hist, const uint8_t *lut_low,
-                                const uint8_t *lut_high, const uint32_t *roi_bits, int4 *thr, const int *pre, int *pre_redo,
-                                int *redo_list, int *redo_count, int *redo_flag, const int *frame_list, int *n_edges,
-                                int *rounds, uint32_t *points, int *n_points, uint32_t *pmask_bits, uint32_t *edge_bits,
-                                uint32_t *c_bits, uint32_t *s_bits, LaneGeom g, int n, cudaStream_t st, int *launches);
+                                const uint8_t *lut_high, const uint32_t *roi_bits, const int *roi_index, size_t roi_stride,
+                                int4 *thr, const int *pre, int *pre_redo, int *redo_list, int *redo_count, int *redo_flag,
+                                const int *frame_list, int *n_edges, int *rounds, uint32_t *points, int *n_points,
+                                uint32_t *pmask_bits, uint32_t *edge_bits, uint32_t *c_bits, uint32_t *s_bits, LaneGeom g, int n,
+                                cudaStream_t st, int *launches);
 void launch_edge_count_rect(const uint32_t *edge_bits, int *counts, int n, int H, int W, int x0, int y0, int x1, int y1,
                             cudaStream_t st);
 void launch_bytes_to_bits(const uint8_t *bytes, uint32_t *bits, int n, int rows, int W, int row_stride,
                           cudaStream_t st, int *launches);
-void launch_mask_rows(const uint32_t *edge_bits, const uint32_t *roi_bits, uint32_t *pmask_bits, LaneGeom g, int n,
-                      cudaStream_t st, int *launches);
+void launch_mask_rows(const uint32_t *edge_bits, const uint32_t *roi_bits, const int *roi_index, size_t roi_stride,
+                      uint32_t *pmask_bits, LaneGeom g, int n, cudaStream_t st, int *launches);
 
 // ---- K3 ---------------------------------------------------------------------------------
 void launch_hough_accum(const uint32_t *points, const int *n_points, int32_t *accum_padded, LaneGeom g,
@@ -110,9 +114,9 @@ void launch_hough_accum(const uint32_t *points, const int *n_points, int32_t *ac
 void launch_hough_peaks(const int32_t *accum_padded, int numrho, int threshold, int2 *peaks, int max_peaks,
                         int *n_peaks, cudaStream_t st);
 // batched form: every frame of the batch, from the edge bit-planes (edge & ROI), peaks ordered on the device
-bool launch_hough_batch(const uint32_t *edge_bits, const uint32_t *roi_bits, int32_t *accum, int2 *peaks_tmp,
-                        int32_t *peaks_sorted, int *n_peaks, LaneGeom g, int threshold, int max_peaks, int n,
-                        cudaStream_t st);
+bool launch_hough_batch(const uint32_t *edge_bits, const uint32_t *roi_bits, const int *roi_index, size_t roi_stride,
+                        int32_t *accum, int2 *peaks_tmp, int32_t *peaks_sorted, int *n_peaks, LaneGeom g, int threshold,
+                        int max_peaks, int n, cudaStream_t st);
 void lane_upload_tables();       // trig tables -> __constant__ (both Hough variants)
 void lane_upload_tables_std();
 

@@ -59,23 +59,61 @@ class LaneDetector:
         self._ctx_key = None
         self._dense_ctx: Optional[_native.LaneContext] = None   # larger max_segments, for frames the default truncated
         self._dense_key = None
+        self._roi_cache = {}        # (h, w, vertex key) -> rasterised ROI mask
         self.dense_reruns = 0       # chunks re-run because HoughLinesP found more segments than max_segments
         self._stream_fit = None     # float64 [S,2,3] for detect_streams
         self._stream_valid = None   # uint8  [S,2]
         self.last_records = None    # RECORD_DTYPE array of the last call (diagnostics)
 
     # ------------------------------------------------------------------ static inputs
-    def _get_roi_mask(self, shape: Tuple[int, int]) -> np.ndarray:
-        """ROI mask exactly as the reference rasterises it (lane_detector.py:47-64)."""
+    def _get_roi_mask(self, shape: Tuple[int, int], vertices=None) -> np.ndarray:
+        """ROI mask exactly as the reference rasterises it (lane_detector.py:47-64), of ``vertices`` when given, else
+        of ``roi_vertices`` or the default trapezoid."""
         h, w = shape[:2]
-        if self.roi_vertices is not None:
+        if vertices is None:
             vertices = self.roi_vertices
-        else:
+        if vertices is None:
             vertices = np.array([[(int(w * 0.1), h), (int(w * 0.4), int(h * 0.6)),
                                   (int(w * 0.6), int(h * 0.6)), (int(w * 0.9), h)]], dtype=np.int32)
         mask = np.zeros((h, w), dtype=np.uint8)
         cv2.fillPoly(mask, vertices, 255)
         return mask
+
+    @staticmethod
+    def _vertex_key(vertices):
+        if vertices is None:
+            return None
+        a = np.asarray(vertices)
+        return a.shape, a.dtype.str, a.tobytes()
+
+    def _roi_key(self, stream_rois, n_masks: int):
+        """Key of the context's mask set: one ROI (``stream_rois`` None), or ``n_masks`` masks, one per stream, where an
+        entry of None is the detector's own ROI and streams past the end of ``stream_rois`` get an empty mask (no frame
+        of the call belongs to them; they only make room for the streams whose smoothing state the detector holds)."""
+        own = self._vertex_key(self.roi_vertices)
+        if stream_rois is None:
+            return (own,)
+        keys = [own if v is None else self._vertex_key(v) for v in stream_rois]
+        return tuple(keys) + ("empty",) * (n_masks - len(keys))
+
+    def _roi_masks(self, h: int, w: int, roi_key, stream_rois) -> np.ndarray:
+        """The masks of ``roi_key``: ``(H, W)`` for one ROI, else ``(R, H, W)``.  Rasterised masks are cached by their
+        vertices, so a rig's masks are drawn once."""
+        if len(self._roi_cache) > 256:
+            self._roi_cache.clear()
+        masks = []
+        for i, k in enumerate(roi_key):
+            ck = (h, w, k)
+            m = self._roi_cache.get(ck)
+            if m is None:
+                if k == "empty":
+                    m = np.zeros((h, w), np.uint8)
+                else:
+                    v = None if stream_rois is None or stream_rois[i] is None else stream_rois[i]
+                    m = self._get_roi_mask((h, w), v)
+                self._roi_cache[ck] = m
+            masks.append(m)
+        return masks[0] if stream_rois is None else np.stack(masks)
 
     def _device_index(self, frames=None) -> int:
         """GPU the context lives on: the device of a CUDA tensor input, else ``device=``, else torch's current one."""
@@ -95,14 +133,14 @@ class LaneDetector:
             pass
         return 0
 
-    def _context(self, h: int, w: int, n: int, frames=None) -> _native.LaneContext:
-        roi_key = None if self.roi_vertices is None else np.asarray(self.roi_vertices).tobytes()
+    def _context(self, h: int, w: int, n: int, frames=None, stream_rois=None, n_masks: int = 1) -> _native.LaneContext:
+        roi_key = self._roi_key(stream_rois, n_masks)
         key = (h, w, roi_key, self._device_index(frames))
         if self._ctx is None or self._ctx_key != key or self._ctx.max_batch < min(n, self._max_batch):
             if self._ctx is not None:
                 self._ctx.close()
             cap = max(min(n, self._max_batch), 1)
-            self._ctx = _native.LaneContext(h, w, cap, self._get_roi_mask((h, w)), device=key[3],
+            self._ctx = _native.LaneContext(h, w, cap, self._roi_masks(h, w, roi_key, stream_rois), device=key[3],
                                             max_segments=self._max_segments, debug=self._debug)
             self._ctx_key = key
         return self._ctx
@@ -140,16 +178,17 @@ class LaneDetector:
         return out
 
     def _run(self, frames, stream_id, n_streams, prev_fit, prev_valid, fmt: int = _native.INPUT_BGR,
-             target_size: Optional[Tuple[int, int]] = None) -> np.ndarray:
+             target_size: Optional[Tuple[int, int]] = None, stream_rois=None) -> np.ndarray:
         """Chunked native calls over frames [N,H,W,3] (numpy or CUDA torch; [N,H*3/2,W] for the YUV 4:2:0 layouts of
         ``fmt``), detected at ``target_size`` = (width, height) when given (the device resizes every frame to it first);
-        state arrays updated in place."""
+        state arrays updated in place.  ``stream_rois``: one ROI per stream (see ``detect_streams``)."""
         n, sh, sw = int(frames.shape[0]), int(frames.shape[1]), int(frames.shape[2])
         if fmt != _native.INPUT_BGR:
             sh = sh * 2 // 3
         fbytes = sh * sw * 3 if fmt == _native.INPUT_BGR else sh * sw * 3 // 2
         h, w = (sh, sw) if target_size is None else (target_size[1], target_size[0])
-        ctx = self._context(h, w, n, frames)
+        n_masks = 1 if stream_rois is None else max(len(stream_rois), n_streams)
+        ctx = self._context(h, w, n, frames, stream_rois, n_masks)
         s, oms = self.smoothing_factor, 1 - self.smoothing_factor
         chunks = []
         on_device = _is_torch_cuda(frames)
@@ -174,7 +213,7 @@ class LaneDetector:
                 # otherwise be fitted on a truncated list.  Re-run the chunk, from the state it started with, on a context
                 # sized for what was found (the reference result, just slower), never return a truncated fit silently.
                 prev_fit[...], prev_valid[...] = fit0, valid0
-                dense = self._dense_context(h, w, int(recs["n_segments_found"].max()), ctx.device)
+                dense = self._dense_context(h, w, int(recs["n_segments_found"].max()), ctx.device, stream_rois, n_masks)
                 recs = np.concatenate([call(dense, i, min(i + dense.max_batch, b)) for i in range(a, b, dense.max_batch)])
                 if recs["flags"].any():
                     raise _native.LaneError(-5, "segment list still truncated after the dense re-run")
@@ -184,15 +223,16 @@ class LaneDetector:
         self.last_records = recs
         return recs
 
-    def _dense_context(self, h: int, w: int, need: int, device: int) -> _native.LaneContext:
+    def _dense_context(self, h: int, w: int, need: int, device: int, stream_rois=None,
+                       n_masks: int = 1) -> _native.LaneContext:
         cap = 1 << max(int(need) - 1, 1).bit_length()
-        roi_key = None if self.roi_vertices is None else np.asarray(self.roi_vertices).tobytes()
+        roi_key = self._roi_key(stream_rois, n_masks)
         key = (h, w, roi_key, device)
         if self._dense_ctx is None or self._dense_key != key or self._dense_ctx.max_segments < need:
             if self._dense_ctx is not None:
                 self._dense_ctx.close()
-            self._dense_ctx = _native.LaneContext(h, w, 8, self._get_roi_mask((h, w)), device=device, max_segments=cap,
-                                                  debug=self._debug)
+            self._dense_ctx = _native.LaneContext(h, w, 8, self._roi_masks(h, w, roi_key, stream_rois), device=device,
+                                                  max_segments=cap, debug=self._debug)
             self._dense_key = key
         self._ctx.copy_settings_to(self._dense_ctx)
         return self._dense_ctx
@@ -352,11 +392,18 @@ class LaneDetector:
         self._adopt_state(lanes)
         return lanes
 
-    def detect_streams(self, frames, stream_ids: Optional[Sequence[int]] = None) -> List[LanePair]:
+    def detect_streams(self, frames, stream_ids: Optional[Sequence[int]] = None, *,
+                       stream_rois: Optional[Sequence[Optional[np.ndarray]]] = None) -> List[LanePair]:
         """Multi-camera form: ``frames`` is [S,T,H,W,3] (stream-major) or [N,H,W,3] with ``stream_ids[N]``.
 
         Every stream keeps its own smoothing state inside this detector (``reset`` clears all of them);
         frames of one stream must be in temporal order.  Returns one pair per frame, in input order.
+
+        ``stream_rois`` gives every camera its own ROI: entry s is stream s's polygon in ``roi_vertices`` form (int32
+        [1,K,2], rasterised with ``cv2.fillPoly`` as the reference does), or None for this detector's own ROI.  It needs
+        an entry for every stream id of the call (``ValueError`` otherwise).  Stream s's results then equal those of
+        ``LaneDetector(roi_vertices=stream_rois[s])`` run on that stream's frames in order, and the whole rig still runs
+        as one batched call.  Without it, every stream uses this detector's ROI.
         """
         if len(frames.shape) == 5:
             s_, t_ = int(frames.shape[0]), int(frames.shape[1])
@@ -371,6 +418,10 @@ class LaneDetector:
         if frames.shape[0] == 0:
             return []
         n_streams = int(stream_ids.max()) + 1
+        if stream_rois is not None:
+            stream_rois = list(stream_rois)
+            if len(stream_rois) < n_streams:
+                raise ValueError(f"stream_rois has {len(stream_rois)} entries; stream id {n_streams - 1} needs {n_streams}")
         if self._stream_fit is None or self._stream_fit.shape[0] < n_streams:
             fit = np.zeros((n_streams, 2, 3), np.float64)
             valid = np.zeros((n_streams, 2), np.uint8)
@@ -378,7 +429,8 @@ class LaneDetector:
                 k = self._stream_fit.shape[0]
                 fit[:k], valid[:k] = self._stream_fit, self._stream_valid
             self._stream_fit, self._stream_valid = fit, valid
-        recs = self._run(frames, stream_ids, self._stream_fit.shape[0], self._stream_fit, self._stream_valid)
+        recs = self._run(frames, stream_ids, self._stream_fit.shape[0], self._stream_fit, self._stream_valid,
+                         stream_rois=stream_rois)
         return self._lanes_from_records(recs)
 
     def draw_lanes(self, frame: np.ndarray, left_lane: Optional[LaneLine], right_lane: Optional[LaneLine],
