@@ -146,6 +146,32 @@ LANE_API int lane_detect_batch_ingest(lane_ctx *ctx, const uint8_t *frames, int 
                                       int src_h, int src_w, const int32_t *stream_id, int n_streams, double *prev_fit,
                                       uint8_t *prev_valid, lane_record *out);
 
+/* One camera of a rig in a lane_detect_rig call. */
+typedef struct lane_rig_source {
+    const uint8_t *frames;   /* n dense frames of one camera in `format` at src_h x src_w (host or device, per the call) */
+    int32_t format;          /* LANE_INPUT_BGR / NV12 / I420 */
+    int32_t src_h, src_w;    /* the camera's own size (even for NV12 / I420) */
+    int32_t n;               /* frames of this camera in the call, in temporal order; 0 = none this tick */
+    int32_t stream_id;       /* the camera: index into prev_fit / prev_valid and the ROI masks */
+} lane_rig_source;
+
+/* A rig whose cameras differ in resolution and decoder layout, in one batched call: every camera's frames as
+ * VideoDataLoader.read_frame delivers them (/root/reference/data/loaders/video_loader.py:96-131, decode + cv2.resize to
+ * target_size) to LaneDetector.detect (lane_detector.py:178-218), with its own smoothing state and, on a context with
+ * one ROI mask per stream (lane_set_roi_masks), its own ROI.  One kernel makes the context's height x width BGR frames of
+ * all sources -- per frame cv2.resize(cv2.cvtColor(f, COLOR_YUV2BGR_NV12 | COLOR_YUV2BGR_I420), (width, height)), or
+ * cv2.resize(f, (width, height)) for BGR -- and the path runs once for the whole rig.  Host sources are copied chunk by
+ * chunk behind the compute; only their own bytes cross PCIe.
+ *   sources        n_sources cameras; frames_on_device selects host or device memory for all of them.
+ *   n_streams, prev_fit, prev_valid   as for lane_detect_batch (both state arrays required).
+ *   out            host lane_record[sum of n], the frames in source order.
+ * Camera s's records equal those of lane_detect_batch_ingest on its frames alone with its stream's state and mask.
+ * Blocking.  LANE_ERR_INVALID: null pointers, a sum of n of 0 or above max_batch, a negative n, an unknown format, a
+ * non-positive size or an odd YUV size, stream_id outside [0, n_streams), n_streams above the context's masks (when
+ * it holds more than one). */
+LANE_API int lane_detect_rig(lane_ctx *ctx, const lane_rig_source *sources, int n_sources, int frames_on_device,
+                             int n_streams, double *prev_fit, uint8_t *prev_valid, lane_record *out);
+
 /* Asynchronous split of the above for pipelined callers: enqueue (device frames only; records
  * land in an internal pinned buffer), then collect (waits for the OLDEST batch in flight and returns
  * its records and the EMA state after it).
@@ -202,6 +228,8 @@ LANE_API int lane_get_stage_ms(lane_ctx *ctx, float ms[LANE_NUM_STAGES], int32_t
 #define LANE_TAP_POINTS 5           /* int32 [n_roi_points][2] (x,y) row-major order of masked edges (:89) */
 #define LANE_TAP_SEGMENTS 6         /* int32 [n_segments][4] HoughLinesP output (:94-101) */
 #define LANE_TAP_GRAY 7             /* uint8 [H][W]   cv2.cvtColor output (:69); recomputed on demand */
+#define LANE_TAP_FRAME 8            /* uint8 [H][W][3] the BGR frame the path ran on (ingest output; device BGR input at
+                                       the context's size is read where the caller keeps it); needs no debug mode */
 /* Copies tap `what` of frame `frame_index` of the last batch to host memory; *bytes_written is set. */
 LANE_API int lane_debug_tap(lane_ctx *ctx, int what, int frame_index, void *host_out, size_t capacity,
                    size_t *bytes_written);

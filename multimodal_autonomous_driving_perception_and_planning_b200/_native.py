@@ -19,7 +19,7 @@ LIB_PATH = os.environ.get("LANE_B200_LIB") or os.path.join(CSRC, "liblane_b200.s
 NUM_POINTS = 50
 NUM_STAGES = 7
 STAGE_NAMES = ("h2d", "blur_hist", "canny", "compact", "ppht", "fit", "d2h")
-TAP_BLUR, TAP_HIST, TAP_CLASS, TAP_EDGES, TAP_POINTS, TAP_SEGMENTS, TAP_GRAY = 1, 2, 3, 4, 5, 6, 7
+TAP_BLUR, TAP_HIST, TAP_CLASS, TAP_EDGES, TAP_POINTS, TAP_SEGMENTS, TAP_GRAY, TAP_FRAME = 1, 2, 3, 4, 5, 6, 7, 8
 FLAG_SEGMENTS_TRUNCATED, FLAG_POINTS_TRUNCATED = 1, 2
 PATH_FUSED_EDGE, PATH_CLUSTER_CANNY, PATH_PPHT_DSMEM = 1, 2, 4
 PATH_ALL_FAST = 7
@@ -38,6 +38,12 @@ class LaneRecord(C.Structure):
                 ("median_x2", C.c_int32), ("low", C.c_int32), ("high", C.c_int32), ("n_edges", C.c_int32),
                 ("n_roi_points", C.c_int32), ("n_segments", C.c_int32), ("hysteresis_rounds", C.c_int32),
                 ("flags", C.c_int32), ("n_segments_found", C.c_int32)]
+
+
+class LaneRigSource(C.Structure):
+    """lane_rig_source: one camera of a lane_detect_rig call."""
+    _fields_ = [("frames", C.c_void_p), ("format", C.c_int32), ("src_h", C.c_int32), ("src_w", C.c_int32),
+                ("n", C.c_int32), ("stream_id", C.c_int32)]
 
 
 # numpy view of lane_record (same layout) so batches decode without a Python loop per field
@@ -96,6 +102,7 @@ _PROTOS = {
                                          C.c_void_p, C.c_void_p]),
     "lane_detect_batch_ingest": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                            C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "lane_detect_rig": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "lane_nv12_to_bgr_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "lane_yuv420_to_bgr_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int,
                                            C.c_int, C.c_int, C.c_void_p]),
@@ -272,6 +279,24 @@ class LaneContext:
                                                _ptr(prev_fit), _ptr(prev_valid), _ptr(self._records)))
         return self._records[:n].copy()
 
+    def detect_rig(self, sources, on_device: bool, n_streams: int, prev_fit: np.ndarray, prev_valid: np.ndarray,
+                   smoothing: float, one_minus: float) -> np.ndarray:
+        """One call for cameras of different sizes and layouts (lane_detect_rig).  ``sources``: one tuple
+        ``(frames, fmt, (h, w), n, stream_id)`` per camera, ``frames`` an int device pointer (on_device) or a C-contiguous
+        uint8 ndarray of ``n`` frames in layout ``fmt`` (INPUT_*) at size (h, w).  State arrays as for ``detect``.
+        Returns the records of all frames in source order (a copy)."""
+        L = lib()
+        self._check(L.lane_set_smoothing(self._h, float(smoothing), float(one_minus)))
+        arr = (LaneRigSource * max(len(sources), 1))()
+        total = 0
+        for i, (frames, fmt, (h, w), n, sid) in enumerate(sources):
+            fp = frames if on_device else (frames.ctypes.data if n else None)
+            arr[i] = LaneRigSource(fp, int(fmt), int(h), int(w), int(n), int(sid))
+            total += int(n)
+        self._check(L.lane_detect_rig(self._h, arr, len(sources), int(on_device), n_streams, _ptr(prev_fit),
+                                      _ptr(prev_valid), _ptr(self._records)))
+        return self._records[:total].copy()
+
     def enqueue(self, frames_ptr: int, n: int, stream_id, n_streams, prev_fit, prev_valid, smoothing, one_minus):
         """Asynchronous form for device-resident frames.  With ``prev_fit`` / ``prev_valid`` the batch starts from that
         state (one batch in flight).  With both ``None`` it continues from the state the previous batch left on the
@@ -300,6 +325,8 @@ class LaneContext:
         h, w = self.height, self.width
         if what in (TAP_BLUR, TAP_CLASS, TAP_EDGES, TAP_GRAY):
             out = np.empty((h, w), np.uint8)
+        elif what == TAP_FRAME:
+            out = np.empty((h, w, 3), np.uint8)
         elif what == TAP_HIST:
             out = np.empty(256, np.uint32)
         elif what == TAP_POINTS:

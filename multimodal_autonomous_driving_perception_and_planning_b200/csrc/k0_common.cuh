@@ -79,6 +79,74 @@ __device__ __forceinline__ uint32_t k0_vmix(int h0, int h1, int b0, int b1)
     return (uint32_t)min(v, 255);
 }
 
+// The per-thread pixel work of the resize kernels (k0_resize, k0_yuv420_resize, k0_rig_ingest): one thread makes PX
+// consecutive destination pixels dx0 .. dx0+PX-1 of destination row dy (columns past dw repeat the last one and are not
+// stored).  yy / b: the row's yofs / beta entries.
+//
+// k0_resize's arithmetic on CN interleaved uint8 channels: r0 / r1 are the two source rows.
+template <int CN, int PX>
+__device__ __forceinline__ void k0_resize_px(const uint8_t *__restrict__ r0, const uint8_t *__restrict__ r1,
+                                             const int *__restrict__ xofs, const short2 *__restrict__ alpha, short2 b, int sw,
+                                             int dx0, int dw, uint8_t (&px)[PX * CN])
+{
+#pragma unroll
+    for (int k = 0; k < PX; k++) {
+        const int dx = min(dx0 + k, dw - 1);
+        const int x0 = __ldg(xofs + dx), x1 = min(x0 + 1, sw - 1);
+        const short2 a = __ldg(alpha + dx);
+#pragma unroll
+        for (int c = 0; c < CN; c++) {
+            const int h0 = (int)__ldg(r0 + x0 * CN + c) * a.x + (int)__ldg(r0 + x1 * CN + c) * a.y;
+            const int h1 = (int)__ldg(r1 + x0 * CN + c) * a.x + (int)__ldg(r1 + x1 * CN + c) * a.y;
+            px[k * CN + c] = (uint8_t)k0_vmix(h0, h1, b.x, b.y);
+        }
+    }
+}
+
+// The same resize of the BGR frame cv2.cvtColor makes of YUV 4:2:0 frame `s` (sh x sw luma, layout FMT): the two source
+// rows x two source columns of every tap are converted on the fly, the converted frame is never stored.
+template <int FMT, int PX>
+__device__ __forceinline__ void k0_yuv420_resize_px(const uint8_t *__restrict__ s, int sh, int sw, int2 yy, short2 b,
+                                                    const int *__restrict__ xofs, const short2 *__restrict__ alpha, int dx0,
+                                                    int dw, uint8_t (&o)[PX * 3])
+{
+    using namespace k0yuv;
+    const uint8_t *l0 = s + (size_t)yy.x * sw, *l1 = s + (size_t)yy.y * sw;
+#pragma unroll
+    for (int k = 0; k < PX; k++) {
+        const int dx = min(dx0 + k, dw - 1);
+        const int x0 = __ldg(xofs + dx), x1 = min(x0 + 1, sw - 1);
+        const short2 a = __ldg(alpha + dx);
+        uint32_t p00[3], p01[3], p10[3], p11[3];     // BGR of (row y0 | y1) x (column x0 | x1)
+        px(__ldg(l0 + x0), chroma<FMT>(s, sh, sw, yy.x >> 1, x0 >> 1), p00[0], p00[1], p00[2]);
+        px(__ldg(l0 + x1), chroma<FMT>(s, sh, sw, yy.x >> 1, x1 >> 1), p01[0], p01[1], p01[2]);
+        px(__ldg(l1 + x0), chroma<FMT>(s, sh, sw, yy.y >> 1, x0 >> 1), p10[0], p10[1], p10[2]);
+        px(__ldg(l1 + x1), chroma<FMT>(s, sh, sw, yy.y >> 1, x1 >> 1), p11[0], p11[1], p11[2]);
+#pragma unroll
+        for (int c = 0; c < 3; c++) {
+            const int h0 = (int)p00[c] * a.x + (int)p01[c] * a.y;
+            const int h1 = (int)p10[c] * a.x + (int)p11[c] * a.y;
+            o[k * 3 + c] = (uint8_t)k0_vmix(h0, h1, b.x, b.y);
+        }
+    }
+}
+
+// Stores one thread's pixels at `out` (destination pixel dx0): packed 4-byte stores when the PX pixels are all inside
+// the row and `out` is aligned, byte stores otherwise.
+template <int CN, int PX>
+__device__ __forceinline__ void k0_store_px(uint8_t *__restrict__ out, const uint8_t (&px)[PX * CN], int dx0, int dw)
+{
+    if (dx0 + PX <= dw && ((uintptr_t)out & 3) == 0 && (PX * CN) % 4 == 0) {
+#pragma unroll
+        for (int q = 0; q < PX * CN / 4; q++)
+            reinterpret_cast<uint32_t *>(out)[q] = (uint32_t)px[4 * q] | ((uint32_t)px[4 * q + 1] << 8) |
+                                                   ((uint32_t)px[4 * q + 2] << 16) | ((uint32_t)px[4 * q + 3] << 24);
+    } else {
+        for (int k = 0; k < PX && dx0 + k < dw; k++)
+            for (int c = 0; c < CN; c++) out[k * CN + c] = px[k * CN + c];
+    }
+}
+
 // Tables for the current device (cached; the first call of a geometry allocates and uploads them synchronously).
 cudaError_t lane_resize_taps(int sh, int sw, int dh, int dw, ResizeTaps *t);
 // k0_resize over n dense frames of `channels` (1 or 3) uint8 planes; device pointers, enqueued on st, no checks.
@@ -94,3 +162,19 @@ void launch_yuv420_to_bgr(const uint8_t *src, int format, uint8_t *dst, int n, i
 // not taken.  Device pointers, enqueued on st; the caller has validated the sizes (even YUV sizes, grid limits).
 cudaError_t launch_ingest(const uint8_t *src, int format, int n, int sh, int sw, uint8_t *dst, int dh, int dw,
                           cudaStream_t st);
+
+// ---- rig ingest: a batch whose frames each have their own layout and size -> BGR at dh x dw, one launch ------------
+// Descriptor of one source frame (device memory, dense); the tap tables are lane_resize_taps' cached ones.
+struct RigFrame {
+    const uint8_t *src;
+    int format, sh, sw;                // LANE_INPUT_*; YUV sizes even
+    const int *xofs;
+    const short2 *alpha;
+    const int2 *yofs;
+    const short2 *beta;
+};
+// The descriptor of frame `src` for a destination of dh x dw (looks up / builds the geometry's tap tables).
+cudaError_t rig_frame(const uint8_t *src, int format, int sh, int sw, int dh, int dw, RigFrame *d);
+// k0_rig_ingest over n frames: frames_dev = device RigFrame[n], dst = [n][dh][dw][3]; enqueued on st, no checks
+// (n and dh up to 65535).
+void launch_rig_ingest(const RigFrame *frames_dev, int n, uint8_t *dst, int dh, int dw, cudaStream_t st);

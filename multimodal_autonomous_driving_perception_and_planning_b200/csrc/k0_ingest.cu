@@ -29,38 +29,57 @@ __global__ void __launch_bounds__(256) k0_yuv420_resize(const uint8_t *__restric
     const int2 yy = __ldg(yofs + dy);
     const short2 b = __ldg(beta + dy);
     const uint8_t *s = src + (size_t)f * sh * sw * 3 / 2;
-    const uint8_t *l0 = s + (size_t)yy.x * sw, *l1 = s + (size_t)yy.y * sw;
     uint8_t *out = dst + (((size_t)f * dh + dy) * dw + dx0) * 3;
     uint8_t o[PX * 3];
-#pragma unroll
-    for (int k = 0; k < PX; k++) {
-        const int dx = min(dx0 + k, dw - 1);
-        const int x0 = __ldg(xofs + dx), x1 = min(x0 + 1, sw - 1);
-        const short2 a = __ldg(alpha + dx);
-        uint32_t p00[3], p01[3], p10[3], p11[3];     // BGR of (row y0 | y1) x (column x0 | x1)
-        px(__ldg(l0 + x0), chroma<FMT>(s, sh, sw, yy.x >> 1, x0 >> 1), p00[0], p00[1], p00[2]);
-        px(__ldg(l0 + x1), chroma<FMT>(s, sh, sw, yy.x >> 1, x1 >> 1), p01[0], p01[1], p01[2]);
-        px(__ldg(l1 + x0), chroma<FMT>(s, sh, sw, yy.y >> 1, x0 >> 1), p10[0], p10[1], p10[2]);
-        px(__ldg(l1 + x1), chroma<FMT>(s, sh, sw, yy.y >> 1, x1 >> 1), p11[0], p11[1], p11[2]);
-#pragma unroll
-        for (int c = 0; c < 3; c++) {
-            const int h0 = (int)p00[c] * a.x + (int)p01[c] * a.y;
-            const int h1 = (int)p10[c] * a.x + (int)p11[c] * a.y;
-            o[k * 3 + c] = (uint8_t)k0_vmix(h0, h1, b.x, b.y);
-        }
-    }
-    if (dx0 + PX <= dw && ((uintptr_t)out & 3) == 0 && (PX * 3) % 4 == 0) {
-#pragma unroll
-        for (int q = 0; q < PX * 3 / 4; q++)
-            reinterpret_cast<uint32_t *>(out)[q] = (uint32_t)o[4 * q] | ((uint32_t)o[4 * q + 1] << 8) |
-                                                   ((uint32_t)o[4 * q + 2] << 16) | ((uint32_t)o[4 * q + 3] << 24);
+    k0_yuv420_resize_px<FMT, PX>(s, sh, sw, yy, b, xofs, alpha, dx0, dw, o);
+    k0_store_px<3, PX>(out, o, dx0, dw);
+}
+
+// The frames of a rig: every frame has its own descriptor (layout, size, tap tables), so cameras of different
+// resolutions and decoders share one launch.  The grid is k0_yuv420_resize's; a block reads its frame's descriptor
+// once, and the branch on the layout is uniform over the block.  A frame already at dh x dw runs on identity taps,
+// which reproduce the source (BGR) or cv2.cvtColor's frame (YUV) exactly.
+template <int PX>
+__global__ void __launch_bounds__(256) k0_rig_ingest(const RigFrame *__restrict__ frames, uint8_t *__restrict__ dst, int dh,
+                                                     int dw)
+{
+    __shared__ RigFrame d;
+    const int dx0 = (blockIdx.x * blockDim.x + threadIdx.x) * PX, dy = blockIdx.y, f = blockIdx.z;
+    if (threadIdx.x == 0) d = frames[f];
+    __syncthreads();
+    if (dx0 >= dw) return;
+    const int2 yy = __ldg(d.yofs + dy);
+    const short2 b = __ldg(d.beta + dy);
+    uint8_t *out = dst + (((size_t)f * dh + dy) * dw + dx0) * 3;
+    uint8_t o[PX * 3];
+    if (d.format == LANE_INPUT_BGR) {
+        const uint8_t *r0 = d.src + (size_t)yy.x * d.sw * 3, *r1 = d.src + (size_t)yy.y * d.sw * 3;
+        k0_resize_px<3, PX>(r0, r1, d.xofs, d.alpha, b, d.sw, dx0, dw, o);
+    } else if (d.format == LANE_INPUT_NV12) {
+        k0_yuv420_resize_px<LANE_INPUT_NV12, PX>(d.src, d.sh, d.sw, yy, b, d.xofs, d.alpha, dx0, dw, o);
     } else {
-        for (int k = 0; k < PX && dx0 + k < dw; k++)
-            for (int c = 0; c < 3; c++) out[k * 3 + c] = o[k * 3 + c];
+        k0_yuv420_resize_px<LANE_INPUT_I420, PX>(d.src, d.sh, d.sw, yy, b, d.xofs, d.alpha, dx0, dw, o);
     }
+    k0_store_px<3, PX>(out, o, dx0, dw);
 }
 
 }  // namespace
+
+cudaError_t rig_frame(const uint8_t *src, int format, int sh, int sw, int dh, int dw, RigFrame *d)
+{
+    ResizeTaps t;
+    const cudaError_t e = lane_resize_taps(sh, sw, dh, dw, &t);
+    if (e) return e;
+    *d = RigFrame{src, format, sh, sw, t.xofs, t.alpha, t.yofs, t.beta};
+    return cudaSuccess;
+}
+
+void launch_rig_ingest(const RigFrame *frames_dev, int n, uint8_t *dst, int dh, int dw, cudaStream_t st)
+{
+    constexpr int PX = 4;
+    const dim3 grid((dw + 256 * PX - 1) / (256 * PX), dh, n);
+    k0_rig_ingest<PX><<<grid, 256, 0, st>>>(frames_dev, dst, dh, dw);
+}
 
 cudaError_t launch_ingest(const uint8_t *src, int format, int n, int sh, int sw, uint8_t *dst, int dh, int dw,
                           cudaStream_t st)

@@ -80,27 +80,8 @@ __global__ void __launch_bounds__(256) k0_resize(const uint8_t *__restrict__ src
     const uint8_t *r0 = src + ((size_t)f * sh + yy.x) * sw * CN, *r1 = src + ((size_t)f * sh + yy.y) * sw * CN;
     uint8_t *out = dst + (((size_t)f * dh + dy) * dw + dx0) * CN;
     uint8_t px[PX * CN];
-#pragma unroll
-    for (int k = 0; k < PX; k++) {
-        const int dx = min(dx0 + k, dw - 1);
-        const int x0 = __ldg(xofs + dx), x1 = min(x0 + 1, sw - 1);
-        const short2 a = __ldg(alpha + dx);
-#pragma unroll
-        for (int c = 0; c < CN; c++) {
-            const int h0 = (int)__ldg(r0 + x0 * CN + c) * a.x + (int)__ldg(r0 + x1 * CN + c) * a.y;
-            const int h1 = (int)__ldg(r1 + x0 * CN + c) * a.x + (int)__ldg(r1 + x1 * CN + c) * a.y;
-            px[k * CN + c] = (uint8_t)k0_vmix(h0, h1, b.x, b.y);
-        }
-    }
-    if (dx0 + PX <= dw && ((uintptr_t)out & 3) == 0 && (PX * CN) % 4 == 0) {
-#pragma unroll
-        for (int q = 0; q < PX * CN / 4; q++)
-            reinterpret_cast<uint32_t *>(out)[q] = (uint32_t)px[4 * q] | ((uint32_t)px[4 * q + 1] << 8) |
-                                                   ((uint32_t)px[4 * q + 2] << 16) | ((uint32_t)px[4 * q + 3] << 24);
-    } else {
-        for (int k = 0; k < PX && dx0 + k < dw; k++)
-            for (int c = 0; c < CN; c++) out[k * CN + c] = px[k * CN + c];
-    }
+    k0_resize_px<CN, PX>(r0, r1, xofs, alpha, b, sw, dx0, dw, px);
+    k0_store_px<CN, PX>(out, px, dx0, dw);
 }
 
 }  // namespace

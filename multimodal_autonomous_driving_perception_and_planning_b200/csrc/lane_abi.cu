@@ -41,6 +41,7 @@ struct lane_ctx {
     // device buffers
     DeviceArray<uint8_t> d_frames;    // staging for host frames / BGR output of the ingest kernels (lazy)
     DeviceArray<uint8_t> d_src;       // staging for host frames the ingest kernels convert / resize (lazy, grows)
+    DeviceArray<RigFrame> d_rig;      // [2][B] frame descriptors of rig batches, per result slot (lazy)
     DeviceArray<uint8_t> d_blur;      // blurred plane: unfused path and verification taps only (lazy)
     DeviceArray<uint32_t> d_kbits;    // [B][H][WW] NMS survivors of the fused edge kernel
     DeviceArray<uint8_t> d_vplane;    // [B][H][W]  their magnitudes (sparse: only survivors' bytes are ever written / read)
@@ -98,6 +99,7 @@ struct lane_ctx {
         PinnedArray<double> h_prev_fit;              // state in (explicit mode) and state out
         PinnedArray<uint8_t> h_prev_valid;
         PinnedArray<int32_t> h_roi_idx;              // staging of d_roi_idx (n_roi > 1 only)
+        PinnedArray<RigFrame> h_rig;                 // staging of the slot's d_rig rows (lazy)
         CudaEvent ev[LANE_NUM_STAGES + 1];
         CudaEvent done;
         CudaEvent reader_done;                       // lane_ctx_fence_records: an outside reader of d_records ends here
@@ -163,11 +165,10 @@ int ensure_streams(lane_ctx *c, int S)
     return LANE_OK;
 }
 
-// Staging for max_batch source frames of `frame_bytes`.  A larger source replaces the buffer once the context's streams
-// are idle (an earlier batch may still be copying into it or converting out of it).
-int ensure_src(lane_ctx *c, size_t frame_bytes)
+// Staging for `need` bytes of host source frames.  A larger need replaces the buffer once the context's streams are
+// idle (an earlier batch may still be copying into it or converting out of it).
+int ensure_src(lane_ctx *c, size_t need)
 {
-    const size_t need = (size_t)c->max_batch * frame_bytes;
     if (c->d_src && need > c->d_src.size()) CU(c->sync());
     CU(c->d_src.grow(need));
     return LANE_OK;
@@ -342,13 +343,11 @@ struct Ingest {
     size_t frame_bytes() const { return format == LANE_INPUT_BGR ? (size_t)h * w * 3 : (size_t)h * w * 3 / 2; }
 };
 
-// Enqueue the whole batch.  Device-resident frames run as one chunk.  Host frames are cut into chunks that are
-// copied on a second stream while the previous chunk computes (the EMA state stays on the device across chunks,
-// which run in order on the compute stream).
-int enqueue(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int32_t *stream_id, int S,
-            const double *prev_fit, const uint8_t *prev_valid, Ingest in)
+// What a batch enqueues before its frames: the stream its back half runs on, its stream ids, every frame's ROI plane
+// and, when given, the explicit EMA state it starts from.
+int begin_batch(lane_ctx *c, bool on_device, int n, const int32_t *stream_id, int S, const double *prev_fit,
+                const uint8_t *prev_valid)
 {
-    int rc = LANE_OK;
     lane_ctx::slot_t &sl = c->slots[c->cur];
     // back half on its own stream: device-resident batches outside profiling / debug mode (stage events and taps assume
     // one stream).  Everything only the back half touches (stream ids, EMA state, records) is ordered on that stream.
@@ -374,6 +373,65 @@ int enqueue(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int
         CU(cudaMemcpyAsync(c->d_prev_fit, sl.h_prev_fit, sizeof(double) * S * 6, cudaMemcpyHostToDevice, hs));
         CU(cudaMemcpyAsync(c->d_prev_valid, sl.h_prev_valid, (size_t)S * 2, cudaMemcpyHostToDevice, hs));
     }
+    return LANE_OK;
+}
+
+// Host frames are cut into chunks that are copied on a second stream while the previous chunk computes (the EMA state
+// stays on the device across chunks, which run in order on the compute stream).  Chunks of this many frames let a copy
+// (~50 GB/s) and the compute of the previous chunk overlap; >= 4 chunks when possible.
+int host_chunk(int n) { return std::max(1, std::min(64, (n + 3) / 4)); }
+
+// The copy stream of chunked host batches (created on first use); the batch's copies start once the work enqueued before
+// it is done with the staging buffers.
+int begin_host_copies(lane_ctx *c)
+{
+    if (!c->copy_st) {
+        for (auto &e : c->copy_ev) CU(e.create(cudaEventDisableTiming));
+        CU(c->start_ev.create(cudaEventDisableTiming));
+        CU(c->copy_st.create(cudaStreamNonBlocking));
+    }
+    CU(cudaEventRecord(c->start_ev, c->st));
+    CU(cudaStreamWaitEvent(c->copy_st, c->start_ev, 0));
+    return LANE_OK;
+}
+
+// The compute stream waits for the copies of chunk k.
+int chunk_copied(lane_ctx *c, int k)
+{
+    cudaEvent_t ev = c->copy_ev[k % LANE_COPY_EVENTS];
+    CU(cudaEventRecord(ev, c->copy_st));
+    CU(cudaStreamWaitEvent(c->st, ev, 0));
+    return LANE_OK;
+}
+
+// What a batch enqueues after its frames: the copies of its records and of the EMA state after it, and its entry in the
+// queue of batches in flight.
+int end_batch(lane_ctx *c, bool on_device, int n, int S, const uint8_t *frames_dev)
+{
+    lane_ctx::slot_t &sl = c->slots[c->cur];
+    cudaStream_t hs = c->overlap_now ? c->st2 : c->st;
+    int rc = mark(c, LANE_STAGE_D2H); if (rc) return rc;
+    CU(cudaMemcpyAsync(sl.h_records, sl.d_records, sizeof(lane_record) * n, cudaMemcpyDeviceToHost, hs));
+    CU(cudaMemcpyAsync(sl.h_prev_fit, c->d_prev_fit, sizeof(double) * S * 6, cudaMemcpyDeviceToHost, hs));
+    CU(cudaMemcpyAsync(sl.h_prev_valid, c->d_prev_valid, (size_t)S * 2, cudaMemcpyDeviceToHost, hs));
+    rc = mark(c, LANE_NUM_STAGES); if (rc) return rc;
+    CU(cudaGetLastError());
+    c->last_frames_dev = frames_dev;
+    CU(cudaEventRecord(sl.done, hs));
+    sl.n = n;
+    sl.S = S;
+    sl.timed = c->profiling && on_device;
+    c->state_on_device = true;
+    c->q_count++;
+    return LANE_OK;
+}
+
+// Enqueue the whole batch.  Device-resident frames run as one chunk, host frames chunk by chunk (host_chunk).
+int enqueue(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int32_t *stream_id, int S,
+            const double *prev_fit, const uint8_t *prev_valid, Ingest in)
+{
+    int rc = begin_batch(c, on_device, n, stream_id, S, prev_fit, prev_valid);
+    if (rc) return rc;
     const int32_t *sid = stream_id ? c->d_stream_id.get() : nullptr;
     const uint8_t *frames_dev = frames;
     const size_t bgr_bytes = (size_t)c->g.H * c->g.W * 3;
@@ -391,21 +449,14 @@ int enqueue(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int
         // converted / resized on the device chunk by chunk
         const size_t bytes = in.frame_bytes();
         CU(c->d_frames.lazy((size_t)c->max_batch * bgr_bytes));
-        if (convert) { rc = ensure_src(c, bytes); if (rc) return rc; }
+        if (convert) { rc = ensure_src(c, (size_t)c->max_batch * bytes); if (rc) return rc; }
         uint8_t *d_in = convert ? c->d_src : c->d_frames;
-        if (!c->copy_st) {
-            for (auto &e : c->copy_ev) CU(e.create(cudaEventDisableTiming));
-            CU(c->start_ev.create(cudaEventDisableTiming));
-            CU(c->copy_st.create(cudaStreamNonBlocking));
-        }
         frames_dev = c->d_frames;
         // pinned (or registered) host memory goes straight to the copy engine; ordinary memory through the device's
         // staging ring.  Decided once for the whole batch: every chunk of a large pageable batch is staged.
         HostStager *ring = HostStager::pageable(frames, bytes * (size_t)n) ? &lane_device_host(c->device).stager : nullptr;
-        // chunk so that a copy (~50 GB/s) and the compute of the previous chunk overlap; >= 4 chunks when possible
-        const int chunk = std::max(1, std::min(64, (n + 3) / 4));
-        CU(cudaEventRecord(c->start_ev, c->st));                 // the staging buffer is free once earlier work is done
-        CU(cudaStreamWaitEvent(c->copy_st, c->start_ev, 0));
+        const int chunk = host_chunk(n);
+        rc = begin_host_copies(c); if (rc) return rc;
         int k = 0;
         for (int off = 0; off < n; off += chunk, k++) {
             const int m = std::min(chunk, n - off);
@@ -415,9 +466,7 @@ int enqueue(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int
                 CU(ring->h2d(to, from, bytes * m, c->copy_st));
             else
                 CU(cudaMemcpyAsync(to, from, bytes * m, cudaMemcpyHostToDevice, c->copy_st));
-            cudaEvent_t ev = c->copy_ev[k % LANE_COPY_EVENTS];
-            CU(cudaEventRecord(ev, c->copy_st));
-            CU(cudaStreamWaitEvent(c->st, ev, 0));
+            rc = chunk_copied(c, k); if (rc) return rc;
             if (convert)
                 CU(launch_ingest(c->d_src + (size_t)off * bytes, in.format, m, in.h, in.w, c->d_frames + (size_t)off * bgr_bytes,
                                  c->g.H, c->g.W, c->st));
@@ -425,20 +474,79 @@ int enqueue(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int
             if (rc) return rc;
         }
     }
-    rc = mark(c, LANE_STAGE_D2H); if (rc) return rc;
-    CU(cudaMemcpyAsync(sl.h_records, sl.d_records, sizeof(lane_record) * n, cudaMemcpyDeviceToHost, hs));
-    CU(cudaMemcpyAsync(sl.h_prev_fit, c->d_prev_fit, sizeof(double) * S * 6, cudaMemcpyDeviceToHost, hs));
-    CU(cudaMemcpyAsync(sl.h_prev_valid, c->d_prev_valid, (size_t)S * 2, cudaMemcpyDeviceToHost, hs));
-    rc = mark(c, LANE_NUM_STAGES); if (rc) return rc;
-    CU(cudaGetLastError());
-    c->last_frames_dev = frames_dev;
-    CU(cudaEventRecord(sl.done, hs));
-    sl.n = n;
-    sl.S = S;
-    sl.timed = c->profiling && on_device;
-    c->state_on_device = true;
-    c->q_count++;
-    return LANE_OK;
+    return end_batch(c, on_device, n, S, frames_dev);
+}
+
+// Bytes of one dense frame of a rig source.
+size_t rig_frame_bytes(const lane_rig_source &r)
+{
+    return r.format == LANE_INPUT_BGR ? (size_t)r.src_h * r.src_w * 3 : (size_t)r.src_h * r.src_w * 3 / 2;
+}
+
+// Enqueue a rig batch (lane_detect_rig, validated): the sources' frames in source order, each camera at its own size and
+// layout.  One k0_rig_ingest launch makes the context's BGR frames of the whole batch (device sources) or of each chunk
+// (host sources), driven by the batch's descriptor table; the rest of the path is enqueue's.
+int enqueue_rig(lane_ctx *c, const lane_rig_source *sources, int n_sources, bool on_device, int n, const int32_t *stream_id,
+                int S, const double *prev_fit, const uint8_t *prev_valid)
+{
+    lane_ctx::slot_t &sl = c->slots[c->cur];
+    const size_t B = (size_t)c->max_batch, bgr_bytes = (size_t)c->g.H * c->g.W * 3;
+    CU(c->d_frames.lazy(B * bgr_bytes));
+    CU(c->d_rig.lazy(2 * B));
+    if (!sl.h_rig) CU(sl.h_rig.alloc(B));
+    // host sources land in d_src one after another in source order: frame f at byte offset at[f]
+    std::vector<size_t> at(n + 1, 0);
+    for (int s = 0, f = 0; s < n_sources; s++)
+        for (int j = 0; j < sources[s].n; j++, f++) at[f + 1] = at[f] + rig_frame_bytes(sources[s]);
+    if (!on_device) { const int rc = ensure_src(c, at[n]); if (rc) return rc; }
+    for (int s = 0, f = 0; s < n_sources; s++) {
+        const lane_rig_source &r = sources[s];
+        if (!r.n) continue;
+        RigFrame d;
+        CU(rig_frame(nullptr, r.format, r.src_h, r.src_w, c->g.H, c->g.W, &d));
+        for (int j = 0; j < r.n; j++, f++) {
+            d.src = on_device ? r.frames + j * rig_frame_bytes(r) : c->d_src + at[f];
+            sl.h_rig[f] = d;
+        }
+    }
+    int rc = begin_batch(c, on_device, n, stream_id, S, prev_fit, prev_valid);
+    if (rc) return rc;
+    RigFrame *rig = c->d_rig + (size_t)c->cur * B;
+    CU(cudaMemcpyAsync(rig, sl.h_rig, sizeof(RigFrame) * n, cudaMemcpyHostToDevice, c->st));
+    const int32_t *sid = c->d_stream_id;
+    if (on_device) {
+        launch_rig_ingest(rig, n, c->d_frames, c->g.H, c->g.W, c->st);
+        rc = run_stages(c, c->d_frames, 0, n, sid, S, c->profiling);
+        if (rc) return rc;
+    } else {
+        // pinned (or registered) sources go straight to the copy engine, ordinary memory through the device's staging
+        // ring when the batch is large; decided once per source for the whole batch
+        HostStager *stager = &lane_device_host(c->device).stager;
+        std::vector<HostStager *> ring(n_sources);
+        for (int s = 0; s < n_sources; s++)
+            ring[s] = sources[s].n && HostStager::pageable(sources[s].frames, at[n]) ? stager : nullptr;
+        const int chunk = host_chunk(n);
+        rc = begin_host_copies(c); if (rc) return rc;
+        int k = 0;
+        for (int off = 0; off < n; off += chunk, k++) {
+            const int m = std::min(chunk, n - off);
+            // the chunk's frames of each source are contiguous on both sides: one copy per source
+            for (int s = 0, first = 0; s < n_sources && first < off + m; first += sources[s].n, s++) {
+                const int lo = std::max(off, first), hi = std::min(off + m, first + sources[s].n);
+                if (lo >= hi) continue;
+                const uint8_t *from = sources[s].frames + (lo - first) * rig_frame_bytes(sources[s]);
+                if (ring[s])
+                    CU(ring[s]->h2d(c->d_src + at[lo], from, at[hi] - at[lo], c->copy_st));
+                else
+                    CU(cudaMemcpyAsync(c->d_src + at[lo], from, at[hi] - at[lo], cudaMemcpyHostToDevice, c->copy_st));
+            }
+            rc = chunk_copied(c, k); if (rc) return rc;
+            launch_rig_ingest(rig + off, m, c->d_frames + (size_t)off * bgr_bytes, c->g.H, c->g.W, c->st);
+            rc = run_stages(c, c->d_frames, off, m, sid, S, false);
+            if (rc) return rc;
+        }
+    }
+    return end_batch(c, on_device, n, S, c->d_frames);
 }
 
 // What every detect call checks and sets up before it enqueues: arguments and context state, the context's device, the
@@ -830,6 +938,36 @@ int lane_detect_batch_ingest(lane_ctx *c, const uint8_t *frames, int frames_on_d
                            Ingest{format, src_h, src_w});
 }
 
+int lane_detect_rig(lane_ctx *c, const lane_rig_source *sources, int n_sources, int frames_on_device, int n_streams,
+                    double *prev_fit, uint8_t *prev_valid, lane_record *out)
+{
+    if (!c || !sources || !out || !prev_fit || !prev_valid)
+        return fail(c, LANE_ERR_INVALID, "lane_detect_rig: ctx, sources, prev_fit, prev_valid and out must not be null");
+    long long n = 0;
+    for (int s = 0; s < n_sources; s++) {
+        const lane_rig_source &r = sources[s];
+        if (r.n < 0) return fail(c, LANE_ERR_INVALID, "source %d: negative frame count %d", s, r.n);
+        if (r.format != LANE_INPUT_BGR && r.format != LANE_INPUT_NV12 && r.format != LANE_INPUT_I420)
+            return fail(c, LANE_ERR_INVALID, "source %d: unknown input format %d", s, r.format);
+        if (r.src_h < 1 || r.src_w < 1) return fail(c, LANE_ERR_INVALID, "source %d: bad size %dx%d", s, r.src_w, r.src_h);
+        if (r.format != LANE_INPUT_BGR && ((r.src_h | r.src_w) & 1))
+            return fail(c, LANE_ERR_INVALID, "source %d: NV12 / I420 needs even width and height (%dx%d)", s, r.src_w, r.src_h);
+        if (r.stream_id < 0 || r.stream_id >= n_streams)
+            return fail(c, LANE_ERR_INVALID, "source %d: stream_id %d outside [0,%d)", s, r.stream_id, n_streams);
+        if (r.n && !r.frames) return fail(c, LANE_ERR_INVALID, "source %d: frames is null", s);
+        n += r.n;
+    }
+    if (n < 1 || n > c->max_batch) return fail(c, LANE_ERR_INVALID, "bad batch: %lld frames (max_batch=%d)", n, c->max_batch);
+    if (n > 65535) return fail(c, LANE_ERR_UNSUPPORTED, "batch %lld above 65535", n);     // the ingest grid's z
+    std::vector<int32_t> stream_id;
+    for (int s = 0; s < n_sources; s++) stream_id.insert(stream_id.end(), sources[s].n, sources[s].stream_id);
+    int rc = check_call(c, sources, (int)n, stream_id.data(), n_streams, prev_fit, prev_valid);
+    if (rc) return rc;
+    rc = enqueue_rig(c, sources, n_sources, frames_on_device != 0, (int)n, stream_id.data(), n_streams, prev_fit, prev_valid);
+    if (rc) return rc;
+    return lane_detect_collect(c, prev_fit, prev_valid, out);
+}
+
 int lane_get_stage_ms(lane_ctx *c, float ms[LANE_NUM_STAGES], int32_t launches[LANE_NUM_STAGES])
 {
     if (!c) return LANE_ERR_INVALID;
@@ -898,6 +1036,7 @@ int lane_debug_tap(lane_ctx *c, int what, int fi, void *host_out, size_t capacit
         if (bytes_written) *bytes_written = bytes;
         return LANE_OK;
     }
+    case LANE_TAP_FRAME: src = c->last_frames_dev + fi * P * 3; bytes = P * 3; break;
     case LANE_TAP_SEGMENTS:
         src = c->d_lines + (size_t)fi * g.max_segments * 4;
         bytes = sizeof(int32_t) * 4 * c->slots[c->cur].h_records[fi].n_segments; break;

@@ -32,6 +32,7 @@ class LaneLine:
 
 LanePair = Tuple[Optional[LaneLine], Optional[LaneLine]]
 _SIDES = ("left", "right")
+_LAYOUTS = {"bgr": _native.INPUT_BGR, "nv12": _native.INPUT_NV12, "i420": _native.INPUT_I420}
 
 
 def _is_torch_cuda(x) -> bool:
@@ -190,7 +191,6 @@ class LaneDetector:
         n_masks = 1 if stream_rois is None else max(len(stream_rois), n_streams)
         ctx = self._context(h, w, n, frames, stream_rois, n_masks)
         s, oms = self.smoothing_factor, 1 - self.smoothing_factor
-        chunks = []
         on_device = _is_torch_cuda(frames)
         if on_device:
             import torch
@@ -204,6 +204,12 @@ class LaneDetector:
             src = frames.data_ptr() + a * fbytes if on_device else frames[a:b]
             return c.detect(src, b - a, on_device, sid, n_streams, prev_fit, prev_valid, s, oms, fmt=fmt, src_hw=(sh, sw))
 
+        return self._chunked(ctx, n, call, h, w, prev_fit, prev_valid, stream_rois, n_masks)
+
+    def _chunked(self, ctx, n, call, h, w, prev_fit, prev_valid, stream_rois, n_masks) -> np.ndarray:
+        """``call(context, a, b)`` -> records of frames [a, b), over frames [0, n) in chunks of the context's max_batch,
+        each chunk re-run on the dense context when its segment lists overflow."""
+        chunks = []
         for a in range(0, n, ctx.max_batch):
             b = min(a + ctx.max_batch, n)
             fit0, valid0 = prev_fit.copy(), prev_valid.copy()
@@ -422,6 +428,13 @@ class LaneDetector:
             stream_rois = list(stream_rois)
             if len(stream_rois) < n_streams:
                 raise ValueError(f"stream_rois has {len(stream_rois)} entries; stream id {n_streams - 1} needs {n_streams}")
+        self._grow_stream_state(n_streams)
+        recs = self._run(frames, stream_ids, self._stream_fit.shape[0], self._stream_fit, self._stream_valid,
+                         stream_rois=stream_rois)
+        return self._lanes_from_records(recs)
+
+    def _grow_stream_state(self, n_streams: int):
+        """Per-stream smoothing state of ``detect_streams`` / ``detect_rig`` for at least ``n_streams`` streams."""
         if self._stream_fit is None or self._stream_fit.shape[0] < n_streams:
             fit = np.zeros((n_streams, 2, 3), np.float64)
             valid = np.zeros((n_streams, 2), np.uint8)
@@ -429,9 +442,109 @@ class LaneDetector:
                 k = self._stream_fit.shape[0]
                 fit[:k], valid[:k] = self._stream_fit, self._stream_valid
             self._stream_fit, self._stream_valid = fit, valid
-        recs = self._run(frames, stream_ids, self._stream_fit.shape[0], self._stream_fit, self._stream_valid,
-                         stream_rois=stream_rois)
-        return self._lanes_from_records(recs)
+
+    def detect_rig(self, frames: Sequence, layouts: Optional[Sequence[str]] = None, *,
+                   target_size: Optional[Tuple[int, int]] = None,
+                   stream_rois: Optional[Sequence[Optional[np.ndarray]]] = None) -> List[List[LanePair]]:
+        """A rig of cameras that differ in resolution and decoder layout, in one batched call.
+
+        ``frames[s]`` is camera s (= stream s of ``detect_streams``): uint8 ``[T_s, H_s, W_s, 3]`` BGR or
+        ``[T_s, H_s*3/2, W_s]`` NV12 / I420, as ``layouts[s]`` ("bgr", "nv12", "i420"; default all "bgr") says, its frames
+        in temporal order.  ``T_s`` may differ between cameras and may be 0, or the entry None: no frame this tick.  Every
+        camera is a numpy array, or every camera is a CUDA tensor on one device.  Every frame is detected at
+        ``target_size`` = (width, height), which may be left out only when all cameras share one size; the device converts
+        and resizes all frames in one kernel (only the source bytes of host frames cross PCIe) and runs the rest of the
+        path once for the rig.  ``stream_rois`` as in ``detect_streams``, polygons in target coordinates.
+
+        Returns one list of pairs per camera.  Camera s's pairs equal those of a fresh
+        ``LaneDetector(roi_vertices=stream_rois[s])`` given its frames through ``detect_batch`` / ``detect_batch_nv12`` /
+        ``detect_batch_i420(frames[s], target_size=target_size)``; its smoothing state is stream s's of ``detect_streams``,
+        so it carries across calls of either kind (``reset`` clears it).
+        """
+        cams = list(frames)
+        layouts = ["bgr"] * len(cams) if layouts is None else list(layouts)
+        if len(layouts) != len(cams):
+            raise ValueError(f"{len(cams)} cameras but {len(layouts)} layouts")
+        if target_size is not None:
+            target_size = check_target_size(target_size)
+        if stream_rois is not None:
+            stream_rois = list(stream_rois)
+            if len(stream_rois) < len(cams):
+                raise ValueError(f"stream_rois has {len(stream_rois)} entries for {len(cams)} cameras")
+        fmts, sizes, counts, kinds = [], [], [], set()
+        for s, (f, lay) in enumerate(zip(cams, layouts)):
+            if lay not in _LAYOUTS:
+                raise ValueError(f"camera {s}: layout {lay!r} is not one of {sorted(_LAYOUTS)}")
+            fmts.append(_LAYOUTS[lay])
+            if f is None:
+                sizes.append(None)
+                counts.append(0)
+                continue
+            kinds.add(("cuda", f.device.index) if _is_torch_cuda(f) else "host" if isinstance(f, np.ndarray) else "other")
+            if len(kinds) > 1 or "other" in kinds:
+                raise ValueError("rig cameras must all be numpy arrays or all CUDA tensors on one device")
+            sizes.append(self._rig_frame_size(f, lay, s))
+            counts.append(int(f.shape[0]))
+        used = {sz for sz, t in zip(sizes, counts) if t}
+        if target_size is None and len(used) > 1:
+            raise ValueError(f"cameras of sizes {sorted(used)} need a target_size")
+        if not used:
+            return [[] for _ in cams]
+        h, w = next(iter(used)) if target_size is None else (target_size[1], target_size[0])
+        on_device = kinds != {"host"}
+        live = [s for s in range(len(cams)) if counts[s]]
+        if on_device:
+            import torch
+            data = {s: cams[s].contiguous() for s in live}
+            torch.cuda.current_stream(data[live[0]].device).synchronize()
+        else:
+            data = {s: np.ascontiguousarray(cams[s]) for s in live}
+        base = [0]                                   # camera s's frames are [base[s], base[s+1]) of the concatenation
+        for t in counts:
+            base.append(base[-1] + t)
+        n = base[-1]
+        self._grow_stream_state(len(cams))
+        fit, valid = self._stream_fit, self._stream_valid
+        n_masks = 1 if stream_rois is None else max(len(stream_rois), fit.shape[0])
+        ctx = self._context(h, w, n, data[live[0]], stream_rois, n_masks)
+        sm, oms = self.smoothing_factor, 1 - self.smoothing_factor
+
+        def call(c, a, b):
+            sources = []
+            for s in live:
+                lo, hi = max(a, base[s]), min(b, base[s + 1])
+                if lo < hi:
+                    sh, sw = sizes[s]
+                    i, j = lo - base[s], hi - base[s]
+                    fb = sh * sw * 3 if fmts[s] == _native.INPUT_BGR else sh * sw * 3 // 2
+                    src = data[s].data_ptr() + i * fb if on_device else data[s][i:j]
+                    sources.append((src, fmts[s], (sh, sw), j - i, s))
+            return c.detect_rig(sources, on_device, fit.shape[0], fit, valid, sm, oms)
+
+        recs = self._chunked(ctx, n, call, h, w, fit, valid, stream_rois, n_masks)
+        lanes = self._lanes_from_records(recs)
+        return [lanes[base[s]:base[s + 1]] for s in range(len(cams))]
+
+    @staticmethod
+    def _rig_frame_size(f, layout: str, s: int) -> Tuple[int, int]:
+        """(H, W) of camera s's frames in ``layout``; ``ValueError`` when the shape is not that layout's, ``cv2.error``
+        for a wrong channel count or dtype (what cv2.cvtColor raises)."""
+        shape = tuple(f.shape)
+        if layout == "bgr":
+            if len(shape) != 4:
+                raise ValueError(f"camera {s}: layout 'bgr' needs frames [T,H,W,3], got {shape}")
+            if shape[-1] != 3:
+                raise cv2.error(f"LaneDetector: camera {s}: expected 3-channel BGR frames, got {shape}")
+            h, w = shape[1], shape[2]
+        else:
+            if len(shape) != 3 or shape[1] % 3:
+                raise ValueError(f"camera {s}: layout {layout!r} needs frames [T,H*3/2,W], got {shape}")
+            h, w = shape[1] * 2 // 3, shape[2]
+            if h % 2 or w % 2:
+                raise ValueError(f"camera {s}: {layout} needs even width and height, got {w}x{h}")
+        if str(f.dtype).replace("torch.", "") != "uint8":
+            raise cv2.error(f"LaneDetector: camera {s}: frames must be uint8, got {f.dtype}")
+        return int(h), int(w)
 
     def draw_lanes(self, frame: np.ndarray, left_lane: Optional[LaneLine], right_lane: Optional[LaneLine],
                    fill_lane: bool = True) -> np.ndarray:
