@@ -184,6 +184,21 @@ LANE_API int lane_detect_enqueue(lane_ctx *ctx, const uint8_t *frames_dev, int n
                         int n_streams, const double *prev_fit, const uint8_t *prev_valid);
 LANE_API int lane_detect_collect(lane_ctx *ctx, double *prev_fit, uint8_t *prev_valid, lane_record *out);
 
+/* lane_detect_enqueue for a rig tick: lane_detect_rig's sources and results, asynchronous, for a recorded multi-camera
+ * drive tagged offline (decode -> LaneDetector.detect per frame per camera, lane_detector.py:178-218) with the device
+ * never waiting for the host between ticks.  Validation and LANE_ERR_INVALID cases are lane_detect_rig's; the state
+ * rules (prev_fit / prev_valid given: one tick in flight; both NULL: continue from the device state, two in flight) and
+ * the result slots are lane_detect_enqueue's, so rig ticks and lane_detect_enqueue batches may share one queue.  The
+ * records come back, in source order, through lane_detect_collect.
+ *   frames_on_device = 1: the sources are read where they are until the tick is collected.
+ *   frames_on_device = 0: every source must be page-locked or registered host memory (cudaHostAlloc,
+ *       cudaHostRegister); pageable memory is LANE_ERR_INVALID.  Each camera is copied whole in one copy, under the
+ *       compute of the tick in flight, into staging of the tick's result slot, so the caller keeps the bytes unchanged
+ *       until the tick is collected.  That staging grows on demand; growing it while a tick is in flight waits for that
+ *       tick. */
+LANE_API int lane_rig_enqueue(lane_ctx *ctx, const lane_rig_source *sources, int n_sources, int frames_on_device,
+                              int n_streams, const double *prev_fit, const uint8_t *prev_valid);
+
 /* The context's CUDA stream (cudaStream_t as void*), so callers can record events on it. */
 LANE_API void *lane_ctx_stream(lane_ctx *ctx);
 /* Device copy of the records lane_detect_collect / lane_detect_batch returned last (lane_record[n]).  It stays valid

@@ -110,6 +110,7 @@ _PROTOS = {
                                            C.c_void_p]),
     "lane_detect_enqueue": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "lane_detect_collect": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "lane_rig_enqueue": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "lane_ctx_stream": (C.c_void_p, [C.c_void_p]),
     "lane_ctx_set_stream": (C.c_int, [C.c_void_p, C.c_void_p]),
     "lane_ctx_records_device": (C.c_void_p, [C.c_void_p]),
@@ -168,6 +169,17 @@ def threshold_lut():
 
 def _ptr(a):
     return a.ctypes.data_as(C.c_void_p) if a is not None else None
+
+
+def _rig_sources(sources, on_device: bool):
+    """The lane_rig_source array of ``LaneContext.detect_rig``'s ``sources``, and their total frame count."""
+    arr = (LaneRigSource * max(len(sources), 1))()
+    total = 0
+    for i, (frames, fmt, (h, w), n, sid) in enumerate(sources):
+        fp = frames if on_device else (frames.ctypes.data if n else None)
+        arr[i] = LaneRigSource(fp, int(fmt), int(h), int(w), int(n), int(sid))
+        total += int(n)
+    return arr, total
 
 
 class LaneContext:
@@ -287,15 +299,21 @@ class LaneContext:
         Returns the records of all frames in source order (a copy)."""
         L = lib()
         self._check(L.lane_set_smoothing(self._h, float(smoothing), float(one_minus)))
-        arr = (LaneRigSource * max(len(sources), 1))()
-        total = 0
-        for i, (frames, fmt, (h, w), n, sid) in enumerate(sources):
-            fp = frames if on_device else (frames.ctypes.data if n else None)
-            arr[i] = LaneRigSource(fp, int(fmt), int(h), int(w), int(n), int(sid))
-            total += int(n)
+        arr, total = _rig_sources(sources, on_device)
         self._check(L.lane_detect_rig(self._h, arr, len(sources), int(on_device), n_streams, _ptr(prev_fit),
                                       _ptr(prev_valid), _ptr(self._records)))
         return self._records[:total].copy()
+
+    def enqueue_rig(self, sources, on_device: bool, n_streams: int, prev_fit, prev_valid, smoothing, one_minus):
+        """Asynchronous ``detect_rig`` (lane_rig_enqueue): ``sources`` as there, host frames in page-locked memory, and
+        the state rules of ``enqueue``.  ``collect`` returns the tick's records in source order.  The frames must stay
+        alive and unchanged until then."""
+        L = lib()
+        self._check(L.lane_set_smoothing(self._h, float(smoothing), float(one_minus)))
+        arr, total = _rig_sources(sources, on_device)
+        self._check(L.lane_rig_enqueue(self._h, arr, len(sources), int(on_device), n_streams, _ptr(prev_fit),
+                                       _ptr(prev_valid)))
+        self._inflight.append(total)
 
     def enqueue(self, frames_ptr: int, n: int, stream_id, n_streams, prev_fit, prev_valid, smoothing, one_minus):
         """Asynchronous form for device-resident frames.  With ``prev_fit`` / ``prev_valid`` the batch starts from that

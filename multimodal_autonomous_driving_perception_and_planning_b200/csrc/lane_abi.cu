@@ -100,6 +100,10 @@ struct lane_ctx {
         PinnedArray<uint8_t> h_prev_valid;
         PinnedArray<int32_t> h_roi_idx;              // staging of d_roi_idx (n_roi > 1 only)
         PinnedArray<RigFrame> h_rig;                 // staging of the slot's d_rig rows (lazy)
+        // lane_rig_enqueue's host ticks: the slot's frames, copied whole while the other slot's tick computes (lazy,
+        // grows), and the event after the ingest launch that last read them
+        DeviceArray<uint8_t> d_src;
+        CudaEvent src_read;
         CudaEvent ev[LANE_NUM_STAGES + 1];
         CudaEvent done;
         CudaEvent reader_done;                       // lane_ctx_fence_records: an outside reader of d_records ends here
@@ -165,12 +169,12 @@ int ensure_streams(lane_ctx *c, int S)
     return LANE_OK;
 }
 
-// Staging for `need` bytes of host source frames.  A larger need replaces the buffer once the context's streams are
-// idle (an earlier batch may still be copying into it or converting out of it).
-int ensure_src(lane_ctx *c, size_t need)
+// Staging `src` (the context's d_src or a slot's) for `need` bytes of host source frames.  A larger need replaces the
+// buffer once the context's streams are idle (an earlier batch may still be copying into it or converting out of it).
+int ensure_src(lane_ctx *c, DeviceArray<uint8_t> &src, size_t need)
 {
-    if (c->d_src && need > c->d_src.size()) CU(c->sync());
-    CU(c->d_src.grow(need));
+    if (src && need > src.size()) CU(c->sync());
+    CU(src.grow(need));
     return LANE_OK;
 }
 
@@ -381,15 +385,23 @@ int begin_batch(lane_ctx *c, bool on_device, int n, const int32_t *stream_id, in
 // (~50 GB/s) and the compute of the previous chunk overlap; >= 4 chunks when possible.
 int host_chunk(int n) { return std::max(1, std::min(64, (n + 3) / 4)); }
 
-// The copy stream of chunked host batches (created on first use); the batch's copies start once the work enqueued before
-// it is done with the staging buffers.
+// The copy stream of host batches and its events, created on first use.
+int ensure_copy_stream(lane_ctx *c)
+{
+    if (c->copy_st) return LANE_OK;
+    for (auto &e : c->copy_ev) CU(e.create(cudaEventDisableTiming));
+    CU(c->start_ev.create(cudaEventDisableTiming));
+    for (auto &sl : c->slots) CU(sl.src_read.create(cudaEventDisableTiming));
+    CU(c->copy_st.create(cudaStreamNonBlocking));
+    return LANE_OK;
+}
+
+// The copy stream of chunked host batches; the batch's copies start once the work enqueued before it is done with the
+// staging buffers.
 int begin_host_copies(lane_ctx *c)
 {
-    if (!c->copy_st) {
-        for (auto &e : c->copy_ev) CU(e.create(cudaEventDisableTiming));
-        CU(c->start_ev.create(cudaEventDisableTiming));
-        CU(c->copy_st.create(cudaStreamNonBlocking));
-    }
+    const int rc = ensure_copy_stream(c);
+    if (rc) return rc;
     CU(cudaEventRecord(c->start_ev, c->st));
     CU(cudaStreamWaitEvent(c->copy_st, c->start_ev, 0));
     return LANE_OK;
@@ -449,7 +461,7 @@ int enqueue(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int
         // converted / resized on the device chunk by chunk
         const size_t bytes = in.frame_bytes();
         CU(c->d_frames.lazy((size_t)c->max_batch * bgr_bytes));
-        if (convert) { rc = ensure_src(c, (size_t)c->max_batch * bytes); if (rc) return rc; }
+        if (convert) { rc = ensure_src(c, c->d_src, (size_t)c->max_batch * bytes); if (rc) return rc; }
         uint8_t *d_in = convert ? c->d_src : c->d_frames;
         frames_dev = c->d_frames;
         // pinned (or registered) host memory goes straight to the copy engine; ordinary memory through the device's
@@ -483,39 +495,58 @@ size_t rig_frame_bytes(const lane_rig_source &r)
     return r.format == LANE_INPUT_BGR ? (size_t)r.src_h * r.src_w * 3 : (size_t)r.src_h * r.src_w * 3 / 2;
 }
 
-// Enqueue a rig batch (lane_detect_rig, validated): the sources' frames in source order, each camera at its own size and
-// layout.  One k0_rig_ingest launch makes the context's BGR frames of the whole batch (device sources) or of each chunk
-// (host sources), driven by the batch's descriptor table; the rest of the path is enqueue's.
+// Enqueue a rig batch (validated): the sources' frames in source order, each camera at its own size and layout.  One
+// k0_rig_ingest launch makes the context's BGR frames of the whole batch, driven by the batch's descriptor table; the rest
+// of the path is enqueue's.  Device sources are read where they are.  Host sources of lane_detect_rig (staged = false)
+// are copied chunk by chunk into the context's d_src behind the compute of the chunk before, one ingest launch per chunk.
+// Host sources of lane_rig_enqueue (staged, page-locked) are copied whole into the slot's own d_src behind the compute
+// of the tick before, and then run like device sources.  `staged` names host sources only: device sources are never
+// copied.
 int enqueue_rig(lane_ctx *c, const lane_rig_source *sources, int n_sources, bool on_device, int n, const int32_t *stream_id,
-                int S, const double *prev_fit, const uint8_t *prev_valid)
+                int S, const double *prev_fit, const uint8_t *prev_valid, bool staged)
 {
+    staged = staged && !on_device;
     lane_ctx::slot_t &sl = c->slots[c->cur];
     const size_t B = (size_t)c->max_batch, bgr_bytes = (size_t)c->g.H * c->g.W * 3;
     CU(c->d_frames.lazy(B * bgr_bytes));
     CU(c->d_rig.lazy(2 * B));
     if (!sl.h_rig) CU(sl.h_rig.alloc(B));
-    // host sources land in d_src one after another in source order: frame f at byte offset at[f]
+    // host sources land in the staging one after another in source order: frame f at byte offset at[f]
+    DeviceArray<uint8_t> &src = staged ? sl.d_src : c->d_src;
     std::vector<size_t> at(n + 1, 0);
     for (int s = 0, f = 0; s < n_sources; s++)
         for (int j = 0; j < sources[s].n; j++, f++) at[f + 1] = at[f] + rig_frame_bytes(sources[s]);
-    if (!on_device) { const int rc = ensure_src(c, at[n]); if (rc) return rc; }
+    if (!on_device) { const int rc = ensure_src(c, src, at[n]); if (rc) return rc; }
     for (int s = 0, f = 0; s < n_sources; s++) {
         const lane_rig_source &r = sources[s];
         if (!r.n) continue;
         RigFrame d;
         CU(rig_frame(nullptr, r.format, r.src_h, r.src_w, c->g.H, c->g.W, &d));
         for (int j = 0; j < r.n; j++, f++) {
-            d.src = on_device ? r.frames + j * rig_frame_bytes(r) : c->d_src + at[f];
+            d.src = on_device ? r.frames + j * rig_frame_bytes(r) : src + at[f];
             sl.h_rig[f] = d;
         }
     }
-    int rc = begin_batch(c, on_device, n, stream_id, S, prev_fit, prev_valid);
+    const bool whole = on_device || staged;          // one ingest launch and one pass of the path for the batch
+    int rc = begin_batch(c, whole, n, stream_id, S, prev_fit, prev_valid);
     if (rc) return rc;
     RigFrame *rig = c->d_rig + (size_t)c->cur * B;
     CU(cudaMemcpyAsync(rig, sl.h_rig, sizeof(RigFrame) * n, cudaMemcpyHostToDevice, c->st));
     const int32_t *sid = c->d_stream_id;
-    if (on_device) {
+    if (whole) {
+        if (staged) {
+            // The copies wait only for the ingest that last read this slot's staging, not for the tick in flight on
+            // the compute stream: they run under it.  The ingest waits for them.
+            rc = ensure_copy_stream(c); if (rc) return rc;
+            CU(cudaStreamWaitEvent(c->copy_st, sl.src_read, 0));
+            for (int s = 0, first = 0; s < n_sources; first += sources[s].n, s++)
+                if (sources[s].n)
+                    CU(cudaMemcpyAsync(src + at[first], sources[s].frames, at[first + sources[s].n] - at[first],
+                                       cudaMemcpyHostToDevice, c->copy_st));
+            rc = chunk_copied(c, c->cur); if (rc) return rc;
+        }
         launch_rig_ingest(rig, n, c->d_frames, c->g.H, c->g.W, c->st);
+        if (staged) CU(cudaEventRecord(sl.src_read, c->st));
         rc = run_stages(c, c->d_frames, 0, n, sid, S, c->profiling);
         if (rc) return rc;
     } else {
@@ -546,7 +577,42 @@ int enqueue_rig(lane_ctx *c, const lane_rig_source *sources, int n_sources, bool
             if (rc) return rc;
         }
     }
-    return end_batch(c, on_device, n, S, c->d_frames);
+    return end_batch(c, whole, n, S, c->d_frames);
+}
+
+// The checks lane_detect_rig and lane_rig_enqueue share before check_call: every source's fields, the batch size, and
+// the stream id of every frame (into `stream_id`).  Returns the batch's frame count or a LANE_ERR_* code.
+int check_rig(lane_ctx *c, const lane_rig_source *sources, int n_sources, int n_streams, std::vector<int32_t> &stream_id)
+{
+    long long n = 0;
+    for (int s = 0; s < n_sources; s++) {
+        const lane_rig_source &r = sources[s];
+        if (r.n < 0) return fail(c, LANE_ERR_INVALID, "source %d: negative frame count %d", s, r.n);
+        if (r.format != LANE_INPUT_BGR && r.format != LANE_INPUT_NV12 && r.format != LANE_INPUT_I420)
+            return fail(c, LANE_ERR_INVALID, "source %d: unknown input format %d", s, r.format);
+        if (r.src_h < 1 || r.src_w < 1) return fail(c, LANE_ERR_INVALID, "source %d: bad size %dx%d", s, r.src_w, r.src_h);
+        if (r.format != LANE_INPUT_BGR && ((r.src_h | r.src_w) & 1))
+            return fail(c, LANE_ERR_INVALID, "source %d: NV12 / I420 needs even width and height (%dx%d)", s, r.src_w, r.src_h);
+        if (r.stream_id < 0 || r.stream_id >= n_streams)
+            return fail(c, LANE_ERR_INVALID, "source %d: stream_id %d outside [0,%d)", s, r.stream_id, n_streams);
+        if (r.n && !r.frames) return fail(c, LANE_ERR_INVALID, "source %d: frames is null", s);
+        n += r.n;
+    }
+    if (n < 1 || n > c->max_batch) return fail(c, LANE_ERR_INVALID, "bad batch: %lld frames (max_batch=%d)", n, c->max_batch);
+    if (n > 65535) return fail(c, LANE_ERR_UNSUPPORTED, "batch %lld above 65535", n);     // the ingest grid's z
+    for (int s = 0; s < n_sources; s++) stream_id.insert(stream_id.end(), sources[s].n, sources[s].stream_id);
+    return (int)n;
+}
+
+// Whether host memory [p, p + bytes) is page-locked or registered, so the copy engine reads it where it is.
+bool page_locked(const void *p, size_t bytes)
+{
+    cudaPointerAttributes first{}, last{};
+    const bool ok = cudaPointerGetAttributes(&first, p) == cudaSuccess && first.type == cudaMemoryTypeHost &&
+                    cudaPointerGetAttributes(&last, (const uint8_t *)p + bytes - 1) == cudaSuccess &&
+                    last.type == cudaMemoryTypeHost;
+    cudaGetLastError();
+    return ok;
 }
 
 // What every detect call checks and sets up before it enqueues: arguments and context state, the context's device, the
@@ -943,29 +1009,31 @@ int lane_detect_rig(lane_ctx *c, const lane_rig_source *sources, int n_sources, 
 {
     if (!c || !sources || !out || !prev_fit || !prev_valid)
         return fail(c, LANE_ERR_INVALID, "lane_detect_rig: ctx, sources, prev_fit, prev_valid and out must not be null");
-    long long n = 0;
-    for (int s = 0; s < n_sources; s++) {
-        const lane_rig_source &r = sources[s];
-        if (r.n < 0) return fail(c, LANE_ERR_INVALID, "source %d: negative frame count %d", s, r.n);
-        if (r.format != LANE_INPUT_BGR && r.format != LANE_INPUT_NV12 && r.format != LANE_INPUT_I420)
-            return fail(c, LANE_ERR_INVALID, "source %d: unknown input format %d", s, r.format);
-        if (r.src_h < 1 || r.src_w < 1) return fail(c, LANE_ERR_INVALID, "source %d: bad size %dx%d", s, r.src_w, r.src_h);
-        if (r.format != LANE_INPUT_BGR && ((r.src_h | r.src_w) & 1))
-            return fail(c, LANE_ERR_INVALID, "source %d: NV12 / I420 needs even width and height (%dx%d)", s, r.src_w, r.src_h);
-        if (r.stream_id < 0 || r.stream_id >= n_streams)
-            return fail(c, LANE_ERR_INVALID, "source %d: stream_id %d outside [0,%d)", s, r.stream_id, n_streams);
-        if (r.n && !r.frames) return fail(c, LANE_ERR_INVALID, "source %d: frames is null", s);
-        n += r.n;
-    }
-    if (n < 1 || n > c->max_batch) return fail(c, LANE_ERR_INVALID, "bad batch: %lld frames (max_batch=%d)", n, c->max_batch);
-    if (n > 65535) return fail(c, LANE_ERR_UNSUPPORTED, "batch %lld above 65535", n);     // the ingest grid's z
     std::vector<int32_t> stream_id;
-    for (int s = 0; s < n_sources; s++) stream_id.insert(stream_id.end(), sources[s].n, sources[s].stream_id);
-    int rc = check_call(c, sources, (int)n, stream_id.data(), n_streams, prev_fit, prev_valid);
+    const int n = check_rig(c, sources, n_sources, n_streams, stream_id);
+    if (n < 0) return n;
+    int rc = check_call(c, sources, n, stream_id.data(), n_streams, prev_fit, prev_valid);
     if (rc) return rc;
-    rc = enqueue_rig(c, sources, n_sources, frames_on_device != 0, (int)n, stream_id.data(), n_streams, prev_fit, prev_valid);
+    rc = enqueue_rig(c, sources, n_sources, frames_on_device != 0, n, stream_id.data(), n_streams, prev_fit, prev_valid, false);
     if (rc) return rc;
     return lane_detect_collect(c, prev_fit, prev_valid, out);
+}
+
+int lane_rig_enqueue(lane_ctx *c, const lane_rig_source *sources, int n_sources, int frames_on_device, int n_streams,
+                     const double *prev_fit, const uint8_t *prev_valid)
+{
+    if (!c || !sources) return fail(c, LANE_ERR_INVALID, "lane_rig_enqueue: ctx and sources must not be null");
+    std::vector<int32_t> stream_id;
+    const int n = check_rig(c, sources, n_sources, n_streams, stream_id);
+    if (n < 0) return n;
+    if (!frames_on_device)
+        for (int s = 0; s < n_sources; s++)
+            if (sources[s].n && !page_locked(sources[s].frames, sources[s].n * rig_frame_bytes(sources[s])))
+                return fail(c, LANE_ERR_INVALID, "source %d: host frames must be page-locked or registered memory "
+                            "(cudaHostAlloc, cudaHostRegister, torch pin_memory)", s);
+    const int rc = check_call(c, sources, n, stream_id.data(), n_streams, prev_fit, prev_valid);
+    if (rc) return rc;
+    return enqueue_rig(c, sources, n_sources, frames_on_device != 0, n, stream_id.data(), n_streams, prev_fit, prev_valid, true);
 }
 
 int lane_get_stage_ms(lane_ctx *c, float ms[LANE_NUM_STAGES], int32_t launches[LANE_NUM_STAGES])

@@ -11,6 +11,8 @@ the ROI polygon mask (``cv2.fillPoly``, built once per frame size) and ``draw_la
 """
 from __future__ import annotations
 
+import os
+from concurrent.futures import ThreadPoolExecutor
 from dataclasses import dataclass
 from typing import List, Optional, Sequence, Tuple
 
@@ -33,10 +35,50 @@ class LaneLine:
 LanePair = Tuple[Optional[LaneLine], Optional[LaneLine]]
 _SIDES = ("left", "right")
 _LAYOUTS = {"bgr": _native.INPUT_BGR, "nv12": _native.INPUT_NV12, "i420": _native.INPUT_I420}
+_COPY_PIECE = 4 << 20         # bytes per host thread task when detect_rig_stream copies a numpy tick into pinned memory
 
 
 def _is_torch_cuda(x) -> bool:
     return type(x).__module__.startswith("torch") and hasattr(x, "is_cuda") and bool(x.is_cuda)
+
+
+def _is_pinned_tensor(x) -> bool:
+    """A contiguous CPU torch tensor in page-locked memory (the copy engine reads it where it is); an empty one has no
+    memory to lock."""
+    return (type(x).__module__.startswith("torch") and hasattr(x, "is_pinned") and not x.is_cuda and x.is_contiguous()
+            and (x.numel() == 0 or bool(x.is_pinned())))
+
+
+@dataclass
+class _RigTick:
+    """One tick of a rig as ``detect_rig``'s checks found it: camera s has ``counts[s]`` frames in layout ``fmts[s]``
+    (INPUT_*) at ``sizes[s]`` = (h, w); every camera with frames is of one ``kind`` (``("cuda", index)``, ``"host"`` for
+    numpy, ``"pinned"``; None when the tick has no frame), detected at ``h`` x ``w``."""
+    cams: list
+    fmts: list
+    sizes: list
+    counts: list
+    kind: object
+    h: Optional[int]
+    w: Optional[int]
+    stream_rois: Optional[list]
+
+    def __post_init__(self):
+        self.base = [0]                              # camera s's frames are [base[s], base[s+1]) of the concatenation
+        for t in self.counts:
+            self.base.append(self.base[-1] + t)
+        self.n = self.base[-1]
+        self.live = [s for s, t in enumerate(self.counts) if t]
+
+    def n_masks(self, n_streams: int) -> int:
+        return 1 if self.stream_rois is None else max(len(self.stream_rois), n_streams)
+
+    def frame_bytes(self, s: int) -> int:
+        sh, sw = self.sizes[s]
+        return sh * sw * 3 if self.fmts[s] == _native.INPUT_BGR else sh * sw * 3 // 2
+
+    def per_camera(self, items):
+        return [items[self.base[s]:self.base[s + 1]] for s in range(len(self.cams))]
 
 
 class LaneDetector:
@@ -461,6 +503,174 @@ class LaneDetector:
         ``detect_batch_i420(frames[s], target_size=target_size)``; its smoothing state is stream s's of ``detect_streams``,
         so it carries across calls of either kind (``reset`` clears it).
         """
+        p = self._rig_plan(frames, layouts, target_size, stream_rois)
+        if not p.n:
+            return [[] for _ in p.cams]
+        on_device = p.kind != "host"
+        if on_device:
+            import torch
+            data = {s: p.cams[s].contiguous() for s in p.live}
+            torch.cuda.current_stream(data[p.live[0]].device).synchronize()
+        else:
+            data = {s: np.ascontiguousarray(p.cams[s]) for s in p.live}
+        self._grow_stream_state(len(p.cams))
+        fit, valid = self._stream_fit, self._stream_valid
+        n_masks = p.n_masks(fit.shape[0])
+        ctx = self._context(p.h, p.w, p.n, data[p.live[0]], p.stream_rois, n_masks)
+        sm, oms = self.smoothing_factor, 1 - self.smoothing_factor
+        base = p.base
+
+        def call(c, a, b):
+            sources = []
+            for s in p.live:
+                lo, hi = max(a, base[s]), min(b, base[s + 1])
+                if lo < hi:
+                    i, j = lo - base[s], hi - base[s]
+                    src = data[s].data_ptr() + i * p.frame_bytes(s) if on_device else data[s][i:j]
+                    sources.append((src, p.fmts[s], p.sizes[s], j - i, s))
+            return c.detect_rig(sources, on_device, fit.shape[0], fit, valid, sm, oms)
+
+        recs = self._chunked(ctx, p.n, call, p.h, p.w, fit, valid, p.stream_rois, n_masks)
+        return p.per_camera(self._lanes_from_records(recs))
+
+    def detect_rig_stream(self, ticks, layouts: Optional[Sequence[str]] = None, *,
+                          target_size: Optional[Tuple[int, int]] = None,
+                          stream_rois: Optional[Sequence[Optional[np.ndarray]]] = None):
+        """Generator: for every tick of ``ticks`` (a per-camera sequence, as ``detect_rig``'s ``frames``) yield what
+        ``detect_rig`` would return for it, with two ticks in flight on the native context.
+
+        The form for a recorded multi-camera drive: the Hough half of tick i runs under the edge kernels of tick i+1, and
+        the host copies of tick i+1 under the compute of tick i (``lane_rig_enqueue``).  Results, the per-camera smoothing
+        state and ``last_records`` are exactly those of calling ``detect_rig`` tick after tick with the same ``layouts`` /
+        ``target_size`` / ``stream_rois``; the state is adopted after every tick, so it carries into later ``detect_rig``
+        / ``detect_streams`` calls.  Ticks may differ in frame counts, and a camera may be None or have 0 frames.
+
+        A tick is every camera a CUDA tensor on one device, every camera a contiguous CPU tensor in pinned memory (read
+        in place), or every camera a numpy array (copied into one of two pinned buffers the generator owns).  Every tick
+        is referenced until it has been yielded; pinned tensors must not change until then.  A tick the pipeline cannot
+        take (more frames than ``max_batch``, another device, a tick without frames) drains it and goes through
+        ``detect_rig``; so do ticks whose segment lists overflow, from the state they started with.  Argument errors are
+        ``detect_rig``'s, raised when the tick's turn comes.
+        """
+        import torch
+        end = object()
+        it = iter(ticks)
+        pending = []                  # ticks taken from `ticks` and not enqueued yet, oldest first
+        queue = []                    # ticks in flight, oldest first: (tick, plan, sources kept alive, pinned buffer)
+        pinned = [None, None]         # pinned host copies of numpy ticks, one per tick in flight
+        copier = [None]               # the host threads of those copies, made by the first tick that needs them
+        ctx, S = None, 0
+        fit = valid = None            # state after the tick collected last
+
+        def take():
+            return pending.pop(0) if pending else next(it, end)
+
+        def plan(tick):
+            return self._rig_plan(tick, layouts, target_size, stream_rois, pinned=True)
+
+        def start(p) -> bool:
+            """Take the detector's state and tick p's context: whether p can be the first tick in flight."""
+            nonlocal ctx, S, fit, valid
+            if not p.n:
+                return False
+            self._grow_stream_state(len(p.cams))
+            S = self._stream_fit.shape[0]
+            ctx = self._context(p.h, p.w, self._max_batch, p.cams[p.live[0]], p.stream_rois, p.n_masks(S))
+            fit, valid = self._stream_fit.copy(), self._stream_valid.copy()
+            return p.n <= ctx.max_batch
+
+        def joins(p) -> bool:
+            """Whether tick p can queue behind the tick in flight: same context and streams, and it fits."""
+            if not p.n or len(p.cams) > S or p.n > ctx.max_batch or self._ctx is not ctx:
+                return False
+            try:
+                dev = self._device_index(p.cams[p.live[0]])
+            except ValueError:
+                return False
+            return self._ctx_key == (p.h, p.w, self._roi_key(p.stream_rois, p.n_masks(S)), dev)
+
+        def enqueue(tick, p, explicit: bool):
+            k = 1 - queue[0][3] if queue else 0      # the pinned buffer the tick in flight does not use
+            if p.kind == "host":
+                need = sum(p.cams[s].nbytes for s in p.live)
+                if pinned[k] is None or pinned[k].numel() < need:
+                    pinned[k] = torch.empty(need, dtype=torch.uint8, pin_memory=True)
+                flat, off, src, pieces = pinned[k].numpy(), 0, {}, []
+                for s in p.live:
+                    cam = np.ascontiguousarray(p.cams[s]).reshape(-1)
+                    src[s] = flat[off:off + cam.nbytes].reshape(p.cams[s].shape)
+                    cuts = list(range(0, cam.nbytes, _COPY_PIECE)) + [cam.nbytes]
+                    pieces += [(flat[off + a:off + b], cam[a:b]) for a, b in zip(cuts, cuts[1:])]
+                    off += cam.nbytes
+                if len(pieces) > 1 and copier[0] is None:
+                    copier[0] = ThreadPoolExecutor(max(1, min(8, (os.cpu_count() or 2) // 2)))
+                # one host thread copies ~10 GB/s: a tick of an 8-camera rig (35 MB) would take longer than its compute
+                list(copier[0].map(lambda ds: np.copyto(*ds), pieces) if len(pieces) > 1 else
+                     (np.copyto(*ds) for ds in pieces))
+            elif p.kind == "pinned":
+                src = {s: p.cams[s].numpy() for s in p.live}
+            else:
+                data = {s: p.cams[s].contiguous() for s in p.live}
+                dev = data[p.live[0]].device
+                torch.cuda.ExternalStream(ctx.stream(), device=dev).wait_stream(torch.cuda.current_stream(dev))
+                src = {s: (data[s], data[s].data_ptr()) for s in p.live}
+            on_device = p.kind not in ("host", "pinned")
+            sources = [(src[s][1] if on_device else src[s], p.fmts[s], p.sizes[s], p.counts[s], s) for s in p.live]
+            ctx.enqueue_rig(sources, on_device, S, fit if explicit else None, valid if explicit else None,
+                            self.smoothing_factor, 1 - self.smoothing_factor)
+            queue.append((tick, p, src, k))
+
+        def blocking(tick, p):
+            if p.kind == "pinned":                   # detect_rig takes host cameras as numpy arrays
+                tick = [None if c is None else c.numpy() for c in p.cams]
+            return self.detect_rig(tick, layouts, target_size=target_size, stream_rois=stream_rois)
+
+        def drain():
+            while ctx is not None and ctx._inflight:
+                ctx.collect(np.zeros((S, 2, 3)), np.zeros((S, 2), np.uint8))
+            queue.clear()
+
+        try:
+            nxt = take()
+            while nxt is not end or queue:
+                if not queue:                        # (re)start the pipeline with the detector's current state
+                    cur, nxt = nxt, take()
+                    p = plan(cur)                    # detect_rig's argument errors, in tick order
+                    if not start(p):
+                        yield blocking(cur, p)
+                        continue
+                    enqueue(cur, p, explicit=True)
+                if nxt is not end and len(queue) < 2:
+                    try:
+                        p = plan(nxt)
+                    except (ValueError, cv2.error):
+                        p = None                     # raised once the ticks before it are out
+                    if p is not None and joins(p):
+                        enqueue(nxt, p, explicit=False)
+                        nxt = take()
+                before = (fit.copy(), valid.copy())
+                recs = ctx.collect(fit, valid)       # fit / valid now hold the state after the oldest tick
+                head = queue.pop(0)
+                if recs["flags"].any():
+                    # truncated segment lists: the ticks behind it started from a wrong state; drain, redo this tick
+                    # the blocking way (dense context) from the state it started with, and restart with the rest
+                    pending[:0] = [q[0] for q in queue] + ([] if nxt is end else [nxt])
+                    drain()
+                    self._stream_fit, self._stream_valid = before
+                    yield blocking(head[0], head[1])
+                    nxt = take()
+                    continue
+                self._stream_fit, self._stream_valid = fit.copy(), valid.copy()
+                self.last_records = recs
+                yield head[1].per_camera(self._lanes_from_records(recs))
+        finally:
+            drain()
+            if copier[0] is not None:
+                copier[0].shutdown()
+
+    def _rig_plan(self, frames, layouts, target_size, stream_rois, pinned: bool = False) -> "_RigTick":
+        """``detect_rig``'s argument checks on one tick, and what they found.  ``pinned``: page-locked contiguous CPU
+        torch tensors are a kind of their own (``detect_rig_stream`` reads them in place)."""
         cams = list(frames)
         layouts = ["bgr"] * len(cams) if layouts is None else list(layouts)
         if len(layouts) != len(cams):
@@ -480,50 +690,18 @@ class LaneDetector:
                 sizes.append(None)
                 counts.append(0)
                 continue
-            kinds.add(("cuda", f.device.index) if _is_torch_cuda(f) else "host" if isinstance(f, np.ndarray) else "other")
+            kinds.add(("cuda", f.device.index) if _is_torch_cuda(f) else "host" if isinstance(f, np.ndarray) else
+                      "pinned" if pinned and _is_pinned_tensor(f) else "other")
             if len(kinds) > 1 or "other" in kinds:
-                raise ValueError("rig cameras must all be numpy arrays or all CUDA tensors on one device")
+                raise ValueError("rig cameras must all be numpy arrays or all CUDA tensors on one device" +
+                                 (", or all pinned contiguous CPU tensors" if pinned else ""))
             sizes.append(self._rig_frame_size(f, lay, s))
             counts.append(int(f.shape[0]))
         used = {sz for sz, t in zip(sizes, counts) if t}
         if target_size is None and len(used) > 1:
             raise ValueError(f"cameras of sizes {sorted(used)} need a target_size")
-        if not used:
-            return [[] for _ in cams]
-        h, w = next(iter(used)) if target_size is None else (target_size[1], target_size[0])
-        on_device = kinds != {"host"}
-        live = [s for s in range(len(cams)) if counts[s]]
-        if on_device:
-            import torch
-            data = {s: cams[s].contiguous() for s in live}
-            torch.cuda.current_stream(data[live[0]].device).synchronize()
-        else:
-            data = {s: np.ascontiguousarray(cams[s]) for s in live}
-        base = [0]                                   # camera s's frames are [base[s], base[s+1]) of the concatenation
-        for t in counts:
-            base.append(base[-1] + t)
-        n = base[-1]
-        self._grow_stream_state(len(cams))
-        fit, valid = self._stream_fit, self._stream_valid
-        n_masks = 1 if stream_rois is None else max(len(stream_rois), fit.shape[0])
-        ctx = self._context(h, w, n, data[live[0]], stream_rois, n_masks)
-        sm, oms = self.smoothing_factor, 1 - self.smoothing_factor
-
-        def call(c, a, b):
-            sources = []
-            for s in live:
-                lo, hi = max(a, base[s]), min(b, base[s + 1])
-                if lo < hi:
-                    sh, sw = sizes[s]
-                    i, j = lo - base[s], hi - base[s]
-                    fb = sh * sw * 3 if fmts[s] == _native.INPUT_BGR else sh * sw * 3 // 2
-                    src = data[s].data_ptr() + i * fb if on_device else data[s][i:j]
-                    sources.append((src, fmts[s], (sh, sw), j - i, s))
-            return c.detect_rig(sources, on_device, fit.shape[0], fit, valid, sm, oms)
-
-        recs = self._chunked(ctx, n, call, h, w, fit, valid, stream_rois, n_masks)
-        lanes = self._lanes_from_records(recs)
-        return [lanes[base[s]:base[s + 1]] for s in range(len(cams))]
+        hw = (None, None) if not used else next(iter(used)) if target_size is None else (target_size[1], target_size[0])
+        return _RigTick(cams, fmts, sizes, counts, next(iter(kinds)) if used else None, *hw, stream_rois)
 
     @staticmethod
     def _rig_frame_size(f, layout: str, s: int) -> Tuple[int, int]:
