@@ -70,6 +70,15 @@ struct CopyPool {
     }
 };
 
+// What the driver knows of host address `p`: cudaMemoryTypeHost for page-locked or registered memory,
+// cudaMemoryTypeUnregistered for ordinary memory (or an address it cannot query).
+inline cudaMemoryType host_memory_type(const void *p)
+{
+    cudaPointerAttributes pa{};
+    const cudaMemoryType t = cudaPointerGetAttributes(&pa, p) == cudaSuccess ? pa.type : cudaMemoryTypeUnregistered;
+    cudaGetLastError();
+    return t;
+}
 
 // One staging ring per device, shared by the contexts and the context-free entry points on it; the worker threads and
 // pinned buffers are created by the first staged copy.  h2d() is blocking on the host side only as far as the memcpy
@@ -101,10 +110,7 @@ struct HostStager {
     // through the driver's own path than through worker wake-ups.
     static bool pageable(const void *p, size_t bytes)
     {
-        cudaPointerAttributes pa{};
-        const bool un = cudaPointerGetAttributes(&pa, p) != cudaSuccess || pa.type == cudaMemoryTypeUnregistered;
-        cudaGetLastError();
-        return un && bytes >= ((size_t)24 << 20);
+        return host_memory_type(p) == cudaMemoryTypeUnregistered && bytes >= ((size_t)24 << 20);
     }
     // Through the ring, whatever the size (the caller has decided with pageable()).
     cudaError_t h2d(uint8_t *dst, const uint8_t *src, size_t bytes, cudaStream_t st)

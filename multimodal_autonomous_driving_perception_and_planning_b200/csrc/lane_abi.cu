@@ -340,13 +340,6 @@ int run_stages(lane_ctx *c, const uint8_t *frames_dev, int off, int m, const int
     return stage_check(c, "fit");
 }
 
-// What the caller's frames are: layout (LANE_INPUT_*) and size.  Unless they already are the context's H x W BGR
-// frames, the ingest kernels (k0_common.cuh) make those from them on the device before the path runs.
-struct Ingest {
-    int format, h, w;
-    size_t frame_bytes() const { return format == LANE_INPUT_BGR ? (size_t)h * w * 3 : (size_t)h * w * 3 / 2; }
-};
-
 // What a batch enqueues before its frames: the stream its back half runs on, its stream ids, every frame's ROI plane
 // and, when given, the explicit EMA state it starts from.
 int begin_batch(lane_ctx *c, bool on_device, int n, const int32_t *stream_id, int S, const double *prev_fit,
@@ -385,25 +378,24 @@ int begin_batch(lane_ctx *c, bool on_device, int n, const int32_t *stream_id, in
 // (~50 GB/s) and the compute of the previous chunk overlap; >= 4 chunks when possible.
 int host_chunk(int n) { return std::max(1, std::min(64, (n + 3) / 4)); }
 
-// The copy stream of host batches and its events, created on first use.
-int ensure_copy_stream(lane_ctx *c)
+// The copy stream of host batches (created on first use), and where a batch's copies start: once the work enqueued
+// before them is done with the staging they write.  That is everything on the compute stream, or for a batch staged
+// in its result slot only the ingest launch that last read the slot's staging: its copies then run under the batch
+// in flight.
+int begin_host_copies(lane_ctx *c, bool staged)
 {
-    if (c->copy_st) return LANE_OK;
-    for (auto &e : c->copy_ev) CU(e.create(cudaEventDisableTiming));
-    CU(c->start_ev.create(cudaEventDisableTiming));
-    for (auto &sl : c->slots) CU(sl.src_read.create(cudaEventDisableTiming));
-    CU(c->copy_st.create(cudaStreamNonBlocking));
-    return LANE_OK;
-}
-
-// The copy stream of chunked host batches; the batch's copies start once the work enqueued before it is done with the
-// staging buffers.
-int begin_host_copies(lane_ctx *c)
-{
-    const int rc = ensure_copy_stream(c);
-    if (rc) return rc;
-    CU(cudaEventRecord(c->start_ev, c->st));
-    CU(cudaStreamWaitEvent(c->copy_st, c->start_ev, 0));
+    if (!c->copy_st) {
+        for (auto &e : c->copy_ev) CU(e.create(cudaEventDisableTiming));
+        CU(c->start_ev.create(cudaEventDisableTiming));
+        for (auto &sl : c->slots) CU(sl.src_read.create(cudaEventDisableTiming));
+        CU(c->copy_st.create(cudaStreamNonBlocking));
+    }
+    if (staged) {
+        CU(cudaStreamWaitEvent(c->copy_st, c->slots[c->cur].src_read, 0));
+    } else {
+        CU(cudaEventRecord(c->start_ev, c->st));
+        CU(cudaStreamWaitEvent(c->copy_st, c->start_ev, 0));
+    }
     return LANE_OK;
 }
 
@@ -438,146 +430,118 @@ int end_batch(lane_ctx *c, bool on_device, int n, int S, const uint8_t *frames_d
     return LANE_OK;
 }
 
-// Enqueue the whole batch.  Device-resident frames run as one chunk, host frames chunk by chunk (host_chunk).
-int enqueue(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int32_t *stream_id, int S,
-            const double *prev_fit, const uint8_t *prev_valid, Ingest in)
-{
-    int rc = begin_batch(c, on_device, n, stream_id, S, prev_fit, prev_valid);
-    if (rc) return rc;
-    const int32_t *sid = stream_id ? c->d_stream_id.get() : nullptr;
-    const uint8_t *frames_dev = frames;
-    const size_t bgr_bytes = (size_t)c->g.H * c->g.W * 3;
-    const bool convert = in.format != LANE_INPUT_BGR || in.h != c->g.H || in.w != c->g.W;
-    if (convert) CU(c->d_frames.lazy((size_t)c->max_batch * bgr_bytes));
-    if (on_device) {
-        if (convert) {                               // source already on the device: one ingest launch, then the usual path
-            CU(launch_ingest(frames, in.format, n, in.h, in.w, c->d_frames, c->g.H, c->g.W, c->st));
-            frames_dev = c->d_frames;
-        }
-        rc = run_stages(c, frames_dev, 0, n, sid, S, c->profiling);
-        if (rc) return rc;
-    } else {
-        // bytes per frame that cross PCIe: the source's own (3 B/px BGR, 1.5 B/px YUV 4:2:0 at the decoder's size),
-        // converted / resized on the device chunk by chunk
-        const size_t bytes = in.frame_bytes();
-        CU(c->d_frames.lazy((size_t)c->max_batch * bgr_bytes));
-        if (convert) { rc = ensure_src(c, c->d_src, (size_t)c->max_batch * bytes); if (rc) return rc; }
-        uint8_t *d_in = convert ? c->d_src : c->d_frames;
-        frames_dev = c->d_frames;
-        // pinned (or registered) host memory goes straight to the copy engine; ordinary memory through the device's
-        // staging ring.  Decided once for the whole batch: every chunk of a large pageable batch is staged.
-        HostStager *ring = HostStager::pageable(frames, bytes * (size_t)n) ? &lane_device_host(c->device).stager : nullptr;
-        const int chunk = host_chunk(n);
-        rc = begin_host_copies(c); if (rc) return rc;
-        int k = 0;
-        for (int off = 0; off < n; off += chunk, k++) {
-            const int m = std::min(chunk, n - off);
-            uint8_t *to = d_in + (size_t)off * bytes;
-            const uint8_t *from = frames + (size_t)off * bytes;
-            if (ring)
-                CU(ring->h2d(to, from, bytes * m, c->copy_st));
-            else
-                CU(cudaMemcpyAsync(to, from, bytes * m, cudaMemcpyHostToDevice, c->copy_st));
-            rc = chunk_copied(c, k); if (rc) return rc;
-            if (convert)
-                CU(launch_ingest(c->d_src + (size_t)off * bytes, in.format, m, in.h, in.w, c->d_frames + (size_t)off * bgr_bytes,
-                                 c->g.H, c->g.W, c->st));
-            rc = run_stages(c, c->d_frames, off, m, sid, S, false);
-            if (rc) return rc;
-        }
-    }
-    return end_batch(c, on_device, n, S, frames_dev);
-}
-
-// Bytes of one dense frame of a rig source.
-size_t rig_frame_bytes(const lane_rig_source &r)
+// Bytes of one dense frame of a source: its own size and layout (3 B/px BGR, 1.5 B/px YUV 4:2:0).
+size_t frame_bytes(const lane_rig_source &r)
 {
     return r.format == LANE_INPUT_BGR ? (size_t)r.src_h * r.src_w * 3 : (size_t)r.src_h * r.src_w * 3 / 2;
 }
 
-// Enqueue a rig batch (validated): the sources' frames in source order, each camera at its own size and layout.  One
-// k0_rig_ingest launch makes the context's BGR frames of the whole batch, driven by the batch's descriptor table; the rest
-// of the path is enqueue's.  Device sources are read where they are.  Host sources of lane_detect_rig (staged = false)
-// are copied chunk by chunk into the context's d_src behind the compute of the chunk before, one ingest launch per chunk.
-// Host sources of lane_rig_enqueue (staged, page-locked) are copied whole into the slot's own d_src behind the compute
-// of the tick before, and then run like device sources.  `staged` names host sources only: device sources are never
-// copied.
-int enqueue_rig(lane_ctx *c, const lane_rig_source *sources, int n_sources, bool on_device, int n, const int32_t *stream_id,
-                int S, const double *prev_fit, const uint8_t *prev_valid, bool staged)
+// How the context's H x W BGR frames are made from the batch's sources before the path runs (k0_common.cuh): they
+// already are those frames; one launch_ingest over frames of one layout and size; or k0_rig_ingest over every frame,
+// each with its own layout and size, driven by the batch's descriptor table.
+enum class Ingest { none, single, rig };
+
+// Enqueue a validated batch: the frames of `sources` in source order, all on the device or all in host memory.  Device
+// frames are read where they are.  Host frames land one after another in a device buffer, behind the compute of what
+// came before.  Host frames `staged` (lane_rig_enqueue, page-locked) are copied whole into the result slot's own
+// staging, after the ingest that last read it; the batch then runs like a device batch.  Other host frames are copied
+// chunk by chunk (host_chunk) into the context's buffers, each chunk behind the compute of the chunk before.
+int enqueue(lane_ctx *c, const lane_rig_source *sources, int n_sources, bool on_device, bool staged, Ingest ingest,
+            int n, const int32_t *stream_id, int S, const double *prev_fit, const uint8_t *prev_valid)
 {
     staged = staged && !on_device;
+    const bool whole = on_device || staged;          // one chunk: one ingest launch and one pass of the path
     lane_ctx::slot_t &sl = c->slots[c->cur];
     const size_t B = (size_t)c->max_batch, bgr_bytes = (size_t)c->g.H * c->g.W * 3;
-    CU(c->d_frames.lazy(B * bgr_bytes));
-    CU(c->d_rig.lazy(2 * B));
-    if (!sl.h_rig) CU(sl.h_rig.alloc(B));
-    // host sources land in the staging one after another in source order: frame f at byte offset at[f]
-    DeviceArray<uint8_t> &src = staged ? sl.d_src : c->d_src;
+    if (ingest != Ingest::none || !on_device) CU(c->d_frames.lazy(B * bgr_bytes));
+    // host frame f lands at byte offset at[f]: in the context's frames when they need no ingest, else in source staging
     std::vector<size_t> at(n + 1, 0);
     for (int s = 0, f = 0; s < n_sources; s++)
-        for (int j = 0; j < sources[s].n; j++, f++) at[f + 1] = at[f] + rig_frame_bytes(sources[s]);
-    if (!on_device) { const int rc = ensure_src(c, src, at[n]); if (rc) return rc; }
-    for (int s = 0, f = 0; s < n_sources; s++) {
-        const lane_rig_source &r = sources[s];
-        if (!r.n) continue;
-        RigFrame d;
-        CU(rig_frame(nullptr, r.format, r.src_h, r.src_w, c->g.H, c->g.W, &d));
-        for (int j = 0; j < r.n; j++, f++) {
-            d.src = on_device ? r.frames + j * rig_frame_bytes(r) : src + at[f];
-            sl.h_rig[f] = d;
+        for (int j = 0; j < sources[s].n; j++, f++) at[f + 1] = at[f] + frame_bytes(sources[s]);
+    uint8_t *land = c->d_frames;
+    if (!on_device && ingest != Ingest::none) {
+        DeviceArray<uint8_t> &src = staged ? sl.d_src : c->d_src;
+        const int rc = ensure_src(c, src, at[n]);
+        if (rc) return rc;
+        land = src;
+    }
+    if (ingest == Ingest::rig) {
+        CU(c->d_rig.lazy(2 * B));
+        if (!sl.h_rig) CU(sl.h_rig.alloc(B));
+        for (int s = 0, f = 0; s < n_sources; s++) {
+            const lane_rig_source &r = sources[s];
+            if (!r.n) continue;
+            RigFrame d;
+            CU(rig_frame(nullptr, r.format, r.src_h, r.src_w, c->g.H, c->g.W, &d));
+            for (int j = 0; j < r.n; j++, f++) {
+                d.src = on_device ? r.frames + j * frame_bytes(r) : land + at[f];
+                sl.h_rig[f] = d;
+            }
         }
     }
-    const bool whole = on_device || staged;          // one ingest launch and one pass of the path for the batch
     int rc = begin_batch(c, whole, n, stream_id, S, prev_fit, prev_valid);
     if (rc) return rc;
-    RigFrame *rig = c->d_rig + (size_t)c->cur * B;
-    CU(cudaMemcpyAsync(rig, sl.h_rig, sizeof(RigFrame) * n, cudaMemcpyHostToDevice, c->st));
-    const int32_t *sid = c->d_stream_id;
-    if (whole) {
-        if (staged) {
-            // The copies wait only for the ingest that last read this slot's staging, not for the tick in flight on
-            // the compute stream: they run under it.  The ingest waits for them.
-            rc = ensure_copy_stream(c); if (rc) return rc;
-            CU(cudaStreamWaitEvent(c->copy_st, sl.src_read, 0));
-            for (int s = 0, first = 0; s < n_sources; first += sources[s].n, s++)
-                if (sources[s].n)
-                    CU(cudaMemcpyAsync(src + at[first], sources[s].frames, at[first + sources[s].n] - at[first],
-                                       cudaMemcpyHostToDevice, c->copy_st));
-            rc = chunk_copied(c, c->cur); if (rc) return rc;
-        }
-        launch_rig_ingest(rig, n, c->d_frames, c->g.H, c->g.W, c->st);
-        if (staged) CU(cudaEventRecord(sl.src_read, c->st));
-        rc = run_stages(c, c->d_frames, 0, n, sid, S, c->profiling);
-        if (rc) return rc;
-    } else {
-        // pinned (or registered) sources go straight to the copy engine, ordinary memory through the device's staging
-        // ring when the batch is large; decided once per source for the whole batch
-        HostStager *stager = &lane_device_host(c->device).stager;
-        std::vector<HostStager *> ring(n_sources);
+    RigFrame *rig = ingest == Ingest::rig ? c->d_rig + (size_t)c->cur * B : nullptr;
+    if (rig) CU(cudaMemcpyAsync(rig, sl.h_rig, sizeof(RigFrame) * n, cudaMemcpyHostToDevice, c->st));
+    const int32_t *sid = stream_id ? c->d_stream_id.get() : nullptr;
+    const uint8_t *frames_dev = on_device && ingest == Ingest::none ? sources[0].frames : c->d_frames.get();
+    // pinned (or registered) host frames go straight to the copy engine, ordinary memory through the device's staging
+    // ring when the batch is large; decided once per source for the whole batch
+    std::vector<HostStager *> ring(n_sources, nullptr);
+    if (!on_device) {
         for (int s = 0; s < n_sources; s++)
-            ring[s] = sources[s].n && HostStager::pageable(sources[s].frames, at[n]) ? stager : nullptr;
-        const int chunk = host_chunk(n);
-        rc = begin_host_copies(c); if (rc) return rc;
-        int k = 0;
-        for (int off = 0; off < n; off += chunk, k++) {
-            const int m = std::min(chunk, n - off);
+            if (sources[s].n && HostStager::pageable(sources[s].frames, at[n])) ring[s] = &lane_device_host(c->device).stager;
+        rc = begin_host_copies(c, staged); if (rc) return rc;
+    }
+    const int chunk = whole ? n : host_chunk(n);
+    for (int off = 0, k = 0; off < n; off += chunk, k++) {
+        const int m = std::min(chunk, n - off);
+        if (!on_device) {
             // the chunk's frames of each source are contiguous on both sides: one copy per source
             for (int s = 0, first = 0; s < n_sources && first < off + m; first += sources[s].n, s++) {
                 const int lo = std::max(off, first), hi = std::min(off + m, first + sources[s].n);
                 if (lo >= hi) continue;
-                const uint8_t *from = sources[s].frames + (lo - first) * rig_frame_bytes(sources[s]);
+                const uint8_t *from = sources[s].frames + (lo - first) * frame_bytes(sources[s]);
                 if (ring[s])
-                    CU(ring[s]->h2d(c->d_src + at[lo], from, at[hi] - at[lo], c->copy_st));
+                    CU(ring[s]->h2d(land + at[lo], from, at[hi] - at[lo], c->copy_st));
                 else
-                    CU(cudaMemcpyAsync(c->d_src + at[lo], from, at[hi] - at[lo], cudaMemcpyHostToDevice, c->copy_st));
+                    CU(cudaMemcpyAsync(land + at[lo], from, at[hi] - at[lo], cudaMemcpyHostToDevice, c->copy_st));
             }
-            rc = chunk_copied(c, k); if (rc) return rc;
-            launch_rig_ingest(rig + off, m, c->d_frames + (size_t)off * bgr_bytes, c->g.H, c->g.W, c->st);
-            rc = run_stages(c, c->d_frames, off, m, sid, S, false);
-            if (rc) return rc;
+            rc = chunk_copied(c, staged ? c->cur : k); if (rc) return rc;
         }
+        uint8_t *to = c->d_frames + (size_t)off * bgr_bytes;
+        if (ingest == Ingest::single) {                // one source: its frames are contiguous on either side
+            const lane_rig_source &r = sources[0];
+            CU(launch_ingest((on_device ? r.frames : land) + at[off], r.format, m, r.src_h, r.src_w, to, c->g.H, c->g.W, c->st));
+        } else if (rig) {
+            launch_rig_ingest(rig + off, m, to, c->g.H, c->g.W, c->st);
+        }
+        if (staged) CU(cudaEventRecord(sl.src_read, c->st));
+        rc = run_stages(c, frames_dev, off, m, sid, S, whole && c->profiling);
+        if (rc) return rc;
     }
-    return end_batch(c, whole, n, S, c->d_frames);
+    return end_batch(c, whole, n, S, frames_dev);
+}
+
+// One source's fields: layout, size (even for YUV 4:2:0) and frames.  `s` numbers it in the message; < 0: the call's
+// only source.
+int check_source(lane_ctx *c, int s, const lane_rig_source &r)
+{
+    char who[32] = "";
+    if (s >= 0) snprintf(who, sizeof(who), "source %d: ", s);
+    if (r.format != LANE_INPUT_BGR && r.format != LANE_INPUT_NV12 && r.format != LANE_INPUT_I420)
+        return fail(c, LANE_ERR_INVALID, "%sunknown input format %d", who, r.format);
+    if (r.src_h < 1 || r.src_w < 1) return fail(c, LANE_ERR_INVALID, "%sbad source size %dx%d", who, r.src_w, r.src_h);
+    if (r.format != LANE_INPUT_BGR && ((r.src_h | r.src_w) & 1))
+        return fail(c, LANE_ERR_INVALID, "%sNV12 / I420 needs even width and height (%dx%d)", who, r.src_w, r.src_h);
+    if (r.n && !r.frames) return fail(c, LANE_ERR_INVALID, "%sframes is null", who);
+    return LANE_OK;
+}
+
+// The ingest kernels that resize put the batch's frames on the grid's z.
+int check_grid(lane_ctx *c, long long n)
+{
+    return n > 65535 ? fail(c, LANE_ERR_UNSUPPORTED, "batch %lld above 65535", n) : LANE_OK;
 }
 
 // The checks lane_detect_rig and lane_rig_enqueue share before check_call: every source's fields, the batch size, and
@@ -588,18 +552,13 @@ int check_rig(lane_ctx *c, const lane_rig_source *sources, int n_sources, int n_
     for (int s = 0; s < n_sources; s++) {
         const lane_rig_source &r = sources[s];
         if (r.n < 0) return fail(c, LANE_ERR_INVALID, "source %d: negative frame count %d", s, r.n);
-        if (r.format != LANE_INPUT_BGR && r.format != LANE_INPUT_NV12 && r.format != LANE_INPUT_I420)
-            return fail(c, LANE_ERR_INVALID, "source %d: unknown input format %d", s, r.format);
-        if (r.src_h < 1 || r.src_w < 1) return fail(c, LANE_ERR_INVALID, "source %d: bad size %dx%d", s, r.src_w, r.src_h);
-        if (r.format != LANE_INPUT_BGR && ((r.src_h | r.src_w) & 1))
-            return fail(c, LANE_ERR_INVALID, "source %d: NV12 / I420 needs even width and height (%dx%d)", s, r.src_w, r.src_h);
+        if (const int rc = check_source(c, s, r)) return rc;
         if (r.stream_id < 0 || r.stream_id >= n_streams)
             return fail(c, LANE_ERR_INVALID, "source %d: stream_id %d outside [0,%d)", s, r.stream_id, n_streams);
-        if (r.n && !r.frames) return fail(c, LANE_ERR_INVALID, "source %d: frames is null", s);
         n += r.n;
     }
     if (n < 1 || n > c->max_batch) return fail(c, LANE_ERR_INVALID, "bad batch: %lld frames (max_batch=%d)", n, c->max_batch);
-    if (n > 65535) return fail(c, LANE_ERR_UNSUPPORTED, "batch %lld above 65535", n);     // the ingest grid's z
+    if (const int rc = check_grid(c, n)) return rc;
     for (int s = 0; s < n_sources; s++) stream_id.insert(stream_id.end(), sources[s].n, sources[s].stream_id);
     return (int)n;
 }
@@ -607,12 +566,7 @@ int check_rig(lane_ctx *c, const lane_rig_source *sources, int n_sources, int n_
 // Whether host memory [p, p + bytes) is page-locked or registered, so the copy engine reads it where it is.
 bool page_locked(const void *p, size_t bytes)
 {
-    cudaPointerAttributes first{}, last{};
-    const bool ok = cudaPointerGetAttributes(&first, p) == cudaSuccess && first.type == cudaMemoryTypeHost &&
-                    cudaPointerGetAttributes(&last, (const uint8_t *)p + bytes - 1) == cudaSuccess &&
-                    last.type == cudaMemoryTypeHost;
-    cudaGetLastError();
-    return ok;
+    return host_memory_type(p) == cudaMemoryTypeHost && host_memory_type((const uint8_t *)p + bytes - 1) == cudaMemoryTypeHost;
 }
 
 // What every detect call checks and sets up before it enqueues: arguments and context state, the context's device, the
@@ -647,18 +601,28 @@ int check_call(lane_ctx *c, const void *frames, int n, const int32_t *stream_id,
     return LANE_OK;
 }
 
-// lane_detect_batch and its ingest forms: validate, enqueue, collect.
-int detect_blocking(lane_ctx *c, const uint8_t *frames, bool on_device, int n, const int32_t *stream_id, int n_streams,
-                    double *prev_fit, uint8_t *prev_valid, lane_record *out, Ingest in)
+// Enqueue the frames of a single-format call (checked by check_call) as a batch of one source, with the caller's
+// stream id per frame.  They need an ingest unless they are BGR at the context's size.
+int enqueue_frames(lane_ctx *c, const lane_rig_source &r, bool on_device, const int32_t *stream_id, int S,
+                   const double *prev_fit, const uint8_t *prev_valid)
 {
-    if (in.format != LANE_INPUT_BGR && ((in.h | in.w) & 1))
-        return fail(c, LANE_ERR_INVALID, "NV12 / I420 needs even width and height (%dx%d)", in.w, in.h);
-    int rc = check_call(c, frames, n, stream_id, n_streams, prev_fit, prev_valid);
+    const bool resize = r.src_h != c->g.H || r.src_w != c->g.W;
+    if (resize)
+        if (const int rc = check_grid(c, r.n)) return rc;
+    const Ingest ingest = r.format == LANE_INPUT_BGR && !resize ? Ingest::none : Ingest::single;
+    return enqueue(c, &r, 1, on_device, false, ingest, r.n, stream_id, S, prev_fit, prev_valid);
+}
+
+// lane_detect_batch and its ingest forms: validate, enqueue, collect.
+int detect_blocking(lane_ctx *c, const lane_rig_source &r, bool on_device, const int32_t *stream_id, int n_streams,
+                    double *prev_fit, uint8_t *prev_valid, lane_record *out)
+{
+    int rc = check_source(c, -1, r);
+    if (rc) return rc;
+    rc = check_call(c, r.frames, r.n, stream_id, n_streams, prev_fit, prev_valid);
     if (rc) return rc;
     if (!out) return fail(c, LANE_ERR_INVALID, "out is null");
-    if (n > 65535 && (in.h != c->g.H || in.w != c->g.W))           // the resize kernels put the batch on the grid's z
-        return fail(c, LANE_ERR_UNSUPPORTED, "batch %d above 65535", n);
-    rc = enqueue(c, frames, on_device, n, stream_id, n_streams, prev_fit, prev_valid, in);
+    rc = enqueue_frames(c, r, on_device, stream_id, n_streams, prev_fit, prev_valid);
     if (rc) return rc;
     return lane_detect_collect(c, prev_fit, prev_valid, out);
 }
@@ -954,7 +918,7 @@ int lane_detect_enqueue(lane_ctx *c, const uint8_t *frames_dev, int n, const int
 {
     const int rc = check_call(c, frames_dev, n, stream_id, n_streams, prev_fit, prev_valid);
     if (rc) return rc;
-    return enqueue(c, frames_dev, true, n, stream_id, n_streams, prev_fit, prev_valid, Ingest{LANE_INPUT_BGR, c->g.H, c->g.W});
+    return enqueue_frames(c, {frames_dev, LANE_INPUT_BGR, c->g.H, c->g.W, n, 0}, true, stream_id, n_streams, prev_fit, prev_valid);
 }
 
 int lane_detect_collect(lane_ctx *c, double *prev_fit, uint8_t *prev_valid, lane_record *out)
@@ -980,16 +944,16 @@ int lane_detect_batch(lane_ctx *c, const uint8_t *frames, int frames_on_device, 
                       int n_streams, double *prev_fit, uint8_t *prev_valid, lane_record *out)
 {
     if (!c) return LANE_ERR_INVALID;
-    return detect_blocking(c, frames, frames_on_device != 0, n, stream_id, n_streams, prev_fit, prev_valid, out,
-                           Ingest{LANE_INPUT_BGR, c->g.H, c->g.W});
+    return detect_blocking(c, {frames, LANE_INPUT_BGR, c->g.H, c->g.W, n, 0}, frames_on_device != 0, stream_id, n_streams,
+                           prev_fit, prev_valid, out);
 }
 
 int lane_detect_batch_nv12(lane_ctx *c, const uint8_t *frames_nv12, int frames_on_device, int n, const int32_t *stream_id,
                            int n_streams, double *prev_fit, uint8_t *prev_valid, lane_record *out)
 {
     if (!c) return LANE_ERR_INVALID;
-    return detect_blocking(c, frames_nv12, frames_on_device != 0, n, stream_id, n_streams, prev_fit, prev_valid, out,
-                           Ingest{LANE_INPUT_NV12, c->g.H, c->g.W});
+    return detect_blocking(c, {frames_nv12, LANE_INPUT_NV12, c->g.H, c->g.W, n, 0}, frames_on_device != 0, stream_id,
+                           n_streams, prev_fit, prev_valid, out);
 }
 
 int lane_detect_batch_ingest(lane_ctx *c, const uint8_t *frames, int frames_on_device, int n, int format, int src_h,
@@ -997,11 +961,8 @@ int lane_detect_batch_ingest(lane_ctx *c, const uint8_t *frames, int frames_on_d
                              lane_record *out)
 {
     if (!c) return LANE_ERR_INVALID;
-    if (format != LANE_INPUT_BGR && format != LANE_INPUT_NV12 && format != LANE_INPUT_I420)
-        return fail(c, LANE_ERR_INVALID, "unknown input format %d", format);
-    if (src_h < 1 || src_w < 1) return fail(c, LANE_ERR_INVALID, "bad source size %dx%d", src_w, src_h);
-    return detect_blocking(c, frames, frames_on_device != 0, n, stream_id, n_streams, prev_fit, prev_valid, out,
-                           Ingest{format, src_h, src_w});
+    return detect_blocking(c, {frames, format, src_h, src_w, n, 0}, frames_on_device != 0, stream_id, n_streams, prev_fit,
+                           prev_valid, out);
 }
 
 int lane_detect_rig(lane_ctx *c, const lane_rig_source *sources, int n_sources, int frames_on_device, int n_streams,
@@ -1014,7 +975,8 @@ int lane_detect_rig(lane_ctx *c, const lane_rig_source *sources, int n_sources, 
     if (n < 0) return n;
     int rc = check_call(c, sources, n, stream_id.data(), n_streams, prev_fit, prev_valid);
     if (rc) return rc;
-    rc = enqueue_rig(c, sources, n_sources, frames_on_device != 0, n, stream_id.data(), n_streams, prev_fit, prev_valid, false);
+    rc = enqueue(c, sources, n_sources, frames_on_device != 0, false, Ingest::rig, n, stream_id.data(), n_streams, prev_fit,
+                 prev_valid);
     if (rc) return rc;
     return lane_detect_collect(c, prev_fit, prev_valid, out);
 }
@@ -1028,12 +990,13 @@ int lane_rig_enqueue(lane_ctx *c, const lane_rig_source *sources, int n_sources,
     if (n < 0) return n;
     if (!frames_on_device)
         for (int s = 0; s < n_sources; s++)
-            if (sources[s].n && !page_locked(sources[s].frames, sources[s].n * rig_frame_bytes(sources[s])))
+            if (sources[s].n && !page_locked(sources[s].frames, sources[s].n * frame_bytes(sources[s])))
                 return fail(c, LANE_ERR_INVALID, "source %d: host frames must be page-locked or registered memory "
                             "(cudaHostAlloc, cudaHostRegister, torch pin_memory)", s);
     const int rc = check_call(c, sources, n, stream_id.data(), n_streams, prev_fit, prev_valid);
     if (rc) return rc;
-    return enqueue_rig(c, sources, n_sources, frames_on_device != 0, n, stream_id.data(), n_streams, prev_fit, prev_valid, true);
+    return enqueue(c, sources, n_sources, frames_on_device != 0, true, Ingest::rig, n, stream_id.data(), n_streams, prev_fit,
+                   prev_valid);
 }
 
 int lane_get_stage_ms(lane_ctx *c, float ms[LANE_NUM_STAGES], int32_t launches[LANE_NUM_STAGES])

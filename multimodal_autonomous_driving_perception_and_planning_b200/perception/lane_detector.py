@@ -49,6 +49,69 @@ def _is_pinned_tensor(x) -> bool:
             and (x.numel() == 0 or bool(x.is_pinned())))
 
 
+def _frame_bytes(fmt: int, h: int, w: int) -> int:
+    """Bytes of one h x w frame in layout ``fmt`` (INPUT_*): 3 B/px BGR, 1.5 B/px YUV 4:2:0."""
+    return h * w * 3 if fmt == _native.INPUT_BGR else h * w * 3 // 2
+
+
+def _two_deep(items, plan, start, joins, enqueue, blocking, restore, adopt):
+    """The queue of ``detect_batches`` and ``detect_rig_stream``: yields one result per item, in order, with up to two
+    items in flight on a native context.  ``plan(item)`` checks an item when its turn comes (raising its argument errors
+    after the items before it are out) and returns ``p``.  ``start(p)`` takes the detector's state for a first item in
+    flight, ``(ctx, fit, valid)`` (the arrays ``ctx.collect`` fills), or None to run it through ``blocking(item, p)``.
+    An item queues behind the one in flight if ``joins(p)``.  ``enqueue(item, p, explicit)`` starts it from ``fit`` /
+    ``valid`` or from the device state, returning what must live until it is collected.  ``restore(fit, valid)`` and
+    ``adopt(recs, p)`` make the state before / after an item the detector's; ``adopt`` returns its result.  An item whose
+    segment lists overflow started the items behind it from a wrong state: the queue is drained, the item redone through
+    ``blocking`` from the state before it, and the items behind it planned again."""
+    it, pending, queue = iter(items), [], []     # queue: (item, plan, what enqueue keeps alive), oldest first
+    end = object()
+    ctx = fit = valid = None
+
+    def take():
+        return pending.pop(0) if pending else next(it, end)
+
+    def drain():
+        while ctx is not None and ctx._inflight:
+            ctx.collect(fit.copy(), valid.copy())
+        queue.clear()
+
+    try:
+        nxt = take()
+        while nxt is not end or queue:
+            if not queue:                            # (re)start with the detector's current state
+                cur, nxt = nxt, take()
+                p = plan(cur)
+                started = start(p)
+                if started is None:
+                    yield blocking(cur, p)
+                    continue
+                ctx, fit, valid = started
+                queue.append((cur, p, enqueue(cur, p, True)))
+            if nxt is not end and len(queue) < 2:
+                try:
+                    p = plan(nxt)
+                except Exception:
+                    p = end                          # planned again, and raised, when its turn comes
+                if p is not end and joins(p):
+                    queue.append((nxt, p, enqueue(nxt, p, False)))
+                    nxt = take()
+            before = (fit.copy(), valid.copy())
+            recs = ctx.collect(fit, valid)           # fit / valid now hold the state after the oldest item
+            item, p, _ = queue.pop(0)
+            if recs["flags"].any():
+                # truncated segment lists: redo the item the blocking way (dense context) and restart with the rest
+                pending[:0] = [q[0] for q in queue] + ([] if nxt is end else [nxt])
+                drain()
+                restore(*before)
+                yield blocking(item, p)
+                nxt = take()
+                continue
+            yield adopt(recs, p)
+    finally:
+        drain()
+
+
 @dataclass
 class _RigTick:
     """One tick of a rig as ``detect_rig``'s checks found it: camera s has ``counts[s]`` frames in layout ``fmts[s]``
@@ -72,10 +135,6 @@ class _RigTick:
 
     def n_masks(self, n_streams: int) -> int:
         return 1 if self.stream_rois is None else max(len(self.stream_rois), n_streams)
-
-    def frame_bytes(self, s: int) -> int:
-        sh, sw = self.sizes[s]
-        return sh * sw * 3 if self.fmts[s] == _native.INPUT_BGR else sh * sw * 3 // 2
 
     def per_camera(self, items):
         return [items[self.base[s]:self.base[s + 1]] for s in range(len(self.cams))]
@@ -228,7 +287,7 @@ class LaneDetector:
         n, sh, sw = int(frames.shape[0]), int(frames.shape[1]), int(frames.shape[2])
         if fmt != _native.INPUT_BGR:
             sh = sh * 2 // 3
-        fbytes = sh * sw * 3 if fmt == _native.INPUT_BGR else sh * sw * 3 // 2
+        fbytes = _frame_bytes(fmt, sh, sw)
         h, w = (sh, sw) if target_size is None else (target_size[1], target_size[0])
         n_masks = 1 if stream_rois is None else max(len(stream_rois), n_streams)
         ctx = self._context(h, w, n, frames, stream_rois, n_masks)
@@ -330,75 +389,48 @@ class LaneDetector:
         waits for the host between batches and the Hough half of batch i runs under the edge kernels of batch i+1.
         Results, state chain and ``prev_*_fit`` are exactly those of calling ``detect_batch`` batch after batch; a batch whose
         segment lists overflow is re-run on the dense context like there (the queue is drained and restarted around it).
-        Batches that are not CUDA tensors of one common shape on one device simply go through ``detect_batch``."""
+        Batches that are not CUDA tensors of one common shape on one device simply go through ``detect_batch``.  A
+        malformed batch raises ``detect_batch``'s error when its turn comes, after the batches before it are yielded."""
         import torch
-        it = iter(batches)
-        queue = []                                   # [tensor, state_before (fit, valid)] of the batches in flight
-        ctx = None
-        fit, valid = self._state_arrays()
+        ctx = fit = valid = None
         s, oms = self.smoothing_factor, 1 - self.smoothing_factor
 
-        def streamable(fr):
+        def plan(fr):
+            self._check_frames(fr, batched=True)
+            return fr
+
+        def joins(fr) -> bool:
             return (_is_torch_cuda(fr) and len(fr.shape) == 4 and fr.shape[0] > 0 and ctx is not None and
                     fr.shape[0] <= ctx.max_batch and (int(fr.shape[1]), int(fr.shape[2])) == (ctx.height, ctx.width) and
                     fr.device.index == ctx.device)
 
-        def enqueue(fr, explicit):
+        def start(fr):
+            nonlocal ctx, fit, valid
+            if _is_torch_cuda(fr) and fr.shape[0] > 0:
+                ctx = self._context(int(fr.shape[1]), int(fr.shape[2]), int(fr.shape[0]), fr)
+            if not joins(fr):
+                return None
+            fit, valid = self._state_arrays()
+            return ctx, fit, valid
+
+        def enqueue(fr, _, explicit: bool):
             fr = fr.contiguous()
             torch.cuda.ExternalStream(ctx.stream(), device=fr.device).wait_stream(torch.cuda.current_stream(fr.device))
-            if explicit:
-                ctx.enqueue(fr.data_ptr(), int(fr.shape[0]), None, 1, fit, valid, s, oms)
-            else:
-                ctx.enqueue(fr.data_ptr(), int(fr.shape[0]), None, 1, None, None, s, oms)
-            queue.append([fr, None])
+            ctx.enqueue(fr.data_ptr(), int(fr.shape[0]), None, 1, fit if explicit else None, valid if explicit else None,
+                        s, oms)
+            return fr
 
-        def drain():
-            while ctx is not None and ctx._inflight:
-                ctx.collect(np.zeros((1, 2, 3)), np.zeros((1, 2), np.uint8))
-            queue.clear()
+        def restore(fit0, valid0):
+            for side, p in enumerate(("prev_left_fit", "prev_right_fit")):
+                setattr(self, p, fit0[0, side].copy() if valid0[0, side] else None)
 
-        try:
-            nxt = next(it, None)
-            while nxt is not None or queue:
-                if not queue:                        # (re)start the pipeline with the detector's current state
-                    cur = nxt
-                    nxt = next(it, None)
-                    self._check_frames(cur, batched=True)
-                    if _is_torch_cuda(cur) and cur.shape[0] > 0:
-                        ctx = self._context(int(cur.shape[1]), int(cur.shape[2]), int(cur.shape[0]), cur)
-                    if not streamable(cur):
-                        yield self.detect_batch(cur)
-                        continue
-                    fit, valid = self._state_arrays()
-                    enqueue(cur, explicit=True)
-                if nxt is not None and len(queue) < 2:
-                    self._check_frames(nxt, batched=True)
-                    if streamable(nxt):
-                        enqueue(nxt, explicit=False)
-                        nxt = next(it, None)
-                head = queue[0][0]
-                state_before = (fit.copy(), valid.copy())
-                recs = ctx.collect(fit, valid)       # fit / valid now hold the state after `head`
-                queue.pop(0)
-                if recs["flags"].any():
-                    # truncated segment lists: the batches behind it started from a wrong state; drain, redo this batch
-                    # the blocking way (dense context) from the state it started with, and restart the pipeline
-                    requeue = [q[0] for q in queue]
-                    drain()
-                    for side, p in enumerate(("prev_left_fit", "prev_right_fit")):
-                        setattr(self, p, state_before[0][0, side].copy() if state_before[1][0, side] else None)
-                    lanes = self.detect_batch(head)
-                    yield lanes
-                    fit, valid = self._state_arrays()
-                    for k, fr in enumerate(requeue):
-                        enqueue(fr, explicit=(k == 0))
-                    continue
-                self.last_records = recs
-                lanes = self._lanes_from_records(recs)
-                self._adopt_state(lanes)
-                yield lanes
-        finally:
-            drain()
+        def adopt(recs, _):
+            self.last_records = recs
+            lanes = self._lanes_from_records(recs)
+            self._adopt_state(lanes)
+            return lanes
+
+        yield from _two_deep(batches, plan, start, joins, enqueue, lambda fr, _: self.detect_batch(fr), restore, adopt)
 
     def _adopt_state(self, lanes: List[LanePair]):
         """Like the reference (:210-216), prev_*_fit aliases the last returned polynomial of that side."""
@@ -526,7 +558,7 @@ class LaneDetector:
                 lo, hi = max(a, base[s]), min(b, base[s + 1])
                 if lo < hi:
                     i, j = lo - base[s], hi - base[s]
-                    src = data[s].data_ptr() + i * p.frame_bytes(s) if on_device else data[s][i:j]
+                    src = data[s].data_ptr() + i * _frame_bytes(p.fmts[s], *p.sizes[s]) if on_device else data[s][i:j]
                     sources.append((src, p.fmts[s], p.sizes[s], j - i, s))
             return c.detect_rig(sources, on_device, fit.shape[0], fit, valid, sm, oms)
 
@@ -553,31 +585,25 @@ class LaneDetector:
         ``detect_rig``'s, raised when the tick's turn comes.
         """
         import torch
-        end = object()
-        it = iter(ticks)
-        pending = []                  # ticks taken from `ticks` and not enqueued yet, oldest first
-        queue = []                    # ticks in flight, oldest first: (tick, plan, sources kept alive, pinned buffer)
         pinned = [None, None]         # pinned host copies of numpy ticks, one per tick in flight
-        copier = [None]               # the host threads of those copies, made by the first tick that needs them
+        last_buf = 1                  # the pinned buffer of the tick enqueued last
+        copier = None                 # the host threads of those copies, made by the first tick that needs them
         ctx, S = None, 0
         fit = valid = None            # state after the tick collected last
-
-        def take():
-            return pending.pop(0) if pending else next(it, end)
 
         def plan(tick):
             return self._rig_plan(tick, layouts, target_size, stream_rois, pinned=True)
 
-        def start(p) -> bool:
-            """Take the detector's state and tick p's context: whether p can be the first tick in flight."""
+        def start(p):
+            """Take the detector's state and tick p's context, unless p cannot be the first tick in flight."""
             nonlocal ctx, S, fit, valid
             if not p.n:
-                return False
+                return None
             self._grow_stream_state(len(p.cams))
             S = self._stream_fit.shape[0]
             ctx = self._context(p.h, p.w, self._max_batch, p.cams[p.live[0]], p.stream_rois, p.n_masks(S))
             fit, valid = self._stream_fit.copy(), self._stream_valid.copy()
-            return p.n <= ctx.max_batch
+            return (ctx, fit, valid) if p.n <= ctx.max_batch else None
 
         def joins(p) -> bool:
             """Whether tick p can queue behind the tick in flight: same context and streams, and it fits."""
@@ -590,7 +616,9 @@ class LaneDetector:
             return self._ctx_key == (p.h, p.w, self._roi_key(p.stream_rois, p.n_masks(S)), dev)
 
         def enqueue(tick, p, explicit: bool):
-            k = 1 - queue[0][3] if queue else 0      # the pinned buffer the tick in flight does not use
+            nonlocal last_buf, copier
+            # a tick that joins queues behind the tick enqueued last: it takes the pinned buffer that one does not use
+            k = last_buf = 0 if explicit else 1 - last_buf
             if p.kind == "host":
                 need = sum(p.cams[s].nbytes for s in p.live)
                 if pinned[k] is None or pinned[k].numel() < need:
@@ -602,10 +630,10 @@ class LaneDetector:
                     cuts = list(range(0, cam.nbytes, _COPY_PIECE)) + [cam.nbytes]
                     pieces += [(flat[off + a:off + b], cam[a:b]) for a, b in zip(cuts, cuts[1:])]
                     off += cam.nbytes
-                if len(pieces) > 1 and copier[0] is None:
-                    copier[0] = ThreadPoolExecutor(max(1, min(8, (os.cpu_count() or 2) // 2)))
+                if len(pieces) > 1 and copier is None:
+                    copier = ThreadPoolExecutor(max(1, min(8, (os.cpu_count() or 2) // 2)))
                 # one host thread copies ~10 GB/s: a tick of an 8-camera rig (35 MB) would take longer than its compute
-                list(copier[0].map(lambda ds: np.copyto(*ds), pieces) if len(pieces) > 1 else
+                list(copier.map(lambda ds: np.copyto(*ds), pieces) if len(pieces) > 1 else
                      (np.copyto(*ds) for ds in pieces))
             elif p.kind == "pinned":
                 src = {s: p.cams[s].numpy() for s in p.live}
@@ -618,55 +646,26 @@ class LaneDetector:
             sources = [(src[s][1] if on_device else src[s], p.fmts[s], p.sizes[s], p.counts[s], s) for s in p.live]
             ctx.enqueue_rig(sources, on_device, S, fit if explicit else None, valid if explicit else None,
                             self.smoothing_factor, 1 - self.smoothing_factor)
-            queue.append((tick, p, src, k))
+            return src
 
         def blocking(tick, p):
             if p.kind == "pinned":                   # detect_rig takes host cameras as numpy arrays
                 tick = [None if c is None else c.numpy() for c in p.cams]
             return self.detect_rig(tick, layouts, target_size=target_size, stream_rois=stream_rois)
 
-        def drain():
-            while ctx is not None and ctx._inflight:
-                ctx.collect(np.zeros((S, 2, 3)), np.zeros((S, 2), np.uint8))
-            queue.clear()
+        def restore(fit0, valid0):
+            self._stream_fit, self._stream_valid = fit0, valid0
+
+        def adopt(recs, p):
+            self._stream_fit, self._stream_valid = fit.copy(), valid.copy()
+            self.last_records = recs
+            return p.per_camera(self._lanes_from_records(recs))
 
         try:
-            nxt = take()
-            while nxt is not end or queue:
-                if not queue:                        # (re)start the pipeline with the detector's current state
-                    cur, nxt = nxt, take()
-                    p = plan(cur)                    # detect_rig's argument errors, in tick order
-                    if not start(p):
-                        yield blocking(cur, p)
-                        continue
-                    enqueue(cur, p, explicit=True)
-                if nxt is not end and len(queue) < 2:
-                    try:
-                        p = plan(nxt)
-                    except (ValueError, cv2.error):
-                        p = None                     # raised once the ticks before it are out
-                    if p is not None and joins(p):
-                        enqueue(nxt, p, explicit=False)
-                        nxt = take()
-                before = (fit.copy(), valid.copy())
-                recs = ctx.collect(fit, valid)       # fit / valid now hold the state after the oldest tick
-                head = queue.pop(0)
-                if recs["flags"].any():
-                    # truncated segment lists: the ticks behind it started from a wrong state; drain, redo this tick
-                    # the blocking way (dense context) from the state it started with, and restart with the rest
-                    pending[:0] = [q[0] for q in queue] + ([] if nxt is end else [nxt])
-                    drain()
-                    self._stream_fit, self._stream_valid = before
-                    yield blocking(head[0], head[1])
-                    nxt = take()
-                    continue
-                self._stream_fit, self._stream_valid = fit.copy(), valid.copy()
-                self.last_records = recs
-                yield head[1].per_camera(self._lanes_from_records(recs))
+            yield from _two_deep(ticks, plan, start, joins, enqueue, blocking, restore, adopt)
         finally:
-            drain()
-            if copier[0] is not None:
-                copier[0].shutdown()
+            if copier is not None:
+                copier.shutdown()
 
     def _rig_plan(self, frames, layouts, target_size, stream_rois, pinned: bool = False) -> "_RigTick":
         """``detect_rig``'s argument checks on one tick, and what they found.  ``pinned``: page-locked contiguous CPU

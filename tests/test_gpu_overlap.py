@@ -98,3 +98,27 @@ def test_detect_batches_generator_equals_detect_batch_batch_after_batch():
     det.detect_batch(batches[0])
     det.close()
     ref_det.close()
+
+
+def test_detect_batches_yields_the_batches_before_a_malformed_one_then_raises():
+    """A malformed batch raises detect_batch's error when its turn comes: the batches before it are yielded first, and
+    nothing is left in flight."""
+    import cv2
+    batches = _batches(640, 480, 8, 2)
+    ref = LaneDetector(max_batch=8)
+    want = [ref.detect_batch(b) for b in batches]
+    det = LaneDetector(max_batch=8)
+    got = []
+    with pytest.raises(cv2.error):
+        for lanes in det.detect_batches(batches + [batches[0][..., :2], batches[0]]):
+            got.append(lanes)
+    assert len(got) == len(want)
+    for a, b in zip(got, want):
+        for pa, pb in zip(a, b):
+            for x, y in zip(pa, pb):
+                assert (x is None) == (y is None)
+                assert x is None or (np.array_equal(x.points, y.points) and np.array_equal(x.polynomial, y.polynomial))
+    assert np.array_equal(det.prev_left_fit, ref.prev_left_fit) and np.array_equal(det.prev_right_fit, ref.prev_right_fit)
+    assert not det._ctx._inflight
+    det.close()
+    ref.close()
