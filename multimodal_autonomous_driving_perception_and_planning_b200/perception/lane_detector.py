@@ -113,10 +113,14 @@ def _two_deep(items, plan, start, joins, enqueue, blocking, restore, adopt):
 
 
 @dataclass
-class _RigTick:
-    """One tick of a rig as ``detect_rig``'s checks found it: camera s has ``counts[s]`` frames in layout ``fmts[s]``
-    (INPUT_*) at ``sizes[s]`` = (h, w); every camera with frames is of one ``kind`` (``("cuda", index)``, ``"host"`` for
-    numpy, ``"pinned"``; None when the tick has no frame), detected at ``h`` x ``w``."""
+class _Plan:
+    """One detect call's batch as its argument checks found it: source s has ``counts[s]`` frames ``cams[s]`` in layout
+    ``fmts[s]`` (INPUT_*) at ``sizes[s]`` = (h, w); every source with frames is of one ``kind`` (``("cuda", index)``,
+    ``"host"`` for numpy, ``"pinned"``; None when the batch has no frame), detected at ``h`` x ``w``.
+
+    ``rig``: the batch takes the rig entries (``lane_detect_rig`` / ``lane_rig_enqueue``), source s being stream s.
+    Otherwise it is one source through ``lane_detect_batch_ingest`` / ``lane_detect_enqueue``, which read BGR frames at
+    the detection size in place, with per-frame stream ids ``frame_sids`` (None: every frame is stream 0)."""
     cams: list
     fmts: list
     sizes: list
@@ -125,19 +129,48 @@ class _RigTick:
     h: Optional[int]
     w: Optional[int]
     stream_rois: Optional[list]
+    rig: bool = True
+    frame_sids: Optional[np.ndarray] = None
 
     def __post_init__(self):
-        self.base = [0]                              # camera s's frames are [base[s], base[s+1]) of the concatenation
+        self.base = [0]                              # source s's frames are [base[s], base[s+1]) of the concatenation
         for t in self.counts:
             self.base.append(self.base[-1] + t)
         self.n = self.base[-1]
         self.live = [s for s, t in enumerate(self.counts) if t]
+        if self.rig:
+            self.n_streams = len(self.cams)
+        else:
+            self.n_streams = 1 if self.frame_sids is None or not self.n else int(self.frame_sids.max()) + 1
+
+    @classmethod
+    def of_frames(cls, frames, fmt: int, target_size=None, frame_sids=None, stream_rois=None) -> "_Plan":
+        """One checked array of frames: [N,H,W,3] BGR, or [N,H*3/2,W] for the YUV 4:2:0 layouts of ``fmt``, detected at
+        ``target_size`` = (width, height) when given."""
+        n, sh, sw = (int(x) for x in frames.shape[:3])
+        if fmt != _native.INPUT_BGR:
+            sh = sh * 2 // 3
+        h, w = (sh, sw) if target_size is None else (target_size[1], target_size[0])
+        kind = ("cuda", frames.device.index) if _is_torch_cuda(frames) else "host"
+        return cls([frames], [fmt], [(sh, sw)], [n], kind, h, w, stream_rois, rig=False, frame_sids=frame_sids)
 
     def n_masks(self, n_streams: int) -> int:
         return 1 if self.stream_rois is None else max(len(self.stream_rois), n_streams)
 
     def per_camera(self, items):
         return [items[self.base[s]:self.base[s + 1]] for s in range(len(self.cams))]
+
+    def sources(self, data, a: int, b: int, on_device: bool) -> list:
+        """``(frames, fmt, (h, w), n, stream id)`` of every source's share of frames [a, b): a device pointer into
+        ``data[s]`` (on_device) or a view of it."""
+        out = []
+        for s in self.live:
+            lo, hi = max(a, self.base[s]), min(b, self.base[s + 1])
+            if lo < hi:
+                i, j = lo - self.base[s], hi - self.base[s]
+                src = data[s].data_ptr() + i * _frame_bytes(self.fmts[s], *self.sizes[s]) if on_device else data[s][i:j]
+                out.append((src, self.fmts[s], self.sizes[s], j - i, s))
+        return out
 
 
 class LaneDetector:
@@ -279,40 +312,33 @@ class LaneDetector:
             out.append((left, right))
         return out
 
-    def _run(self, frames, stream_id, n_streams, prev_fit, prev_valid, fmt: int = _native.INPUT_BGR,
-             target_size: Optional[Tuple[int, int]] = None, stream_rois=None) -> np.ndarray:
-        """Chunked native calls over frames [N,H,W,3] (numpy or CUDA torch; [N,H*3/2,W] for the YUV 4:2:0 layouts of
-        ``fmt``), detected at ``target_size`` = (width, height) when given (the device resizes every frame to it first);
-        state arrays updated in place.  ``stream_rois``: one ROI per stream (see ``detect_streams``)."""
-        n, sh, sw = int(frames.shape[0]), int(frames.shape[1]), int(frames.shape[2])
-        if fmt != _native.INPUT_BGR:
-            sh = sh * 2 // 3
-        fbytes = _frame_bytes(fmt, sh, sw)
-        h, w = (sh, sw) if target_size is None else (target_size[1], target_size[0])
-        n_masks = 1 if stream_rois is None else max(len(stream_rois), n_streams)
-        ctx = self._context(h, w, n, frames, stream_rois, n_masks)
-        s, oms = self.smoothing_factor, 1 - self.smoothing_factor
-        on_device = _is_torch_cuda(frames)
+    def _run(self, p: _Plan, prev_fit: np.ndarray, prev_valid: np.ndarray) -> np.ndarray:
+        """Plan ``p`` through its blocking entry in chunks of the context's max_batch, from the state ``prev_fit`` /
+        ``prev_valid`` (one row per stream, updated in place); each chunk is re-run on the dense context when its segment
+        lists overflow."""
+        on_device = p.kind not in ("host", "pinned")
         if on_device:
             import torch
-            frames = frames.contiguous()
-            torch.cuda.current_stream(frames.device).synchronize()
+            data = {s: p.cams[s].contiguous() for s in p.live}
+            torch.cuda.current_stream(data[p.live[0]].device).synchronize()
         else:
-            frames = np.ascontiguousarray(frames)
+            data = {s: np.ascontiguousarray(p.cams[s]) for s in p.live}
+        n_streams = prev_fit.shape[0]
+        n_masks = p.n_masks(n_streams)
+        ctx = self._context(p.h, p.w, p.n, data[p.live[0]], p.stream_rois, n_masks)
+        sm, oms = self.smoothing_factor, 1 - self.smoothing_factor
 
         def call(c, a, b):
-            sid = None if stream_id is None else stream_id[a:b]
-            src = frames.data_ptr() + a * fbytes if on_device else frames[a:b]
-            return c.detect(src, b - a, on_device, sid, n_streams, prev_fit, prev_valid, s, oms, fmt=fmt, src_hw=(sh, sw))
+            sources = p.sources(data, a, b, on_device)
+            if p.rig:
+                return c.detect_rig(sources, on_device, n_streams, prev_fit, prev_valid, sm, oms)
+            (src, fmt, hw, k, _), = sources
+            sid = None if p.frame_sids is None else p.frame_sids[a:b]
+            return c.detect(src, k, on_device, sid, n_streams, prev_fit, prev_valid, sm, oms, fmt=fmt, src_hw=hw)
 
-        return self._chunked(ctx, n, call, h, w, prev_fit, prev_valid, stream_rois, n_masks)
-
-    def _chunked(self, ctx, n, call, h, w, prev_fit, prev_valid, stream_rois, n_masks) -> np.ndarray:
-        """``call(context, a, b)`` -> records of frames [a, b), over frames [0, n) in chunks of the context's max_batch,
-        each chunk re-run on the dense context when its segment lists overflow."""
         chunks = []
-        for a in range(0, n, ctx.max_batch):
-            b = min(a + ctx.max_batch, n)
+        for a in range(0, p.n, ctx.max_batch):
+            b = min(a + ctx.max_batch, p.n)
             fit0, valid0 = prev_fit.copy(), prev_valid.copy()
             recs = call(ctx, a, b)
             if recs["flags"].any():
@@ -320,7 +346,8 @@ class LaneDetector:
                 # otherwise be fitted on a truncated list.  Re-run the chunk, from the state it started with, on a context
                 # sized for what was found (the reference result, just slower), never return a truncated fit silently.
                 prev_fit[...], prev_valid[...] = fit0, valid0
-                dense = self._dense_context(h, w, int(recs["n_segments_found"].max()), ctx.device, stream_rois, n_masks)
+                dense = self._dense_context(p.h, p.w, int(recs["n_segments_found"].max()), ctx.device, p.stream_rois,
+                                            n_masks)
                 recs = np.concatenate([call(dense, i, min(i + dense.max_batch, b)) for i in range(a, b, dense.max_batch)])
                 if recs["flags"].any():
                     raise _native.LaneError(-5, "segment list still truncated after the dense re-run")
@@ -370,13 +397,16 @@ class LaneDetector:
         ``np.stack([cv2.resize(f, target_size) for f in frames])`` (``roi_vertices`` are in target coordinates).
         """
         self._check_frames(frames, batched=True)
+        return self._detect_frames(frames, _native.INPUT_BGR, target_size)
+
+    def _detect_frames(self, frames, fmt: int, target_size) -> List[LanePair]:
+        """``detect_batch`` and its decoder-layout forms, on frames checked for layout ``fmt`` (INPUT_*)."""
         if target_size is not None:
             target_size = check_target_size(target_size)
         if frames.shape[0] == 0:
             return []
         fit, valid = self._state_arrays()
-        recs = self._run(frames, None, 1, fit, valid, target_size=target_size)
-        lanes = self._lanes_from_records(recs)
+        lanes = self._lanes_from_records(self._run(_Plan.of_frames(frames, fmt, target_size), fit, valid))
         self._adopt_state(lanes)
         return lanes
 
@@ -391,46 +421,78 @@ class LaneDetector:
         segment lists overflow is re-run on the dense context like there (the queue is drained and restarted around it).
         Batches that are not CUDA tensors of one common shape on one device simply go through ``detect_batch``.  A
         malformed batch raises ``detect_batch``'s error when its turn comes, after the batches before it are yielded."""
-        import torch
-        ctx = fit = valid = None
-        s, oms = self.smoothing_factor, 1 - self.smoothing_factor
-
         def plan(fr):
             self._check_frames(fr, batched=True)
-            return fr
-
-        def joins(fr) -> bool:
-            return (_is_torch_cuda(fr) and len(fr.shape) == 4 and fr.shape[0] > 0 and ctx is not None and
-                    fr.shape[0] <= ctx.max_batch and (int(fr.shape[1]), int(fr.shape[2])) == (ctx.height, ctx.width) and
-                    fr.device.index == ctx.device)
-
-        def start(fr):
-            nonlocal ctx, fit, valid
-            if _is_torch_cuda(fr) and fr.shape[0] > 0:
-                ctx = self._context(int(fr.shape[1]), int(fr.shape[2]), int(fr.shape[0]), fr)
-            if not joins(fr):
-                return None
-            fit, valid = self._state_arrays()
-            return ctx, fit, valid
-
-        def enqueue(fr, _, explicit: bool):
-            fr = fr.contiguous()
-            torch.cuda.ExternalStream(ctx.stream(), device=fr.device).wait_stream(torch.cuda.current_stream(fr.device))
-            ctx.enqueue(fr.data_ptr(), int(fr.shape[0]), None, 1, fit if explicit else None, valid if explicit else None,
-                        s, oms)
-            return fr
+            return _Plan.of_frames(fr, _native.INPUT_BGR)
 
         def restore(fit0, valid0):
             for side, p in enumerate(("prev_left_fit", "prev_right_fit")):
                 setattr(self, p, fit0[0, side].copy() if valid0[0, side] else None)
 
-        def adopt(recs, _):
-            self.last_records = recs
-            lanes = self._lanes_from_records(recs)
+        def adopt(lanes, p, fit, valid):
             self._adopt_state(lanes)
             return lanes
 
-        yield from _two_deep(batches, plan, start, joins, enqueue, lambda fr, _: self.detect_batch(fr), restore, adopt)
+        yield from self._stream(batches, plan, lambda p: self._state_arrays(), lambda fr, p: self.detect_batch(fr),
+                                restore, adopt)
+
+    def _stream(self, items, plan, state, blocking, restore, adopt, cap: Optional[int] = None, stage=None):
+        """``_two_deep`` over plans, the queue of ``detect_batches`` and ``detect_rig_stream``.  ``plan(item)`` checks an
+        item and returns its ``_Plan``; ``state(p)`` returns ``(fit, valid)``, the detector's state for a first item in
+        flight as arrays ``collect`` may fill; ``blocking`` and ``restore`` are ``_two_deep``'s; ``adopt(lanes, p, fit,
+        valid)`` makes the state after an item (its pairs ``lanes``) the detector's and returns the item's result.  The
+        context is sized for ``cap`` frames (None: the first item's).  CUDA frames are read in place once the work on the
+        caller's stream is done, pinned ones in place, and host (numpy) frames only through ``stage(p, explicit)``, which
+        copies them into page-locked memory and returns them per source; without it host items run blocking."""
+        import torch
+        ctx = fit = valid = None
+
+        def streams(p) -> bool:
+            return bool(p.n) and (p.kind != "host" or stage is not None)
+
+        def start(p):
+            nonlocal ctx, fit, valid
+            if not streams(p):
+                return None
+            fit, valid = state(p)
+            ctx = self._context(p.h, p.w, cap or p.n, p.cams[p.live[0]], p.stream_rois, p.n_masks(len(fit)))
+            return (ctx, fit, valid) if joins(p) else None
+
+        def joins(p) -> bool:
+            """Whether p can queue behind the item in flight: same context and streams, and it fits."""
+            if not streams(p) or p.n_streams > len(fit) or p.n > ctx.max_batch or self._ctx is not ctx:
+                return False
+            try:
+                dev = self._device_index(p.cams[p.live[0]])
+            except ValueError:
+                return False
+            return self._ctx_key == (p.h, p.w, self._roi_key(p.stream_rois, p.n_masks(len(fit))), dev)
+
+        def enqueue(item, p, explicit: bool):
+            on_device = p.kind not in ("host", "pinned")
+            if p.kind == "host":
+                data = stage(p, explicit)
+            elif p.kind == "pinned":
+                data = {s: p.cams[s].numpy() for s in p.live}
+            else:
+                data = {s: p.cams[s].contiguous() for s in p.live}
+                dev = data[p.live[0]].device
+                torch.cuda.ExternalStream(ctx.stream(), device=dev).wait_stream(torch.cuda.current_stream(dev))
+            sources = p.sources(data, 0, p.n, on_device)
+            fit0, valid0 = (fit, valid) if explicit else (None, None)
+            sm, oms = self.smoothing_factor, 1 - self.smoothing_factor
+            if p.rig:
+                ctx.enqueue_rig(sources, on_device, len(fit), fit0, valid0, sm, oms)
+            else:
+                (src, _, _, k, _), = sources
+                ctx.enqueue(src, k, p.frame_sids, len(fit), fit0, valid0, sm, oms)
+            return data
+
+        def adopt_records(recs, p):
+            self.last_records = recs
+            return adopt(self._lanes_from_records(recs), p, fit, valid)
+
+        yield from _two_deep(items, plan, start, joins, enqueue, blocking, restore, adopt_records)
 
     def _adopt_state(self, lanes: List[LanePair]):
         """Like the reference (:210-216), prev_*_fit aliases the last returned polynomial of that side."""
@@ -452,25 +514,15 @@ class LaneDetector:
         ``target_size`` = (width, height): the decoder's frames at camera resolution are detected at that size, equal to
         ``detect_batch`` of ``cv2.resize(cv2.cvtColor(f, COLOR_YUV2BGR_NV12), target_size)`` (``VideoDataLoader`` with
         ``target_size``); conversion and resize are one kernel and only the NV12 bytes cross PCIe."""
-        return self._detect_yuv420(frames, _native.INPUT_NV12, target_size)
+        check_yuv420(frames, "LaneDetector")
+        return self._detect_frames(frames, _native.INPUT_NV12, target_size)
 
     def detect_batch_i420(self, frames, *, target_size: Optional[Tuple[int, int]] = None) -> List[LanePair]:
         """``detect_batch_nv12`` for the planar layout software decoders hand out (FFmpeg / PyAV ``yuv420p``): uint8
         ``[N, H*3/2, W]`` = Y plane, U plane, V plane; equal to ``detect_batch`` on
         ``cv2.cvtColor(f, cv2.COLOR_YUV2BGR_I420)`` of every frame, resized to ``target_size`` when given."""
-        return self._detect_yuv420(frames, _native.INPUT_I420, target_size)
-
-    def _detect_yuv420(self, frames, fmt: int, target_size) -> List[LanePair]:
         check_yuv420(frames, "LaneDetector")
-        if target_size is not None:
-            target_size = check_target_size(target_size)
-        if frames.shape[0] == 0:
-            return []
-        fit, valid = self._state_arrays()
-        recs = self._run(frames, None, 1, fit, valid, fmt=fmt, target_size=target_size)
-        lanes = self._lanes_from_records(recs)
-        self._adopt_state(lanes)
-        return lanes
+        return self._detect_frames(frames, _native.INPUT_I420, target_size)
 
     def detect_streams(self, frames, stream_ids: Optional[Sequence[int]] = None, *,
                        stream_rois: Optional[Sequence[Optional[np.ndarray]]] = None) -> List[LanePair]:
@@ -497,15 +549,13 @@ class LaneDetector:
             raise ValueError("stream_ids must be non-negative int32[N]")
         if frames.shape[0] == 0:
             return []
-        n_streams = int(stream_ids.max()) + 1
-        if stream_rois is not None:
-            stream_rois = list(stream_rois)
-            if len(stream_rois) < n_streams:
-                raise ValueError(f"stream_rois has {len(stream_rois)} entries; stream id {n_streams - 1} needs {n_streams}")
-        self._grow_stream_state(n_streams)
-        recs = self._run(frames, stream_ids, self._stream_fit.shape[0], self._stream_fit, self._stream_valid,
-                         stream_rois=stream_rois)
-        return self._lanes_from_records(recs)
+        p = _Plan.of_frames(frames, _native.INPUT_BGR, frame_sids=stream_ids,
+                            stream_rois=None if stream_rois is None else list(stream_rois))
+        if p.stream_rois is not None and len(p.stream_rois) < p.n_streams:
+            raise ValueError(f"stream_rois has {len(p.stream_rois)} entries; stream id {p.n_streams - 1} needs "
+                             f"{p.n_streams}")
+        self._grow_stream_state(p.n_streams)
+        return self._lanes_from_records(self._run(p, self._stream_fit, self._stream_valid))
 
     def _grow_stream_state(self, n_streams: int):
         """Per-stream smoothing state of ``detect_streams`` / ``detect_rig`` for at least ``n_streams`` streams."""
@@ -535,35 +585,13 @@ class LaneDetector:
         ``detect_batch_i420(frames[s], target_size=target_size)``; its smoothing state is stream s's of ``detect_streams``,
         so it carries across calls of either kind (``reset`` clears it).
         """
-        p = self._rig_plan(frames, layouts, target_size, stream_rois)
+        return self._detect_rig(self._rig_plan(frames, layouts, target_size, stream_rois))
+
+    def _detect_rig(self, p: _Plan) -> List[List[LanePair]]:
         if not p.n:
             return [[] for _ in p.cams]
-        on_device = p.kind != "host"
-        if on_device:
-            import torch
-            data = {s: p.cams[s].contiguous() for s in p.live}
-            torch.cuda.current_stream(data[p.live[0]].device).synchronize()
-        else:
-            data = {s: np.ascontiguousarray(p.cams[s]) for s in p.live}
-        self._grow_stream_state(len(p.cams))
-        fit, valid = self._stream_fit, self._stream_valid
-        n_masks = p.n_masks(fit.shape[0])
-        ctx = self._context(p.h, p.w, p.n, data[p.live[0]], p.stream_rois, n_masks)
-        sm, oms = self.smoothing_factor, 1 - self.smoothing_factor
-        base = p.base
-
-        def call(c, a, b):
-            sources = []
-            for s in p.live:
-                lo, hi = max(a, base[s]), min(b, base[s + 1])
-                if lo < hi:
-                    i, j = lo - base[s], hi - base[s]
-                    src = data[s].data_ptr() + i * _frame_bytes(p.fmts[s], *p.sizes[s]) if on_device else data[s][i:j]
-                    sources.append((src, p.fmts[s], p.sizes[s], j - i, s))
-            return c.detect_rig(sources, on_device, fit.shape[0], fit, valid, sm, oms)
-
-        recs = self._chunked(ctx, p.n, call, p.h, p.w, fit, valid, p.stream_rois, n_masks)
-        return p.per_camera(self._lanes_from_records(recs))
+        self._grow_stream_state(p.n_streams)
+        return p.per_camera(self._lanes_from_records(self._run(p, self._stream_fit, self._stream_valid)))
 
     def detect_rig_stream(self, ticks, layouts: Optional[Sequence[str]] = None, *,
                           target_size: Optional[Tuple[int, int]] = None,
@@ -586,88 +614,51 @@ class LaneDetector:
         """
         import torch
         pinned = [None, None]         # pinned host copies of numpy ticks, one per tick in flight
-        last_buf = 1                  # the pinned buffer of the tick enqueued last
+        last_buf = 1                  # the pinned buffer of the numpy tick enqueued last
         copier = None                 # the host threads of those copies, made by the first tick that needs them
-        ctx, S = None, 0
-        fit = valid = None            # state after the tick collected last
 
-        def plan(tick):
-            return self._rig_plan(tick, layouts, target_size, stream_rois, pinned=True)
-
-        def start(p):
-            """Take the detector's state and tick p's context, unless p cannot be the first tick in flight."""
-            nonlocal ctx, S, fit, valid
-            if not p.n:
-                return None
-            self._grow_stream_state(len(p.cams))
-            S = self._stream_fit.shape[0]
-            ctx = self._context(p.h, p.w, self._max_batch, p.cams[p.live[0]], p.stream_rois, p.n_masks(S))
-            fit, valid = self._stream_fit.copy(), self._stream_valid.copy()
-            return (ctx, fit, valid) if p.n <= ctx.max_batch else None
-
-        def joins(p) -> bool:
-            """Whether tick p can queue behind the tick in flight: same context and streams, and it fits."""
-            if not p.n or len(p.cams) > S or p.n > ctx.max_batch or self._ctx is not ctx:
-                return False
-            try:
-                dev = self._device_index(p.cams[p.live[0]])
-            except ValueError:
-                return False
-            return self._ctx_key == (p.h, p.w, self._roi_key(p.stream_rois, p.n_masks(S)), dev)
-
-        def enqueue(tick, p, explicit: bool):
+        def stage(p, explicit: bool):
             nonlocal last_buf, copier
-            # a tick that joins queues behind the tick enqueued last: it takes the pinned buffer that one does not use
+            # a tick that joins takes the pinned buffer the numpy tick enqueued last does not use (only that one can still
+            # be in flight)
             k = last_buf = 0 if explicit else 1 - last_buf
-            if p.kind == "host":
-                need = sum(p.cams[s].nbytes for s in p.live)
-                if pinned[k] is None or pinned[k].numel() < need:
-                    pinned[k] = torch.empty(need, dtype=torch.uint8, pin_memory=True)
-                flat, off, src, pieces = pinned[k].numpy(), 0, {}, []
-                for s in p.live:
-                    cam = np.ascontiguousarray(p.cams[s]).reshape(-1)
-                    src[s] = flat[off:off + cam.nbytes].reshape(p.cams[s].shape)
-                    cuts = list(range(0, cam.nbytes, _COPY_PIECE)) + [cam.nbytes]
-                    pieces += [(flat[off + a:off + b], cam[a:b]) for a, b in zip(cuts, cuts[1:])]
-                    off += cam.nbytes
-                if len(pieces) > 1 and copier is None:
-                    copier = ThreadPoolExecutor(max(1, min(8, (os.cpu_count() or 2) // 2)))
-                # one host thread copies ~10 GB/s: a tick of an 8-camera rig (35 MB) would take longer than its compute
-                list(copier.map(lambda ds: np.copyto(*ds), pieces) if len(pieces) > 1 else
-                     (np.copyto(*ds) for ds in pieces))
-            elif p.kind == "pinned":
-                src = {s: p.cams[s].numpy() for s in p.live}
-            else:
-                data = {s: p.cams[s].contiguous() for s in p.live}
-                dev = data[p.live[0]].device
-                torch.cuda.ExternalStream(ctx.stream(), device=dev).wait_stream(torch.cuda.current_stream(dev))
-                src = {s: (data[s], data[s].data_ptr()) for s in p.live}
-            on_device = p.kind not in ("host", "pinned")
-            sources = [(src[s][1] if on_device else src[s], p.fmts[s], p.sizes[s], p.counts[s], s) for s in p.live]
-            ctx.enqueue_rig(sources, on_device, S, fit if explicit else None, valid if explicit else None,
-                            self.smoothing_factor, 1 - self.smoothing_factor)
+            need = sum(p.cams[s].nbytes for s in p.live)
+            if pinned[k] is None or pinned[k].numel() < need:
+                pinned[k] = torch.empty(need, dtype=torch.uint8, pin_memory=True)
+            flat, off, src, pieces = pinned[k].numpy(), 0, {}, []
+            for s in p.live:
+                cam = np.ascontiguousarray(p.cams[s]).reshape(-1)
+                src[s] = flat[off:off + cam.nbytes].reshape(p.cams[s].shape)
+                cuts = list(range(0, cam.nbytes, _COPY_PIECE)) + [cam.nbytes]
+                pieces += [(flat[off + a:off + b], cam[a:b]) for a, b in zip(cuts, cuts[1:])]
+                off += cam.nbytes
+            if len(pieces) > 1 and copier is None:
+                copier = ThreadPoolExecutor(max(1, min(8, (os.cpu_count() or 2) // 2)))
+            # one host thread copies ~10 GB/s: a tick of an 8-camera rig (35 MB) would take longer than its compute
+            list(copier.map(lambda ds: np.copyto(*ds), pieces) if len(pieces) > 1 else
+                 (np.copyto(*ds) for ds in pieces))
             return src
 
-        def blocking(tick, p):
-            if p.kind == "pinned":                   # detect_rig takes host cameras as numpy arrays
-                tick = [None if c is None else c.numpy() for c in p.cams]
-            return self.detect_rig(tick, layouts, target_size=target_size, stream_rois=stream_rois)
+        def state(p):
+            self._grow_stream_state(p.n_streams)
+            return self._stream_fit.copy(), self._stream_valid.copy()
 
         def restore(fit0, valid0):
             self._stream_fit, self._stream_valid = fit0, valid0
 
-        def adopt(recs, p):
+        def adopt(lanes, p, fit, valid):
             self._stream_fit, self._stream_valid = fit.copy(), valid.copy()
-            self.last_records = recs
-            return p.per_camera(self._lanes_from_records(recs))
+            return p.per_camera(lanes)
 
         try:
-            yield from _two_deep(ticks, plan, start, joins, enqueue, blocking, restore, adopt)
+            yield from self._stream(ticks, lambda t: self._rig_plan(t, layouts, target_size, stream_rois, pinned=True),
+                                    state, lambda t, p: self._detect_rig(p), restore, adopt, cap=self._max_batch,
+                                    stage=stage)
         finally:
             if copier is not None:
                 copier.shutdown()
 
-    def _rig_plan(self, frames, layouts, target_size, stream_rois, pinned: bool = False) -> "_RigTick":
+    def _rig_plan(self, frames, layouts, target_size, stream_rois, pinned: bool = False) -> _Plan:
         """``detect_rig``'s argument checks on one tick, and what they found.  ``pinned``: page-locked contiguous CPU
         torch tensors are a kind of their own (``detect_rig_stream`` reads them in place)."""
         cams = list(frames)
@@ -700,7 +691,7 @@ class LaneDetector:
         if target_size is None and len(used) > 1:
             raise ValueError(f"cameras of sizes {sorted(used)} need a target_size")
         hw = (None, None) if not used else next(iter(used)) if target_size is None else (target_size[1], target_size[0])
-        return _RigTick(cams, fmts, sizes, counts, next(iter(kinds)) if used else None, *hw, stream_rois)
+        return _Plan(cams, fmts, sizes, counts, next(iter(kinds)) if used else None, *hw, stream_rois)
 
     @staticmethod
     def _rig_frame_size(f, layout: str, s: int) -> Tuple[int, int]:
