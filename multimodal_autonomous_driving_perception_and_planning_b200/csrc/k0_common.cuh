@@ -1,5 +1,6 @@
 // Shared pieces of the frame-ingest kernels (K0): the YUV 4:2:0 -> BGR arithmetic of k0_nv12.cu / k0_ingest.cu, its
-// inverse for the egress kernel (k8_egress.cu) and the INTER_LINEAR tap tables and vertical step of k0_resize.cu.
+// inverse for the egress kernel (k8_egress.cu), the Bayer demosaic of k0_ingest.cu and the INTER_LINEAR tap tables and
+// vertical step of k0_resize.cu.
 #pragma once
 #include "lane_common.cuh"
 
@@ -79,9 +80,9 @@ __device__ __forceinline__ uint32_t k0_vmix(int h0, int h1, int b0, int b1)
     return (uint32_t)min(v, 255);
 }
 
-// The per-thread pixel work of the resize kernels (k0_resize, k0_yuv420_resize, k0_rig_ingest): one thread makes PX
-// consecutive destination pixels dx0 .. dx0+PX-1 of destination row dy (columns past dw repeat the last one and are not
-// stored).  yy / b: the row's yofs / beta entries.
+// The per-thread pixel work of the resize kernels (k0_resize, k0_yuv420_resize, k0_bayer_resize, k0_rig_ingest): one
+// thread makes PX consecutive destination pixels dx0 .. dx0+PX-1 of destination row dy (columns past dw repeat the last
+// one and are not stored).  yy / b: the row's yofs / beta entries.
 //
 // k0_resize's arithmetic on CN interleaved uint8 channels: r0 / r1 are the two source rows.
 template <int CN, int PX>
@@ -131,6 +132,93 @@ __device__ __forceinline__ void k0_yuv420_resize_px(const uint8_t *__restrict__ 
     }
 }
 
+// ---- raw Bayer -> BGR, bit-exact with cv2.cvtColor(f, COLOR_Bayer{RGGB,BGGR,GRBG,GBRG}2BGR) (oracle/bayer.py) -------
+// The bilinear demosaic.  Pixel (y, x) of an H x W mosaic (H, W >= 3) is the interior formula at (clamp(y, 1, H-2),
+// clamp(x, 1, W-2)): its own colour is the raw value; at an R or B site G = (4 neighbours + 2) >> 2 and the other chroma
+// = (4 diagonals + 2) >> 2; at a G site the colour of the horizontal neighbours = (left + right + 1) >> 1 and that of
+// the vertical ones = (up + down + 1) >> 1.  The four patterns are one RGGB mosaic read at a phase (py, px).
+__host__ __device__ constexpr bool lane_input_bayer(int format)
+{
+    return format >= LANE_INPUT_BAYER_RGGB && format <= LANE_INPUT_BAYER_GBRG;
+}
+
+// (py, px) of a LANE_INPUT_BAYER_* layout as bits 1 and 0: RGGB 0, GRBG 1, GBRG 2, BGGR 3.
+__host__ __device__ constexpr int lane_bayer_phase(int format)
+{
+    return format == LANE_INPUT_BAYER_RGGB ? 0 : format == LANE_INPUT_BAYER_GRBG ? 1 : format == LANE_INPUT_BAYER_GBRG ? 2 : 3;
+}
+
+namespace k0bayer {
+
+// BGR of the centre of the 3x3 window of w at column J (columns J-1..J+1), whose site is at parity (ry, rx) of the RGGB
+// mosaic.
+template <int J>
+__device__ __forceinline__ void px(const int (&w)[3][4], int ry, int rx, int &b, int &g, int &r)
+{
+    const int own = w[1][J], h = w[1][J - 1] + w[1][J + 1], v = w[0][J] + w[2][J];
+    const int d = w[0][J - 1] + w[0][J + 1] + w[2][J - 1] + w[2][J + 1];
+    const bool chroma_site = ry == rx;                       // R (0, 0) or B (1, 1); else G
+    const int near = chroma_site ? own : (h + 1) >> 1;      // R on a red row, B on a blue row
+    const int far = chroma_site ? (d + 2) >> 2 : (v + 1) >> 1;
+    g = chroma_site ? (h + v + 2) >> 2 : own;
+    r = ry ? far : near;
+    b = ry ? near : far;
+}
+
+// k0_resize's horizontal step on the demosaiced row cy (clamped, 1 <= cy <= sh-2; site parity ry): the two source
+// columns of the tap are the clamped centres cx0 and cx0 + ddx (ddx 0 or 1), demosaiced from the 3x4 raw window at
+// rows cy-1..cy+1, columns cx0-1..cx0+2.  `up` points at row cy-1.
+__device__ __forceinline__ void hmix(const uint8_t *__restrict__ up, int sw, int cx0, int ddx, int ry, int rx, short2 a,
+                                     int (&h)[3])
+{
+    const int x3 = min(cx0 + 2, sw - 1);                    // columns cx0-1 .. cx0+1 are inside the row
+    int w[3][4];
+#pragma unroll
+    for (int i = 0; i < 3; i++) {
+        const uint8_t *r = up + i * sw;
+        w[i][0] = __ldg(r + cx0 - 1); w[i][1] = __ldg(r + cx0); w[i][2] = __ldg(r + cx0 + 1); w[i][3] = __ldg(r + x3);
+    }
+    int p0[3], p1[3];
+    px<1>(w, ry, rx, p0[0], p0[1], p0[2]);
+    px<2>(w, ry, rx ^ 1, p1[0], p1[1], p1[2]);
+#pragma unroll
+    for (int c = 0; c < 3; c++) h[c] = p0[c] * a.x + (ddx ? p1[c] : p0[c]) * a.y;
+}
+
+}  // namespace k0bayer
+
+// The same resize of the BGR frame cv2.cvtColor makes of Bayer mosaic `s` (sh x sw, sh and sw >= 3, phase as
+// lane_bayer_phase): the two source rows x two source columns of every tap are demosaiced on the fly from their raw
+// neighbourhood (the clamped centres of y1 / x1 are those of y0 / x0 or one further), the demosaiced frame is never
+// stored.  At identity taps this is cv2.cvtColor's frame itself.  dy below is uniform over a destination row.
+template <int PX>
+__device__ __forceinline__ void k0_bayer_resize_px(const uint8_t *__restrict__ s, int sh, int sw, int phase, int2 yy,
+                                                   short2 b, const int *__restrict__ xofs, const short2 *__restrict__ alpha,
+                                                   int dx0, int dw, uint8_t (&o)[PX * 3])
+{
+    const int cy0 = min(max(yy.x, 1), sh - 2), dy = min(max(yy.y, 1), sh - 2) - cy0;        // dy: 0 or 1
+    const uint8_t *up = s + (size_t)(cy0 - 1) * sw;
+    const int ry = (cy0 + (phase >> 1)) & 1;
+#pragma unroll
+    for (int k = 0; k < PX; k++) {
+        const int dx = min(dx0 + k, dw - 1);
+        const int x0 = __ldg(xofs + dx), x1 = min(x0 + 1, sw - 1);
+        const short2 a = __ldg(alpha + dx);
+        const int cx0 = min(max(x0, 1), sw - 2), ddx = min(max(x1, 1), sw - 2) - cx0;
+        const int rx = (cx0 + phase) & 1;
+        int h0[3], h1[3];
+        k0bayer::hmix(up, sw, cx0, ddx, ry, rx, a, h0);
+        if (dy) {
+            k0bayer::hmix(up + sw, sw, cx0, ddx, ry ^ 1, rx, a, h1);
+        } else {
+#pragma unroll
+            for (int c = 0; c < 3; c++) h1[c] = h0[c];
+        }
+#pragma unroll
+        for (int c = 0; c < 3; c++) o[k * 3 + c] = (uint8_t)k0_vmix(h0[c], h1[c], b.x, b.y);
+    }
+}
+
 // Stores one thread's pixels at `out` (destination pixel dx0): packed 4-byte stores when the PX pixels are all inside
 // the row and `out` is aligned, byte stores otherwise.
 template <int CN, int PX>
@@ -158,8 +246,9 @@ void launch_yuv420_to_bgr(const uint8_t *src, int format, uint8_t *dst, int n, i
 
 // ---- ingest: any LANE_INPUT_* layout at any size -> BGR at dh x dw --------------------------------------------------
 // NV12 / I420 at the destination size: k0_nv12's conversion kernels; NV12 / I420 at another size: the fused
-// conversion + resize kernel (k0_ingest.cu); BGR at another size: k0_resize.  BGR at its own size needs no kernel and is
-// not taken.  Device pointers, enqueued on st; the caller has validated the sizes (even YUV sizes, grid limits).
+// conversion + resize kernel (k0_ingest.cu); Bayer at any size: the fused demosaic + resize kernel (identity taps at its
+// own size); BGR at another size: k0_resize.  BGR at its own size needs no kernel and is not taken.  Device pointers,
+// enqueued on st; the caller has validated the sizes (even YUV sizes, Bayer sizes >= 3, grid limits).
 cudaError_t launch_ingest(const uint8_t *src, int format, int n, int sh, int sw, uint8_t *dst, int dh, int dw,
                           cudaStream_t st);
 
@@ -167,7 +256,7 @@ cudaError_t launch_ingest(const uint8_t *src, int format, int n, int sh, int sw,
 // Descriptor of one source frame (device memory, dense); the tap tables are lane_resize_taps' cached ones.
 struct RigFrame {
     const uint8_t *src;
-    int format, sh, sw;                // LANE_INPUT_*; YUV sizes even
+    int format, sh, sw;                // LANE_INPUT_*; YUV sizes even, Bayer sizes >= 3
     const int *xofs;
     const short2 *alpha;
     const int2 *yofs;

@@ -8,6 +8,11 @@
 // and the 2x2 block's (U, V), k0_common.cuh) and apply k0_resize's 11-bit horizontal taps and vertical step to them:
 // the full-resolution BGR frame is never written.  HBM-bound: reads the touched 1.5 B/px of the source once, writes
 // 3 B per destination pixel.
+//
+// K0e: raw camera frames (8-bit Bayer mosaics, 1 B/px) the same way: per destination pixel
+//     cv2.resize(cv2.cvtColor(src, COLOR_Bayer{RGGB,BGGR,GRBG,GBRG}2BGR), (dw, dh))      (INTER_LINEAR)
+// with the two source rows x two source columns of every tap demosaiced from their 4x4 raw neighbourhood
+// (k0_bayer_resize_px).  A frame at the destination size runs on identity taps: the demosaic alone.
 #include "host_stage.h"
 #include "k0_common.cuh"
 
@@ -35,10 +40,54 @@ __global__ void __launch_bounds__(256) k0_yuv420_resize(const uint8_t *__restric
     k0_store_px<3, PX>(out, o, dx0, dw);
 }
 
+// k0_yuv420_resize for Bayer mosaics of one pattern (phase: lane_bayer_phase), at any size including the source's own.
+template <int PX>
+__global__ void __launch_bounds__(256) k0_bayer_resize(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst,
+                                                       const int *__restrict__ xofs, const short2 *__restrict__ alpha,
+                                                       const int2 *__restrict__ yofs, const short2 *__restrict__ beta,
+                                                       int phase, int sh, int sw, int dh, int dw)
+{
+    const int dx0 = (blockIdx.x * blockDim.x + threadIdx.x) * PX, dy = blockIdx.y, f = blockIdx.z;
+    if (dx0 >= dw) return;
+    const int2 yy = __ldg(yofs + dy);
+    const short2 b = __ldg(beta + dy);
+    const uint8_t *s = src + (size_t)f * sh * sw;
+    uint8_t *out = dst + (((size_t)f * dh + dy) * dw + dx0) * 3;
+    uint8_t o[PX * 3];
+    k0_bayer_resize_px<PX>(s, sh, sw, phase, yy, b, xofs, alpha, dx0, dw, o);
+    k0_store_px<3, PX>(out, o, dx0, dw);
+}
+
 // The frames of a rig: every frame has its own descriptor (layout, size, tap tables), so cameras of different
 // resolutions and decoders share one launch.  The grid is k0_yuv420_resize's; a block reads its frame's descriptor
 // once, and the branch on the layout is uniform over the block.  A frame already at dh x dw runs on identity taps,
-// which reproduce the source (BGR) or cv2.cvtColor's frame (YUV) exactly.
+// which reproduce the source (BGR) or cv2.cvtColor's frame (YUV, Bayer) exactly.
+//
+// The Bayer and the BGR / YUV pixel work are separate functions kept out of line: inlined side by side they need 60
+// registers, which would drop the kernel from 5 to 4 blocks per SM; apart, each fits the kernel's 48.
+template <int PX>
+__device__ __noinline__ void rig_bgr_yuv420(const RigFrame &d, int2 yy, short2 b, int dx0, int dw, uint8_t *out)
+{
+    uint8_t o[PX * 3];
+    if (d.format == LANE_INPUT_BGR) {
+        const uint8_t *r0 = d.src + (size_t)yy.x * d.sw * 3, *r1 = d.src + (size_t)yy.y * d.sw * 3;
+        k0_resize_px<3, PX>(r0, r1, d.xofs, d.alpha, b, d.sw, dx0, dw, o);
+    } else if (d.format == LANE_INPUT_NV12) {
+        k0_yuv420_resize_px<LANE_INPUT_NV12, PX>(d.src, d.sh, d.sw, yy, b, d.xofs, d.alpha, dx0, dw, o);
+    } else {
+        k0_yuv420_resize_px<LANE_INPUT_I420, PX>(d.src, d.sh, d.sw, yy, b, d.xofs, d.alpha, dx0, dw, o);
+    }
+    k0_store_px<3, PX>(out, o, dx0, dw);
+}
+
+template <int PX>
+__device__ __noinline__ void rig_bayer(const RigFrame &d, int2 yy, short2 b, int dx0, int dw, uint8_t *out)
+{
+    uint8_t o[PX * 3];
+    k0_bayer_resize_px<PX>(d.src, d.sh, d.sw, lane_bayer_phase(d.format), yy, b, d.xofs, d.alpha, dx0, dw, o);
+    k0_store_px<3, PX>(out, o, dx0, dw);
+}
+
 template <int PX>
 __global__ void __launch_bounds__(256) k0_rig_ingest(const RigFrame *__restrict__ frames, uint8_t *__restrict__ dst, int dh,
                                                      int dw)
@@ -51,16 +100,10 @@ __global__ void __launch_bounds__(256) k0_rig_ingest(const RigFrame *__restrict_
     const int2 yy = __ldg(d.yofs + dy);
     const short2 b = __ldg(d.beta + dy);
     uint8_t *out = dst + (((size_t)f * dh + dy) * dw + dx0) * 3;
-    uint8_t o[PX * 3];
-    if (d.format == LANE_INPUT_BGR) {
-        const uint8_t *r0 = d.src + (size_t)yy.x * d.sw * 3, *r1 = d.src + (size_t)yy.y * d.sw * 3;
-        k0_resize_px<3, PX>(r0, r1, d.xofs, d.alpha, b, d.sw, dx0, dw, o);
-    } else if (d.format == LANE_INPUT_NV12) {
-        k0_yuv420_resize_px<LANE_INPUT_NV12, PX>(d.src, d.sh, d.sw, yy, b, d.xofs, d.alpha, dx0, dw, o);
-    } else {
-        k0_yuv420_resize_px<LANE_INPUT_I420, PX>(d.src, d.sh, d.sw, yy, b, d.xofs, d.alpha, dx0, dw, o);
-    }
-    k0_store_px<3, PX>(out, o, dx0, dw);
+    if (lane_input_bayer(d.format))
+        rig_bayer<PX>(d, yy, b, dx0, dw, out);
+    else
+        rig_bgr_yuv420<PX>(d, yy, b, dx0, dw, out);
 }
 
 }  // namespace
@@ -84,7 +127,8 @@ void launch_rig_ingest(const RigFrame *frames_dev, int n, uint8_t *dst, int dh, 
 cudaError_t launch_ingest(const uint8_t *src, int format, int n, int sh, int sw, uint8_t *dst, int dh, int dw,
                           cudaStream_t st)
 {
-    if (format != LANE_INPUT_BGR && sh == dh && sw == dw) {       // INTER_LINEAR at scale 1 is the identity
+    const bool yuv = format == LANE_INPUT_NV12 || format == LANE_INPUT_I420;
+    if (yuv && sh == dh && sw == dw) {                             // INTER_LINEAR at scale 1 is the identity
         launch_yuv420_to_bgr(src, format, dst, n, sh, sw, st);
         return cudaGetLastError();
     }
@@ -97,7 +141,10 @@ cudaError_t launch_ingest(const uint8_t *src, int format, int n, int sh, int sw,
     }
     constexpr int PX = 4;
     const dim3 grid((dw + 256 * PX - 1) / (256 * PX), dh, n);
-    if (format == LANE_INPUT_I420)
+    if (lane_input_bayer(format))
+        k0_bayer_resize<PX><<<grid, 256, 0, st>>>(src, dst, t.xofs, t.alpha, t.yofs, t.beta, lane_bayer_phase(format), sh, sw,
+                                                  dh, dw);
+    else if (format == LANE_INPUT_I420)
         k0_yuv420_resize<LANE_INPUT_I420, PX><<<grid, 256, 0, st>>>(src, dst, t.xofs, t.alpha, t.yofs, t.beta, sh, sw, dh, dw);
     else
         k0_yuv420_resize<LANE_INPUT_NV12, PX><<<grid, 256, 0, st>>>(src, dst, t.xofs, t.alpha, t.yofs, t.beta, sh, sw, dh, dw);
@@ -135,6 +182,25 @@ extern "C" int lane_yuv420_to_bgr_batch(const uint8_t *src, int format, int n, i
 {
     return yuv420_to_bgr("lane_yuv420_to_bgr_batch", src, format, n, src_h, src_w, dst, dst_h, dst_w, on_device, device,
                          cuda_stream);
+}
+
+extern "C" int lane_bayer_to_bgr_batch(const uint8_t *src, int format, int n, int src_h, int src_w, uint8_t *dst,
+                                       int dst_h, int dst_w, int on_device, int device, void *cuda_stream)
+{
+    const char *who = "lane_bayer_to_bgr_batch";
+    if (!src || !dst || n < 1 || src_h < 1 || src_w < 1 || dst_h < 1 || dst_w < 1)
+        return lane_api_fail(LANE_ERR_INVALID, who, "bad arguments (non-null pointers, positive sizes)");
+    if (!lane_input_bayer(format)) return lane_api_fail(LANE_ERR_INVALID, who, "format must be a LANE_INPUT_BAYER_* layout");
+    if (src_h < 3 || src_w < 3) return lane_api_fail(LANE_ERR_INVALID, who, "a Bayer frame needs at least 3 rows and 3 columns");
+    if (dst_h > 65535 || n > 65535) return lane_api_fail(LANE_ERR_UNSUPPORTED, who, "destination height / batch above 65535");
+    if (int rc = lane_api_device(who, device)) return rc;
+    cudaStream_t st = (cudaStream_t)cuda_stream;
+    auto launch = [&](const uint8_t *s, uint8_t *d) {
+        const cudaError_t e = launch_ingest(s, format, n, src_h, src_w, d, dst_h, dst_w, st);
+        return e ? lane_api_fail(LANE_ERR_CUDA, who, "launch", e) : LANE_OK;
+    };
+    if (on_device) return launch(src, dst);
+    return lane_host_round_trip(who, device, st, src, (size_t)n * src_h * src_w, dst, (size_t)n * dst_h * dst_w * 3, launch);
 }
 
 extern "C" int lane_nv12_to_bgr_batch(const uint8_t *src, int n, int height, int width, uint8_t *dst, int on_device,

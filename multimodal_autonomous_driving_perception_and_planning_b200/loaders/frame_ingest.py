@@ -85,12 +85,27 @@ class FrameIngest:
         check_yuv420(frames, "FrameIngest")
         n, h, w = int(frames.shape[0]), int(frames.shape[1]) * 2 // 3, int(frames.shape[2])
         dw, dh = (w, h) if self.target_size is None else self.target_size
-        lib = _native.lib()
+        return self._convert(_native.lib().lane_yuv420_to_bgr_batch, frames, fmt, n, h, w, dh, dw)
+
+    def from_bayer(self, frames, pattern: str):
+        """Raw camera frames -> BGR: ``frames`` uint8 ``[N, H, W]`` 8-bit Bayer mosaics (numpy or CUDA tensor, H and W
+        at least 3) whose top-left 2x2 is ``pattern`` ("rggb", "bggr", "grbg" or "gbrg") become ``[N, H, W, 3]``, equal
+        to ``cv2.cvtColor(f, cv2.COLOR_Bayer<P>2BGR)`` per frame, followed by the resize when ``target_size`` is set.
+        Demosaic and resize are one kernel: the full-resolution BGR frame is never stored."""
+        fmt = bayer_format(pattern)
+        check_bayer(frames, "FrameIngest")
+        n, h, w = (int(x) for x in frames.shape)
+        dw, dh = (w, h) if self.target_size is None else self.target_size
+        return self._convert(_native.lib().lane_bayer_to_bgr_batch, frames, fmt, n, h, w, dh, dw)
+
+    def _convert(self, entry, frames, fmt, n, h, w, dh, dw):
+        """One context-free conversion entry (``lane_yuv420_to_bgr_batch`` / ``lane_bayer_to_bgr_batch``): numpy in,
+        numpy out; CUDA tensor in, CUDA tensor out on torch's current stream."""
         if isinstance(frames, np.ndarray):
             src = np.ascontiguousarray(frames)
             dst = np.empty((n, dh, dw, 3), np.uint8)
-            rc = lib.lane_yuv420_to_bgr_batch(src.ctypes.data_as(C.c_void_p), fmt, n, h, w, dst.ctypes.data_as(C.c_void_p),
-                                              dh, dw, 0, self._device_index(), None)
+            rc = entry(src.ctypes.data_as(C.c_void_p), fmt, n, h, w, dst.ctypes.data_as(C.c_void_p), dh, dw, 0,
+                       self._device_index(), None)
         else:
             import torch
             if not frames.is_cuda:
@@ -98,8 +113,8 @@ class FrameIngest:
             src = frames.contiguous()
             dst = torch.empty((n, dh, dw, 3), dtype=torch.uint8, device=src.device)
             stream = torch.cuda.current_stream(src.device).cuda_stream
-            rc = lib.lane_yuv420_to_bgr_batch(C.c_void_p(src.data_ptr()), fmt, n, h, w, C.c_void_p(dst.data_ptr()), dh, dw,
-                                              1, src.device.index, C.c_void_p(stream))
+            rc = entry(C.c_void_p(src.data_ptr()), fmt, n, h, w, C.c_void_p(dst.data_ptr()), dh, dw, 1, src.device.index,
+                       C.c_void_p(stream))
         _native.check_global(rc)
         return dst
 
@@ -113,6 +128,23 @@ def check_yuv420(frames, who: str):
     shape = tuple(frames.shape)
     if len(shape) != 3 or shape[1] % 3 or shape[2] % 2 or (shape[1] * 2 // 3) % 2:
         raise cv2.error(f"{who}: expected NV12 / I420 frames [N, H*3/2, W] with even H and W, got {shape}")
+    if str(frames.dtype).replace("torch.", "") != "uint8":
+        raise cv2.error(f"{who}: expected uint8 frames, got {frames.dtype}")
+
+
+def bayer_format(pattern) -> int:
+    """LANE_INPUT_BAYER_* of a pattern name ("rggb", "bggr", "grbg", "gbrg"), else ``ValueError``."""
+    if not isinstance(pattern, str) or pattern not in _native.BAYER:
+        raise ValueError(f"Bayer pattern {pattern!r} is not one of {sorted(_native.BAYER)}")
+    return _native.BAYER[pattern]
+
+
+def check_bayer(frames, who: str):
+    """uint8 ``[N, H, W]`` with H, W >= 3 (raw Bayer mosaics), else ``cv2.error``.  cv2.cvtColor returns an all-zero
+    frame below 3 rows or columns; such frames are refused rather than emulated."""
+    shape = tuple(frames.shape)
+    if len(shape) != 3 or shape[1] < 3 or shape[2] < 3:
+        raise cv2.error(f"{who}: expected Bayer frames [N, H, W] with H, W >= 3, got {shape}")
     if str(frames.dtype).replace("torch.", "") != "uint8":
         raise cv2.error(f"{who}: expected uint8 frames, got {frames.dtype}")
 

@@ -20,7 +20,7 @@ import cv2
 import numpy as np
 
 from .. import _native
-from ..loaders.frame_ingest import check_target_size, check_yuv420
+from ..loaders.frame_ingest import bayer_format, check_bayer, check_target_size, check_yuv420
 
 
 @dataclass
@@ -34,7 +34,9 @@ class LaneLine:
 
 LanePair = Tuple[Optional[LaneLine], Optional[LaneLine]]
 _SIDES = ("left", "right")
-_LAYOUTS = {"bgr": _native.INPUT_BGR, "nv12": _native.INPUT_NV12, "i420": _native.INPUT_I420}
+_LAYOUTS = {"bgr": _native.INPUT_BGR, "nv12": _native.INPUT_NV12, "i420": _native.INPUT_I420,
+            **{"bayer_" + p: fmt for p, fmt in _native.BAYER.items()}}
+_BAYER_FORMATS = frozenset(_native.BAYER.values())
 _COPY_PIECE = 4 << 20         # bytes per host thread task when detect_rig_stream copies a numpy tick into pinned memory
 
 
@@ -50,8 +52,8 @@ def _is_pinned_tensor(x) -> bool:
 
 
 def _frame_bytes(fmt: int, h: int, w: int) -> int:
-    """Bytes of one h x w frame in layout ``fmt`` (INPUT_*): 3 B/px BGR, 1.5 B/px YUV 4:2:0."""
-    return h * w * 3 if fmt == _native.INPUT_BGR else h * w * 3 // 2
+    """Bytes of one h x w frame in layout ``fmt`` (INPUT_*): 3 B/px BGR, 1.5 B/px YUV 4:2:0, 1 B/px Bayer."""
+    return h * w * 3 if fmt == _native.INPUT_BGR else h * w if fmt in _BAYER_FORMATS else h * w * 3 // 2
 
 
 def _two_deep(items, plan, start, joins, enqueue, blocking, restore, adopt):
@@ -145,10 +147,10 @@ class _Plan:
 
     @classmethod
     def of_frames(cls, frames, fmt: int, target_size=None, frame_sids=None, stream_rois=None) -> "_Plan":
-        """One checked array of frames: [N,H,W,3] BGR, or [N,H*3/2,W] for the YUV 4:2:0 layouts of ``fmt``, detected at
-        ``target_size`` = (width, height) when given."""
+        """One checked array of frames: [N,H,W,3] BGR, [N,H*3/2,W] for the YUV 4:2:0 layouts or [N,H,W] for the Bayer
+        layouts of ``fmt``, detected at ``target_size`` = (width, height) when given."""
         n, sh, sw = (int(x) for x in frames.shape[:3])
-        if fmt != _native.INPUT_BGR:
+        if fmt not in (_native.INPUT_BGR, *_BAYER_FORMATS):
             sh = sh * 2 // 3
         h, w = (sh, sw) if target_size is None else (target_size[1], target_size[0])
         kind = ("cuda", frames.device.index) if _is_torch_cuda(frames) else "host"
@@ -524,6 +526,16 @@ class LaneDetector:
         check_yuv420(frames, "LaneDetector")
         return self._detect_frames(frames, _native.INPUT_I420, target_size)
 
+    def detect_batch_bayer(self, frames, pattern: str, *, target_size: Optional[Tuple[int, int]] = None) -> List[LanePair]:
+        """``detect_batch`` for raw camera frames: uint8 ``[N, H, W]`` 8-bit Bayer mosaics (numpy or CUDA tensor, H and W
+        at least 3) whose top-left 2x2 is ``pattern`` ("rggb", "bggr", "grbg" or "gbrg"; no default).  Equal to
+        ``detect_batch`` of ``cv2.cvtColor(f, cv2.COLOR_Bayer<P>2BGR)`` of every frame, resized to ``target_size`` =
+        (width, height) when given, with the same ``prev_*_fit`` after it.  Demosaic and resize are one kernel on the
+        device, so a host batch moves 1 B/px over PCIe."""
+        fmt = bayer_format(pattern)
+        check_bayer(frames, "LaneDetector")
+        return self._detect_frames(frames, fmt, target_size)
+
     def detect_streams(self, frames, stream_ids: Optional[Sequence[int]] = None, *,
                        stream_rois: Optional[Sequence[Optional[np.ndarray]]] = None) -> List[LanePair]:
         """Multi-camera form: ``frames`` is [S,T,H,W,3] (stream-major) or [N,H,W,3] with ``stream_ids[N]``.
@@ -572,9 +584,9 @@ class LaneDetector:
                    stream_rois: Optional[Sequence[Optional[np.ndarray]]] = None) -> List[List[LanePair]]:
         """A rig of cameras that differ in resolution and decoder layout, in one batched call.
 
-        ``frames[s]`` is camera s (= stream s of ``detect_streams``): uint8 ``[T_s, H_s, W_s, 3]`` BGR or
-        ``[T_s, H_s*3/2, W_s]`` NV12 / I420, as ``layouts[s]`` ("bgr", "nv12", "i420"; default all "bgr") says, its frames
-        in temporal order.  ``T_s`` may differ between cameras and may be 0, or the entry None: no frame this tick.  Every
+        ``frames[s]`` is camera s (= stream s of ``detect_streams``): uint8 ``[T_s, H_s, W_s, 3]`` BGR,
+        ``[T_s, H_s*3/2, W_s]`` NV12 / I420 or ``[T_s, H_s, W_s]`` raw Bayer, as ``layouts[s]`` ("bgr", "nv12", "i420",
+        "bayer_rggb", "bayer_bggr", "bayer_grbg", "bayer_gbrg"; default all "bgr") says, its frames in temporal order.  ``T_s`` may differ between cameras and may be 0, or the entry None: no frame this tick.  Every
         camera is a numpy array, or every camera is a CUDA tensor on one device.  Every frame is detected at
         ``target_size`` = (width, height), which may be left out only when all cameras share one size; the device converts
         and resizes all frames in one kernel (only the source bytes of host frames cross PCIe) and runs the rest of the
@@ -582,7 +594,7 @@ class LaneDetector:
 
         Returns one list of pairs per camera.  Camera s's pairs equal those of a fresh
         ``LaneDetector(roi_vertices=stream_rois[s])`` given its frames through ``detect_batch`` / ``detect_batch_nv12`` /
-        ``detect_batch_i420(frames[s], target_size=target_size)``; its smoothing state is stream s's of ``detect_streams``,
+        ``detect_batch_i420(frames[s], target_size=target_size)`` / ``detect_batch_bayer``; its smoothing state is stream s's of ``detect_streams``,
         so it carries across calls of either kind (``reset`` clears it).
         """
         return self._detect_rig(self._rig_plan(frames, layouts, target_size, stream_rois))
@@ -704,6 +716,12 @@ class LaneDetector:
             if shape[-1] != 3:
                 raise cv2.error(f"LaneDetector: camera {s}: expected 3-channel BGR frames, got {shape}")
             h, w = shape[1], shape[2]
+        elif layout.startswith("bayer_"):
+            if len(shape) != 3:
+                raise ValueError(f"camera {s}: layout {layout!r} needs frames [T,H,W], got {shape}")
+            h, w = shape[1], shape[2]
+            if h < 3 or w < 3:
+                raise ValueError(f"camera {s}: {layout} needs at least 3 rows and 3 columns, got {w}x{h}")
         else:
             if len(shape) != 3 or shape[1] % 3:
                 raise ValueError(f"camera {s}: layout {layout!r} needs frames [T,H*3/2,W], got {shape}")
