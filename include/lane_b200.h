@@ -141,6 +141,12 @@ LANE_API int lane_detect_batch_nv12(lane_ctx *ctx, const uint8_t *frames_nv12, i
 #define LANE_INPUT_BAYER_BGGR 17
 #define LANE_INPUT_BAYER_GRBG 18
 #define LANE_INPUT_BAYER_GBRG 19
+/* Packed YUV 4:2:2, uint8 [n][src_h][src_w][2] (2 B/px), src_w even, src_h >= 1: every horizontal pixel pair shares one
+ * (U, V), nothing is shared vertically.  UYVY (GMSL / FPD-Link camera deserializers) stores each pair as U Y0 V Y1,
+ * YUYV (V4L2 USB cameras, cv2's YUY2) as Y0 U Y1 V.  Such a frame becomes cv2.cvtColor(f, COLOR_YUV2BGR_UYVY |
+ * COLOR_YUV2BGR_YUY2): the BT.601 arithmetic of NV12. */
+#define LANE_INPUT_UYVY 8
+#define LANE_INPUT_YUYV 9
 
 /* lane_detect_batch on frames of another size and/or layout, as VideoDataLoader.read_frame delivers them
  * (/root/reference/data/loaders/video_loader.py:96-131: decode, then cv2.resize(frame, target_size) at :108, :128) to
@@ -148,8 +154,8 @@ LANE_API int lane_detect_batch_nv12(lane_ctx *ctx, const uint8_t *frames_nv12, i
  * -- cv2.resize(cv2.cvtColor(f, COLOR_YUV2BGR_NV12 | COLOR_YUV2BGR_I420), (width, height)) in one kernel for YUV, the
  * lane_resize_batch kernel for BGR -- and the usual path runs on it: only the source bytes cross PCIe, and the records
  * equal those of lane_detect_batch on the cv2-prepared frames.  format: LANE_INPUT_*; src_h / src_w: the frames' own
- * size (even for NV12 / I420, at least 3 for Bayer, whose frames are demosaiced and resized in one kernel at any size).
- * Other arguments as for lane_detect_batch. */
+ * size (even for NV12 / I420, at least 3 for Bayer, whose frames are demosaiced and resized in one kernel at any size,
+ * an even width for UYVY / YUYV).  Other arguments as for lane_detect_batch. */
 LANE_API int lane_detect_batch_ingest(lane_ctx *ctx, const uint8_t *frames, int frames_on_device, int n, int format,
                                       int src_h, int src_w, const int32_t *stream_id, int n_streams, double *prev_fit,
                                       uint8_t *prev_valid, lane_record *out);
@@ -157,8 +163,8 @@ LANE_API int lane_detect_batch_ingest(lane_ctx *ctx, const uint8_t *frames, int 
 /* One camera of a rig in a lane_detect_rig call. */
 typedef struct lane_rig_source {
     const uint8_t *frames;   /* n dense frames of one camera in `format` at src_h x src_w (host or device, per the call) */
-    int32_t format;          /* LANE_INPUT_BGR / NV12 / I420 / BAYER_* */
-    int32_t src_h, src_w;    /* the camera's own size (even for NV12 / I420, at least 3 for Bayer) */
+    int32_t format;          /* LANE_INPUT_BGR / NV12 / I420 / BAYER_* / UYVY / YUYV */
+    int32_t src_h, src_w;    /* the camera's own size (even for NV12 / I420, at least 3 for Bayer, even width for UYVY / YUYV) */
     int32_t n;               /* frames of this camera in the call, in temporal order; 0 = none this tick */
     int32_t stream_id;       /* the camera: index into prev_fit / prev_valid and the ROI masks */
 } lane_rig_source;
@@ -174,10 +180,11 @@ typedef struct lane_rig_source {
  *   n_streams, prev_fit, prev_valid   as for lane_detect_batch (both state arrays required).
  *   out            host lane_record[sum of n], the frames in source order.
  * Camera s's records equal those of lane_detect_batch_ingest on its frames alone with its stream's state and mask.
- * Bayer sources (LANE_INPUT_BAYER_*) become cv2.resize(cv2.cvtColor(f, COLOR_Bayer<P>2BGR), (width, height)).
+ * Bayer sources (LANE_INPUT_BAYER_*) become cv2.resize(cv2.cvtColor(f, COLOR_Bayer<P>2BGR), (width, height)), packed
+ * 4:2:2 sources (LANE_INPUT_UYVY / YUYV) cv2.resize(cv2.cvtColor(f, COLOR_YUV2BGR_UYVY | COLOR_YUV2BGR_YUY2), ...).
  * Blocking.  LANE_ERR_INVALID: null pointers, a sum of n of 0 or above max_batch, a negative n, an unknown format, a
- * non-positive size, an odd YUV size or a Bayer size below 3, stream_id outside [0, n_streams), n_streams above the context's masks (when
- * it holds more than one). */
+ * non-positive size, an odd YUV 4:2:0 size, a Bayer size below 3 or an odd 4:2:2 width, stream_id outside
+ * [0, n_streams), n_streams above the context's masks (when it holds more than one). */
 LANE_API int lane_detect_rig(lane_ctx *ctx, const lane_rig_source *sources, int n_sources, int frames_on_device,
                              int n_streams, double *prev_fit, uint8_t *prev_valid, lane_record *out);
 
@@ -320,6 +327,16 @@ LANE_API int lane_yuv420_to_bgr_batch(const uint8_t *src, int format, int n, int
  * cuda_stream as for lane_resize_batch.  Needs no context; errors via lane_last_error(NULL). */
 LANE_API int lane_bayer_to_bgr_batch(const uint8_t *src, int format, int n, int src_h, int src_w, uint8_t *dst,
                                      int dst_h, int dst_w, int on_device, int device, void *cuda_stream);
+
+/* Packed 4:2:2 camera frames -> the frame VideoDataLoader.read_frame returns with target_size set: per frame
+ * cv2.resize(cv2.cvtColor(f, COLOR_YUV2BGR_UYVY | COLOR_YUV2BGR_YUY2), (dst_w, dst_h)), bit-exact, in one pass that
+ * reads the 2 B/px source and writes only the destination (the full-resolution BGR frame is never stored).
+ * src: uint8 [n][src_h][src_w][2] in `format` (LANE_INPUT_UYVY or LANE_INPUT_YUYV), src_w even; dst: uint8
+ * [n][dst_h][dst_w][3], any positive size (equal to the source size: conversion only).  When resizing, dst_h and n up
+ * to 65535.  on_device / device / cuda_stream as for lane_resize_batch.  Needs no context; errors via
+ * lane_last_error(NULL). */
+LANE_API int lane_yuv422_to_bgr_batch(const uint8_t *src, int format, int n, int src_h, int src_w, uint8_t *dst,
+                                      int dst_h, int dst_w, int on_device, int device, void *cuda_stream);
 
 /* ---- frame egress (SURVEY.md 8f rank 3: the step after the overlays when annotated video is written) ---------------
  * cv2.cvtColor(f, COLOR_BGR2YUV_I420) per frame (NV12: the same samples, U and V interleaved), for annotated frames

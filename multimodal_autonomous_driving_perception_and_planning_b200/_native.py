@@ -28,6 +28,9 @@ INPUT_BGR, INPUT_NV12, INPUT_I420 = 0, 1, 2          # LANE_INPUT_*: frame layou
 # raw 8-bit Bayer mosaics [n][h][w], named by the sensor's top-left 2x2 (cv2.COLOR_Bayer<P>2BGR)
 INPUT_BAYER_RGGB, INPUT_BAYER_BGGR, INPUT_BAYER_GRBG, INPUT_BAYER_GBRG = 16, 17, 18, 19
 BAYER = {"rggb": INPUT_BAYER_RGGB, "bggr": INPUT_BAYER_BGGR, "grbg": INPUT_BAYER_GRBG, "gbrg": INPUT_BAYER_GBRG}
+# packed YUV 4:2:2 camera frames [n][h][w][2], w even: UYVY (U Y0 V Y1, GMSL / FPD-Link) and YUYV (Y0 U Y1 V, V4L2)
+INPUT_UYVY, INPUT_YUYV = 8, 9
+YUV422 = {"uyvy": INPUT_UYVY, "yuyv": INPUT_YUYV}
 
 
 class LaneSide(C.Structure):
@@ -111,6 +114,8 @@ _PROTOS = {
                                            C.c_int, C.c_int, C.c_void_p]),
     "lane_bayer_to_bgr_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int,
                                           C.c_int, C.c_int, C.c_void_p]),
+    "lane_yuv422_to_bgr_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int,
+                                           C.c_int, C.c_int, C.c_void_p]),
     "lane_bgr_to_yuv420_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int,
                                            C.c_void_p]),
     "lane_detect_enqueue": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
@@ -283,8 +288,9 @@ class LaneContext:
                prev_valid: np.ndarray, smoothing: float, one_minus: float, fmt: int = INPUT_BGR,
                src_hw=None) -> np.ndarray:
         """frames: int device pointer (on_device) or C-contiguous uint8 ndarray in layout ``fmt`` (INPUT_*) at size
-        ``src_hw`` = (h, w) (None: the context's) -- BGR [n,h,w,3], the decoder layouts [n,h*3/2,w] or Bayer [n,h,w].  Frames of
-        another layout or size become the context's BGR frames on the device first (lane_detect_batch_ingest).
+        ``src_hw`` = (h, w) (None: the context's) -- BGR [n,h,w,3], the decoder layouts [n,h*3/2,w], Bayer [n,h,w] or
+        YUV 4:2:2 [n,h,w,2].  Frames of another layout or size become the context's BGR frames on the device first
+        (lane_detect_batch_ingest).
         prev_fit float64[S,2,3] and prev_valid uint8[S,2] are updated in place.  Returns a RECORD_DTYPE array of n
         records (a copy)."""
         L = lib()

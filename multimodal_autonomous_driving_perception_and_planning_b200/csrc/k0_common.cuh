@@ -1,6 +1,6 @@
 // Shared pieces of the frame-ingest kernels (K0): the YUV 4:2:0 -> BGR arithmetic of k0_nv12.cu / k0_ingest.cu, its
-// inverse for the egress kernel (k8_egress.cu), the Bayer demosaic of k0_ingest.cu and the INTER_LINEAR tap tables and
-// vertical step of k0_resize.cu.
+// inverse for the egress kernel (k8_egress.cu), the packed 4:2:2 addressing and the Bayer demosaic of k0_ingest.cu and
+// the INTER_LINEAR tap tables and vertical step of k0_resize.cu.
 #pragma once
 #include "lane_common.cuh"
 
@@ -132,6 +132,55 @@ __device__ __forceinline__ void k0_yuv420_resize_px(const uint8_t *__restrict__ 
     }
 }
 
+// ---- packed YUV 4:2:2 -> BGR, bit-exact with cv2.cvtColor(f, COLOR_YUV2BGR_UYVY / COLOR_YUV2BGR_YUY2) (oracle/yuv422.py)
+// The per-pixel arithmetic of NV12 (k0yuv::px / uv_terms); each horizontal pixel pair shares the (U, V) of its 4-byte
+// group, nothing is shared vertically.  Within a group UYVY stores U Y0 V Y1 and YUYV Y0 U Y1 V: with yo the offset of
+// Y0 (1 for UYVY, 0 for YUYV), Y of pixel x is byte 2x + yo of its row, U byte (x & ~1) * 2 + 1 - yo and V the byte two
+// after U.
+__host__ __device__ constexpr bool lane_input_yuv422(int format)
+{
+    return format == LANE_INPUT_UYVY || format == LANE_INPUT_YUYV;
+}
+
+// yo of a LANE_INPUT_UYVY / YUYV layout: the byte offset of Y0 in each 4-byte group.
+__host__ __device__ constexpr int lane_yuv422_y0(int format) { return format == LANE_INPUT_UYVY ? 1 : 0; }
+
+// BGR of pixel x of a 4:2:2 row whose Y bytes are ly[2x] and whose pair (U, V) bytes are lc[(x & ~1) * 2] and two after.
+__device__ __forceinline__ void k0_yuv422_px(const uint8_t *__restrict__ ly, const uint8_t *__restrict__ lc, int x,
+                                             uint32_t (&p)[3])
+{
+    const uint8_t *c = lc + (x & ~1) * 2;
+    k0yuv::px(__ldg(ly + 2 * x), k0yuv::uv_terms(__ldg(c), __ldg(c + 2)), p[0], p[1], p[2]);
+}
+
+// The same resize of the BGR frame cv2.cvtColor makes of packed 4:2:2 frame `s` (sw pixels wide, Y0 at byte offset yo
+// of each group): the two source rows x two source columns of every tap are converted on the fly, the converted frame
+// is never stored.  At identity taps this is cv2.cvtColor's frame itself.
+template <int PX>
+__device__ __forceinline__ void k0_yuv422_resize_px(const uint8_t *__restrict__ s, int sw, int yo, int2 yy, short2 b,
+                                                    const int *__restrict__ xofs, const short2 *__restrict__ alpha, int dx0,
+                                                    int dw, uint8_t (&o)[PX * 3])
+{
+    const uint8_t *l0 = s + (size_t)yy.x * sw * 2, *l1 = s + (size_t)yy.y * sw * 2;
+#pragma unroll
+    for (int k = 0; k < PX; k++) {
+        const int dx = min(dx0 + k, dw - 1);
+        const int x0 = __ldg(xofs + dx), x1 = min(x0 + 1, sw - 1);
+        const short2 a = __ldg(alpha + dx);
+        uint32_t p00[3], p01[3], p10[3], p11[3];     // BGR of (row y0 | y1) x (column x0 | x1)
+        k0_yuv422_px(l0 + yo, l0 + 1 - yo, x0, p00);
+        k0_yuv422_px(l0 + yo, l0 + 1 - yo, x1, p01);
+        k0_yuv422_px(l1 + yo, l1 + 1 - yo, x0, p10);
+        k0_yuv422_px(l1 + yo, l1 + 1 - yo, x1, p11);
+#pragma unroll
+        for (int c = 0; c < 3; c++) {
+            const int h0 = (int)p00[c] * a.x + (int)p01[c] * a.y;
+            const int h1 = (int)p10[c] * a.x + (int)p11[c] * a.y;
+            o[k * 3 + c] = (uint8_t)k0_vmix(h0, h1, b.x, b.y);
+        }
+    }
+}
+
 // ---- raw Bayer -> BGR, bit-exact with cv2.cvtColor(f, COLOR_Bayer{RGGB,BGGR,GRBG,GBRG}2BGR) (oracle/bayer.py) -------
 // The bilinear demosaic.  Pixel (y, x) of an H x W mosaic (H, W >= 3) is the interior formula at (clamp(y, 1, H-2),
 // clamp(x, 1, W-2)): its own colour is the raw value; at an R or B site G = (4 neighbours + 2) >> 2 and the other chroma
@@ -243,12 +292,15 @@ void launch_resize(const uint8_t *src, uint8_t *dst, int n, int channels, int sh
 
 // k0_nv12: YUV 4:2:0 -> BGR at the source size
 void launch_yuv420_to_bgr(const uint8_t *src, int format, uint8_t *dst, int n, int H, int W, cudaStream_t st);
+// k0_nv12: packed YUV 4:2:2 (LANE_INPUT_UYVY / YUYV) -> BGR at the source size (W even)
+void launch_yuv422_to_bgr(const uint8_t *src, int format, uint8_t *dst, int n, int H, int W, cudaStream_t st);
 
 // ---- ingest: any LANE_INPUT_* layout at any size -> BGR at dh x dw --------------------------------------------------
-// NV12 / I420 at the destination size: k0_nv12's conversion kernels; NV12 / I420 at another size: the fused
-// conversion + resize kernel (k0_ingest.cu); Bayer at any size: the fused demosaic + resize kernel (identity taps at its
+// NV12 / I420 / UYVY / YUYV at the destination size: k0_nv12's conversion kernels; at another size: the fused
+// conversion + resize kernels (k0_ingest.cu); Bayer at any size: the fused demosaic + resize kernel (identity taps at its
 // own size); BGR at another size: k0_resize.  BGR at its own size needs no kernel and is not taken.  Device pointers,
-// enqueued on st; the caller has validated the sizes (even YUV sizes, Bayer sizes >= 3, grid limits).
+// enqueued on st; the caller has validated the sizes (even 4:2:0 sizes, Bayer sizes >= 3, even 4:2:2 widths, grid
+// limits).
 cudaError_t launch_ingest(const uint8_t *src, int format, int n, int sh, int sw, uint8_t *dst, int dh, int dw,
                           cudaStream_t st);
 
@@ -256,7 +308,7 @@ cudaError_t launch_ingest(const uint8_t *src, int format, int n, int sh, int sw,
 // Descriptor of one source frame (device memory, dense); the tap tables are lane_resize_taps' cached ones.
 struct RigFrame {
     const uint8_t *src;
-    int format, sh, sw;                // LANE_INPUT_*; YUV sizes even, Bayer sizes >= 3
+    int format, sh, sw;                // LANE_INPUT_*; 4:2:0 sizes even, Bayer sizes >= 3, 4:2:2 widths even
     const int *xofs;
     const short2 *alpha;
     const int2 *yofs;

@@ -13,6 +13,11 @@
 //     cv2.resize(cv2.cvtColor(src, COLOR_Bayer{RGGB,BGGR,GRBG,GBRG}2BGR), (dw, dh))      (INTER_LINEAR)
 // with the two source rows x two source columns of every tap demosaiced from their 4x4 raw neighbourhood
 // (k0_bayer_resize_px).  A frame at the destination size runs on identity taps: the demosaic alone.
+//
+// K0f: packed YUV 4:2:2 camera frames (UYVY / YUYV, 2 B/px) the same way as K0c: per destination pixel
+//     cv2.resize(cv2.cvtColor(src, COLOR_YUV2BGR_UYVY | COLOR_YUV2BGR_YUY2), (dw, dh))      (INTER_LINEAR)
+// with the two source rows x two source columns of every tap converted from their Y and their pair's (U, V)
+// (k0_yuv422_resize_px).  At the destination size launch_ingest takes k0_nv12.cu's conversion kernels instead.
 #include "host_stage.h"
 #include "k0_common.cuh"
 
@@ -58,13 +63,32 @@ __global__ void __launch_bounds__(256) k0_bayer_resize(const uint8_t *__restrict
     k0_store_px<3, PX>(out, o, dx0, dw);
 }
 
+// k0_yuv420_resize for packed 4:2:2 frames whose Y0 sits at byte YO of each 4-byte group (lane_yuv422_y0).
+template <int YO, int PX>
+__global__ void __launch_bounds__(256) k0_yuv422_resize(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst,
+                                                        const int *__restrict__ xofs, const short2 *__restrict__ alpha,
+                                                        const int2 *__restrict__ yofs, const short2 *__restrict__ beta,
+                                                        int sh, int sw, int dh, int dw)
+{
+    const int dx0 = (blockIdx.x * blockDim.x + threadIdx.x) * PX, dy = blockIdx.y, f = blockIdx.z;
+    if (dx0 >= dw) return;
+    const int2 yy = __ldg(yofs + dy);
+    const short2 b = __ldg(beta + dy);
+    const uint8_t *s = src + (size_t)f * sh * sw * 2;
+    uint8_t *out = dst + (((size_t)f * dh + dy) * dw + dx0) * 3;
+    uint8_t o[PX * 3];
+    k0_yuv422_resize_px<PX>(s, sw, YO, yy, b, xofs, alpha, dx0, dw, o);
+    k0_store_px<3, PX>(out, o, dx0, dw);
+}
+
 // The frames of a rig: every frame has its own descriptor (layout, size, tap tables), so cameras of different
 // resolutions and decoders share one launch.  The grid is k0_yuv420_resize's; a block reads its frame's descriptor
 // once, and the branch on the layout is uniform over the block.  A frame already at dh x dw runs on identity taps,
 // which reproduce the source (BGR) or cv2.cvtColor's frame (YUV, Bayer) exactly.
 //
-// The Bayer and the BGR / YUV pixel work are separate functions kept out of line: inlined side by side they need 60
-// registers, which would drop the kernel from 5 to 4 blocks per SM; apart, each fits the kernel's 48.
+// The Bayer, the packed 4:2:2 and the BGR / YUV 4:2:0 pixel work are separate functions kept out of line: inlined side
+// by side the first and the last need 60 registers, which would drop the kernel from 5 to 4 blocks per SM; apart, each
+// fits the kernel's 48.
 template <int PX>
 __device__ __noinline__ void rig_bgr_yuv420(const RigFrame &d, int2 yy, short2 b, int dx0, int dw, uint8_t *out)
 {
@@ -88,6 +112,19 @@ __device__ __noinline__ void rig_bayer(const RigFrame &d, int2 yy, short2 b, int
     k0_store_px<3, PX>(out, o, dx0, dw);
 }
 
+// The frame's layout picks a constant Y0 offset: with the offset a run-time value in the addresses the branch needs 64
+// registers.
+template <int PX>
+__device__ __noinline__ void rig_yuv422(const RigFrame &d, int2 yy, short2 b, int dx0, int dw, uint8_t *out)
+{
+    uint8_t o[PX * 3];
+    if (lane_yuv422_y0(d.format))
+        k0_yuv422_resize_px<PX>(d.src, d.sw, 1, yy, b, d.xofs, d.alpha, dx0, dw, o);
+    else
+        k0_yuv422_resize_px<PX>(d.src, d.sw, 0, yy, b, d.xofs, d.alpha, dx0, dw, o);
+    k0_store_px<3, PX>(out, o, dx0, dw);
+}
+
 template <int PX>
 __global__ void __launch_bounds__(256) k0_rig_ingest(const RigFrame *__restrict__ frames, uint8_t *__restrict__ dst, int dh,
                                                      int dw)
@@ -102,6 +139,8 @@ __global__ void __launch_bounds__(256) k0_rig_ingest(const RigFrame *__restrict_
     uint8_t *out = dst + (((size_t)f * dh + dy) * dw + dx0) * 3;
     if (lane_input_bayer(d.format))
         rig_bayer<PX>(d, yy, b, dx0, dw, out);
+    else if (lane_input_yuv422(d.format))
+        rig_yuv422<PX>(d, yy, b, dx0, dw, out);
     else
         rig_bgr_yuv420<PX>(d, yy, b, dx0, dw, out);
 }
@@ -132,6 +171,10 @@ cudaError_t launch_ingest(const uint8_t *src, int format, int n, int sh, int sw,
         launch_yuv420_to_bgr(src, format, dst, n, sh, sw, st);
         return cudaGetLastError();
     }
+    if (lane_input_yuv422(format) && sh == dh && sw == dw) {
+        launch_yuv422_to_bgr(src, format, dst, n, sh, sw, st);
+        return cudaGetLastError();
+    }
     ResizeTaps t;
     cudaError_t e = lane_resize_taps(sh, sw, dh, dw, &t);
     if (e) return e;
@@ -144,6 +187,10 @@ cudaError_t launch_ingest(const uint8_t *src, int format, int n, int sh, int sw,
     if (lane_input_bayer(format))
         k0_bayer_resize<PX><<<grid, 256, 0, st>>>(src, dst, t.xofs, t.alpha, t.yofs, t.beta, lane_bayer_phase(format), sh, sw,
                                                   dh, dw);
+    else if (format == LANE_INPUT_UYVY)
+        k0_yuv422_resize<1, PX><<<grid, 256, 0, st>>>(src, dst, t.xofs, t.alpha, t.yofs, t.beta, sh, sw, dh, dw);
+    else if (format == LANE_INPUT_YUYV)
+        k0_yuv422_resize<0, PX><<<grid, 256, 0, st>>>(src, dst, t.xofs, t.alpha, t.yofs, t.beta, sh, sw, dh, dw);
     else if (format == LANE_INPUT_I420)
         k0_yuv420_resize<LANE_INPUT_I420, PX><<<grid, 256, 0, st>>>(src, dst, t.xofs, t.alpha, t.yofs, t.beta, sh, sw, dh, dw);
     else
@@ -201,6 +248,29 @@ extern "C" int lane_bayer_to_bgr_batch(const uint8_t *src, int format, int n, in
     };
     if (on_device) return launch(src, dst);
     return lane_host_round_trip(who, device, st, src, (size_t)n * src_h * src_w, dst, (size_t)n * dst_h * dst_w * 3, launch);
+}
+
+extern "C" int lane_yuv422_to_bgr_batch(const uint8_t *src, int format, int n, int src_h, int src_w, uint8_t *dst,
+                                        int dst_h, int dst_w, int on_device, int device, void *cuda_stream)
+{
+    const char *who = "lane_yuv422_to_bgr_batch";
+    if (!src || !dst || n < 1 || src_h < 1 || src_w < 1 || dst_h < 1 || dst_w < 1)
+        return lane_api_fail(LANE_ERR_INVALID, who, "bad arguments (non-null pointers, positive sizes)");
+    if (!lane_input_yuv422(format))
+        return lane_api_fail(LANE_ERR_INVALID, who, "format must be LANE_INPUT_UYVY or LANE_INPUT_YUYV");
+    if (src_w & 1) return lane_api_fail(LANE_ERR_INVALID, who, "YUV 4:2:2 needs an even width");
+    const bool resize = dst_h != src_h || dst_w != src_w;
+    if (resize && (dst_h > 65535 || n > 65535))
+        return lane_api_fail(LANE_ERR_UNSUPPORTED, who, "destination height / batch above 65535");
+    if (int rc = lane_api_device(who, device)) return rc;
+    cudaStream_t st = (cudaStream_t)cuda_stream;
+    auto launch = [&](const uint8_t *s, uint8_t *d) {
+        const cudaError_t e = launch_ingest(s, format, n, src_h, src_w, d, dst_h, dst_w, st);
+        return e ? lane_api_fail(LANE_ERR_CUDA, who, "launch", e) : LANE_OK;
+    };
+    if (on_device) return launch(src, dst);
+    return lane_host_round_trip(who, device, st, src, (size_t)n * src_h * src_w * 2, dst, (size_t)n * dst_h * dst_w * 3,
+                                launch);
 }
 
 extern "C" int lane_nv12_to_bgr_batch(const uint8_t *src, int n, int height, int width, uint8_t *dst, int on_device,

@@ -13,6 +13,11 @@
 // HBM-bound: 1.5 B/px read + 3 B/px written.  A thread converts a 2 x 8 pixel block: one 8-byte load per luma row,
 // one 8-byte load of the four (U, V) pairs the block shares, three 8-byte stores per output row; a warp covers
 // 256 px of two rows, so every access is a full, aligned segment.
+//
+// K0f at the source size: packed YUV 4:2:2 (UYVY / YUYV, 2 B/px) -> BGR with the same arithmetic.  Nothing is shared
+// between rows, so a batch of dense frames is one run of pixel pairs: a thread converts 8 pixels with one 16-byte load,
+// PRMT splits it into the 8 Y bytes and the 4 (U, V) pairs, and row8 makes the 24 BGR bytes (three 8-byte stores).
+// 2 B/px read + 3 B/px written.
 #include <algorithm>
 
 #include "k0_common.cuh"
@@ -107,6 +112,57 @@ __global__ void __launch_bounds__(256) k0_nv12_generic(const uint8_t *__restrict
     }
 }
 
+// PRMT selectors of a 16-byte 4:2:2 group of 8 pixels (words w0..w3, little-endian) by Y0 offset YO: the Y bytes of
+// words (w0, w1) / (w2, w3), and the (U, V) bytes of one word pair as U0 V0 U1 V1.
+template <int YO> constexpr uint32_t Y_SEL = YO ? 0x7531u : 0x6420u;
+template <int YO> constexpr uint32_t UV_SEL = YO ? 0x6420u : 0x7531u;
+
+// 8 pixels of one 4:2:2 row (16 source bytes) -> 24 BGR bytes at d (8-byte aligned)
+template <int YO>
+__device__ __forceinline__ void yuv422_8px(uint4 w, uint2 *__restrict__ d)
+{
+    const uint2 yy = make_uint2(__byte_perm(w.x, w.y, Y_SEL<YO>), __byte_perm(w.z, w.w, Y_SEL<YO>));
+    const uint32_t uv01 = __byte_perm(w.x, w.y, UV_SEL<YO>), uv23 = __byte_perm(w.z, w.w, UV_SEL<YO>);
+    UV t[4];
+    t[0] = uv_terms((int)(uv01 & 0xFFu), (int)((uv01 >> 8) & 0xFFu));
+    t[1] = uv_terms((int)((uv01 >> 16) & 0xFFu), (int)(uv01 >> 24));
+    t[2] = uv_terms((int)(uv23 & 0xFFu), (int)((uv23 >> 8) & 0xFFu));
+    t[3] = uv_terms((int)((uv23 >> 16) & 0xFFu), (int)(uv23 >> 24));
+    uint32_t o[6];
+    row8(yy, t, o);
+    d[0] = make_uint2(o[0], o[1]); d[1] = make_uint2(o[2], o[3]); d[2] = make_uint2(o[4], o[5]);
+}
+
+// W % 8 == 0, 16-byte aligned source, 8-byte aligned destination: one thread = 8 pixels of one row
+template <int YO>
+__global__ void __launch_bounds__(256) k0_yuv422_vec(const uint4 *__restrict__ src, uint2 *__restrict__ dst, long long groups)
+{
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < groups; i += (long long)gridDim.x * blockDim.x)
+        yuv422_8px<YO>(__ldg(src + i), dst + 3 * i);
+}
+
+// any even W and alignment: one thread per pixel pair (4 source bytes, 6 destination bytes)
+__global__ void __launch_bounds__(256) k0_yuv422_generic(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst, int yo,
+                                                         long long pairs)
+{
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < pairs; i += (long long)gridDim.x * blockDim.x) {
+        const uint8_t *g = src + 4 * i;
+        const UV t = uv_terms(__ldg(g + 1 - yo), __ldg(g + 3 - yo));
+        uint8_t *d = dst + 6 * i;
+#pragma unroll
+        for (int k = 0; k < 2; k++) {
+            uint32_t b, gr, r;
+            px(__ldg(g + yo + 2 * k), t, b, gr, r);
+            d[3 * k] = (uint8_t)b; d[3 * k + 1] = (uint8_t)gr; d[3 * k + 2] = (uint8_t)r;
+        }
+    }
+}
+
+int grid_for(long long threads)
+{
+    return (int)std::max<long long>(1, std::min<long long>((threads + 255) / 256, (long long)lane_sm_count() * 16));
+}
+
 template <int FMT>
 void launch_fmt(const uint8_t *src, uint8_t *dst, int n, int H, int W, cudaStream_t st)
 {
@@ -131,4 +187,20 @@ void launch_yuv420_to_bgr(const uint8_t *src, int format, uint8_t *dst, int n, i
         launch_fmt<LANE_INPUT_I420>(src, dst, n, H, W, st);
     else
         launch_fmt<LANE_INPUT_NV12>(src, dst, n, H, W, st);
+}
+
+// packed YUV 4:2:2 (LANE_INPUT_UYVY / LANE_INPUT_YUYV) -> BGR at the same size (W even); device pointers, enqueued on st
+void launch_yuv422_to_bgr(const uint8_t *src, int format, uint8_t *dst, int n, int H, int W, cudaStream_t st)
+{
+    const long long px = (long long)n * H * W;
+    if (W % 8 == 0 && (uintptr_t)src % 16 == 0 && (uintptr_t)dst % 8 == 0) {
+        const auto *s = reinterpret_cast<const uint4 *>(src);
+        auto *d = reinterpret_cast<uint2 *>(dst);
+        if (format == LANE_INPUT_UYVY)
+            k0_yuv422_vec<1><<<grid_for(px / 8), 256, 0, st>>>(s, d, px / 8);
+        else
+            k0_yuv422_vec<0><<<grid_for(px / 8), 256, 0, st>>>(s, d, px / 8);
+    } else {
+        k0_yuv422_generic<<<grid_for(px / 2), 256, 0, st>>>(src, dst, lane_yuv422_y0(format), px / 2);
+    }
 }

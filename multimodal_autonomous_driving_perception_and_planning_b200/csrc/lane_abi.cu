@@ -430,11 +430,13 @@ int end_batch(lane_ctx *c, bool on_device, int n, int S, const uint8_t *frames_d
     return LANE_OK;
 }
 
-// Bytes of one dense frame of a source: its own size and layout (3 B/px BGR, 1.5 B/px YUV 4:2:0, 1 B/px Bayer).
+// Bytes of one dense frame of a source: its own size and layout (3 B/px BGR, 1.5 B/px YUV 4:2:0, 1 B/px Bayer,
+// 2 B/px YUV 4:2:2).
 size_t frame_bytes(const lane_rig_source &r)
 {
     const size_t px = (size_t)r.src_h * r.src_w;
-    return r.format == LANE_INPUT_BGR ? px * 3 : lane_input_bayer(r.format) ? px : px * 3 / 2;
+    return r.format == LANE_INPUT_BGR ? px * 3 : lane_input_bayer(r.format) ? px : lane_input_yuv422(r.format) ? px * 2
+                                                                                                               : px * 3 / 2;
 }
 
 // How the context's H x W BGR frames are made from the batch's sources before the path runs (k0_common.cuh): they
@@ -524,20 +526,22 @@ int enqueue(lane_ctx *c, const lane_rig_source *sources, int n_sources, bool on_
     return end_batch(c, whole, n, S, frames_dev);
 }
 
-// One source's fields: layout, size (even for YUV 4:2:0, at least 3 x 3 for Bayer) and frames.  `s` numbers it in the
-// message; < 0: the call's only source.
+// One source's fields: layout, size (even for YUV 4:2:0, at least 3 x 3 for Bayer, an even width for YUV 4:2:2) and
+// frames.  `s` numbers it in the message; < 0: the call's only source.
 int check_source(lane_ctx *c, int s, const lane_rig_source &r)
 {
     char who[32] = "";
     if (s >= 0) snprintf(who, sizeof(who), "source %d: ", s);
     const bool yuv = r.format == LANE_INPUT_NV12 || r.format == LANE_INPUT_I420;
-    if (r.format != LANE_INPUT_BGR && !yuv && !lane_input_bayer(r.format))
+    if (r.format != LANE_INPUT_BGR && !yuv && !lane_input_bayer(r.format) && !lane_input_yuv422(r.format))
         return fail(c, LANE_ERR_INVALID, "%sunknown input format %d", who, r.format);
     if (r.src_h < 1 || r.src_w < 1) return fail(c, LANE_ERR_INVALID, "%sbad source size %dx%d", who, r.src_w, r.src_h);
     if (yuv && ((r.src_h | r.src_w) & 1))
         return fail(c, LANE_ERR_INVALID, "%sNV12 / I420 needs even width and height (%dx%d)", who, r.src_w, r.src_h);
     if (lane_input_bayer(r.format) && (r.src_h < 3 || r.src_w < 3))
         return fail(c, LANE_ERR_INVALID, "%sa Bayer frame needs at least 3 rows and 3 columns (%dx%d)", who, r.src_w, r.src_h);
+    if (lane_input_yuv422(r.format) && (r.src_w & 1))
+        return fail(c, LANE_ERR_INVALID, "%sUYVY / YUYV needs an even width (%dx%d)", who, r.src_w, r.src_h);
     if (r.n && !r.frames) return fail(c, LANE_ERR_INVALID, "%sframes is null", who);
     return LANE_OK;
 }

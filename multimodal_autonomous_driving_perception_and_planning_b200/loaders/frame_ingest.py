@@ -98,9 +98,21 @@ class FrameIngest:
         dw, dh = (w, h) if self.target_size is None else self.target_size
         return self._convert(_native.lib().lane_bayer_to_bgr_batch, frames, fmt, n, h, w, dh, dw)
 
+    def from_yuv422(self, frames, order: str):
+        """Packed 4:2:2 camera frames -> BGR: ``frames`` uint8 ``[N, H, W, 2]`` (numpy or CUDA tensor, W even) in byte
+        order ``order`` ("uyvy": U Y0 V Y1, what GMSL / FPD-Link cameras deliver; "yuyv": Y0 U Y1 V, a V4L2 USB camera's
+        default) become ``[N, H, W, 3]``, equal to ``cv2.cvtColor(f, cv2.COLOR_YUV2BGR_UYVY | COLOR_YUV2BGR_YUY2)`` per
+        frame, followed by the resize when ``target_size`` is set.  Conversion and resize are one kernel: the
+        full-resolution BGR frame is never stored."""
+        fmt = yuv422_format(order)
+        check_yuv422(frames, "FrameIngest")
+        n, h, w = (int(x) for x in frames.shape[:3])
+        dw, dh = (w, h) if self.target_size is None else self.target_size
+        return self._convert(_native.lib().lane_yuv422_to_bgr_batch, frames, fmt, n, h, w, dh, dw)
+
     def _convert(self, entry, frames, fmt, n, h, w, dh, dw):
-        """One context-free conversion entry (``lane_yuv420_to_bgr_batch`` / ``lane_bayer_to_bgr_batch``): numpy in,
-        numpy out; CUDA tensor in, CUDA tensor out on torch's current stream."""
+        """One context-free conversion entry (``lane_yuv420_to_bgr_batch`` / ``lane_bayer_to_bgr_batch`` /
+        ``lane_yuv422_to_bgr_batch``): numpy in, numpy out; CUDA tensor in, CUDA tensor out on torch's current stream."""
         if isinstance(frames, np.ndarray):
             src = np.ascontiguousarray(frames)
             dst = np.empty((n, dh, dw, 3), np.uint8)
@@ -145,6 +157,22 @@ def check_bayer(frames, who: str):
     shape = tuple(frames.shape)
     if len(shape) != 3 or shape[1] < 3 or shape[2] < 3:
         raise cv2.error(f"{who}: expected Bayer frames [N, H, W] with H, W >= 3, got {shape}")
+    if str(frames.dtype).replace("torch.", "") != "uint8":
+        raise cv2.error(f"{who}: expected uint8 frames, got {frames.dtype}")
+
+
+def yuv422_format(order) -> int:
+    """LANE_INPUT_UYVY / LANE_INPUT_YUYV of a byte order name ("uyvy", "yuyv"), else ``ValueError``."""
+    if not isinstance(order, str) or order not in _native.YUV422:
+        raise ValueError(f"YUV 4:2:2 order {order!r} is not one of {sorted(_native.YUV422)}")
+    return _native.YUV422[order]
+
+
+def check_yuv422(frames, who: str):
+    """uint8 ``[N, H, W, 2]`` with even W (packed UYVY / YUYV), else ``cv2.error`` (what cv2.cvtColor raises)."""
+    shape = tuple(frames.shape)
+    if len(shape) != 4 or shape[3] != 2 or shape[2] % 2:
+        raise cv2.error(f"{who}: expected YUV 4:2:2 frames [N, H, W, 2] with even W, got {shape}")
     if str(frames.dtype).replace("torch.", "") != "uint8":
         raise cv2.error(f"{who}: expected uint8 frames, got {frames.dtype}")
 

@@ -20,7 +20,8 @@ import cv2
 import numpy as np
 
 from .. import _native
-from ..loaders.frame_ingest import bayer_format, check_bayer, check_target_size, check_yuv420
+from ..loaders.frame_ingest import (bayer_format, check_bayer, check_target_size, check_yuv420, check_yuv422,
+                                    yuv422_format)
 
 
 @dataclass
@@ -35,8 +36,9 @@ class LaneLine:
 LanePair = Tuple[Optional[LaneLine], Optional[LaneLine]]
 _SIDES = ("left", "right")
 _LAYOUTS = {"bgr": _native.INPUT_BGR, "nv12": _native.INPUT_NV12, "i420": _native.INPUT_I420,
-            **{"bayer_" + p: fmt for p, fmt in _native.BAYER.items()}}
+            **{"bayer_" + p: fmt for p, fmt in _native.BAYER.items()}, **_native.YUV422}
 _BAYER_FORMATS = frozenset(_native.BAYER.values())
+_YUV422_FORMATS = frozenset(_native.YUV422.values())
 _COPY_PIECE = 4 << 20         # bytes per host thread task when detect_rig_stream copies a numpy tick into pinned memory
 
 
@@ -52,8 +54,13 @@ def _is_pinned_tensor(x) -> bool:
 
 
 def _frame_bytes(fmt: int, h: int, w: int) -> int:
-    """Bytes of one h x w frame in layout ``fmt`` (INPUT_*): 3 B/px BGR, 1.5 B/px YUV 4:2:0, 1 B/px Bayer."""
-    return h * w * 3 if fmt == _native.INPUT_BGR else h * w if fmt in _BAYER_FORMATS else h * w * 3 // 2
+    """Bytes of one h x w frame in layout ``fmt`` (INPUT_*): 3 B/px BGR, 1.5 B/px YUV 4:2:0, 1 B/px Bayer, 2 B/px
+    YUV 4:2:2."""
+    if fmt == _native.INPUT_BGR:
+        return h * w * 3
+    if fmt in _BAYER_FORMATS:
+        return h * w
+    return h * w * 2 if fmt in _YUV422_FORMATS else h * w * 3 // 2
 
 
 def _two_deep(items, plan, start, joins, enqueue, blocking, restore, adopt):
@@ -147,10 +154,11 @@ class _Plan:
 
     @classmethod
     def of_frames(cls, frames, fmt: int, target_size=None, frame_sids=None, stream_rois=None) -> "_Plan":
-        """One checked array of frames: [N,H,W,3] BGR, [N,H*3/2,W] for the YUV 4:2:0 layouts or [N,H,W] for the Bayer
-        layouts of ``fmt``, detected at ``target_size`` = (width, height) when given."""
+        """One checked array of frames: [N,H,W,3] BGR, [N,H*3/2,W] for the YUV 4:2:0 layouts, [N,H,W] for the Bayer
+        layouts or [N,H,W,2] for the YUV 4:2:2 layouts of ``fmt``, detected at ``target_size`` = (width, height) when
+        given."""
         n, sh, sw = (int(x) for x in frames.shape[:3])
-        if fmt not in (_native.INPUT_BGR, *_BAYER_FORMATS):
+        if fmt not in (_native.INPUT_BGR, *_BAYER_FORMATS, *_YUV422_FORMATS):
             sh = sh * 2 // 3
         h, w = (sh, sw) if target_size is None else (target_size[1], target_size[0])
         kind = ("cuda", frames.device.index) if _is_torch_cuda(frames) else "host"
@@ -536,6 +544,16 @@ class LaneDetector:
         check_bayer(frames, "LaneDetector")
         return self._detect_frames(frames, fmt, target_size)
 
+    def detect_batch_yuv422(self, frames, order: str, *, target_size: Optional[Tuple[int, int]] = None) -> List[LanePair]:
+        """``detect_batch`` for packed YUV 4:2:2 camera frames: uint8 ``[N, H, W, 2]`` (numpy or CUDA tensor, W even) in
+        byte order ``order`` ("uyvy": U Y0 V Y1, GMSL / FPD-Link cameras; "yuyv": Y0 U Y1 V, V4L2 USB cameras; no
+        default).  Equal to ``detect_batch`` of ``cv2.cvtColor(f, cv2.COLOR_YUV2BGR_UYVY | COLOR_YUV2BGR_YUY2)`` of every
+        frame, resized to ``target_size`` = (width, height) when given, with the same ``prev_*_fit`` after it.
+        Conversion and resize are one kernel on the device, so a host batch moves 2 B/px over PCIe instead of 3."""
+        fmt = yuv422_format(order)
+        check_yuv422(frames, "LaneDetector")
+        return self._detect_frames(frames, fmt, target_size)
+
     def detect_streams(self, frames, stream_ids: Optional[Sequence[int]] = None, *,
                        stream_rois: Optional[Sequence[Optional[np.ndarray]]] = None) -> List[LanePair]:
         """Multi-camera form: ``frames`` is [S,T,H,W,3] (stream-major) or [N,H,W,3] with ``stream_ids[N]``.
@@ -585,8 +603,9 @@ class LaneDetector:
         """A rig of cameras that differ in resolution and decoder layout, in one batched call.
 
         ``frames[s]`` is camera s (= stream s of ``detect_streams``): uint8 ``[T_s, H_s, W_s, 3]`` BGR,
-        ``[T_s, H_s*3/2, W_s]`` NV12 / I420 or ``[T_s, H_s, W_s]`` raw Bayer, as ``layouts[s]`` ("bgr", "nv12", "i420",
-        "bayer_rggb", "bayer_bggr", "bayer_grbg", "bayer_gbrg"; default all "bgr") says, its frames in temporal order.  ``T_s`` may differ between cameras and may be 0, or the entry None: no frame this tick.  Every
+        ``[T_s, H_s*3/2, W_s]`` NV12 / I420, ``[T_s, H_s, W_s]`` raw Bayer or ``[T_s, H_s, W_s, 2]`` packed YUV 4:2:2, as
+        ``layouts[s]`` ("bgr", "nv12", "i420", "bayer_rggb", "bayer_bggr", "bayer_grbg", "bayer_gbrg", "uyvy", "yuyv";
+        default all "bgr") says, its frames in temporal order.  ``T_s`` may differ between cameras and may be 0, or the entry None: no frame this tick.  Every
         camera is a numpy array, or every camera is a CUDA tensor on one device.  Every frame is detected at
         ``target_size`` = (width, height), which may be left out only when all cameras share one size; the device converts
         and resizes all frames in one kernel (only the source bytes of host frames cross PCIe) and runs the rest of the
@@ -594,8 +613,9 @@ class LaneDetector:
 
         Returns one list of pairs per camera.  Camera s's pairs equal those of a fresh
         ``LaneDetector(roi_vertices=stream_rois[s])`` given its frames through ``detect_batch`` / ``detect_batch_nv12`` /
-        ``detect_batch_i420(frames[s], target_size=target_size)`` / ``detect_batch_bayer``; its smoothing state is stream s's of ``detect_streams``,
-        so it carries across calls of either kind (``reset`` clears it).
+        ``detect_batch_i420(frames[s], target_size=target_size)`` / ``detect_batch_bayer`` / ``detect_batch_yuv422``; its
+        smoothing state is stream s's of ``detect_streams``, so it carries across calls of either kind (``reset`` clears
+        it).
         """
         return self._detect_rig(self._rig_plan(frames, layouts, target_size, stream_rois))
 
@@ -722,6 +742,12 @@ class LaneDetector:
             h, w = shape[1], shape[2]
             if h < 3 or w < 3:
                 raise ValueError(f"camera {s}: {layout} needs at least 3 rows and 3 columns, got {w}x{h}")
+        elif layout in _native.YUV422:
+            if len(shape) != 4 or shape[-1] != 2:
+                raise ValueError(f"camera {s}: layout {layout!r} needs frames [T,H,W,2], got {shape}")
+            h, w = shape[1], shape[2]
+            if w % 2:
+                raise ValueError(f"camera {s}: {layout} needs an even width, got {w}x{h}")
         else:
             if len(shape) != 3 or shape[1] % 3:
                 raise ValueError(f"camera {s}: layout {layout!r} needs frames [T,H*3/2,W], got {shape}")
