@@ -80,7 +80,7 @@ __device__ __forceinline__ uint32_t k0_vmix(int h0, int h1, int b0, int b1)
     return (uint32_t)min(v, 255);
 }
 
-// The per-thread pixel work of the resize kernels (k0_resize, k0_yuv420_resize, k0_bayer_resize, k0_rig_ingest): one
+// The per-thread pixel work of the resize kernels (k0_resize, k0_ingest_resize, k0_rig_ingest): one
 // thread makes PX consecutive destination pixels dx0 .. dx0+PX-1 of destination row dy (columns past dw repeat the last
 // one and are not stored).  yy / b: the row's yofs / beta entries.
 //
@@ -197,6 +197,38 @@ __host__ __device__ constexpr int lane_bayer_phase(int format)
     return format == LANE_INPUT_BAYER_RGGB ? 0 : format == LANE_INPUT_BAYER_GRBG ? 1 : format == LANE_INPUT_BAYER_GBRG ? 2 : 3;
 }
 
+// ---- the LANE_INPUT_* layouts: what the host checks, byte counts and kernel choices of every ingest path ask ---------
+// (loaders/frame_layout.py is the Python side's table.)
+__host__ __device__ constexpr bool lane_input_yuv420(int format)
+{
+    return format == LANE_INPUT_NV12 || format == LANE_INPUT_I420;
+}
+
+// Bytes of n dense h x w frames: 3 B/px BGR, 1.5 B/px YUV 4:2:0, 1 B/px Bayer, 2 B/px YUV 4:2:2.
+__host__ __device__ constexpr size_t lane_input_frame_bytes(int format, int h, int w, size_t n = 1)
+{
+    const size_t px = n * h * w;
+    return format == LANE_INPUT_BGR ? px * 3 : lane_input_bayer(format) ? px : lane_input_yuv422(format) ? px * 2 : px * 3 / 2;
+}
+
+// Why h x w frames (h, w >= 1) of `format` cannot be taken, or null: an unknown layout, odd 4:2:0 sizes (the chroma
+// blocks are 2 x 2), Bayer frames below 3 x 3 (cv2.cvtColor makes an all-zero frame of them), odd 4:2:2 widths.
+inline const char *lane_input_refusal(int format, int h, int w)
+{
+    if (lane_input_yuv420(format)) return (h | w) & 1 ? "YUV 4:2:0 needs even width and height" : nullptr;
+    if (lane_input_bayer(format)) return h < 3 || w < 3 ? "a Bayer frame needs at least 3 rows and 3 columns" : nullptr;
+    if (lane_input_yuv422(format)) return w & 1 ? "YUV 4:2:2 needs an even width" : nullptr;
+    return format == LANE_INPUT_BGR ? nullptr : "unknown input format";
+}
+
+// Whether sh x sw frames of `format` become dh x dw BGR on a resizing grid (one block row per destination row, one z
+// per frame: dh and the batch up to 65535): at every other size, and Bayer frames at every size (their demosaic is that
+// kernel on identity taps).  Otherwise BGR needs no kernel and YUV takes k0_nv12's conversion.
+__host__ __device__ constexpr bool lane_input_resizes(int format, int sh, int sw, int dh, int dw)
+{
+    return sh != dh || sw != dw || lane_input_bayer(format);
+}
+
 namespace k0bayer {
 
 // BGR of the centre of the 3x3 window of w at column J (columns J-1..J+1), whose site is at parity (ry, rx) of the RGGB
@@ -297,10 +329,9 @@ void launch_yuv422_to_bgr(const uint8_t *src, int format, uint8_t *dst, int n, i
 
 // ---- ingest: any LANE_INPUT_* layout at any size -> BGR at dh x dw --------------------------------------------------
 // NV12 / I420 / UYVY / YUYV at the destination size: k0_nv12's conversion kernels; at another size: the fused
-// conversion + resize kernels (k0_ingest.cu); Bayer at any size: the fused demosaic + resize kernel (identity taps at its
-// own size); BGR at another size: k0_resize.  BGR at its own size needs no kernel and is not taken.  Device pointers,
-// enqueued on st; the caller has validated the sizes (even 4:2:0 sizes, Bayer sizes >= 3, even 4:2:2 widths, grid
-// limits).
+// conversion + resize kernel (k0_ingest_resize); Bayer at any size: the fused demosaic + resize kernel (identity taps at
+// its own size); BGR at another size: k0_resize.  BGR at its own size needs no kernel and is not taken.  Device pointers,
+// enqueued on st; the caller has validated the sizes (lane_input_refusal) and the grid (lane_input_resizes).
 cudaError_t launch_ingest(const uint8_t *src, int format, int n, int sh, int sw, uint8_t *dst, int dh, int dw,
                           cudaStream_t st);
 
@@ -308,7 +339,7 @@ cudaError_t launch_ingest(const uint8_t *src, int format, int n, int sh, int sw,
 // Descriptor of one source frame (device memory, dense); the tap tables are lane_resize_taps' cached ones.
 struct RigFrame {
     const uint8_t *src;
-    int format, sh, sw;                // LANE_INPUT_*; 4:2:0 sizes even, Bayer sizes >= 3, 4:2:2 widths even
+    int format, sh, sw;                // LANE_INPUT_*, at a size lane_input_refusal takes
     const int *xofs;
     const short2 *alpha;
     const int2 *yofs;

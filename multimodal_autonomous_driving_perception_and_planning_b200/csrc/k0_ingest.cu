@@ -26,63 +26,34 @@ namespace {
 using namespace k0yuv;
 
 // k0_resize's thread shape: one thread = PX consecutive destination pixels of one row, packed 4-byte stores when
-// aligned, byte stores otherwise; a warp covers a contiguous run of the row, so its source reads (two short luma row
-// segments and the chroma rows under them) stay in L1 across the PX pixels.
+// aligned, byte stores otherwise; a warp covers a contiguous run of the row, so its source reads (two short source row
+// segments, and for 4:2:0 the chroma rows under them) stay in L1 across the PX pixels.  FMT: the layout
+// (LANE_INPUT_NV12 / I420 / UYVY / YUYV, or LANE_INPUT_BAYER_RGGB for every Bayer pattern, read at run-time `phase`:
+// lane_bayer_phase).
 template <int FMT, int PX>
-__global__ void __launch_bounds__(256) k0_yuv420_resize(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst,
+__global__ void __launch_bounds__(256) k0_ingest_resize(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst,
                                                         const int *__restrict__ xofs, const short2 *__restrict__ alpha,
                                                         const int2 *__restrict__ yofs, const short2 *__restrict__ beta,
-                                                        int sh, int sw, int dh, int dw)
+                                                        int sh, int sw, int dh, int dw, int phase)
 {
     const int dx0 = (blockIdx.x * blockDim.x + threadIdx.x) * PX, dy = blockIdx.y, f = blockIdx.z;
     if (dx0 >= dw) return;
     const int2 yy = __ldg(yofs + dy);
     const short2 b = __ldg(beta + dy);
-    const uint8_t *s = src + (size_t)f * sh * sw * 3 / 2;
+    const uint8_t *s = src + lane_input_frame_bytes(FMT, sh, sw, f);
     uint8_t *out = dst + (((size_t)f * dh + dy) * dw + dx0) * 3;
     uint8_t o[PX * 3];
-    k0_yuv420_resize_px<FMT, PX>(s, sh, sw, yy, b, xofs, alpha, dx0, dw, o);
-    k0_store_px<3, PX>(out, o, dx0, dw);
-}
-
-// k0_yuv420_resize for Bayer mosaics of one pattern (phase: lane_bayer_phase), at any size including the source's own.
-template <int PX>
-__global__ void __launch_bounds__(256) k0_bayer_resize(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst,
-                                                       const int *__restrict__ xofs, const short2 *__restrict__ alpha,
-                                                       const int2 *__restrict__ yofs, const short2 *__restrict__ beta,
-                                                       int phase, int sh, int sw, int dh, int dw)
-{
-    const int dx0 = (blockIdx.x * blockDim.x + threadIdx.x) * PX, dy = blockIdx.y, f = blockIdx.z;
-    if (dx0 >= dw) return;
-    const int2 yy = __ldg(yofs + dy);
-    const short2 b = __ldg(beta + dy);
-    const uint8_t *s = src + (size_t)f * sh * sw;
-    uint8_t *out = dst + (((size_t)f * dh + dy) * dw + dx0) * 3;
-    uint8_t o[PX * 3];
-    k0_bayer_resize_px<PX>(s, sh, sw, phase, yy, b, xofs, alpha, dx0, dw, o);
-    k0_store_px<3, PX>(out, o, dx0, dw);
-}
-
-// k0_yuv420_resize for packed 4:2:2 frames whose Y0 sits at byte YO of each 4-byte group (lane_yuv422_y0).
-template <int YO, int PX>
-__global__ void __launch_bounds__(256) k0_yuv422_resize(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst,
-                                                        const int *__restrict__ xofs, const short2 *__restrict__ alpha,
-                                                        const int2 *__restrict__ yofs, const short2 *__restrict__ beta,
-                                                        int sh, int sw, int dh, int dw)
-{
-    const int dx0 = (blockIdx.x * blockDim.x + threadIdx.x) * PX, dy = blockIdx.y, f = blockIdx.z;
-    if (dx0 >= dw) return;
-    const int2 yy = __ldg(yofs + dy);
-    const short2 b = __ldg(beta + dy);
-    const uint8_t *s = src + (size_t)f * sh * sw * 2;
-    uint8_t *out = dst + (((size_t)f * dh + dy) * dw + dx0) * 3;
-    uint8_t o[PX * 3];
-    k0_yuv422_resize_px<PX>(s, sw, YO, yy, b, xofs, alpha, dx0, dw, o);
+    if constexpr (lane_input_bayer(FMT))
+        k0_bayer_resize_px<PX>(s, sh, sw, phase, yy, b, xofs, alpha, dx0, dw, o);
+    else if constexpr (lane_input_yuv422(FMT))
+        k0_yuv422_resize_px<PX>(s, sw, lane_yuv422_y0(FMT), yy, b, xofs, alpha, dx0, dw, o);
+    else
+        k0_yuv420_resize_px<FMT, PX>(s, sh, sw, yy, b, xofs, alpha, dx0, dw, o);
     k0_store_px<3, PX>(out, o, dx0, dw);
 }
 
 // The frames of a rig: every frame has its own descriptor (layout, size, tap tables), so cameras of different
-// resolutions and decoders share one launch.  The grid is k0_yuv420_resize's; a block reads its frame's descriptor
+// resolutions and decoders share one launch.  The grid is k0_ingest_resize's; a block reads its frame's descriptor
 // once, and the branch on the layout is uniform over the block.  A frame already at dh x dw runs on identity taps,
 // which reproduce the source (BGR) or cv2.cvtColor's frame (YUV, Bayer) exactly.
 //
@@ -166,13 +137,11 @@ void launch_rig_ingest(const RigFrame *frames_dev, int n, uint8_t *dst, int dh, 
 cudaError_t launch_ingest(const uint8_t *src, int format, int n, int sh, int sw, uint8_t *dst, int dh, int dw,
                           cudaStream_t st)
 {
-    const bool yuv = format == LANE_INPUT_NV12 || format == LANE_INPUT_I420;
-    if (yuv && sh == dh && sw == dw) {                             // INTER_LINEAR at scale 1 is the identity
-        launch_yuv420_to_bgr(src, format, dst, n, sh, sw, st);
-        return cudaGetLastError();
-    }
-    if (lane_input_yuv422(format) && sh == dh && sw == dw) {
-        launch_yuv422_to_bgr(src, format, dst, n, sh, sw, st);
+    if (!lane_input_resizes(format, sh, sw, dh, dw)) {            // INTER_LINEAR at scale 1 is the identity
+        if (lane_input_yuv422(format))
+            launch_yuv422_to_bgr(src, format, dst, n, sh, sw, st);
+        else
+            launch_yuv420_to_bgr(src, format, dst, n, sh, sw, st);
         return cudaGetLastError();
     }
     ResizeTaps t;
@@ -184,32 +153,31 @@ cudaError_t launch_ingest(const uint8_t *src, int format, int n, int sh, int sw,
     }
     constexpr int PX = 4;
     const dim3 grid((dw + 256 * PX - 1) / (256 * PX), dh, n);
-    if (lane_input_bayer(format))
-        k0_bayer_resize<PX><<<grid, 256, 0, st>>>(src, dst, t.xofs, t.alpha, t.yofs, t.beta, lane_bayer_phase(format), sh, sw,
-                                                  dh, dw);
-    else if (format == LANE_INPUT_UYVY)
-        k0_yuv422_resize<1, PX><<<grid, 256, 0, st>>>(src, dst, t.xofs, t.alpha, t.yofs, t.beta, sh, sw, dh, dw);
-    else if (format == LANE_INPUT_YUYV)
-        k0_yuv422_resize<0, PX><<<grid, 256, 0, st>>>(src, dst, t.xofs, t.alpha, t.yofs, t.beta, sh, sw, dh, dw);
-    else if (format == LANE_INPUT_I420)
-        k0_yuv420_resize<LANE_INPUT_I420, PX><<<grid, 256, 0, st>>>(src, dst, t.xofs, t.alpha, t.yofs, t.beta, sh, sw, dh, dw);
-    else
-        k0_yuv420_resize<LANE_INPUT_NV12, PX><<<grid, 256, 0, st>>>(src, dst, t.xofs, t.alpha, t.yofs, t.beta, sh, sw, dh, dw);
+    auto launch = [&](auto kernel) {
+        kernel<<<grid, 256, 0, st>>>(src, dst, t.xofs, t.alpha, t.yofs, t.beta, sh, sw, dh, dw, lane_bayer_phase(format));
+    };
+    switch (format) {
+    case LANE_INPUT_NV12: launch(k0_ingest_resize<LANE_INPUT_NV12, PX>); break;
+    case LANE_INPUT_I420: launch(k0_ingest_resize<LANE_INPUT_I420, PX>); break;
+    case LANE_INPUT_UYVY: launch(k0_ingest_resize<LANE_INPUT_UYVY, PX>); break;
+    case LANE_INPUT_YUYV: launch(k0_ingest_resize<LANE_INPUT_YUYV, PX>); break;
+    default: launch(k0_ingest_resize<LANE_INPUT_BAYER_RGGB, PX>);
+    }
     return cudaGetLastError();
 }
 
 namespace {
 
-int yuv420_to_bgr(const char *who, const uint8_t *src, int format, int n, int src_h, int src_w, uint8_t *dst, int dst_h,
-                  int dst_w, int on_device, int device, void *cuda_stream)
+// The context-free conversion entries: n frames of a layout `accepts` takes (`formats` names them), checked against
+// the layout table, become BGR at dst_h x dst_w on the device or through a host round trip.  `who` starts every message.
+int to_bgr(const char *who, bool (*accepts)(int), const char *formats, const uint8_t *src, int format, int n, int src_h,
+           int src_w, uint8_t *dst, int dst_h, int dst_w, int on_device, int device, void *cuda_stream)
 {
     if (!src || !dst || n < 1 || src_h < 1 || src_w < 1 || dst_h < 1 || dst_w < 1)
         return lane_api_fail(LANE_ERR_INVALID, who, "bad arguments (non-null pointers, positive sizes)");
-    if (format != LANE_INPUT_NV12 && format != LANE_INPUT_I420)
-        return lane_api_fail(LANE_ERR_INVALID, who, "format must be LANE_INPUT_NV12 or LANE_INPUT_I420");
-    if ((src_h | src_w) & 1) return lane_api_fail(LANE_ERR_INVALID, who, "YUV 4:2:0 needs even width and height");
-    const bool resize = dst_h != src_h || dst_w != src_w;
-    if (resize && (dst_h > 65535 || n > 65535))
+    if (!accepts(format)) return lane_api_fail(LANE_ERR_INVALID, who, formats);
+    if (const char *why = lane_input_refusal(format, src_h, src_w)) return lane_api_fail(LANE_ERR_INVALID, who, why);
+    if (lane_input_resizes(format, src_h, src_w, dst_h, dst_w) && (dst_h > 65535 || n > 65535))
         return lane_api_fail(LANE_ERR_UNSUPPORTED, who, "destination height / batch above 65535");
     if (int rc = lane_api_device(who, device)) return rc;
     cudaStream_t st = (cudaStream_t)cuda_stream;
@@ -218,8 +186,8 @@ int yuv420_to_bgr(const char *who, const uint8_t *src, int format, int n, int sr
         return e ? lane_api_fail(LANE_ERR_CUDA, who, "launch", e) : LANE_OK;
     };
     if (on_device) return launch(src, dst);
-    return lane_host_round_trip(who, device, st, src, (size_t)n * src_h * src_w * 3 / 2, dst, (size_t)n * dst_h * dst_w * 3,
-                                launch);
+    return lane_host_round_trip(who, device, st, src, lane_input_frame_bytes(format, src_h, src_w, n), dst,
+                                (size_t)n * dst_h * dst_w * 3, launch);
 }
 
 }  // namespace
@@ -227,55 +195,27 @@ int yuv420_to_bgr(const char *who, const uint8_t *src, int format, int n, int sr
 extern "C" int lane_yuv420_to_bgr_batch(const uint8_t *src, int format, int n, int src_h, int src_w, uint8_t *dst,
                                         int dst_h, int dst_w, int on_device, int device, void *cuda_stream)
 {
-    return yuv420_to_bgr("lane_yuv420_to_bgr_batch", src, format, n, src_h, src_w, dst, dst_h, dst_w, on_device, device,
-                         cuda_stream);
+    return to_bgr("lane_yuv420_to_bgr_batch", lane_input_yuv420, "format must be LANE_INPUT_NV12 or LANE_INPUT_I420", src,
+                  format, n, src_h, src_w, dst, dst_h, dst_w, on_device, device, cuda_stream);
 }
 
 extern "C" int lane_bayer_to_bgr_batch(const uint8_t *src, int format, int n, int src_h, int src_w, uint8_t *dst,
                                        int dst_h, int dst_w, int on_device, int device, void *cuda_stream)
 {
-    const char *who = "lane_bayer_to_bgr_batch";
-    if (!src || !dst || n < 1 || src_h < 1 || src_w < 1 || dst_h < 1 || dst_w < 1)
-        return lane_api_fail(LANE_ERR_INVALID, who, "bad arguments (non-null pointers, positive sizes)");
-    if (!lane_input_bayer(format)) return lane_api_fail(LANE_ERR_INVALID, who, "format must be a LANE_INPUT_BAYER_* layout");
-    if (src_h < 3 || src_w < 3) return lane_api_fail(LANE_ERR_INVALID, who, "a Bayer frame needs at least 3 rows and 3 columns");
-    if (dst_h > 65535 || n > 65535) return lane_api_fail(LANE_ERR_UNSUPPORTED, who, "destination height / batch above 65535");
-    if (int rc = lane_api_device(who, device)) return rc;
-    cudaStream_t st = (cudaStream_t)cuda_stream;
-    auto launch = [&](const uint8_t *s, uint8_t *d) {
-        const cudaError_t e = launch_ingest(s, format, n, src_h, src_w, d, dst_h, dst_w, st);
-        return e ? lane_api_fail(LANE_ERR_CUDA, who, "launch", e) : LANE_OK;
-    };
-    if (on_device) return launch(src, dst);
-    return lane_host_round_trip(who, device, st, src, (size_t)n * src_h * src_w, dst, (size_t)n * dst_h * dst_w * 3, launch);
+    return to_bgr("lane_bayer_to_bgr_batch", lane_input_bayer, "format must be a LANE_INPUT_BAYER_* layout", src, format,
+                  n, src_h, src_w, dst, dst_h, dst_w, on_device, device, cuda_stream);
 }
 
 extern "C" int lane_yuv422_to_bgr_batch(const uint8_t *src, int format, int n, int src_h, int src_w, uint8_t *dst,
                                         int dst_h, int dst_w, int on_device, int device, void *cuda_stream)
 {
-    const char *who = "lane_yuv422_to_bgr_batch";
-    if (!src || !dst || n < 1 || src_h < 1 || src_w < 1 || dst_h < 1 || dst_w < 1)
-        return lane_api_fail(LANE_ERR_INVALID, who, "bad arguments (non-null pointers, positive sizes)");
-    if (!lane_input_yuv422(format))
-        return lane_api_fail(LANE_ERR_INVALID, who, "format must be LANE_INPUT_UYVY or LANE_INPUT_YUYV");
-    if (src_w & 1) return lane_api_fail(LANE_ERR_INVALID, who, "YUV 4:2:2 needs an even width");
-    const bool resize = dst_h != src_h || dst_w != src_w;
-    if (resize && (dst_h > 65535 || n > 65535))
-        return lane_api_fail(LANE_ERR_UNSUPPORTED, who, "destination height / batch above 65535");
-    if (int rc = lane_api_device(who, device)) return rc;
-    cudaStream_t st = (cudaStream_t)cuda_stream;
-    auto launch = [&](const uint8_t *s, uint8_t *d) {
-        const cudaError_t e = launch_ingest(s, format, n, src_h, src_w, d, dst_h, dst_w, st);
-        return e ? lane_api_fail(LANE_ERR_CUDA, who, "launch", e) : LANE_OK;
-    };
-    if (on_device) return launch(src, dst);
-    return lane_host_round_trip(who, device, st, src, (size_t)n * src_h * src_w * 2, dst, (size_t)n * dst_h * dst_w * 3,
-                                launch);
+    return to_bgr("lane_yuv422_to_bgr_batch", lane_input_yuv422, "format must be LANE_INPUT_UYVY or LANE_INPUT_YUYV", src,
+                  format, n, src_h, src_w, dst, dst_h, dst_w, on_device, device, cuda_stream);
 }
 
 extern "C" int lane_nv12_to_bgr_batch(const uint8_t *src, int n, int height, int width, uint8_t *dst, int on_device,
                                       int device, void *cuda_stream)
 {
-    return yuv420_to_bgr("lane_nv12_to_bgr_batch", src, LANE_INPUT_NV12, n, height, width, dst, height, width, on_device,
-                         device, cuda_stream);
+    return to_bgr("lane_nv12_to_bgr_batch", lane_input_yuv420, "format must be LANE_INPUT_NV12 or LANE_INPUT_I420", src,
+                  LANE_INPUT_NV12, n, height, width, dst, height, width, on_device, device, cuda_stream);
 }

@@ -430,15 +430,6 @@ int end_batch(lane_ctx *c, bool on_device, int n, int S, const uint8_t *frames_d
     return LANE_OK;
 }
 
-// Bytes of one dense frame of a source: its own size and layout (3 B/px BGR, 1.5 B/px YUV 4:2:0, 1 B/px Bayer,
-// 2 B/px YUV 4:2:2).
-size_t frame_bytes(const lane_rig_source &r)
-{
-    const size_t px = (size_t)r.src_h * r.src_w;
-    return r.format == LANE_INPUT_BGR ? px * 3 : lane_input_bayer(r.format) ? px : lane_input_yuv422(r.format) ? px * 2
-                                                                                                               : px * 3 / 2;
-}
-
 // How the context's H x W BGR frames are made from the batch's sources before the path runs (k0_common.cuh): they
 // already are those frames; one launch_ingest over frames of one layout and size; or k0_rig_ingest over every frame,
 // each with its own layout and size, driven by the batch's descriptor table.
@@ -459,8 +450,10 @@ int enqueue(lane_ctx *c, const lane_rig_source *sources, int n_sources, bool on_
     if (ingest != Ingest::none || !on_device) CU(c->d_frames.lazy(B * bgr_bytes));
     // host frame f lands at byte offset at[f]: in the context's frames when they need no ingest, else in source staging
     std::vector<size_t> at(n + 1, 0);
-    for (int s = 0, f = 0; s < n_sources; s++)
-        for (int j = 0; j < sources[s].n; j++, f++) at[f + 1] = at[f] + frame_bytes(sources[s]);
+    for (int s = 0, f = 0; s < n_sources; s++) {
+        const lane_rig_source &r = sources[s];
+        for (int j = 0; j < r.n; j++, f++) at[f + 1] = at[f] + lane_input_frame_bytes(r.format, r.src_h, r.src_w);
+    }
     uint8_t *land = c->d_frames;
     if (!on_device && ingest != Ingest::none) {
         DeviceArray<uint8_t> &src = staged ? sl.d_src : c->d_src;
@@ -477,7 +470,7 @@ int enqueue(lane_ctx *c, const lane_rig_source *sources, int n_sources, bool on_
             RigFrame d;
             CU(rig_frame(nullptr, r.format, r.src_h, r.src_w, c->g.H, c->g.W, &d));
             for (int j = 0; j < r.n; j++, f++) {
-                d.src = on_device ? r.frames + j * frame_bytes(r) : land + at[f];
+                d.src = on_device ? r.frames + j * lane_input_frame_bytes(r.format, r.src_h, r.src_w) : land + at[f];
                 sl.h_rig[f] = d;
             }
         }
@@ -504,7 +497,8 @@ int enqueue(lane_ctx *c, const lane_rig_source *sources, int n_sources, bool on_
             for (int s = 0, first = 0; s < n_sources && first < off + m; first += sources[s].n, s++) {
                 const int lo = std::max(off, first), hi = std::min(off + m, first + sources[s].n);
                 if (lo >= hi) continue;
-                const uint8_t *from = sources[s].frames + (lo - first) * frame_bytes(sources[s]);
+                const lane_rig_source &r = sources[s];
+                const uint8_t *from = r.frames + (lo - first) * lane_input_frame_bytes(r.format, r.src_h, r.src_w);
                 if (ring[s])
                     CU(ring[s]->h2d(land + at[lo], from, at[hi] - at[lo], c->copy_st));
                 else
@@ -526,22 +520,15 @@ int enqueue(lane_ctx *c, const lane_rig_source *sources, int n_sources, bool on_
     return end_batch(c, whole, n, S, frames_dev);
 }
 
-// One source's fields: layout, size (even for YUV 4:2:0, at least 3 x 3 for Bayer, an even width for YUV 4:2:2) and
-// frames.  `s` numbers it in the message; < 0: the call's only source.
+// One source's fields: layout and size (lane_input_refusal) and frames.  `s` numbers it in the message; < 0: the call's
+// only source.
 int check_source(lane_ctx *c, int s, const lane_rig_source &r)
 {
     char who[32] = "";
     if (s >= 0) snprintf(who, sizeof(who), "source %d: ", s);
-    const bool yuv = r.format == LANE_INPUT_NV12 || r.format == LANE_INPUT_I420;
-    if (r.format != LANE_INPUT_BGR && !yuv && !lane_input_bayer(r.format) && !lane_input_yuv422(r.format))
-        return fail(c, LANE_ERR_INVALID, "%sunknown input format %d", who, r.format);
     if (r.src_h < 1 || r.src_w < 1) return fail(c, LANE_ERR_INVALID, "%sbad source size %dx%d", who, r.src_w, r.src_h);
-    if (yuv && ((r.src_h | r.src_w) & 1))
-        return fail(c, LANE_ERR_INVALID, "%sNV12 / I420 needs even width and height (%dx%d)", who, r.src_w, r.src_h);
-    if (lane_input_bayer(r.format) && (r.src_h < 3 || r.src_w < 3))
-        return fail(c, LANE_ERR_INVALID, "%sa Bayer frame needs at least 3 rows and 3 columns (%dx%d)", who, r.src_w, r.src_h);
-    if (lane_input_yuv422(r.format) && (r.src_w & 1))
-        return fail(c, LANE_ERR_INVALID, "%sUYVY / YUYV needs an even width (%dx%d)", who, r.src_w, r.src_h);
+    if (const char *why = lane_input_refusal(r.format, r.src_h, r.src_w))
+        return fail(c, LANE_ERR_INVALID, "%s%s (format %d, %dx%d)", who, why, r.format, r.src_w, r.src_h);
     if (r.n && !r.frames) return fail(c, LANE_ERR_INVALID, "%sframes is null", who);
     return LANE_OK;
 }
@@ -614,10 +601,10 @@ int check_call(lane_ctx *c, const void *frames, int n, const int32_t *stream_id,
 int enqueue_frames(lane_ctx *c, const lane_rig_source &r, bool on_device, const int32_t *stream_id, int S,
                    const double *prev_fit, const uint8_t *prev_valid)
 {
-    const bool resize = r.src_h != c->g.H || r.src_w != c->g.W;
-    if (resize || lane_input_bayer(r.format))          // Bayer frames take the resizing kernel at every size
+    const bool resizes = lane_input_resizes(r.format, r.src_h, r.src_w, c->g.H, c->g.W);
+    if (resizes)
         if (const int rc = check_grid(c, r.n)) return rc;
-    const Ingest ingest = r.format == LANE_INPUT_BGR && !resize ? Ingest::none : Ingest::single;
+    const Ingest ingest = r.format == LANE_INPUT_BGR && !resizes ? Ingest::none : Ingest::single;
     return enqueue(c, &r, 1, on_device, false, ingest, r.n, stream_id, S, prev_fit, prev_valid);
 }
 
@@ -998,7 +985,8 @@ int lane_rig_enqueue(lane_ctx *c, const lane_rig_source *sources, int n_sources,
     if (n < 0) return n;
     if (!frames_on_device)
         for (int s = 0; s < n_sources; s++)
-            if (sources[s].n && !page_locked(sources[s].frames, sources[s].n * frame_bytes(sources[s])))
+            if (const lane_rig_source &r = sources[s];
+                r.n && !page_locked(r.frames, lane_input_frame_bytes(r.format, r.src_h, r.src_w, r.n)))
                 return fail(c, LANE_ERR_INVALID, "source %d: host frames must be page-locked or registered memory "
                             "(cudaHostAlloc, cudaHostRegister, torch pin_memory)", s);
     const int rc = check_call(c, sources, n, stream_id.data(), n_streams, prev_fit, prev_valid);

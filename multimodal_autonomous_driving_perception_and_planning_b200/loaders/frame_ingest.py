@@ -15,6 +15,7 @@ import cv2
 import numpy as np
 
 from .. import _native
+from .frame_layout import LAYOUTS, Layout, check_frames, named
 
 
 class FrameIngest:
@@ -73,30 +74,20 @@ class FrameIngest:
         ``[N, H, W, 3]``, equal to ``cv2.cvtColor(f, cv2.COLOR_YUV2BGR_NV12)`` per frame, followed by the resize when
         ``target_size`` is set (what ``VideoDataLoader.read_frame`` returns for that frame).  With ``target_size`` the
         conversion and the resize are one kernel: the full-resolution BGR frame is never stored."""
-        return self._from_yuv420(frames, _native.INPUT_NV12)
+        return self._to_bgr(frames, LAYOUTS["nv12"])
 
     def from_i420(self, frames):
         """``from_nv12`` for the planar layout software decoders hand out (FFmpeg / PyAV ``yuv420p``): uint8
         ``[N, H*3/2, W]`` = Y plane, then the U plane, then the V plane (each ``H/2 x W/2``); equal to
         ``cv2.cvtColor(f, cv2.COLOR_YUV2BGR_I420)`` per frame, resized when ``target_size`` is set."""
-        return self._from_yuv420(frames, _native.INPUT_I420)
-
-    def _from_yuv420(self, frames, fmt):
-        check_yuv420(frames, "FrameIngest")
-        n, h, w = int(frames.shape[0]), int(frames.shape[1]) * 2 // 3, int(frames.shape[2])
-        dw, dh = (w, h) if self.target_size is None else self.target_size
-        return self._convert(_native.lib().lane_yuv420_to_bgr_batch, frames, fmt, n, h, w, dh, dw)
+        return self._to_bgr(frames, LAYOUTS["i420"])
 
     def from_bayer(self, frames, pattern: str):
         """Raw camera frames -> BGR: ``frames`` uint8 ``[N, H, W]`` 8-bit Bayer mosaics (numpy or CUDA tensor, H and W
         at least 3) whose top-left 2x2 is ``pattern`` ("rggb", "bggr", "grbg" or "gbrg") become ``[N, H, W, 3]``, equal
         to ``cv2.cvtColor(f, cv2.COLOR_Bayer<P>2BGR)`` per frame, followed by the resize when ``target_size`` is set.
         Demosaic and resize are one kernel: the full-resolution BGR frame is never stored."""
-        fmt = bayer_format(pattern)
-        check_bayer(frames, "FrameIngest")
-        n, h, w = (int(x) for x in frames.shape)
-        dw, dh = (w, h) if self.target_size is None else self.target_size
-        return self._convert(_native.lib().lane_bayer_to_bgr_batch, frames, fmt, n, h, w, dh, dw)
+        return self._to_bgr(frames, named(pattern, _native.BAYER, "Bayer pattern"))
 
     def from_yuv422(self, frames, order: str):
         """Packed 4:2:2 camera frames -> BGR: ``frames`` uint8 ``[N, H, W, 2]`` (numpy or CUDA tensor, W even) in byte
@@ -104,19 +95,19 @@ class FrameIngest:
         default) become ``[N, H, W, 3]``, equal to ``cv2.cvtColor(f, cv2.COLOR_YUV2BGR_UYVY | COLOR_YUV2BGR_YUY2)`` per
         frame, followed by the resize when ``target_size`` is set.  Conversion and resize are one kernel: the
         full-resolution BGR frame is never stored."""
-        fmt = yuv422_format(order)
-        check_yuv422(frames, "FrameIngest")
-        n, h, w = (int(x) for x in frames.shape[:3])
-        dw, dh = (w, h) if self.target_size is None else self.target_size
-        return self._convert(_native.lib().lane_yuv422_to_bgr_batch, frames, fmt, n, h, w, dh, dw)
+        return self._to_bgr(frames, named(order, _native.YUV422, "YUV 4:2:2 order"))
 
-    def _convert(self, entry, frames, fmt, n, h, w, dh, dw):
-        """One context-free conversion entry (``lane_yuv420_to_bgr_batch`` / ``lane_bayer_to_bgr_batch`` /
-        ``lane_yuv422_to_bgr_batch``): numpy in, numpy out; CUDA tensor in, CUDA tensor out on torch's current stream."""
+    def _to_bgr(self, frames, layout: Layout):
+        """Frames in a camera ``layout`` through its context-free conversion entry: numpy in, numpy out; CUDA tensor
+        in, CUDA tensor out on torch's current stream."""
+        h, w = check_frames(frames, layout, "FrameIngest")
+        n = int(frames.shape[0])
+        dw, dh = (w, h) if self.target_size is None else self.target_size
+        entry = getattr(_native.lib(), layout.entry)
         if isinstance(frames, np.ndarray):
             src = np.ascontiguousarray(frames)
             dst = np.empty((n, dh, dw, 3), np.uint8)
-            rc = entry(src.ctypes.data_as(C.c_void_p), fmt, n, h, w, dst.ctypes.data_as(C.c_void_p), dh, dw, 0,
+            rc = entry(src.ctypes.data_as(C.c_void_p), layout.fmt, n, h, w, dst.ctypes.data_as(C.c_void_p), dh, dw, 0,
                        self._device_index(), None)
         else:
             import torch
@@ -125,56 +116,14 @@ class FrameIngest:
             src = frames.contiguous()
             dst = torch.empty((n, dh, dw, 3), dtype=torch.uint8, device=src.device)
             stream = torch.cuda.current_stream(src.device).cuda_stream
-            rc = entry(C.c_void_p(src.data_ptr()), fmt, n, h, w, C.c_void_p(dst.data_ptr()), dh, dw, 1, src.device.index,
-                       C.c_void_p(stream))
+            rc = entry(C.c_void_p(src.data_ptr()), layout.fmt, n, h, w, C.c_void_p(dst.data_ptr()), dh, dw, 1,
+                       src.device.index, C.c_void_p(stream))
         _native.check_global(rc)
         return dst
 
     def resize(self, frame: np.ndarray) -> np.ndarray:
         """One frame, as ``read_frame`` does it."""
         return self.resize_batch(frame[None])[0]
-
-
-def check_yuv420(frames, who: str):
-    """uint8 ``[N, H*3/2, W]`` with even H and W (NV12 / I420), else ``cv2.error`` (what cv2.cvtColor raises)."""
-    shape = tuple(frames.shape)
-    if len(shape) != 3 or shape[1] % 3 or shape[2] % 2 or (shape[1] * 2 // 3) % 2:
-        raise cv2.error(f"{who}: expected NV12 / I420 frames [N, H*3/2, W] with even H and W, got {shape}")
-    if str(frames.dtype).replace("torch.", "") != "uint8":
-        raise cv2.error(f"{who}: expected uint8 frames, got {frames.dtype}")
-
-
-def bayer_format(pattern) -> int:
-    """LANE_INPUT_BAYER_* of a pattern name ("rggb", "bggr", "grbg", "gbrg"), else ``ValueError``."""
-    if not isinstance(pattern, str) or pattern not in _native.BAYER:
-        raise ValueError(f"Bayer pattern {pattern!r} is not one of {sorted(_native.BAYER)}")
-    return _native.BAYER[pattern]
-
-
-def check_bayer(frames, who: str):
-    """uint8 ``[N, H, W]`` with H, W >= 3 (raw Bayer mosaics), else ``cv2.error``.  cv2.cvtColor returns an all-zero
-    frame below 3 rows or columns; such frames are refused rather than emulated."""
-    shape = tuple(frames.shape)
-    if len(shape) != 3 or shape[1] < 3 or shape[2] < 3:
-        raise cv2.error(f"{who}: expected Bayer frames [N, H, W] with H, W >= 3, got {shape}")
-    if str(frames.dtype).replace("torch.", "") != "uint8":
-        raise cv2.error(f"{who}: expected uint8 frames, got {frames.dtype}")
-
-
-def yuv422_format(order) -> int:
-    """LANE_INPUT_UYVY / LANE_INPUT_YUYV of a byte order name ("uyvy", "yuyv"), else ``ValueError``."""
-    if not isinstance(order, str) or order not in _native.YUV422:
-        raise ValueError(f"YUV 4:2:2 order {order!r} is not one of {sorted(_native.YUV422)}")
-    return _native.YUV422[order]
-
-
-def check_yuv422(frames, who: str):
-    """uint8 ``[N, H, W, 2]`` with even W (packed UYVY / YUYV), else ``cv2.error`` (what cv2.cvtColor raises)."""
-    shape = tuple(frames.shape)
-    if len(shape) != 4 or shape[3] != 2 or shape[2] % 2:
-        raise cv2.error(f"{who}: expected YUV 4:2:2 frames [N, H, W, 2] with even W, got {shape}")
-    if str(frames.dtype).replace("torch.", "") != "uint8":
-        raise cv2.error(f"{who}: expected uint8 frames, got {frames.dtype}")
 
 
 def check_target_size(target_size) -> Tuple[int, int]:

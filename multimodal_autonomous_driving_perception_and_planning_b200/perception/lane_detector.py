@@ -20,8 +20,8 @@ import cv2
 import numpy as np
 
 from .. import _native
-from ..loaders.frame_ingest import (bayer_format, check_bayer, check_target_size, check_yuv420, check_yuv422,
-                                    yuv422_format)
+from ..loaders.frame_ingest import check_target_size
+from ..loaders.frame_layout import BY_FORMAT, LAYOUTS, Layout, check_frames, named
 
 
 @dataclass
@@ -35,10 +35,6 @@ class LaneLine:
 
 LanePair = Tuple[Optional[LaneLine], Optional[LaneLine]]
 _SIDES = ("left", "right")
-_LAYOUTS = {"bgr": _native.INPUT_BGR, "nv12": _native.INPUT_NV12, "i420": _native.INPUT_I420,
-            **{"bayer_" + p: fmt for p, fmt in _native.BAYER.items()}, **_native.YUV422}
-_BAYER_FORMATS = frozenset(_native.BAYER.values())
-_YUV422_FORMATS = frozenset(_native.YUV422.values())
 _COPY_PIECE = 4 << 20         # bytes per host thread task when detect_rig_stream copies a numpy tick into pinned memory
 
 
@@ -54,13 +50,8 @@ def _is_pinned_tensor(x) -> bool:
 
 
 def _frame_bytes(fmt: int, h: int, w: int) -> int:
-    """Bytes of one h x w frame in layout ``fmt`` (INPUT_*): 3 B/px BGR, 1.5 B/px YUV 4:2:0, 1 B/px Bayer, 2 B/px
-    YUV 4:2:2."""
-    if fmt == _native.INPUT_BGR:
-        return h * w * 3
-    if fmt in _BAYER_FORMATS:
-        return h * w
-    return h * w * 2 if fmt in _YUV422_FORMATS else h * w * 3 // 2
+    """Bytes of one h x w frame in layout ``fmt`` (INPUT_*), from the layout table."""
+    return BY_FORMAT[fmt].frame_bytes(h, w)
 
 
 def _two_deep(items, plan, start, joins, enqueue, blocking, restore, adopt):
@@ -154,12 +145,9 @@ class _Plan:
 
     @classmethod
     def of_frames(cls, frames, fmt: int, target_size=None, frame_sids=None, stream_rois=None) -> "_Plan":
-        """One checked array of frames: [N,H,W,3] BGR, [N,H*3/2,W] for the YUV 4:2:0 layouts, [N,H,W] for the Bayer
-        layouts or [N,H,W,2] for the YUV 4:2:2 layouts of ``fmt``, detected at ``target_size`` = (width, height) when
+        """One checked array of frames in layout ``fmt`` (INPUT_*), detected at ``target_size`` = (width, height) when
         given."""
-        n, sh, sw = (int(x) for x in frames.shape[:3])
-        if fmt not in (_native.INPUT_BGR, *_BAYER_FORMATS, *_YUV422_FORMATS):
-            sh = sh * 2 // 3
+        n, (sh, sw) = int(frames.shape[0]), BY_FORMAT[fmt].hw(frames.shape)
         h, w = (sh, sw) if target_size is None else (target_size[1], target_size[0])
         kind = ("cuda", frames.device.index) if _is_torch_cuda(frames) else "host"
         return cls([frames], [fmt], [(sh, sw)], [n], kind, h, w, stream_rois, rig=False, frame_sids=frame_sids)
@@ -524,15 +512,13 @@ class LaneDetector:
         ``target_size`` = (width, height): the decoder's frames at camera resolution are detected at that size, equal to
         ``detect_batch`` of ``cv2.resize(cv2.cvtColor(f, COLOR_YUV2BGR_NV12), target_size)`` (``VideoDataLoader`` with
         ``target_size``); conversion and resize are one kernel and only the NV12 bytes cross PCIe."""
-        check_yuv420(frames, "LaneDetector")
-        return self._detect_frames(frames, _native.INPUT_NV12, target_size)
+        return self._detect_camera(frames, LAYOUTS["nv12"], target_size)
 
     def detect_batch_i420(self, frames, *, target_size: Optional[Tuple[int, int]] = None) -> List[LanePair]:
         """``detect_batch_nv12`` for the planar layout software decoders hand out (FFmpeg / PyAV ``yuv420p``): uint8
         ``[N, H*3/2, W]`` = Y plane, U plane, V plane; equal to ``detect_batch`` on
         ``cv2.cvtColor(f, cv2.COLOR_YUV2BGR_I420)`` of every frame, resized to ``target_size`` when given."""
-        check_yuv420(frames, "LaneDetector")
-        return self._detect_frames(frames, _native.INPUT_I420, target_size)
+        return self._detect_camera(frames, LAYOUTS["i420"], target_size)
 
     def detect_batch_bayer(self, frames, pattern: str, *, target_size: Optional[Tuple[int, int]] = None) -> List[LanePair]:
         """``detect_batch`` for raw camera frames: uint8 ``[N, H, W]`` 8-bit Bayer mosaics (numpy or CUDA tensor, H and W
@@ -540,9 +526,7 @@ class LaneDetector:
         ``detect_batch`` of ``cv2.cvtColor(f, cv2.COLOR_Bayer<P>2BGR)`` of every frame, resized to ``target_size`` =
         (width, height) when given, with the same ``prev_*_fit`` after it.  Demosaic and resize are one kernel on the
         device, so a host batch moves 1 B/px over PCIe."""
-        fmt = bayer_format(pattern)
-        check_bayer(frames, "LaneDetector")
-        return self._detect_frames(frames, fmt, target_size)
+        return self._detect_camera(frames, named(pattern, _native.BAYER, "Bayer pattern"), target_size)
 
     def detect_batch_yuv422(self, frames, order: str, *, target_size: Optional[Tuple[int, int]] = None) -> List[LanePair]:
         """``detect_batch`` for packed YUV 4:2:2 camera frames: uint8 ``[N, H, W, 2]`` (numpy or CUDA tensor, W even) in
@@ -550,9 +534,12 @@ class LaneDetector:
         default).  Equal to ``detect_batch`` of ``cv2.cvtColor(f, cv2.COLOR_YUV2BGR_UYVY | COLOR_YUV2BGR_YUY2)`` of every
         frame, resized to ``target_size`` = (width, height) when given, with the same ``prev_*_fit`` after it.
         Conversion and resize are one kernel on the device, so a host batch moves 2 B/px over PCIe instead of 3."""
-        fmt = yuv422_format(order)
-        check_yuv422(frames, "LaneDetector")
-        return self._detect_frames(frames, fmt, target_size)
+        return self._detect_camera(frames, named(order, _native.YUV422, "YUV 4:2:2 order"), target_size)
+
+    def _detect_camera(self, frames, layout: Layout, target_size) -> List[LanePair]:
+        """``detect_batch`` of frames in a camera ``layout``, checked against it."""
+        check_frames(frames, layout, "LaneDetector")
+        return self._detect_frames(frames, layout.fmt, target_size)
 
     def detect_streams(self, frames, stream_ids: Optional[Sequence[int]] = None, *,
                        stream_rois: Optional[Sequence[Optional[np.ndarray]]] = None) -> List[LanePair]:
@@ -705,9 +692,9 @@ class LaneDetector:
                 raise ValueError(f"stream_rois has {len(stream_rois)} entries for {len(cams)} cameras")
         fmts, sizes, counts, kinds = [], [], [], set()
         for s, (f, lay) in enumerate(zip(cams, layouts)):
-            if lay not in _LAYOUTS:
-                raise ValueError(f"camera {s}: layout {lay!r} is not one of {sorted(_LAYOUTS)}")
-            fmts.append(_LAYOUTS[lay])
+            if lay not in LAYOUTS:
+                raise ValueError(f"camera {s}: layout {lay!r} is not one of {sorted(LAYOUTS)}")
+            fmts.append(LAYOUTS[lay].fmt)
             if f is None:
                 sizes.append(None)
                 counts.append(0)
@@ -727,36 +714,19 @@ class LaneDetector:
 
     @staticmethod
     def _rig_frame_size(f, layout: str, s: int) -> Tuple[int, int]:
-        """(H, W) of camera s's frames in ``layout``; ``ValueError`` when the shape is not that layout's, ``cv2.error``
-        for a wrong channel count or dtype (what cv2.cvtColor raises)."""
-        shape = tuple(f.shape)
-        if layout == "bgr":
-            if len(shape) != 4:
-                raise ValueError(f"camera {s}: layout 'bgr' needs frames [T,H,W,3], got {shape}")
-            if shape[-1] != 3:
-                raise cv2.error(f"LaneDetector: camera {s}: expected 3-channel BGR frames, got {shape}")
-            h, w = shape[1], shape[2]
-        elif layout.startswith("bayer_"):
-            if len(shape) != 3:
-                raise ValueError(f"camera {s}: layout {layout!r} needs frames [T,H,W], got {shape}")
-            h, w = shape[1], shape[2]
-            if h < 3 or w < 3:
-                raise ValueError(f"camera {s}: {layout} needs at least 3 rows and 3 columns, got {w}x{h}")
-        elif layout in _native.YUV422:
-            if len(shape) != 4 or shape[-1] != 2:
-                raise ValueError(f"camera {s}: layout {layout!r} needs frames [T,H,W,2], got {shape}")
-            h, w = shape[1], shape[2]
-            if w % 2:
-                raise ValueError(f"camera {s}: {layout} needs an even width, got {w}x{h}")
-        else:
-            if len(shape) != 3 or shape[1] % 3:
-                raise ValueError(f"camera {s}: layout {layout!r} needs frames [T,H*3/2,W], got {shape}")
-            h, w = shape[1] * 2 // 3, shape[2]
-            if h % 2 or w % 2:
-                raise ValueError(f"camera {s}: {layout} needs even width and height, got {w}x{h}")
+        """(H, W) of camera s's frames in ``layout``; ``ValueError`` when the shape or size is not that layout's,
+        ``cv2.error`` for a BGR camera's channel count or any dtype (what cv2.cvtColor raises)."""
+        lay, shape = LAYOUTS[layout], tuple(f.shape)
+        hw = lay.hw(shape)
+        if hw is None and layout == "bgr" and len(shape) == 4:
+            raise cv2.error(f"LaneDetector: camera {s}: expected 3-channel BGR frames, got {shape}")
+        if hw is None:
+            raise ValueError(f"camera {s}: layout {layout!r} needs frames [T,{lay.dims}], got {shape}")
+        if lay.refuses(*hw):
+            raise ValueError(f"camera {s}: {layout} needs {lay.rule}, got {hw[1]}x{hw[0]}")
         if str(f.dtype).replace("torch.", "") != "uint8":
             raise cv2.error(f"LaneDetector: camera {s}: frames must be uint8, got {f.dtype}")
-        return int(h), int(w)
+        return hw
 
     def draw_lanes(self, frame: np.ndarray, left_lane: Optional[LaneLine], right_lane: Optional[LaneLine],
                    fill_lane: bool = True) -> np.ndarray:

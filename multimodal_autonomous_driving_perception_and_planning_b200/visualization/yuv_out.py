@@ -17,6 +17,7 @@ import cv2
 import numpy as np
 
 from .. import _native
+from ..loaders.frame_layout import BY_FORMAT
 
 
 def bgr_to_i420(frames, out=None):
@@ -55,7 +56,7 @@ def _host(frames, out, fmt):
     n, h, w = frames.shape[:3]
     if h % 2 or w % 2:
         raise ValueError(("NV12" if fmt == _native.INPUT_NV12 else "I420") + " needs even width and height")
-    shape = (n, h * 3 // 2, w)
+    shape = (n, *BY_FORMAT[fmt].frame_shape(h, w))
     if out is None:
         out = np.empty(shape, np.uint8)
     elif not isinstance(out, np.ndarray) or out.shape != shape or out.dtype != np.uint8:
@@ -101,7 +102,7 @@ def _device(frames, out, fmt, who):
     import torch
     check_bgr(frames, who)
     n, h, w = (int(s) for s in frames.shape[:3])
-    shape = (n, h * 3 // 2, w)
+    shape = (n, *BY_FORMAT[fmt].frame_shape(h, w))
     if out is not None:
         _check_out(out, shape, frames, who)
     if not frames.is_cuda:

@@ -13,7 +13,7 @@ The rig: 1 x 3840x2160 NV12 (front), 4 x 1936x1216 NV12 (surround), 2 x 1280x720
 - ``throughput_fps``: frames/s with 32 device-resident frames per camera (256 per step), over ``steps`` steps
   (default 30) after two warm-up steps; the frames (1.3 GB) are more than L2 holds.
 - ``ingest_kernel_ms``: device time of k0_rig_ingest for the 256 frames, against the sum of the per-camera ingest
-  kernels (k0_yuv420_resize / k0_resize) for the same frames, from torch.profiler's CUDA activity in a pass of its own,
+  kernels (k0_ingest_resize / k0_resize) for the same frames, from torch.profiler's CUDA activity in a pass of its own,
   averaged over 10 calls.
 Before anything is timed, (a) and (b) are compared: every camera's records must be equal byte for byte."""
 import json
@@ -163,7 +163,7 @@ def ingest_kernels(calls=10):
     for e in prof.key_averages():
         if "k0_rig_ingest" in e.key:
             rig_us += e.device_time_total
-        elif "k0_yuv420_resize" in e.key or "k0_resize" in e.key:
+        elif "k0_ingest_resize" in e.key or "k0_resize" in e.key:
             per_cam_us += e.device_time_total
     return {"k0_rig_ingest": round(rig_us / calls / 1e3, 4), "per_camera_sum": round(per_cam_us / calls / 1e3, 4)}
 
